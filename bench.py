@@ -73,6 +73,41 @@ def stored_digest(key):
     return None
 
 
+DUMP_BYTES = 64_000_000
+UNSCORED = -1.0          # dumped score of a point without a finite normal; real scores 1 - votes/ntrees lie in [0, 1]
+
+
+def dump_scores(sc):
+    """scores as dumped: the NaN of an unscored point becomes UNSCORED, so that every dumped value is finite"""
+    out = np.ascontiguousarray(sc, np.float32).copy()
+    out[np.isnan(out)] = UNSCORED
+    return out
+
+
+def dump_outputs(directory, arrays):
+    """Writes each array as <directory>/<name>.npy, floats as float32 and integers (indices) as float64, so that two builds
+    can be compared output for output.  At most DUMP_BYTES in all: an array larger than its share of what is left is
+    replaced by a fixed, seeded sample of its elements in ascending index order (the same elements on every run).
+    Every value must be finite."""
+    for name, a in arrays.items():
+        if not np.isfinite(a).all():
+            raise ValueError("--dump-outputs: %s holds values that are not finite" % name)
+    os.makedirs(directory, exist_ok=True)
+    items = sorted(((name, np.ascontiguousarray(a).ravel()) for name, a in arrays.items()), key=lambda t: t[1].nbytes)
+    left = DUMP_BYTES - 4096 * len(items)                       # .npy headers
+    for i, (name, a) in enumerate(items):
+        a = a.astype(np.float32 if a.dtype.kind == "f" else np.float64)
+        share = left // (len(items) - i)
+        note = ""
+        if a.nbytes > share:
+            keep = share // a.itemsize
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+            note = " (seeded sample of %d elements)" % keep
+        np.save(os.path.join(directory, name + ".npy"), a)
+        left -= a.nbytes
+        sys.stderr.write("bench.py: wrote %s.npy, %d x %s%s\n" % (name, a.size, a.dtype, note))
+
+
 # ---------------------------------------------------------------------------------------------------------------
 # workloads
 # ---------------------------------------------------------------------------------------------------------------
@@ -311,8 +346,9 @@ def roofline_record(acc, per_call_views, peak_gbs, peak_src, workload, world):
             "stage_ms": {k: v / calls for k, v in (acc.stage or {}).items()}, "host_syncs_per_call": acc.syncs / calls}
 
 
-def single_cloud_leg(torch, K, dev, local, stream, xyz, vp, args, steps, warmup, sampler=None, flush=False):
-    """One cloud on one GPU: device-resident `value`, host-buffer `e2e`, digests.  Returns a dict."""
+def single_cloud_leg(torch, K, dev, local, stream, xyz, vp, args, steps, warmup, sampler=None, flush=False, dump=False):
+    """One cloud on one GPU: device-resident `value`, host-buffer `e2e`, digests.  Returns a dict; with `dump`, its
+    "outputs" are the scores and keypoint indices of the last timed step."""
     n = len(xyz)
     det = make_detector(K, local, vp, args.cpr)
     det.setStream(stream.cuda_stream)
@@ -335,6 +371,7 @@ def single_cloud_leg(torch, K, dev, local, stream, xyz, vp, args, steps, warmup,
         step()
     acc.reset()
     ms, wall_ms, nkp, clocks = time_steps(torch, None, dev, stream, 1, step, steps, sampler)
+    outputs = {"scores": dump_scores(d_scores.cpu().numpy()), "keypoints": d_kp[:nkp].cpu().numpy()} if dump else None
     if flush_buf is not None:                                  # the flush is not part of the path: time it alone and take it out
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         torch.cuda.synchronize(dev); e0.record(stream)
@@ -367,11 +404,12 @@ def single_cloud_leg(torch, K, dev, local, stream, xyz, vp, args, steps, warmup,
     det.close()
     del d_xyz4, d_scores, d_kp, flush_buf
     return dict(n=n, ms=ms, wall_ms=wall_ms, nkp=int(nkp), clocks=clocks, acc=snap, stats=st, e2e_ms=e2e_ms, idx=idx, scores=scores,
-                fragile=int(fragile), h2d=int(n * 16), d2h=int(n * 4 + len(idx) * 4))
+                fragile=int(fragile), h2d=int(n * 16), d2h=int(n * 4 + len(idx) * 4), outputs=outputs)
 
 
-def views_leg(torch, dist, K, dev, local, stream, rank, world, args, steps, warmup, views_per_gpu, sampler=None):
-    """configs[4]: `views_per_gpu` independent views per GPU per step in ONE kpl_detect_batch call."""
+def views_leg(torch, dist, K, dev, local, stream, rank, world, args, steps, warmup, views_per_gpu, sampler=None, dump=False):
+    """configs[4]: `views_per_gpu` independent views per GPU per step in ONE kpl_detect_batch call.  With `dump`, the
+    result's "outputs" are the scores, view-local keypoint indices and keypoint offsets of the last timed step."""
     host_views, vp = make_views(rank, args.distinct_views)
     pts = len(host_views[0])
     det = make_detector(K, local, vp, args.cpr)
@@ -396,6 +434,10 @@ def views_leg(torch, dist, K, dev, local, stream, rank, world, args, steps, warm
         step()
     acc.reset()
     ms, wall_ms, nkp, clocks = time_steps(torch, dist, dev, stream, world, step, steps, sampler)
+    outputs = None
+    if dump:
+        kpo = d_kpo.cpu().numpy()
+        outputs = {"scores": dump_scores(d_scores.cpu().numpy()), "keypoints": d_kp[:int(kpo[-1])].cpu().numpy(), "keypoint_offsets": kpo}
     snap = acc
     st = det.stats()
     sc_host = torch.empty(n_local, dtype=torch.float32).pin_memory().numpy()
@@ -421,7 +463,8 @@ def views_leg(torch, dist, K, dev, local, stream, rank, world, args, steps, warm
               "scores": sha(canon_scores(np.concatenate(scores_v[:len(host_views)]))) if views_per_gpu >= len(host_views) else None}
     det.close()
     return dict(pts_view=pts, n_local=n_local, ms=ms, wall_ms=wall_ms, nkp=int(nkp), clocks=clocks, acc=snap, stats=st, e2e_ms=e2e_ms,
-                batch_equals_single=bool(same), digest=digest, h2d=int(n_local * 16), d2h=int(n_local * 4 + nk_total * 4 + (views_per_gpu + 1) * 8))
+                batch_equals_single=bool(same), digest=digest, h2d=int(n_local * 16), d2h=int(n_local * 4 + nk_total * 4 + (views_per_gpu + 1) * 8),
+                outputs=outputs)
 
 
 def run_b200(args):
@@ -444,9 +487,12 @@ def run_b200(args):
     config = make_config(args, world)
     line = None
     rc = 0
+    dump = bool(args.dump_outputs)
+    outputs = None
 
     if args.workload == "views":
-        r = views_leg(torch, dist, K, dev, local, stream, rank, world, args, args.steps, args.warmup, args.views_per_gpu, sampler)
+        r = views_leg(torch, dist, K, dev, local, stream, rank, world, args, args.steps, args.warmup, args.views_per_gpu, sampler, dump=dump)
+        outputs = r["outputs"]
         n_total = r["n_local"] * world
         value = n_total / (r["ms"] * 1e-3)
         e2e_ms = r["e2e_ms"]
@@ -487,15 +533,18 @@ def run_b200(args):
         host_np = pinned.numpy()
         acc = Acc()
         exch = []
+        last_kp = [None]
 
         def step():
-            nk, _ = job.detect()                                # slab resident in HBM, results stay on the device
+            nk, last_kp[0] = job.detect()                       # slab resident in HBM; rank 0 receives the global keypoint list
             acc.add(det); exch.append(job.info()["exchange_ms"])
             return nk
         for _ in range(args.warmup):
             step()
         acc.reset(); exch.clear()
         ms, wall_ms, nkp, clocks = time_steps(torch, dist, dev, stream, world, step, args.steps, sampler)
+        if dump and rank == 0:
+            outputs = {"keypoints": last_kp[0].copy()}
         snap_calls, snap_dev = acc.calls, acc.dev_ms
         st = det.stats()
         box = [None]
@@ -550,7 +599,8 @@ def run_b200(args):
         xyz, vp, _ = make_workload(args.workload, args.points)
         n_total = len(xyz)
         flush = n_total * 64 < 126e6
-        r = single_cloud_leg(torch, K, dev, local, stream, xyz, vp, args, args.steps, args.warmup, sampler, flush=flush)
+        r = single_cloud_leg(torch, K, dev, local, stream, xyz, vp, args, args.steps, args.warmup, sampler, flush=flush, dump=dump)
+        outputs = r["outputs"]
         roof = roofline_record(r["acc"], 1, peak_gbs, peak_src, args.workload, 1)
         pts = r["acc"].scored / max(1, r["acc"].calls)
         pipe_bytes = roof["algorithmic_bytes_per_launch"] + 16.0 * K_NORMALS * pts + 200.0 * pts
@@ -621,6 +671,8 @@ def run_b200(args):
                 rc = 3
             line["extra"] = extra
 
+    if rank == 0 and outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if rank == 0 and line is not None:
         line["impl_details"] = {"cells_per_radius": args.cpr, "library": "keypoint_learning_b200/libkpl_b200.so (C ABI include/kpl.h)",
                                 "multi_gpu": "kpl_shard_* : NCCL ncclSend/ncclRecv inside the library; torch.distributed (gloo) only for barriers and the NCCL id"
@@ -650,7 +702,13 @@ def main():
     ap.add_argument("--parity-sample", type=int, default=400_000, help="points of the crop on which the CUDA path is compared with the oracle")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", dest="extras", action="store_false", help="skip the sub-records of the other single-GPU configurations")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path returned in its last timed step as DIR/<name>.npy "
+                                                          "(scores, -1 for an unscored point; keypoint indices; at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm runs on a crop sized from its own timing, so its outputs are not reproducible")
     if args.impl == "reference":
         run_reference(args)
     else:

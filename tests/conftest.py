@@ -1,3 +1,5 @@
+import hashlib
+import json
 import os
 import sys
 
@@ -19,6 +21,38 @@ def oracle():
     from oracle import oracle as O
     O.lib()
     return O
+
+
+def digest(arrays):
+    """sha256 over the bytes of one array or of a tuple of arrays, in order."""
+    h = hashlib.sha256()
+    for a in arrays if isinstance(arrays, tuple) else (arrays,):
+        h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
+
+
+class Reference:
+    """What the reference's own code (oracle/_ref) returns.  Where oracle/_ref is built, check() runs it and also holds
+    the recorded digest to it; elsewhere check() compares with the digest recorded in golden/reference_digests.json."""
+
+    def __init__(self, oracle):
+        self.live = oracle.ref_lib() is not None
+        with open(os.path.join(GOLDEN, "reference_digests.json")) as f:
+            self.digests = json.load(f)
+
+    def check(self, key, got, ref_fn):
+        """`got` (an array or a tuple of arrays) must be bit-identical to the reference's result `ref_fn()`."""
+        d = digest(got)
+        if self.live:
+            assert d == digest(ref_fn()), key
+            assert self.digests.get(key) == d, "reference_digests.json is stale for %s: the reference gives %s" % (key, d)
+        else:
+            assert d == self.digests[key], key
+
+
+@pytest.fixture(scope="session")
+def reference(oracle):
+    return Reference(oracle)
 
 
 @pytest.fixture(scope="session")

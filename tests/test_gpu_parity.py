@@ -339,12 +339,10 @@ def test_uniform_sampling_matches_restatement(kpl, views, oracle):
     d.close()
 
 
-def test_cuda_path_against_the_reference_templates(kpl, views, oracle):
+def test_cuda_path_against_the_reference_templates(kpl, views, oracle, reference):
     """The CUDA path against oracle/_ref DIRECTLY: the reference's own computePointFeatures / runForest /
-    detectKeypoints templates (compiled from the mounted tree; the prebuilt library travels with the repo),
-    fed with the canonical neighbour order the device uses."""
-    if oracle.ref_lib() is None:
-        pytest.skip("oracle/_ref was not built (reference tree not mounted)")
+    detectKeypoints templates (or their recorded results where oracle/_ref is not built), fed with the canonical
+    neighbour order the device uses."""
     xyz = np.ascontiguousarray(views["cheff002"][:3000])
     nrm = oracle.normals_knn(xyz, 10)
     forest = oracle.load_forest_yaml(forest_path("synthetic-SHOT-like-T50-D10"))
@@ -354,16 +352,14 @@ def test_cuda_path_against_the_reference_templates(kpl, views, oracle):
     d.keepIntermediates(True)
     d.setInputCloud(xyz); d.setNormals(nrm)
     _, idx = d.compute()
-    f_ref = oracle.ref_features(xyz, nrm, R_FEAT, 5, 10, lf)
-    assert np.array_equal(d.fetch("features", len(xyz), 50).view(np.uint32), f_ref.view(np.uint32))
-    all_idx, sc_ref = oracle.ref_detect(xyz, nrm, forest, R_FEAT, R_NMS, 0.5, 5, 10, lf, None, non_maxima=False)
-    assert np.array_equal(d.getResponse().view(np.uint32), sc_ref.view(np.uint32))
-    kp_ref, _ = oracle.ref_detect(xyz, nrm, forest, R_FEAT, R_NMS, 0.5, 5, 10, lf, ln)
-    assert np.array_equal(idx, kp_ref)
+    reference.check("cheff002_3k/features", d.fetch("features", len(xyz), 50), lambda: oracle.ref_features(xyz, nrm, R_FEAT, 5, 10, lf))
+    reference.check("cheff002_3k/scores", d.getResponse(),
+                    lambda: oracle.ref_detect(xyz, nrm, forest, R_FEAT, R_NMS, 0.5, 5, 10, lf, None, non_maxima=False)[1])
+    reference.check("cheff002_3k/keypoints", idx, lambda: oracle.ref_detect(xyz, nrm, forest, R_FEAT, R_NMS, 0.5, 5, 10, lf, ln)[0])
     d.setNonMaximaDrawsRemove(True); d.setNonMaximaDrawsThreshold(1.5)
     _, idx_d = d.compute()
-    kp_d, _ = oracle.ref_detect(xyz, nrm, forest, R_FEAT, R_NMS, 0.5, 5, 10, lf, ln, draws_remove=True, draws_thr=1.5)
-    assert np.array_equal(idx_d, kp_d)
+    reference.check("cheff002_3k/keypoints_draws", idx_d,
+                    lambda: oracle.ref_detect(xyz, nrm, forest, R_FEAT, R_NMS, 0.5, 5, 10, lf, ln, draws_remove=True, draws_thr=1.5)[0])
     d.close()
 
 
@@ -683,10 +679,8 @@ def test_scene_closed_surfaces_vs_oracle(kpl, oracle, main_forest):
     d.close()
 
 
-def test_scene_crop_against_the_reference_templates(kpl, oracle):
+def test_scene_crop_against_the_reference_templates(kpl, oracle, reference):
     """A 3 k-point crop of the closed-surface scene through oracle/_ref (the reference's own templates)."""
-    if oracle.ref_lib() is None:
-        pytest.skip("oracle/_ref was not built (reference tree not mounted)")
     xyz, vp = scene_crop(1_250_000, 3000)
     nrm = oracle.normals_knn(xyz, 10, vp)
     fname = "synthetic-SHOT-like-T50-D10"
@@ -697,12 +691,10 @@ def test_scene_crop_against_the_reference_templates(kpl, oracle):
     d.keepIntermediates(True)
     d.setInputCloud(xyz); d.setNormals(nrm)
     _, idx = d.compute()
-    f_ref = oracle.ref_features(xyz, nrm, R_FEAT, 5, 10, lf)
-    assert np.array_equal(d.fetch("features", len(xyz), 50).view(np.uint32), f_ref.view(np.uint32))
-    _, sc_ref = oracle.ref_detect(xyz, nrm, forest, R_FEAT, R_NMS, 0.5, 5, 10, lf, None, non_maxima=False)
-    assert np.array_equal(d.getResponse().view(np.uint32), sc_ref.view(np.uint32))
-    kp_ref, _ = oracle.ref_detect(xyz, nrm, forest, R_FEAT, R_NMS, 0.5, 5, 10, lf, ln)
-    assert np.array_equal(idx, kp_ref)
+    reference.check("scene_crop_3k/features", d.fetch("features", len(xyz), 50), lambda: oracle.ref_features(xyz, nrm, R_FEAT, 5, 10, lf))
+    reference.check("scene_crop_3k/scores", d.getResponse(),
+                    lambda: oracle.ref_detect(xyz, nrm, forest, R_FEAT, R_NMS, 0.5, 5, 10, lf, None, non_maxima=False)[1])
+    reference.check("scene_crop_3k/keypoints", idx, lambda: oracle.ref_detect(xyz, nrm, forest, R_FEAT, R_NMS, 0.5, 5, 10, lf, ln)[0])
     d.close()
 
 

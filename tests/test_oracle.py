@@ -175,12 +175,10 @@ def test_normals_radius_mode_runs(oracle, views):
     assert np.allclose(np.linalg.norm(nrm[ok, :3], axis=1), 1.0, atol=1e-5)
 
 
-def test_binning_helpers_match_the_reference_build(oracle):
+def test_binning_helpers_match_the_reference_build(oracle, reference):
     """oracle/_ref: the reference's OWN src/KeypointLearning.cpp compiled from the mounted tree.  The oracle's
     restatement of findAnnulusPair / findBinPair must agree with it bit for bit on a dense sweep that includes
     every bin boundary +- a few ulps, the clamps and the centre-of-bin cases."""
-    if oracle.ref_lib() is None:
-        pytest.skip("oracle/_ref was not built (reference tree not mounted)")
     rng = np.random.default_rng(5)
 
     def around(values, span=3):
@@ -199,23 +197,29 @@ def test_binning_helpers_match_the_reference_build(oracle):
         edges = around(np.arange(0, 2 * A + 1, dtype=np.float32) * dim / np.float32(2))        # boundaries and centres
         d = np.concatenate([edges[(edges >= 0) & (edges <= np.float32(support))],
                             rng.uniform(0, support, 200_000).astype(np.float32), np.float32([0.0, support])])
-        got, ref = oracle.annulus_sweep(A, support, d), oracle.ref_annulus_sweep(A, support, d)
-        for g, r in zip(got, ref):
-            assert np.array_equal(g.view(np.uint32), r.view(np.uint32)), (A, support)
+        reference.check("annulus_sweep/A=%d,support=%g" % (A, support), oracle.annulus_sweep(A, support, d),
+                        lambda: oracle.ref_annulus_sweep(A, support, d))
     for B in (10, 5, 8, 16, 1, 3):
         dim = np.float32(2) / np.float32(B)
         edges = around(np.arange(0, 2 * B + 1, dtype=np.float32) * dim / np.float32(2))
         c = np.concatenate([edges, rng.uniform(-0.5, 2.5, 200_000).astype(np.float32), np.float32([-1.0, 0.0, 2.0, 3.0, -0.0])])
-        got, ref = oracle.bin_sweep(B, c), oracle.ref_bin_sweep(B, c)
-        for g, r in zip(got, ref):
-            assert np.array_equal(g.view(np.uint32), r.view(np.uint32)), B
+        reference.check("bin_sweep/B=%d" % B, oracle.bin_sweep(B, c), lambda: oracle.ref_bin_sweep(B, c))
 
 
-def test_binning_helpers_match_the_reference_build_random_shapes(oracle):
-    """hypothesis: arbitrary (n_annulus, support) / n_bins, not just the shapes the detector is used with."""
+def test_binning_helpers_match_the_reference_build_random_shapes(oracle, reference):
+    """arbitrary (n_annulus, support) / n_bins, not just the shapes the detector is used with: 60 seeded draws of each,
+    and hypothesis on top where oracle/_ref is built."""
+    rng = np.random.default_rng(11)
+    for k in range(60):
+        A, B, seed = int(rng.integers(1, 65)), int(rng.integers(1, 65)), int(rng.integers(0, 2**31 - 1))
+        support = float(np.float32(2.0 ** rng.uniform(-6, 12)))
+        d = np.minimum(np.random.default_rng(seed).uniform(0, support, 2000).astype(np.float32), np.float32(support))
+        reference.check("annulus_random/%d" % k, oracle.annulus_sweep(A, support, d), lambda: oracle.ref_annulus_sweep(A, support, d))
+        c = np.random.default_rng(seed).uniform(-1.0, 3.0, 2000).astype(np.float32)
+        reference.check("bin_random/%d" % k, oracle.bin_sweep(B, c), lambda: oracle.ref_bin_sweep(B, c))
+    if not reference.live:
+        return
     from hypothesis import given, settings, strategies as st
-    if oracle.ref_lib() is None:
-        pytest.skip("oracle/_ref was not built (reference tree not mounted)")
 
     @settings(max_examples=60, deadline=None)
     @given(st.integers(1, 64), st.floats(0.015625, 4096.0, allow_nan=False, width=32), st.integers(0, 2**31 - 1))
@@ -248,9 +252,7 @@ def _ref_case(views, n=2500):
     return xyz
 
 
-def test_features_match_the_reference_templates(oracle, views):
-    if oracle.ref_lib() is None:
-        pytest.skip("oracle/_ref was not built (reference tree not mounted)")
+def test_features_match_the_reference_templates(oracle, views, reference):
     xyz = _ref_case(views)
     nrm = oracle.normals_knn(xyz, 10)
     nrm[7::53, 0] = np.nan                                      # neighbours (and queries) without a finite normal
@@ -258,19 +260,18 @@ def test_features_match_the_reference_templates(oracle, views):
     q = q[np.isfinite(nrm[q, 0])]                               # runForest never asks for such a query (hpp:277)
     for r_feat, A, B in ((20.0, 5, 10), (9.0, 4, 8), (14.0, 10, 5)):
         for order in (0, 1):
-            lists = oracle.ref_neighbour_lists(xyz, r_feat, order)
-            f_ref = oracle.ref_features(xyz, nrm, r_feat, A, B, lists, q)
             f_orc = oracle.features(xyz, nrm, r_feat, A, B, order=order, qidx=q)
-            assert np.array_equal(f_ref.view(np.uint32), f_orc.view(np.uint32)), (r_feat, A, B, order)
+            reference.check("features/r=%g,A=%d,B=%d,order=%d" % (r_feat, A, B, order), f_orc,
+                            lambda: oracle.ref_features(xyz, nrm, r_feat, A, B, oracle.ref_neighbour_lists(xyz, r_feat, order), q))
+    if not reference.live:
+        return
     # the order really matters at the last bit: a sorted-kd-tree order gives different (close) rows
     f_sorted = oracle.ref_features(xyz, nrm, 20.0, 5, 10, oracle.ref_neighbour_lists(xyz, 20.0, 2), q)
     f_canon = oracle.features(xyz, nrm, 20.0, 5, 10, order=1, qidx=q)
     assert np.abs(f_sorted - f_canon).max() < 1e-5 and not np.array_equal(f_sorted, f_canon)
 
 
-def test_detection_matches_the_reference_templates(oracle, views):
-    if oracle.ref_lib() is None:
-        pytest.skip("oracle/_ref was not built (reference tree not mounted)")
+def test_detection_matches_the_reference_templates(oracle, views, reference):
     xyz = _ref_case(views)
     nrm = oracle.normals_knn(xyz, 10)
     assert np.isfinite(nrm[:, :3]).all()                        # the reference mis-aligns its response cloud otherwise (hpp:277 vs :203)
@@ -280,16 +281,17 @@ def test_detection_matches_the_reference_templates(oracle, views):
     feat = oracle.features(xyz, nrm, r_feat, A, B, order=1)
     sc = oracle.scores(forest, feat, nrm)
     # runForest: setNonMaxima(false) hands back the response cloud (hpp:189-196)
-    idx, sc_ref = oracle.ref_detect(xyz, nrm, forest, r_feat, 4.0, 0.5, A, B, lf, None, non_maxima=False)
-    assert np.array_equal(idx, np.arange(len(xyz))) and np.array_equal(sc_ref.view(np.uint32), sc.view(np.uint32))
+    reference.check("detect/all", (np.arange(len(xyz), dtype=np.int32), sc),
+                    lambda: oracle.ref_detect(xyz, nrm, forest, r_feat, 4.0, 0.5, A, B, lf, None, non_maxima=False))
     for r_nms, th in ((4.0, 0.85), (2.0, 0.5), (6.0, 0.3), (4.0, 0.0)):
         ln = oracle.ref_neighbour_lists(xyz, r_nms, 0)
-        idx, s = oracle.ref_detect(xyz, nrm, forest, r_feat, r_nms, th, A, B, lf, ln, non_maxima=True, draws_remove=False)
-        assert np.array_equal(idx, oracle.nms(xyz, sc, r_nms, th)), (r_nms, th)
-        assert np.array_equal(s.view(np.uint32), sc[idx].view(np.uint32))
+        idx = oracle.nms(xyz, sc, r_nms, th)
+        reference.check("detect/nms=%g,th=%g" % (r_nms, th), (idx, sc[idx]),
+                        lambda: oracle.ref_detect(xyz, nrm, forest, r_feat, r_nms, th, A, B, lf, ln, non_maxima=True, draws_remove=False))
         for dthr in (0.0, 1.0, 3.0):
-            idx_d, _ = oracle.ref_detect(xyz, nrm, forest, r_feat, r_nms, th, A, B, lf, ln, non_maxima=True, draws_remove=True, draws_thr=dthr)
-            assert np.array_equal(idx_d, oracle.nms(xyz, sc, r_nms, th, draws_remove=True, draws_thr=dthr)), (r_nms, th, dthr)
+            reference.check("detect/nms=%g,th=%g,draws=%g" % (r_nms, th, dthr), oracle.nms(xyz, sc, r_nms, th, draws_remove=True, draws_thr=dthr),
+                            lambda: oracle.ref_detect(xyz, nrm, forest, r_feat, r_nms, th, A, B, lf, ln, non_maxima=True, draws_remove=True,
+                                                      draws_thr=dthr)[0])
 
 
 def test_normals_radius_order_deviation_is_small(oracle, views):
@@ -482,13 +484,11 @@ def test_integral_image_normals_restatement(oracle):
     assert checked > 300
 
 
-def test_eigen_normalize_variants_against_the_reference_templates(oracle, views):
+def test_eigen_normalize_variants_against_the_reference_templates(oracle, views, reference):
     """`row.normalize()` (hpp:360-365) is Eigen code whose arithmetic changed between versions: >= 3.3 divides by the norm,
     3.2.x multiplies by 1/norm.  The reference pins no Eigen version, so both are restated; the reference's own
     computePointFeatures (oracle/_ref) run over either stub variant must equal the oracle in that mode, and the two
     variants differ by at most one ulp per feature."""
-    if oracle.ref_lib() is None:
-        pytest.skip("oracle/_ref was not built (reference tree not mounted)")
     xyz = np.ascontiguousarray(views["cheff000"][:2500])
     nrm = oracle.normals_knn(xyz, 10)
     lf = oracle.ref_neighbour_lists(xyz, 20.0, 1)
@@ -497,8 +497,7 @@ def test_eigen_normalize_variants_against_the_reference_templates(oracle, views)
         for recip in (False, True):
             oracle.set_normalize_mode(recip)
             f = oracle.features(xyz, nrm, 20.0, 5, 10, order=1)
-            r = oracle.ref_features(xyz, nrm, 20.0, 5, 10, lf)
-            assert np.array_equal(f.view(np.uint32), r.view(np.uint32)), recip
+            reference.check("features_normalize/reciprocal=%d" % recip, f, lambda: oracle.ref_features(xyz, nrm, 20.0, 5, 10, lf))
             rows[recip] = f
     finally:
         oracle.set_normalize_mode(False)
