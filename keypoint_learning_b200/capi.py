@@ -17,6 +17,7 @@ KPL_OK = 0
 STATUS = {0: "KPL_OK", 1: "KPL_E_INVALID", 2: "KPL_E_FOREST", 3: "KPL_E_SIZE_MISMATCH", 4: "KPL_E_NONFINITE",
           5: "KPL_E_VARCOUNT", 6: "KPL_E_CUDA", 7: "KPL_E_GRID", 8: "KPL_E_NOMEM", 9: "KPL_E_IO", 10: "KPL_E_UNSUPPORTED",
           11: "KPL_E_NCCL", 12: "KPL_E_HALO"}
+KPL_E_HALO = 12
 NORMALS_GIVEN, NORMALS_KNN, NORMALS_RADIUS = 0, 1, 2
 ROLE_HALO, ROLE_SCORE, ROLE_OWNED = 0, 1, 3
 

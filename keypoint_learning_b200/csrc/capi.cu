@@ -227,11 +227,15 @@ int kpl_forest_info(const kpl_ctx* ctx, int32_t* ntrees, int32_t* nnodes, int32_
 static const double CELL_PAD = 1.0 + 9.5367431640625e-07;    // 1 + 2^-20: points closer than r never lie more than cells_per_radius cells apart
 static const double REACH_PAD = 1.0 + 4.76837158203125e-07;   // 1 + 2^-21
 
+double kpl::canonical_cell(const kpl_params& P) { return (double)P.radius_features * CELL_PAD / (double)P.cells_per_radius; }
+int32_t kpl::grid_dim(double lo, double hi, double cell) { return (int32_t)std::min(2147483000.0, std::floor((hi - lo) / cell) + 1.0); }
+int kpl::grid_reach(double radius, double cell) { return (int)std::floor(radius * REACH_PAD / cell) + 1; }
+
 static void clear_batch(GridDesc& g)
 {
     g.views = nullptr; g.layer_view = nullptr; g.view_offsets = nullptr; g.nviews = 0;
     g.interior_lo = g.interior_hi = 0; g.guard_cells = 0;
-    g.owned_lo = g.owned_hi = 0;
+    g.forced = 0;
 }
 
 static int finish_grid(kpl_ctx* ctx, int64_t n)
@@ -245,8 +249,8 @@ static int finish_grid(kpl_ctx* ctx, int64_t n)
     }
     if (ncells > 2147483646.0) return fail(ctx, KPL_E_GRID, "uniform grid would exceed 2^31-2 cells: cloud too sparse for radius_features/cells_per_radius");
     g.ncells = (int64_t)ncells;
-    g.reach_feat = (int)std::floor((double)P.radius_features * REACH_PAD / g.cell) + 1;
-    g.reach_nms = (int)std::floor((double)P.radius_nms * REACH_PAD / g.cell) + 1;
+    g.reach_feat = grid_reach(P.radius_features, g.cell);
+    g.reach_nms = grid_reach(P.radius_nms, g.cell);
     ctx->stats.grid_cells = g.ncells;
     for (int a = 0; a < 3; ++a) { ctx->stats.grid_dims[a] = g.dim[a]; ctx->stats.grid_origin[a] = g.org[a]; }
     ctx->stats.grid_cell = g.cell;
@@ -256,19 +260,18 @@ static int finish_grid(kpl_ctx* ctx, int64_t n)
 
 // Grid of ONE cloud.  A forced grid (slab of a larger cloud) is known a priori: no bounding-box pass and no host
 // synchronisation; a non-finite point or a point outside the forced grid is reported by the flags cell_key_kernel
-// raises, which finish_call() reads together with the counters.  cell_override > 0 replaces the canonical cell size
+// raises, which detect_finish() / check_forced_grid() read.  cell_override > 0 replaces the canonical cell size
 // (kpl_normals sizes its k-NN grid from the data).
-static int prepare_grid(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, const uint8_t* d_role, int64_t n, double cell_override = 0.0)
+int kpl::prepare_grid(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, const uint8_t* d_role, int64_t n, const ForcedGrid* forced, double cell_override)
 {
-    const kpl_params& P = ctx->params;
     GridDesc& g = ctx->grid;
     clear_batch(g);
-    g.cell = cell_override > 0.0 ? cell_override : (double)P.radius_features * CELL_PAD / (double)P.cells_per_radius;
-    if (P.grid_forced) {
+    g.cell = cell_override > 0.0 ? cell_override : canonical_cell(ctx->params);
+    if (forced) {
         KPL_CUDA(launch_bbox_init(ctx));
-        for (int a = 0; a < 3; ++a) { g.org[a] = P.grid_origin[a]; g.dim[a] = P.grid_dims[a]; g.off[a] = P.grid_offset[a]; }
-        g.interior_lo = P.slab_interior_lo; g.interior_hi = P.slab_interior_hi; g.guard_cells = P.slab_guard_cells;
-        if (P.slab_owned_hi > P.slab_owned_lo) { g.owned_lo = std::max(P.slab_owned_lo, 0); g.owned_hi = std::min(P.slab_owned_hi, g.dim[0]); }
+        for (int a = 0; a < 3; ++a) { g.org[a] = forced->origin[a]; g.dim[a] = forced->dims[a]; g.off[a] = forced->offset[a]; }
+        g.interior_lo = forced->interior_lo; g.interior_hi = forced->interior_hi; g.guard_cells = forced->guard_cells;
+        g.forced = 1;
     } else {
         KPL_CUDA(launch_bbox(ctx, d_xyz, n, ctx->d_bbox));
         uint32_t hb[8];
@@ -279,7 +282,7 @@ static int prepare_grid(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, 
         for (int a = 0; a < 3; ++a) {
             const double lo = (double)dec_float(hb[a]), hi = (double)dec_float(hb[3 + a]);
             g.off[a] = 0; g.org[a] = lo;
-            g.dim[a] = (int32_t)std::min(2147483000.0, std::floor((hi - lo) / g.cell) + 1.0);
+            g.dim[a] = grid_dim(lo, hi, g.cell);
         }
     }
     int rc = finish_grid(ctx, n);
@@ -288,6 +291,18 @@ static int prepare_grid(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, 
     ctx->cur_nrm = d_nrm;
     KPL_CUDA(build_grid(ctx, d_xyz, d_nrm, d_role, n));
     return KPL_OK;
+}
+
+// Grid of a cloud passed to a public entry point: the one kpl_params force (setForcedGrid, a role slab through
+// kpl_detect), else the canonical grid of its bounding box.
+static int prepare_params_grid(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, const uint8_t* d_role, int64_t n)
+{
+    const kpl_params& P = ctx->params;
+    if (!P.grid_forced) return prepare_grid(ctx, d_xyz, d_nrm, d_role, n, nullptr);
+    ForcedGrid f;
+    for (int a = 0; a < 3; ++a) { f.origin[a] = P.grid_origin[a]; f.dims[a] = P.grid_dims[a]; f.offset[a] = P.grid_offset[a]; }
+    f.interior_lo = P.slab_interior_lo; f.interior_hi = P.slab_interior_hi; f.guard_cells = P.slab_guard_cells;
+    return prepare_grid(ctx, d_xyz, d_nrm, d_role, n, &f);
 }
 
 // Grid of a batch of independent views (kpl_detect_batch): view v keeps the cells of its own canonical grid (origin =
@@ -299,7 +314,7 @@ static int prepare_grid_batch(kpl_ctx* ctx, const float4* d_xyz, const float4* d
     const kpl_params& P = ctx->params;
     GridDesc& g = ctx->grid;
     clear_batch(g);
-    g.cell = (double)P.radius_features * CELL_PAD / (double)P.cells_per_radius;
+    g.cell = canonical_cell(P);
     KPL_CUDA(ensure(ctx->view_offsets, (size_t)nviews + 1));
     KPL_CUDA(ensure(ctx->views, (size_t)nviews));
     KPL_CUDA(ensure(ctx->scratch_i, (size_t)nviews * 8 + 16));
@@ -311,9 +326,7 @@ static int prepare_grid_batch(kpl_ctx* ctx, const float4* d_xyz, const float4* d
     KPL_CUDA(cudaMemcpyAsync(hb.data(), d_boxes, hb.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
     KPL_CUDA(cudaStreamSynchronize(ctx->stream));
     ctx->syncs++;
-    const int reach_f = (int)std::floor((double)P.radius_features * REACH_PAD / g.cell) + 1;
-    const int reach_n = (int)std::floor((double)P.radius_nms * REACH_PAD / g.cell) + 1;
-    const int pad = std::max(std::max(reach_f, reach_n), 1);
+    const int pad = std::max(std::max(grid_reach(P.radius_features, g.cell), grid_reach(P.radius_nms, g.cell)), 1);
     std::vector<ViewDesc> hv((size_t)nviews);
     int64_t z = 0;
     int dimx = 1, dimy = 1;
@@ -324,7 +337,7 @@ static int prepare_grid_batch(kpl_ctx* ctx, const float4* d_xyz, const float4* d
         for (int a = 0; a < 3; ++a) {
             const double lo = (double)dec_float(b[a]), hi = (double)dec_float(b[3 + a]);
             hv[(size_t)v].org[a] = lo;
-            d[a] = (int)std::min(2147483000.0, std::floor((hi - lo) / g.cell) + 1.0);
+            d[a] = grid_dim(lo, hi, g.cell);
         }
         dimx = std::max(dimx, d[0]); dimy = std::max(dimy, d[1]);
         hv[(size_t)v].zoff = (int32_t)z; hv[(size_t)v].dimz = d[2];
@@ -382,7 +395,7 @@ static int prepare_normals(kpl_ctx* ctx, bool given, int64_t n)
     return KPL_OK;
 }
 
-static void begin_call(kpl_ctx* ctx)
+void kpl::detect_reset(kpl_ctx* ctx)
 {
     (void)cudaGetLastError();      // a stale error of an earlier, unrelated runtime call must not be blamed on this call
     ctx->launches = 0;
@@ -461,7 +474,7 @@ int detect_finish(kpl_ctx* ctx, int64_t n, int64_t* n_kp_out)
     KPL_CUDA(cudaMemcpyAsync(hb, ctx->d_bbox, sizeof hb, cudaMemcpyDeviceToHost, ctx->stream));
     KPL_CUDA(cudaStreamSynchronize(ctx->stream));
     ctx->syncs++;
-    if (ctx->params.grid_forced && hb[7]) return fail(ctx, KPL_E_GRID, "a point lies outside the forced grid (or is not finite)");
+    if (ctx->grid.forced && hb[7]) return fail(ctx, KPL_E_GRID, "a point lies outside the forced grid (or is not finite)");
     if (hc[9]) {
         char b[256];
         snprintf(b, sizeof b, "%llu k-NN normals that kept points depend on were clipped by a slab face: widen normal_support_cells", hc[9]);
@@ -494,24 +507,19 @@ int detect_begin(kpl_ctx* ctx)
     return KPL_OK;
 }
 
-int detect_grid_phase(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, const uint8_t* d_role, int64_t n)
-{
-    return prepare_grid(ctx, d_xyz, d_nrm, d_role, n);
-}
-
 }  // namespace kpl
 
 static int run_detect(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, const uint8_t* d_role, int64_t n,
                       float* d_scores_out, int32_t* d_kp_out, int64_t* n_kp_out)
 {
-    begin_call(ctx);
+    detect_reset(ctx);
     if (n_kp_out) *n_kp_out = 0;
     int rc = detect_check(ctx, n, d_role != nullptr);
     if (rc) return rc;
     ctx->stats.n_points = n;
     if (n == 0) return KPL_OK;
     if ((rc = detect_begin(ctx))) return rc;
-    if ((rc = prepare_grid(ctx, d_xyz, d_nrm, d_role, n))) return rc;
+    if ((rc = prepare_params_grid(ctx, d_xyz, d_nrm, d_role, n))) return rc;
     if ((rc = detect_score_phase(ctx, d_nrm != nullptr, d_role != nullptr, n))) return rc;
     if ((rc = detect_nms_phase(ctx, d_role != nullptr, n, d_kp_out))) return rc;
     if (d_scores_out) KPL_CUDA(cudaMemcpyAsync(d_scores_out, ctx->score.p, (size_t)n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
@@ -523,7 +531,7 @@ static int run_detect(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, co
 static int run_detect_batch(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, int64_t n, const int64_t* h_offsets, int nviews,
                             float* d_scores_out, int32_t* d_kp_out, int64_t* d_kp_offsets_out, int64_t* n_kp_out)
 {
-    begin_call(ctx);
+    detect_reset(ctx);
     if (n_kp_out) *n_kp_out = 0;
     int rc = detect_check(ctx, n, false);
     if (rc) return rc;
@@ -617,7 +625,7 @@ int kpl_detect_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, 
 // out-of-grid flag here.
 static int check_forced_grid(kpl_ctx* ctx)
 {
-    if (!ctx->params.grid_forced) return KPL_OK;
+    if (!ctx->grid.forced) return KPL_OK;
     uint32_t hb[8];
     KPL_CUDA(cudaMemcpyAsync(hb, ctx->d_bbox, sizeof hb, cudaMemcpyDeviceToHost, ctx->stream));
     KPL_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -634,7 +642,7 @@ static const double KNN_TARGET = 14.0;
 static int prepare_knn_grid(kpl_ctx* ctx, int64_t n)
 {
     const kpl_params& P = ctx->params;
-    if (P.grid_forced || P.normals_mode != KPL_NORMALS_KNN) return prepare_grid(ctx, ctx->in_xyz.p, nullptr, nullptr, n);
+    if (P.grid_forced || P.normals_mode != KPL_NORMALS_KNN) return prepare_params_grid(ctx, ctx->in_xyz.p, nullptr, nullptr, n);
     // first guess from the bounding box as if the points filled it; surfaces and curves then show far more points per
     // occupied cell than wanted, and the cell is refined from the measured occupancy (occupancy ~ cell^2 on a surface)
     KPL_CUDA(launch_bbox(ctx, ctx->in_xyz.p, n, ctx->d_bbox));
@@ -652,7 +660,7 @@ static int prepare_knn_grid(kpl_ctx* ctx, int64_t n)
     const double min_cell = std::cbrt(vol / 1.0e9) * 1.001 + longest * 1e-7;  // at most ~1e9 cells
     double cell = std::max(std::cbrt(vol * target / (double)n), min_cell);
     for (int pass = 0; pass < 3; ++pass) {
-        int rc = prepare_grid(ctx, ctx->in_xyz.p, nullptr, nullptr, n, cell);
+        int rc = prepare_grid(ctx, ctx->in_xyz.p, nullptr, nullptr, n, nullptr, cell);
         if (rc) return rc;
         if (pass == 2) break;
         KPL_CUDA(cudaMemsetAsync(ctx->counters.p + 10, 0, sizeof(unsigned long long), ctx->stream));
@@ -716,7 +724,7 @@ int kpl_detect_batch_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_norm
 int kpl_normals(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, int64_t n, float* normals_out)
 {
     if (!ctx || (n > 0 && !normals_out)) return KPL_E_INVALID;
-    begin_call(ctx);
+    detect_reset(ctx);
     if (n == 0) return KPL_OK;
     if (ctx->params.normals_mode == KPL_NORMALS_GIVEN) return fail(ctx, KPL_E_INVALID, "normals_mode must be KNN or RADIUS");
     int rc = upload_inputs(ctx, xyz, xyz_stride, nullptr, 0, nullptr, n);
@@ -745,7 +753,7 @@ int kpl_normals(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, int64_t n, f
 int kpl_normals_organized(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, int32_t width, int32_t height, float smoothing_size, float* normals_out)
 {
     if (!ctx || width < 1 || height < 1 || !xyz || !normals_out) return KPL_E_INVALID;
-    begin_call(ctx);
+    detect_reset(ctx);
     if (!(smoothing_size > 0.f) || !std::isfinite(smoothing_size)) return fail(ctx, KPL_E_INVALID, "normal smoothing size must be > 0");
     const int64_t n = (int64_t)width * height;
     if (n > 2147483000ll) return fail(ctx, KPL_E_INVALID, "point count out of range");
@@ -767,7 +775,7 @@ int kpl_features(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float
                  int64_t n, const int32_t* indices, int64_t m, float* features_out)
 {
     if (!ctx || m < 0 || (m > 0 && !features_out)) return KPL_E_INVALID;
-    begin_call(ctx);
+    detect_reset(ctx);
     if (!indices && m != n) return fail(ctx, KPL_E_INVALID, "indices == NULL requires m == n");
     if (n == 0 || m == 0) return KPL_OK;
     if (m > 2147483000ll) return fail(ctx, KPL_E_INVALID, "too many feature indices");
@@ -778,7 +786,7 @@ int kpl_features(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float
     int rc = upload_inputs(ctx, xyz, xyz_stride, normals, normals_stride, nullptr, n);
     if (rc) return rc;
     KPL_CUDA(cudaMemsetAsync(ctx->counters.p, 0, kpl_ctx::NCOUNTERS * sizeof(unsigned long long), ctx->stream));
-    if ((rc = prepare_grid(ctx, ctx->in_xyz.p, normals ? ctx->in_nrm.p : nullptr, nullptr, n))) return rc;
+    if ((rc = prepare_params_grid(ctx, ctx->in_xyz.p, normals ? ctx->in_nrm.p : nullptr, nullptr, n))) return rc;
     if ((rc = check_forced_grid(ctx))) return rc;
     if ((rc = prepare_lists(ctx, normals != nullptr, indices == nullptr, false))) return rc;
     if ((rc = prepare_normals(ctx, normals != nullptr, n))) return rc;
@@ -813,11 +821,11 @@ int kpl_features(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float
 int kpl_radius_stats(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, int64_t n, double radius, int32_t* counts_out, uint64_t* hash_out)
 {
     if (!ctx || !(radius >= 0)) return KPL_E_INVALID;
-    begin_call(ctx);
+    detect_reset(ctx);
     if (n == 0) return KPL_OK;
     int rc = upload_inputs(ctx, xyz, xyz_stride, nullptr, 0, nullptr, n);
     if (rc) return rc;
-    if ((rc = prepare_grid(ctx, ctx->in_xyz.p, nullptr, nullptr, n))) return rc;
+    if ((rc = prepare_params_grid(ctx, ctx->in_xyz.p, nullptr, nullptr, n))) return rc;
     if ((rc = check_forced_grid(ctx))) return rc;
     KPL_CUDA(ensure(ctx->scratch_i, (size_t)n * 3 + 2));
     int32_t* d_counts = ctx->scratch_i.p;
@@ -834,12 +842,12 @@ int kpl_nearest(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, int64_t n, c
                 int32_t* idx_out, float* d2_out)
 {
     if (!ctx || m < 0 || (m > 0 && (!queries || !idx_out))) return KPL_E_INVALID;
-    begin_call(ctx);
+    detect_reset(ctx);
     if (m == 0) return KPL_OK;
     if (n <= 0) return fail(ctx, KPL_E_INVALID, "the cloud is empty");
     int rc = upload_inputs(ctx, xyz, xyz_stride, nullptr, 0, nullptr, n);
     if (rc) return rc;
-    if ((rc = prepare_grid(ctx, ctx->in_xyz.p, nullptr, nullptr, n))) return rc;
+    if ((rc = prepare_params_grid(ctx, ctx->in_xyz.p, nullptr, nullptr, n))) return rc;
     if ((rc = check_forced_grid(ctx))) return rc;
     if ((rc = upload_vec3(ctx, ctx->in_nrm, queries, q_stride, m))) return rc;          // the normals staging buffer is free here
     KPL_CUDA(ensure(ctx->scratch_i, (size_t)m + 2));
@@ -856,13 +864,13 @@ int kpl_radius_neighbors(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, int
                          const int32_t* queries, int64_t m, int64_t* offsets_out, int32_t* indices_out)
 {
     if (!ctx || !(radius >= 0) || m < 0 || !offsets_out || (m > 0 && !queries)) return KPL_E_INVALID;
-    begin_call(ctx);
+    detect_reset(ctx);
     offsets_out[0] = 0;
     if (n == 0 || m == 0) { for (int64_t k = 0; k <= m; ++k) offsets_out[k] = 0; return KPL_OK; }
     for (int64_t k = 0; k < m; ++k) if (queries[k] < 0 || queries[k] >= n) return fail(ctx, KPL_E_INVALID, "query index out of range");
     int rc = upload_inputs(ctx, xyz, xyz_stride, nullptr, 0, nullptr, n);
     if (rc) return rc;
-    if ((rc = prepare_grid(ctx, ctx->in_xyz.p, nullptr, nullptr, n))) return rc;
+    if ((rc = prepare_params_grid(ctx, ctx->in_xyz.p, nullptr, nullptr, n))) return rc;
     if ((rc = check_forced_grid(ctx))) return rc;
     KPL_CUDA(ensure(ctx->scratch_i, (size_t)n + 2));
     KPL_CUDA(launch_radius_stats(ctx, n, radius, ctx->scratch_i.p, nullptr));
@@ -896,7 +904,7 @@ int kpl_radius_neighbors(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, int
 int kpl_uniform_sample(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, int64_t n, float leaf, int32_t* idx_out, int64_t* m_out)
 {
     if (!ctx || !m_out || (n > 0 && !idx_out)) return KPL_E_INVALID;
-    begin_call(ctx);
+    detect_reset(ctx);
     *m_out = 0;
     if (!(leaf > 0.f) || !std::isfinite(leaf)) return fail(ctx, KPL_E_INVALID, "leaf must be > 0");
     if (n < 0 || n > 2147483000ll) return fail(ctx, KPL_E_INVALID, "point count out of range");

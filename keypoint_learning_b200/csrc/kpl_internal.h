@@ -38,7 +38,14 @@ struct GridDesc {
     // search that would have to look beyond such a face cannot be exact (normals.cu)
     int32_t interior_lo, interior_hi;
     int32_t guard_cells;  // points in the outermost guard_cells columns next to an interior face are expected to be clipped
-    int32_t owned_lo, owned_hi;   // local columns holding every point with a scoring role (0,0: not stated)
+    int32_t forced;       // 1: a ForcedGrid, whose points no bounding-box pass has checked (grid.cu: cell_key_kernel flags them)
+};
+
+// A grid given by the caller (a slab of a larger cloud) instead of the canonical grid of the cloud's bounding box
+struct ForcedGrid {
+    double origin[3];                                // the GLOBAL origin: a point's cell is floor((v - origin) / cell) - offset
+    int32_t dims[3], offset[3];
+    int32_t interior_lo, interior_hi, guard_cells;   // as in GridDesc
 };
 
 // One forest node, 8 bytes: thr_or_value + packed(child_block_offset << 10 | var); var == 1023 => leaf.
@@ -170,10 +177,18 @@ cudaError_t launch_radius_lists(kpl_ctx* c, int64_t n, double radius, const int3
 cudaError_t launch_unsort_rows(kpl_ctx* c, const float* d_sorted_rows, int64_t n, int width, float* d_out_orig_order);
 cudaError_t launch_unsort_normals(kpl_ctx* c, int64_t n, float4* d_out_orig_order);
 
-// detection phases (capi.cu), shared with the slab-sharded driver (shard.cu); all return kpl_status
+// canonical grid (capi.cu): the cell of kpl_params, the cells spanned by a bounding box [lo, hi], the cells a search
+// of `radius` has to visit on each side.  The same expressions make a slab plan the grid of the unsharded run.
+double canonical_cell(const kpl_params& P);
+int32_t grid_dim(double lo, double hi, double cell);
+int grid_reach(double radius, double cell);
+
+// detection phases (capi.cu), shared with the slab-sharded driver (shard.cu); all but detect_reset return kpl_status
+void detect_reset(kpl_ctx* ctx);
 int detect_check(kpl_ctx* ctx, int64_t n, bool sharded);
 int detect_begin(kpl_ctx* ctx);
-int detect_grid_phase(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, const uint8_t* d_role, int64_t n);
+// forced == nullptr: the canonical grid of the cloud's bounding box; cell_override > 0 replaces the canonical cell
+int prepare_grid(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, const uint8_t* d_role, int64_t n, const ForcedGrid* forced, double cell_override = 0.0);
 int detect_score_phase(kpl_ctx* ctx, bool normals_given, bool use_role, int64_t n);
 int detect_nms_phase(kpl_ctx* ctx, bool use_role, int64_t n, int32_t* d_kp_out);
 int detect_finish(kpl_ctx* ctx, int64_t n, int64_t* n_kp_out);

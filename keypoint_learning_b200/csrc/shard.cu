@@ -93,7 +93,7 @@ struct kpl_shard {
     ncclComm_t comm = nullptr;
     int64_t n_own = 0, n_l = 0, n_r = 0, n_loc = 0;     // owned / received left / received right / all local points
     int64_t send_l = 0, send_r = 0;                      // strip sizes sent to the left / right neighbour
-    int32_t x0 = 0, x1 = 0;                              // local grid columns [x0, x1) of the global grid
+    ForcedGrid grid{};                                   // local grid: columns [offset[0], offset[0] + dims[0]) of the global grid
     bool has_slab = false;
     DevBuf<float4> loc_xyz;                              // [left halo | owned | right halo]
     DevBuf<uint8_t> role;
@@ -108,8 +108,6 @@ struct kpl_shard {
     std::vector<ShardRecord> h_rec;
     cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     float exchange_ms = 0.f, gather_ms = 0.f;
-    kpl_params saved;
-    std::string err;
 };
 
 namespace {
@@ -180,48 +178,113 @@ __global__ void record_kernel(const unsigned long long* __restrict__ counters, c
     rec->reserved = 0;
 }
 
-// ---- exchanges -------------------------------------------------------------------------------------------------
-// Both neighbours at once: grouped ncclSend / ncclRecv on the context stream.
-int exchange_nccl(kpl_shard* s, const void* send_l, void* recv_l, const void* send_r, void* recv_r, size_t bytes_per_item)
+// ---- transport -------------------------------------------------------------------------------------------------
+// A call drives the ranks S[0..n): the one rank of an NCCL communicator, or every rank of an in-process group from
+// one host thread.  Errors are reported on S[0]'s context.
+int on_rank(kpl_shard** S, int r, int rc)
 {
-    cudaStream_t st = s->ctx->stream;
-    KS_NCCL(s->nccl->GroupStart());
-    if (s->rank > 0) {
-        if (s->send_l) KS_NCCL(s->nccl->Send(send_l, (size_t)s->send_l * bytes_per_item, ncclChar, s->rank - 1, s->comm, st));
-        if (s->n_l) KS_NCCL(s->nccl->Recv(recv_l, (size_t)s->n_l * bytes_per_item, ncclChar, s->rank - 1, s->comm, st));
-    }
-    if (s->rank < s->world - 1) {
-        if (s->send_r) KS_NCCL(s->nccl->Send(send_r, (size_t)s->send_r * bytes_per_item, ncclChar, s->rank + 1, s->comm, st));
-        if (s->n_r) KS_NCCL(s->nccl->Recv(recv_r, (size_t)s->n_r * bytes_per_item, ncclChar, s->rank + 1, s->comm, st));
-    }
-    KS_NCCL(s->nccl->GroupEnd());
+    if (rc && r) S[0]->ctx->err = S[r]->ctx->err;
+    return rc;
+}
+
+// f on every rank of the call, in rank order, up to the first failure
+template <typename F>
+int each_rank(kpl_shard** S, int n, F f)
+{
+    for (int r = 0; r < n; ++r)
+        if (int rc = f(S[r])) return on_rank(S, r, rc);
     return KPL_OK;
 }
 
-int set_forced_grid(kpl_shard* s)
+// the buffers of one exchange: the packed strips a rank sends, the ends of its local array that receive
+struct Strips {
+    const void *send_l, *send_r;
+    void *recv_l, *recv_r;
+    size_t item;
+};
+
+Strips strips(kpl_shard* t, bool scores)
 {
-    kpl_ctx* c = s->ctx;
-    s->saved = c->params;
-    kpl_params& P = c->params;
-    const kpl_slab_plan& L = s->plan;
-    P.grid_forced = 1;
-    for (int a = 0; a < 3; ++a) { P.grid_origin[a] = L.origin[a]; P.grid_dims[a] = L.dims[a]; P.grid_offset[a] = 0; }
-    P.grid_dims[0] = s->x1 - s->x0;
-    P.grid_offset[0] = s->x0;
-    P.slab_interior_lo = s->rank > 0;
-    P.slab_interior_hi = s->rank < s->world - 1;
-    P.slab_guard_cells = L.normal_support_cells;
-    P.slab_owned_lo = L.cuts[s->rank] - s->x0;
-    P.slab_owned_hi = L.cuts[s->rank + 1] - s->x0;
+    const int64_t hi = t->n_l + t->n_own;
+    if (scores) return {t->ssc_l.p, t->ssc_r.p, t->ctx->score.p, t->ctx->score.p + hi, sizeof(float)};
+    return {t->sbuf_l.p, t->sbuf_r.p, t->loc_xyz.p, t->loc_xyz.p + hi, sizeof(float4)};
+}
+
+// Position strips (scores == false) or score strips with both neighbours: a rank receives the right strip of its left
+// neighbour and the left strip of its right neighbour.  NCCL: grouped ncclSend / ncclRecv on the context stream.
+// In-process group: every stream is synchronised, then peer copies.
+int exchange(kpl_shard** S, int n, bool scores)
+{
+    kpl_shard* s = S[0];
+    if (!s->in_process) {
+        const Strips b = strips(s, scores);
+        cudaStream_t st = s->ctx->stream;
+        KS_NCCL(s->nccl->GroupStart());
+        if (s->rank > 0) {
+            if (s->send_l) KS_NCCL(s->nccl->Send(b.send_l, (size_t)s->send_l * b.item, ncclChar, s->rank - 1, s->comm, st));
+            if (s->n_l) KS_NCCL(s->nccl->Recv(b.recv_l, (size_t)s->n_l * b.item, ncclChar, s->rank - 1, s->comm, st));
+        }
+        if (s->rank < s->world - 1) {
+            if (s->send_r) KS_NCCL(s->nccl->Send(b.send_r, (size_t)s->send_r * b.item, ncclChar, s->rank + 1, s->comm, st));
+            if (s->n_r) KS_NCCL(s->nccl->Recv(b.recv_r, (size_t)s->n_r * b.item, ncclChar, s->rank + 1, s->comm, st));
+        }
+        KS_NCCL(s->nccl->GroupEnd());
+        return KPL_OK;
+    }
+    for (int r = 0; r < n; ++r) {
+        kpl_ctx* c = S[r]->ctx;
+        if (cudaSetDevice(c->device) != cudaSuccess || cudaStreamSynchronize(c->stream) != cudaSuccess)
+            return sfail(s, KPL_E_CUDA, "kpl_shard_detect_group: stream synchronisation failed");
+        c->syncs++;
+    }
+    for (int r = 0; r < n; ++r) {
+        kpl_shard* t = S[r];
+        const Strips b = strips(t, scores);
+        cudaError_t e = cudaSetDevice(t->ctx->device);
+        if (!e && r > 0 && t->n_l)
+            e = cudaMemcpyAsync(b.recv_l, strips(S[r - 1], scores).send_r, (size_t)t->n_l * b.item, cudaMemcpyDefault, t->ctx->stream);
+        if (!e && r < n - 1 && t->n_r)
+            e = cudaMemcpyAsync(b.recv_r, strips(S[r + 1], scores).send_l, (size_t)t->n_r * b.item, cudaMemcpyDefault, t->ctx->stream);
+        if (e) return sfail(s, KPL_E_CUDA, std::string("peer copy: ") + cudaGetErrorString(e));
+    }
+    return KPL_OK;
+}
+
+// The keypoint lists of all ranks into rank 0's kp_all, in rank order: NCCL send / receive, or peer copies.
+int gather_keypoints(kpl_shard** S, int n, const std::vector<int64_t>& counts)
+{
+    kpl_shard* s = S[0];
+    cudaStream_t st = s->ctx->stream;
+    if (s->in_process) {
+        int64_t off = 0;
+        for (int r = 0; r < n; ++r) {
+            if (counts[(size_t)r]) KS_CUDA(cudaMemcpyAsync(s->kp_all.p + off, S[r]->kp_global.p, (size_t)counts[(size_t)r] * sizeof(int32_t), cudaMemcpyDefault, st));
+            off += counts[(size_t)r];
+        }
+        return KPL_OK;
+    }
+    KS_NCCL(s->nccl->GroupStart());
+    if (s->rank == 0) {
+        int64_t off = counts[0];
+        for (int p = 1; p < s->world; ++p) {
+            if (counts[(size_t)p]) KS_NCCL(s->nccl->Recv(s->kp_all.p + off, (size_t)counts[(size_t)p], ncclInt32, p, s->comm, st));
+            off += counts[(size_t)p];
+        }
+    } else if (counts[(size_t)s->rank]) {
+        KS_NCCL(s->nccl->Send(s->kp_global.p, (size_t)counts[(size_t)s->rank], ncclInt32, 0, s->comm, st));
+    }
+    KS_NCCL(s->nccl->GroupEnd());
+    if (s->rank == 0 && counts[0]) KS_CUDA(cudaMemcpyAsync(s->kp_all.p, s->kp_global.p, (size_t)counts[0] * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
     return KPL_OK;
 }
 
 // ---- the phases of one detection (everything is enqueued on the context stream) --------------------------------
+// the per-call reset of the rank's context, then its position strips
 int phase_pack(kpl_shard* s)
 {
     kpl_ctx* c = s->ctx;
+    detect_reset(c);
     KS_CUDA(cudaSetDevice(c->device));
-    (void)cudaGetLastError();                      // a stale error of an earlier, unrelated runtime call must not be blamed on this step
     KS_CUDA(cudaEventRecord(s->ev[0], c->stream));
     const float4* owned = s->loc_xyz.p + s->n_l;
     if (s->send_l) {
@@ -243,7 +306,7 @@ int phase_score(kpl_shard* s)
     int rc = detect_begin(c);
     if (rc) return rc;
     c->launches += 2;
-    if ((rc = detect_grid_phase(c, s->loc_xyz.p, nullptr, s->role.p, s->n_loc))) return rc;
+    if ((rc = prepare_grid(c, s->loc_xyz.p, nullptr, s->role.p, s->n_loc, &s->grid))) return rc;
     if ((rc = detect_score_phase(c, false, true, s->n_loc))) return rc;
     KS_CUDA(cudaEventRecord(s->ev[2], c->stream));
     const float* owned_scores = c->score.p + s->n_l;
@@ -329,6 +392,69 @@ void finish_timings(kpl_shard* s, bool gathered)
     (void)cudaGetLastError();
 }
 
+int copy_out(kpl_shard* s, float* scores_owned_out, int32_t* kp_global_out, int64_t kp_capacity, int64_t total)
+{
+    kpl_ctx* c = s->ctx;
+    KS_CUDA(cudaSetDevice(c->device));
+    if (scores_owned_out)
+        KS_CUDA(cudaMemcpyAsync(scores_owned_out, c->score.p + s->n_l, (size_t)s->n_own * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    if (s->rank == 0 && kp_global_out && total > 0) {
+        if (kp_capacity < total) return sfail(s, KPL_E_INVALID, "kp_global_out is too small");
+        KS_CUDA(cudaMemcpyAsync(kp_global_out, s->kp_sorted.p, (size_t)total * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    }
+    KS_CUDA(cudaStreamSynchronize(c->stream));
+    c->syncs++;
+    c->stats.host_syncs = c->syncs;
+    c->stats.kernel_launches = c->launches;
+    return KPL_OK;
+}
+
+// One sharded detection over the ranks S[0..n) of this call.  The verdict over the records of all ranks comes before a
+// rank-local error of detect_finish, so that every rank returns the same status.
+int detect_step(kpl_shard** S, int n, float* const* scores_owned_out, int32_t* kp_global_out, int64_t kp_capacity, int64_t* n_kp_out)
+{
+    kpl_shard* s = S[0];
+    kpl_ctx* c = s->ctx;
+    int rc;
+    if ((rc = each_rank(S, n, check_ready)) || (rc = each_rank(S, n, phase_pack)) || (rc = exchange(S, n, false)) ||
+        (rc = each_rank(S, n, phase_score)) || (rc = exchange(S, n, true)) || (rc = each_rank(S, n, phase_nms)))
+        return rc;
+    // the records of all ranks to S[0]'s host: all-gathered, or one copy per in-process rank
+    if (!s->in_process) {
+        KS_NCCL(s->nccl->AllGather(s->rec.p, s->rec_all.p, sizeof(ShardRecord), ncclChar, s->comm, c->stream));
+        KS_CUDA(cudaMemcpyAsync(s->h_rec.data(), s->rec_all.p, (size_t)s->world * sizeof(ShardRecord), cudaMemcpyDeviceToHost, c->stream));
+    }
+    int local_err = KPL_OK, err_rank = 0;
+    for (int r = 0; r < n; ++r) {
+        kpl_ctx* t = S[r]->ctx;
+        if (s->in_process) {
+            KS_CUDA(cudaSetDevice(t->device));
+            KS_CUDA(cudaMemcpyAsync(&s->h_rec[(size_t)r], S[r]->rec.p, sizeof(ShardRecord), cudaMemcpyDeviceToHost, t->stream));
+        }
+        int64_t local_kp = 0;
+        const int e = detect_finish(t, S[r]->n_loc, &local_kp);      // the synchronisation; also fills stats / timings of the rank
+        if (e && !local_err && e != KPL_E_HALO && e != KPL_E_GRID) { local_err = e; err_rank = r; }
+    }
+    int64_t total = 0;
+    std::vector<int64_t> counts;
+    if ((rc = verdict(s, total, counts))) return rc;                   // identical on every rank: nobody is left waiting in a collective
+    if (local_err) return on_rank(S, err_rank, local_err);
+    if (n_kp_out) *n_kp_out = total;
+    // keypoint lists to rank 0 (sizes are known everywhere now), then one sort into ascending global index
+    KS_CUDA(cudaSetDevice(c->device));
+    KS_CUDA(cudaEventRecord(s->ev[4], c->stream));
+    if (s->rank == 0) { KS_CUDA(ensure(s->kp_all, (size_t)total + 1)); KS_CUDA(ensure(s->kp_sorted, (size_t)total + 1)); }
+    if ((rc = gather_keypoints(S, n, counts))) return rc;
+    if (s->rank == 0 && (rc = sort_keypoints(s, total))) return rc;
+    KS_CUDA(cudaEventRecord(s->ev[5], c->stream));
+    for (int r = 0; r < n; ++r) {
+        rc = copy_out(S[r], scores_owned_out ? scores_owned_out[r] : nullptr, r == 0 ? kp_global_out : nullptr, kp_capacity, total);
+        if (rc) return on_rank(S, r, rc);
+        finish_timings(S[r], r == 0);
+    }
+    return KPL_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -350,18 +476,18 @@ int kpl_slab_plan_make(const float* xyz, int32_t stride, int64_t n, const kpl_pa
             lo[a] = std::min(lo[a], v[a]); hi[a] = std::max(hi[a], v[a]);
         }
     }
-    // the same expressions as prepare_grid (capi.cu): the plan IS the grid of the unsharded run
-    const double cell = (double)p->radius_features * (1.0 + 9.5367431640625e-07) / (double)p->cells_per_radius;
+    // the canonical grid of the whole cloud: the plan IS the grid of the unsharded run
+    const double cell = canonical_cell(*p);
     out->cell = cell; out->world = world; out->n_points = n;
     double ncells = 1.0;
     for (int a = 0; a < 3; ++a) {
         out->origin[a] = (double)lo[a];
-        out->dims[a] = (int32_t)std::min(2147483000.0, std::floor(((double)hi[a] - (double)lo[a]) / cell) + 1.0);
+        out->dims[a] = grid_dim(lo[a], hi[a], cell);
         ncells *= (double)out->dims[a];
     }
     if (ncells > 2147483646.0) return KPL_E_GRID;
-    out->reach_feat = (int)std::floor((double)p->radius_features * (1.0 + 4.76837158203125e-07) / cell) + 1;
-    out->reach_nms = (int)std::floor((double)p->radius_nms * (1.0 + 4.76837158203125e-07) / cell) + 1;
+    out->reach_feat = grid_reach(p->radius_features, cell);
+    out->reach_nms = grid_reach(p->radius_nms, cell);
     out->normal_support_cells = normal_support_cells;
     out->halo = std::max(out->reach_feat + normal_support_cells, out->reach_nms);
     const int nx = out->dims[0], ny = out->dims[1], nz = out->dims[2];
@@ -547,9 +673,12 @@ static int set_slab_local(kpl_shard* s, const float* xyz, int32_t stride, const 
         if (s->rank < s->world - 1 && cx >= c1 - H) sr.push_back((int32_t)i);
     }
     s->n_own = n_own; s->send_l = (int64_t)sl.size(); s->send_r = (int64_t)sr.size();
-    s->x0 = std::max(c0 - H, 0); s->x1 = std::min(c1 + H, L.dims[0]);
-    if (s->rank == 0) s->x0 = 0;
-    if (s->rank == s->world - 1) s->x1 = L.dims[0];
+    // the local grid: this rank's columns and the halo columns beyond its interior faces
+    const int x0 = s->rank > 0 ? std::max(c0 - H, 0) : 0, x1 = s->rank < s->world - 1 ? std::min(c1 + H, L.dims[0]) : L.dims[0];
+    ForcedGrid& g = s->grid;
+    for (int a = 0; a < 3; ++a) { g.origin[a] = L.origin[a]; g.dims[a] = L.dims[a]; g.offset[a] = 0; }
+    g.dims[0] = x1 - x0; g.offset[0] = x0;
+    g.interior_lo = s->rank > 0; g.interior_hi = s->rank < s->world - 1; g.guard_cells = L.normal_support_cells;
     KS_CUDA(ensure(s->gidx, (size_t)n_own));
     KS_CUDA(ensure(s->sel_l, sl.size() + 1)); KS_CUDA(ensure(s->sel_r, sr.size() + 1));
     KS_CUDA(ensure(s->sbuf_l, sl.size() + 1)); KS_CUDA(ensure(s->sbuf_r, sr.size() + 1));
@@ -562,18 +691,26 @@ static int set_slab_local(kpl_shard* s, const float* xyz, int32_t stride, const 
     return KPL_OK;
 }
 
-// once n_l / n_r are known: the local cloud buffer, the roles, the owned coordinates
-static int set_slab_layout(kpl_shard* s, const float* xyz, int32_t stride)
+// [left halo | owned | right halo] once the strip sizes n_l / n_r are known: the local cloud buffer and the roles.
+// An in-process rank's owned points, which kpl_shard_set_slab staged at the start of loc_xyz, move to their place.
+static int set_slab_layout(kpl_shard* s, int64_t n_l, int64_t n_r)
 {
     kpl_ctx* c = s->ctx;
-    s->n_loc = s->n_l + s->n_own + s->n_r;
+    s->n_l = n_l; s->n_r = n_r; s->n_loc = n_l + s->n_own + n_r;
     if (s->n_loc > 2147483000ll) return sfail(s, KPL_E_INVALID, "slab too large");
-    KS_CUDA(ensure(s->loc_xyz, (size_t)s->n_loc));
+    KS_CUDA(cudaSetDevice(c->device));
+    DevBuf<float4> staged;
+    if (s->in_process) std::swap(staged, s->loc_xyz);
+    cudaError_t e = ensure(s->loc_xyz, (size_t)s->n_loc);
+    if (!e && staged.p) e = cudaMemcpyAsync(s->loc_xyz.p + n_l, staged.p, (size_t)s->n_own * sizeof(float4), cudaMemcpyDeviceToDevice, c->stream);
+    if (!e && staged.p) e = cudaStreamSynchronize(c->stream);
+    srelease(staged);
+    KS_CUDA(e);
     KS_CUDA(ensure(s->role, (size_t)s->n_loc));
     KS_CUDA(cudaMemsetAsync(s->role.p, KPL_ROLE_HALO, (size_t)s->n_loc, c->stream));
-    KS_CUDA(cudaMemsetAsync(s->role.p + s->n_l, KPL_ROLE_OWNED, (size_t)s->n_own, c->stream));
+    KS_CUDA(cudaMemsetAsync(s->role.p + n_l, KPL_ROLE_OWNED, (size_t)s->n_own, c->stream));
     s->has_slab = true;
-    return kpl_shard_upload(s, xyz, stride);
+    return KPL_OK;
 }
 
 int kpl_shard_set_slab(kpl_shard* s, const float* xyz, int32_t stride, const int32_t* gidx, int64_t n_own)
@@ -583,7 +720,7 @@ int kpl_shard_set_slab(kpl_shard* s, const float* xyz, int32_t stride, const int
     int rc = set_slab_local(s, xyz, stride, gidx, n_own);
     if (rc) return rc;
     if (s->in_process) {
-        // the group driver fills n_l / n_r from its peers; the layout follows there (kpl_shard_detect_group)
+        // the group driver takes n_l / n_r from the peers; the layout follows there (kpl_shard_detect_group)
         s->n_l = s->n_r = -1;
         KS_CUDA(ensure(s->loc_xyz, (size_t)n_own));
         if (stride == 16) KS_CUDA(cudaMemcpy(s->loc_xyz.p, xyz, (size_t)n_own * 16, cudaMemcpyHostToDevice));
@@ -597,9 +734,9 @@ int kpl_shard_set_slab(kpl_shard* s, const float* xyz, int32_t stride, const int
     std::vector<unsigned long long> all(2 * (size_t)s->world);
     KS_CUDA(cudaMemcpyAsync(all.data(), s->sizes_all.p, all.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
     KS_CUDA(cudaStreamSynchronize(c->stream));
-    s->n_l = s->rank > 0 ? (int64_t)all[2 * (size_t)(s->rank - 1) + 1] : 0;            // the left neighbour's RIGHT strip
-    s->n_r = s->rank < s->world - 1 ? (int64_t)all[2 * (size_t)(s->rank + 1)] : 0;     // the right neighbour's LEFT strip
-    return set_slab_layout(s, xyz, stride);
+    rc = set_slab_layout(s, s->rank > 0 ? (int64_t)all[2 * (size_t)(s->rank - 1) + 1] : 0,     // the left neighbour's RIGHT strip
+                         s->rank < s->world - 1 ? (int64_t)all[2 * (size_t)(s->rank + 1)] : 0); // the right neighbour's LEFT strip
+    return rc ? rc : kpl_shard_upload(s, xyz, stride);
 }
 
 int kpl_shard_upload(kpl_shard* s, const float* xyz, int32_t stride)
@@ -615,80 +752,12 @@ int kpl_shard_upload(kpl_shard* s, const float* xyz, int32_t stride)
     return KPL_OK;
 }
 
-static int copy_out(kpl_shard* s, float* scores_owned_out, int32_t* kp_global_out, int64_t kp_capacity, int64_t total)
-{
-    kpl_ctx* c = s->ctx;
-    KS_CUDA(cudaSetDevice(c->device));
-    if (scores_owned_out)
-        KS_CUDA(cudaMemcpyAsync(scores_owned_out, c->score.p + s->n_l, (size_t)s->n_own * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    if (s->rank == 0 && kp_global_out && total > 0) {
-        if (kp_capacity < total) return sfail(s, KPL_E_INVALID, "kp_global_out is too small");
-        KS_CUDA(cudaMemcpyAsync(kp_global_out, s->kp_sorted.p, (size_t)total * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
-    }
-    KS_CUDA(cudaStreamSynchronize(c->stream));
-    c->syncs++;
-    c->stats.host_syncs = c->syncs;
-    c->stats.kernel_launches = c->launches;
-    return KPL_OK;
-}
-
 int kpl_shard_detect(kpl_shard* s, float* scores_owned_out, int32_t* kp_global_out, int64_t kp_capacity, int64_t* n_kp_out)
 {
     if (!s) return KPL_E_INVALID;
     if (n_kp_out) *n_kp_out = 0;
     if (s->in_process) return sfail(s, KPL_E_INVALID, "ranks of an in-process group are driven by kpl_shard_detect_group");
-    int rc = check_ready(s);
-    if (rc) return rc;
-    kpl_ctx* c = s->ctx;
-    c->launches = 0; c->syncs = 0; c->err.clear();
-    memset(&c->timings, 0, sizeof c->timings);
-    memset(&c->stats, 0, sizeof c->stats);
-    c->stats.n_views = 1;
-    c->last_has_normals = c->last_has_features = c->last_has_fragile = false;
-    set_forced_grid(s);
-    auto body = [&]() -> int {
-        int r;
-        if ((r = phase_pack(s))) return r;
-        if ((r = exchange_nccl(s, s->sbuf_l.p, s->loc_xyz.p, s->sbuf_r.p, s->loc_xyz.p + s->n_l + s->n_own, sizeof(float4)))) return r;
-        if ((r = phase_score(s))) return r;
-        if ((r = exchange_nccl(s, s->ssc_l.p, c->score.p, s->ssc_r.p, c->score.p + s->n_l + s->n_own, sizeof(float)))) return r;
-        if ((r = phase_nms(s))) return r;
-        KS_NCCL(s->nccl->AllGather(s->rec.p, s->rec_all.p, sizeof(ShardRecord), ncclChar, s->comm, c->stream));
-        KS_CUDA(cudaMemcpyAsync(s->h_rec.data(), s->rec_all.p, (size_t)s->world * sizeof(ShardRecord), cudaMemcpyDeviceToHost, c->stream));
-        int64_t local_kp = 0;
-        r = detect_finish(c, s->n_loc, &local_kp);            // the synchronisation; also fills stats / timings of this rank
-        int64_t total = 0;
-        std::vector<int64_t> counts;
-        const int rv = verdict(s, total, counts);                 // identical on every rank: nobody is left waiting in a collective
-        if (rv) return rv;
-        if (r) return r;
-        if (n_kp_out) *n_kp_out = total;
-        // keypoint lists to rank 0 (sizes are known everywhere now), then one sort into ascending global index
-        KS_CUDA(cudaEventRecord(s->ev[4], c->stream));
-        if (s->rank == 0) { KS_CUDA(ensure(s->kp_all, (size_t)total + 1)); KS_CUDA(ensure(s->kp_sorted, (size_t)total + 1)); }
-        KS_NCCL(s->nccl->GroupStart());
-        if (s->rank == 0) {
-            int64_t off = counts[0];
-            for (int p = 1; p < s->world; ++p) {
-                if (counts[(size_t)p]) KS_NCCL(s->nccl->Recv(s->kp_all.p + off, (size_t)counts[(size_t)p], ncclInt32, p, s->comm, c->stream));
-                off += counts[(size_t)p];
-            }
-        } else if (counts[(size_t)s->rank]) {
-            KS_NCCL(s->nccl->Send(s->kp_global.p, (size_t)counts[(size_t)s->rank], ncclInt32, 0, s->comm, c->stream));
-        }
-        KS_NCCL(s->nccl->GroupEnd());
-        if (s->rank == 0) {
-            if (counts[0]) KS_CUDA(cudaMemcpyAsync(s->kp_all.p, s->kp_global.p, (size_t)counts[0] * sizeof(int32_t), cudaMemcpyDeviceToDevice, c->stream));
-            if ((r = sort_keypoints(s, total))) return r;
-        }
-        KS_CUDA(cudaEventRecord(s->ev[5], c->stream));
-        if ((r = copy_out(s, scores_owned_out, kp_global_out, kp_capacity, total))) return r;
-        finish_timings(s, true);
-        return KPL_OK;
-    };
-    rc = body();
-    c->params = s->saved;
-    return rc;
+    return detect_step(&s, 1, &scores_owned_out, kp_global_out, kp_capacity, n_kp_out);
 }
 
 // All ranks of an in-process group from one host thread: the same phases, strips moved by peer copies.  The streams
@@ -700,110 +769,17 @@ int kpl_shard_detect_group(kpl_shard** S, int32_t world, float** scores_owned_ou
     if (!S || world < 1 || !S[0]) return KPL_E_INVALID;
     if (n_kp_out) *n_kp_out = 0;
     kpl_shard* s = S[0];                       // errors are reported on rank 0's context
-    for (int r = 0; r < world; ++r) {
+    for (int r = 0; r < world; ++r)
         if (!S[r] || !S[r]->in_process || S[r]->world != world || S[r]->rank != r) return sfail(s, KPL_E_INVALID, "kpl_shard_detect_group: not the ranks 0..world-1 of one in-process group");
-    }
-    auto sync_all = [&]() -> int {
-        for (int r = 0; r < world; ++r) {
-            if (cudaSetDevice(S[r]->ctx->device) != cudaSuccess || cudaStreamSynchronize(S[r]->ctx->stream) != cudaSuccess)
-                return sfail(s, KPL_E_CUDA, "kpl_shard_detect_group: stream synchronisation failed");
-            S[r]->ctx->syncs++;
-        }
-        return KPL_OK;
-    };
-    int rc;
-    // first call after set_slab: strip sizes from the peers, then the layout (owned points move to their final place)
+    // first call after set_slab: the strip sizes come from the peers
     for (int r = 0; r < world; ++r) {
         kpl_shard* t = S[r];
-        if (t->n_l >= 0 && t->has_slab) continue;
+        if (t->has_slab) continue;
         if (t->n_own < 1) return sfail(s, KPL_E_INVALID, "kpl_shard_set_slab was not called on every rank");
-        const int64_t n_l = r > 0 ? S[r - 1]->send_r : 0, n_r = r < world - 1 ? S[r + 1]->send_l : 0;
-        t->n_l = n_l; t->n_r = n_r; t->n_loc = n_l + t->n_own + n_r;
-        {
-            kpl_shard* s = t;
-            KS_CUDA(cudaSetDevice(t->ctx->device));
-            DevBuf<float4> fresh;
-            KS_CUDA(ensure(fresh, (size_t)t->n_loc));
-            KS_CUDA(cudaMemcpy(fresh.p + n_l, t->loc_xyz.p, (size_t)t->n_own * sizeof(float4), cudaMemcpyDeviceToDevice));
-            srelease(t->loc_xyz);
-            t->loc_xyz = fresh;
-            KS_CUDA(ensure(t->role, (size_t)t->n_loc));
-            KS_CUDA(cudaMemset(t->role.p, KPL_ROLE_HALO, (size_t)t->n_loc));
-            KS_CUDA(cudaMemset(t->role.p + n_l, KPL_ROLE_OWNED, (size_t)t->n_own));
-            t->has_slab = true;
-        }
+        const int rc = set_slab_layout(t, r > 0 ? S[r - 1]->send_r : 0, r < world - 1 ? S[r + 1]->send_l : 0);
+        if (rc) return on_rank(S, r, rc);
     }
-    for (int r = 0; r < world; ++r) {
-        if ((rc = check_ready(S[r]))) { if (r) s->ctx->err = S[r]->ctx->err; return rc; }
-        kpl_ctx* c = S[r]->ctx;
-        c->launches = 0; c->syncs = 0; c->err.clear();
-        memset(&c->timings, 0, sizeof c->timings);
-        memset(&c->stats, 0, sizeof c->stats);
-        c->stats.n_views = 1;
-        c->last_has_normals = c->last_has_features = c->last_has_fragile = false;
-        set_forced_grid(S[r]);
-    }
-    auto restore = [&]() { for (int r = 0; r < world; ++r) S[r]->ctx->params = S[r]->saved; };
-    auto fail_rank = [&](int r, int code) { if (r) s->ctx->err = S[r]->ctx->err; restore(); return code; };
-    // the strip a rank RECEIVES from its left neighbour is that neighbour's right strip, and vice versa
-    auto move = [&](int bytes_per_item, auto sendbuf_l, auto sendbuf_r, auto recv_l, auto recv_r) -> int {
-        for (int r = 0; r < world; ++r) {
-            kpl_shard* t = S[r];
-            if (cudaSetDevice(t->ctx->device) != cudaSuccess) return KPL_E_CUDA;
-            cudaError_t e = cudaSuccess;
-            if (r > 0 && t->n_l) e = cudaMemcpyAsync(recv_l(t), sendbuf_r(S[r - 1]), (size_t)t->n_l * bytes_per_item, cudaMemcpyDefault, t->ctx->stream);
-            if (!e && r < world - 1 && t->n_r) e = cudaMemcpyAsync(recv_r(t), sendbuf_l(S[r + 1]), (size_t)t->n_r * bytes_per_item, cudaMemcpyDefault, t->ctx->stream);
-            if (e) return sfail(s, KPL_E_CUDA, std::string("peer copy: ") + cudaGetErrorString(e));
-        }
-        return KPL_OK;
-    };
-    for (int r = 0; r < world; ++r) if ((rc = phase_pack(S[r]))) return fail_rank(r, rc);
-    if ((rc = sync_all())) { restore(); return rc; }
-    if ((rc = move((int)sizeof(float4), [](kpl_shard* t) { return (const void*)t->sbuf_l.p; }, [](kpl_shard* t) { return (const void*)t->sbuf_r.p; },
-                   [](kpl_shard* t) { return (void*)t->loc_xyz.p; }, [](kpl_shard* t) { return (void*)(t->loc_xyz.p + t->n_l + t->n_own); }))) { restore(); return rc; }
-    for (int r = 0; r < world; ++r) if ((rc = phase_score(S[r]))) return fail_rank(r, rc);
-    if ((rc = sync_all())) { restore(); return rc; }
-    if ((rc = move((int)sizeof(float), [](kpl_shard* t) { return (const void*)t->ssc_l.p; }, [](kpl_shard* t) { return (const void*)t->ssc_r.p; },
-                   [](kpl_shard* t) { return (void*)t->ctx->score.p; }, [](kpl_shard* t) { return (void*)(t->ctx->score.p + t->n_l + t->n_own); }))) { restore(); return rc; }
-    for (int r = 0; r < world; ++r) if ((rc = phase_nms(S[r]))) return fail_rank(r, rc);
-    std::vector<int64_t> counts((size_t)world, 0);
-    int first_err = KPL_OK, err_rank = 0;
-    std::vector<ShardRecord> recs((size_t)world);
-    for (int r = 0; r < world; ++r) {
-        kpl_shard* t = S[r];
-        kpl_shard* s = t;
-        KS_CUDA(cudaSetDevice(t->ctx->device));
-        KS_CUDA(cudaMemcpyAsync(&recs[(size_t)r], t->rec.p, sizeof(ShardRecord), cudaMemcpyDeviceToHost, t->ctx->stream));
-        int64_t local_kp = 0;
-        const int e = detect_finish(t->ctx, t->n_loc, &local_kp);
-        if (e && !first_err && e != KPL_E_HALO && e != KPL_E_GRID) { first_err = e; err_rank = r; }
-    }
-    for (int r = 0; r < world; ++r) S[r]->h_rec = recs;
-    int64_t total = 0;
-    rc = verdict(s, total, counts);
-    if (rc) { restore(); return rc; }
-    if (first_err) return fail_rank(err_rank, first_err);
-    if (n_kp_out) *n_kp_out = total;
-    {
-        kpl_ctx* c = s->ctx;
-        KS_CUDA(cudaSetDevice(c->device));
-        KS_CUDA(cudaEventRecord(s->ev[4], c->stream));
-        KS_CUDA(ensure(s->kp_all, (size_t)total + 1)); KS_CUDA(ensure(s->kp_sorted, (size_t)total + 1));
-        int64_t off = 0;
-        for (int r = 0; r < world; ++r) {
-            if (counts[(size_t)r]) KS_CUDA(cudaMemcpyAsync(s->kp_all.p + off, S[r]->kp_global.p, (size_t)counts[(size_t)r] * sizeof(int32_t), cudaMemcpyDefault, c->stream));
-            off += counts[(size_t)r];
-        }
-        if ((rc = sort_keypoints(s, total))) { restore(); return rc; }
-        KS_CUDA(cudaEventRecord(s->ev[5], c->stream));
-    }
-    for (int r = 0; r < world; ++r) {
-        rc = copy_out(S[r], scores_owned_out ? scores_owned_out[r] : nullptr, r == 0 ? kp_global_out : nullptr, kp_capacity, total);
-        if (rc) return fail_rank(r, rc);
-        finish_timings(S[r], r == 0);
-    }
-    restore();
-    return KPL_OK;
+    return detect_step(S, world, scores_owned_out, kp_global_out, kp_capacity, n_kp_out);
 }
 
 int kpl_shard_get_info(const kpl_shard* s, kpl_shard_info* out)
@@ -813,8 +789,8 @@ int kpl_shard_get_info(const kpl_shard* s, kpl_shard_info* out)
     out->n_owned = s->n_own; out->n_left = std::max<int64_t>(s->n_l, 0); out->n_right = std::max<int64_t>(s->n_r, 0);
     out->send_left = s->send_l; out->send_right = s->send_r;
     out->halo_bytes = (s->send_l + s->send_r) * (int64_t)(sizeof(float4) + sizeof(float));
-    out->local_dims[0] = s->x1 - s->x0; out->local_dims[1] = s->plan.dims[1]; out->local_dims[2] = s->plan.dims[2];
-    out->local_offset[0] = s->x0;
+    out->local_dims[0] = s->grid.dims[0]; out->local_dims[1] = s->plan.dims[1]; out->local_dims[2] = s->plan.dims[2];
+    out->local_offset[0] = s->grid.offset[0];
     out->rank = s->rank; out->world = s->world;
     out->exchange_ms = s->exchange_ms; out->gather_ms = s->gather_ms;
     return KPL_OK;

@@ -22,8 +22,6 @@ import numpy as np
 
 from . import capi
 
-ROLE_HALO, ROLE_SCORE, ROLE_OWNED = 0, 1, 3
-
 
 @dataclass
 class SlabPlan:
@@ -166,34 +164,29 @@ class SlabJob:
             pass
 
 
-KPL_E_HALO = 12
+def _widening(detect, jobs, xyz, r_feat, r_nms, cpr, max_support):
+    """detect(); on KPL_E_HALO (a k-NN normal that matters was clipped by a slab face -- every rank reports it) re-plan
+    `jobs` with twice the k-NN support and try again.  The support is thereby derived from the data."""
+    while True:
+        try:
+            return detect()
+        except capi.KplError as e:
+            ns = jobs[0].plan.normal_support_cells * 2
+            if e.code != capi.KPL_E_HALO or ns > max_support:
+                raise
+            plan = plan_slabs(xyz, r_feat, r_nms, cpr, jobs[0].world, ns)
+            for j in jobs:
+                j.replan(xyz, plan)
 
 
 def detect_widening(job, xyz, r_feat, r_nms, cpr, max_support=64, **kw):
-    """job.detect(); on KPL_E_HALO (a k-NN normal that matters was clipped by a slab face -- every rank reports it)
-    re-plan with twice the k-NN support and try again.  The support is thereby derived from the data."""
-    while True:
-        try:
-            return job.detect(**kw)
-        except capi.KplError as e:
-            ns = job.plan.normal_support_cells * 2
-            if e.code != KPL_E_HALO or ns > max_support:
-                raise
-            job.replan(xyz, plan_slabs(xyz, r_feat, r_nms, cpr, job.world, ns))
+    """job.detect() with the widening loop of _widening (every rank of an NCCL job runs it in lockstep)."""
+    return _widening(lambda: job.detect(**kw), [job], xyz, r_feat, r_nms, cpr, max_support)
 
 
 def detect_group_widening(jobs, xyz, r_feat, r_nms, cpr, max_support=64, want_scores=True):
-    """detect_group() with the same widening loop for an in-process group."""
-    while True:
-        try:
-            return detect_group(jobs, want_scores)
-        except capi.KplError as e:
-            ns = jobs[0].plan.normal_support_cells * 2
-            if e.code != KPL_E_HALO or ns > max_support:
-                raise
-            plan = plan_slabs(xyz, r_feat, r_nms, cpr, len(jobs), ns)
-            for j in jobs:
-                j.replan(xyz, plan)
+    """detect_group() with the widening loop of _widening for an in-process group."""
+    return _widening(lambda: detect_group(jobs, want_scores), jobs, xyz, r_feat, r_nms, cpr, max_support)
 
 
 def detect_group(jobs, want_scores=True):
@@ -244,7 +237,7 @@ class HostSlab:
         self.n_r = 0 if from_right is None else len(from_right)
         self.local = np.ascontiguousarray(np.concatenate(parts))
         self.role = np.zeros(len(self.local), np.uint8)
-        self.role[self.n_l:self.n_l + len(self.own)] = ROLE_OWNED
+        self.role[self.n_l:self.n_l + len(self.own)] = capi.ROLE_OWNED
         return self.local, self.role
 
     def score_strips(self, scores_local):

@@ -1,6 +1,7 @@
 """N-GPU result == 1-GPU result, bit for bit (BASELINE.md s5), through the C entry points kpl_shard_* of include/kpl.h.
 On a single GPU: the ranks of an in-process group (peer copies instead of NCCL; every kernel and all host logic of the
 sharded step) and a one-rank NCCL communicator.  With 2+ GPUs: real NCCL halo / score exchange under torchrun."""
+import ctypes
 import os
 import socket
 import subprocess
@@ -73,6 +74,14 @@ def _single_gpu_reference(kpl, xyz, forest="synthetic-T100-D15"):
     return det
 
 
+def _ctx_params(det):
+    """kpl_get_params of the detector's context, field by field (a sharded call must leave it untouched)."""
+    from keypoint_learning_b200 import capi
+    p = capi.KplParams()
+    assert capi.load_library().kpl_get_params(det._h, ctypes.byref(p)) == 0
+    return {f: (list(v) if isinstance(v, ctypes.Array) else v) for f, v in ((f, getattr(p, f)) for f, _ in p._fields_)}
+
+
 @pytest.mark.parametrize("world", [1, 2, 3, 4])
 def test_in_process_group_equals_single_gpu(kpl, world):
     """All ranks of an in-process group on ONE device: same kernels, same host logic, strips moved by device copies."""
@@ -113,21 +122,27 @@ def test_clipped_knn_support_is_detected(kpl):
     rng = np.random.default_rng(5)
     # ~6 mm spacing: the 10th neighbour lies ~11 mm away, far beyond one 5 mm cell column
     xyz = np.stack([rng.uniform(-400, 400, 4000), rng.uniform(-100, 100, 4000), rng.uniform(-3, 3, 4000)], axis=1).astype(np.float32)
+    ref = _single_gpu_reference(kpl, xyz)
+    ref.setInputCloud(xyz)
+    _, idx_full = ref.compute()
     plan = shard.plan_slabs(xyz, 20.0, 4.0, 4, 2, normal_support_cells=1)
     dets = [_single_gpu_reference(kpl, xyz) for _ in range(2)]
     jobs = [shard.SlabJob(d, xyz, plan, r, None) for r, d in enumerate(dets)]
+    before = [_ctx_params(d) for d in dets]
     with pytest.raises(kpl.KplError) as e:
         shard.detect_group(jobs)
     assert e.value.code == 12
+    # the failed call left every context as it was: a plain detection on it is the single-GPU one
+    for d, p in zip(dets, before):
+        assert _ctx_params(d) == p
+        d.setInputCloud(xyz)
+        assert np.array_equal(d.compute()[1], idx_full)
     for j in jobs:
         j.close()
     # a wide enough support passes and reproduces the single-GPU result
     plan = shard.plan_slabs(xyz, 20.0, 4.0, 4, 2, normal_support_cells=40)
     jobs = [shard.SlabJob(d, xyz, plan, r, None) for r, d in enumerate(dets)]
     kp, scores = shard.detect_group(jobs)
-    ref = _single_gpu_reference(kpl, xyz)
-    ref.setInputCloud(xyz)
-    _, idx_full = ref.compute()
     assert np.array_equal(kp, idx_full)
     for j, sc in zip(jobs, scores):
         full = ref.getResponse()[j.gidx]
@@ -147,10 +162,14 @@ def test_one_rank_nccl_communicator(kpl):
     _, idx_full = ref.compute()
     sc_full = ref.getResponse().copy()
     plan = shard.plan_slabs(xyz, 20.0, 4.0, 4, 1)
+    before = _ctx_params(ref)
     job = shard.SlabJob(ref, xyz, plan, 0, shard.nccl_unique_id())
     sc = np.empty(job.n_owned, np.float32)
     n, kp = job.detect(scores_out=sc)
     assert n == len(idx_full) and np.array_equal(kp, idx_full)
     assert np.array_equal(sc.view(np.uint32), sc_full.view(np.uint32))
+    # the sharded call left the context as it was: a plain detection on it is the single-GPU one
+    assert _ctx_params(ref) == before
+    assert np.array_equal(ref.compute()[1], idx_full)
     job.close()
     ref.close()
