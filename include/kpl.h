@@ -54,7 +54,9 @@ enum kpl_normals_mode {
     KPL_NORMALS_RADIUS = 2   /* NormalEstimation::setRadiusSearch(r_feat)    (impl/KeypointLearning.hpp:130-137) */
 };
 
-/* Per-point roles for slab-sharded clouds (no counterpart in the reference, which is single process). */
+/* Per-point roles for slab-sharded clouds (no counterpart in the reference, which is single process).  kpl_detect* with a
+ * role array refuses draws-remove NMS (KPL_E_UNSUPPORTED): such a caller drives one slab by itself and cannot see the
+ * neighbours' decisions its own depend on; the kpl_shard_* entry points exchange them. */
 enum kpl_role { KPL_ROLE_HALO = 0, KPL_ROLE_SCORE = 1, KPL_ROLE_OWNED = 3 };
 
 /* Mirrors the detector's setters (include/KeypointLearning.h:81-90,102-155) and the TestDetector
@@ -111,7 +113,7 @@ typedef struct kpl_stats {
     double grid_origin[3];
     double grid_cell;
     int32_t fast_math;        /* 1: the self-tested FMA-corrected sqrt/div sequences were used (bit-identical) */
-    int32_t reserved;
+    int32_t nms_rounds;       /* draws-remove NMS: resolution rounds of the last call (one host synchronisation each); 0 without */
     int64_t n_unscored;       /* points without a finite normal: score NaN, never a keypoint (hpp:277)        */
     int64_t n_near_threshold; /* scored points with |score - threshold| <= 1e-5: the decisions a 1e-5 score
                                  difference against another implementation could flip                         */
@@ -215,6 +217,8 @@ KPL_API int kpl_detect_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_no
  * [view_offsets[v], view_offsets[v+1]) of xyz (and of normals when given).  Every view is processed exactly as a
  * kpl_detect call on it alone would (own bounding box, own canonical grid and accumulation order: bit-identical
  * scores and keypoints), but all views share one stacked grid, one launch per stage and one set of host round trips.
+ * Draws-remove NMS included: no r_nms neighbourhood spans two views and every view keeps its own index order, so the
+ * resolution rounds over the stacked grid decide all views at once (one host round trip per round for the whole batch).
  * scores_out: NULL or n floats.  kp_idx_out (capacity n): VIEW-LOCAL keypoint indices, view after view, ascending
  * inside a view; kp_offsets_out[n_views + 1]: view v's keypoints are kp_idx_out[kp_offsets_out[v] .. kp_offsets_out[v+1]). */
 KPL_API int kpl_detect_batch(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
@@ -236,7 +240,10 @@ KPL_API int kpl_detect_batch_device(kpl_ctx* ctx, const void* d_xyz4, const void
  *   3. exchanges the 4-byte scores of the strips, so that NMS sees the neighbours' scores  [ncclSend/ncclRecv]
  *   4. runs threshold + NMS for its owned points; rank 0 gathers the ascending GLOBAL keypoint index list.
  * A k-NN normal search that the slab edge would clip fails the call on every rank with KPL_E_HALO (widen
- * normal_support_cells).  draws-remove NMS is not available (its dependency chain crosses slabs). */
+ * normal_support_cells).  draws-remove NMS: every rank classifies and decides its OWNED points only; the states of the
+ * strip points (1 B per point) go to the neighbours after the classification and after every resolution round, and all
+ * ranks stop on the same global count of undecided candidates -- one host synchronisation per round
+ * (kpl_stats.nms_rounds).  The result is the single-GPU one. */
 #define KPL_MAX_RANKS 64
 typedef struct kpl_slab_plan {
     double origin[3];              /* grid origin = bounding-box minimum of the whole cloud                        */

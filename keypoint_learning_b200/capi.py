@@ -51,7 +51,7 @@ class KplStats(C.Structure):
     _fields_ = [("n_points", C.c_int64), ("n_scored", C.c_int64), ("feature_pairs", C.c_int64), ("candidate_pairs", C.c_int64),
                 ("n_above_threshold", C.c_int64), ("n_keypoints", C.c_int64), ("grid_cells", C.c_int64),
                 ("grid_dims", C.c_int32 * 3), ("kernel_launches", C.c_int32), ("grid_origin", C.c_double * 3), ("grid_cell", C.c_double),
-                ("fast_math", C.c_int32), ("reserved", C.c_int32), ("n_unscored", C.c_int64),
+                ("fast_math", C.c_int32), ("nms_rounds", C.c_int32), ("n_unscored", C.c_int64),
                 ("n_near_threshold", C.c_int64), ("n_fragile_points", C.c_int64), ("host_syncs", C.c_int32), ("n_views", C.c_int32)]
 
 

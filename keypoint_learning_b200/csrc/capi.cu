@@ -409,13 +409,15 @@ void kpl::detect_reset(kpl_ctx* ctx)
 
 namespace kpl {
 
-int detect_check(kpl_ctx* ctx, int64_t n, bool sharded)
+int detect_check(kpl_ctx* ctx, int64_t n, bool with_role)
 {
     const kpl_params& P = ctx->params;
     if (n < 0 || n > 2147483000ll) return fail(ctx, KPL_E_INVALID, "point count out of range");
     if (ctx->forest.ntrees < 1) return fail(ctx, KPL_E_FOREST, "no forest loaded");
-    if (P.draws_remove && P.non_maxima && sharded)
-        return fail(ctx, KPL_E_UNSUPPORTED, "draws-remove NMS walks the whole cloud in index order (hpp:233-250): not available for slab-sharded calls");
+    // a caller that drives a slab by itself cannot see the neighbours' decisions, which its own depend on (the kpl_shard_*
+    // entry points exchange them between the resolution rounds)
+    if (P.draws_remove && P.non_maxima && with_role)
+        return fail(ctx, KPL_E_UNSUPPORTED, "draws-remove NMS walks the whole cloud in index order (hpp:233-250): not available with a role array; use the kpl_shard_* entry points");
     const int F = P.n_annulus * P.n_bins;
     if (ctx->forest.var_count > 0 && ctx->forest.var_count != F) return fail(ctx, KPL_E_VARCOUNT, "annuli*bins does not match the forest's var_count");
     // whatever var_count says, no split may read beyond the A*B floats of a feature row
@@ -536,8 +538,6 @@ static int run_detect_batch(kpl_ctx* ctx, const float4* d_xyz, const float4* d_n
     int rc = detect_check(ctx, n, false);
     if (rc) return rc;
     if (ctx->params.grid_forced) return fail(ctx, KPL_E_INVALID, "a forced grid cannot be combined with a batch of views");
-    if (ctx->params.draws_remove && ctx->params.non_maxima)
-        return fail(ctx, KPL_E_UNSUPPORTED, "draws-remove NMS is not available for batched calls");
     ctx->stats.n_points = n; ctx->stats.n_views = nviews;
     if (n == 0) return KPL_OK;
     if ((rc = detect_begin(ctx))) return rc;

@@ -166,6 +166,13 @@ cudaError_t launch_forest(kpl_ctx* c, int64_t n, bool use_role);
 #endif
 cudaError_t launch_nms(kpl_ctx* c, int64_t n, bool use_role);
 cudaError_t launch_nms_draws(kpl_ctx* c, int64_t n, bool use_role);
+// the pieces of launch_nms_draws, for a caller that exchanges halo states between rounds (shard.cu); gidx: global index of
+// every local original index (nullptr: the identity)
+cudaError_t launch_nms_draws_classify(kpl_ctx* c, int64_t n, bool use_role);
+cudaError_t launch_nms_draws_round(kpl_ctx* c, int64_t n, bool use_role, const int32_t* gidx);
+cudaError_t launch_nms_draws_flags(kpl_ctx* c, int64_t n, bool use_role);
+// resolution rounds of a cloud of n points never exceed this cap (the lowest undecided index resolves in every round)
+inline int nms_round_cap(int64_t n) { return (int)(n < (1 << 20) ? n : (1 << 20)); }
 cudaError_t launch_compact(kpl_ctx* c, int64_t n, int32_t* d_kp_idx_out);
 
 cudaError_t uniform_sample(kpl_ctx* c, const float4* xyz, int64_t n, float leaf, const float mn[3], const float mx[3],
@@ -185,7 +192,8 @@ int grid_reach(double radius, double cell);
 
 // detection phases (capi.cu), shared with the slab-sharded driver (shard.cu); all but detect_reset return kpl_status
 void detect_reset(kpl_ctx* ctx);
-int detect_check(kpl_ctx* ctx, int64_t n, bool sharded);
+// with_role: a caller-supplied role array (kpl_detect*), which rules out draws-remove NMS; the kpl_shard_* driver passes false
+int detect_check(kpl_ctx* ctx, int64_t n, bool with_role);
 int detect_begin(kpl_ctx* ctx);
 // forced == nullptr: the canonical grid of the cloud's bounding box; cell_override > 0 replaces the canonical cell
 int prepare_grid(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, const uint8_t* d_role, int64_t n, const ForcedGrid* forced, double cell_override = 0.0);

@@ -85,6 +85,10 @@ cudaError_t launch_nms(kpl_ctx* c, int64_t n, bool use_role)
 // draw is active, and active once all of them are decided; the lowest undecided index always resolves, so
 // the loop ends, and decisions never change once made (stale reads only postpone a decision).
 // state: 0 not a keypoint, 1 keypoint, 2 undecided candidate, 3 skipped candidate.
+// With roles (a slab of a sharded cloud) only OWNED points are classified and decided: a halo point's own
+// lower-index draws may lie beyond the halo, so its state is always its owner's decision, copied in by the
+// caller between rounds.  "Lower index" is then the GLOBAL index: gidx maps a local original index to it
+// (nullptr: the identity, a single cloud or a batch, whose views keep their own index order).
 __device__ __forceinline__ float draw_distance(const float4& p, const float4& c)
 {
     // (pointIn.getVector3fMap() - drawPoint.getVector3fMap()).norm(): Eigen reduction order a0 + (a1 + a2)
@@ -96,8 +100,8 @@ template <int PASS>   // 0: classify, 1: one resolution round
 __global__ void __launch_bounds__(128)
 nms_draws_kernel(const float4* __restrict__ s_pos, const float* __restrict__ s_score, const uint32_t* __restrict__ skey,
                  const int32_t* __restrict__ cell_start, const uint8_t* __restrict__ s_role, int dimx, int dimy, int dimz,
-                 int n, float rn2, int reach, double th, float draws_thr, uint8_t* __restrict__ s_state,
-                 unsigned long long* __restrict__ counters)
+                 int n, float rn2, int reach, double th, float draws_thr, const int32_t* __restrict__ gidx,
+                 uint8_t* __restrict__ s_state, unsigned long long* __restrict__ counters)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     bool above = false, near = false;
@@ -105,12 +109,12 @@ nms_draws_kernel(const float4* __restrict__ s_pos, const float* __restrict__ s_s
         const float4 p = __ldg(s_pos + i);
         const uint32_t orig = __float_as_uint(p.w);
         const float my = __ldg(s_score + i);
+        const bool owned = !s_role || ((s_role[i] & 3) == 3);
         if (PASS == 0) {
-            const bool owned = !s_role || ((s_role[i] & 3) == 3);
             above = owned && isfinite(my) && !((double)my < th);
             near = owned && isfinite(my) && fabs((double)my - th) <= 1e-5;
         }
-        const bool work = PASS == 0 ? above : (s_state[i] == 2);
+        const bool work = PASS == 0 ? above : (owned && s_state[i] == 2);
         if (work) {
             int cx, cy, cz;
             key_to_cell_n(__ldg(skey + i), dimx, dimy, cx, cy, cz);
@@ -119,6 +123,7 @@ nms_draws_kernel(const float4* __restrict__ s_pos, const float* __restrict__ s_s
             const int x0 = max(cx - reach, 0), x1 = min(cx + reach, dimx - 1);
             bool is_max = true, has_draw = false, close_draw = false;   // PASS 0
             bool lower_active = false, lower_undecided = false;         // PASS 1
+            const uint32_t my_order = PASS == 1 && gidx ? (uint32_t)__ldg(gidx + orig) : orig;
             for (int z = z0; z <= z1 && is_max; ++z)
                 for (int y = y0; y <= y1 && is_max; ++y) {
                     const int64_t base = ((int64_t)z * dimy + y) * dimx;
@@ -133,7 +138,8 @@ nms_draws_kernel(const float4* __restrict__ s_pos, const float* __restrict__ s_s
                                 has_draw = true;
                                 if (draw_distance(p, c) < draws_thr) close_draw = true;
                             }
-                        } else if (my == sj && __float_as_uint(c.w) < orig && draw_distance(p, c) < draws_thr) {
+                        } else if (my == sj && (gidx ? (uint32_t)__ldg(gidx + __float_as_uint(c.w)) : __float_as_uint(c.w)) < my_order &&
+                                   draw_distance(p, c) < draws_thr) {
                             // a lower-index close draw: active (1) skips this point, undecided (2) postpones it;
                             // a close draw that is a keypoint without draws cannot exist (it ties with this point)
                             const uint8_t st = s_state[j];
@@ -156,39 +162,66 @@ nms_draws_kernel(const float4* __restrict__ s_pos, const float* __restrict__ s_s
     }
 }
 
-__global__ void __launch_bounds__(256) state_to_flag_kernel(const float4* __restrict__ s_pos, const uint8_t* __restrict__ s_state, int n,
-                                                            uint8_t* __restrict__ flag)
+__global__ void __launch_bounds__(256) state_to_flag_kernel(const float4* __restrict__ s_pos, const uint8_t* __restrict__ s_role,
+                                                            const uint8_t* __restrict__ s_state, int n, uint8_t* __restrict__ flag)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) flag[__float_as_uint(__ldg(&s_pos[i].w))] = s_state[i] == 1 ? 1 : 0;
+    if (i < n) flag[__float_as_uint(__ldg(&s_pos[i].w))] = s_state[i] == 1 && (!s_role || (s_role[i] & 3) == 3) ? 1 : 0;
 }
 
-cudaError_t launch_nms_draws(kpl_ctx* c, int64_t n, bool use_role)
+cudaError_t launch_nms_draws_classify(kpl_ctx* c, int64_t n, bool use_role)
 {
     const kpl_params& U = c->params;
     cudaError_t e;
     if ((e = ensure(c->flag, n)) || (e = ensure(c->s_state, n))) return e;
     const double rn = (double)U.radius_nms;
-    const unsigned blocks = (unsigned)((n + 127) / 128);
-    const uint8_t* role = use_role ? c->s_role.p : nullptr;
-    nms_draws_kernel<0><<<blocks, 128, 0, c->stream>>>(c->s_pos.p, c->s_score.p, c->key_b.p, c->cell_start.p, role,
-                                                        c->grid.dim[0], c->grid.dim[1], c->grid.dim[2], (int)n, (float)(rn * rn),
-                                                        c->grid.reach_nms, U.threshold, U.draws_threshold, c->s_state.p, c->counters.p);
+    nms_draws_kernel<0><<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(c->s_pos.p, c->s_score.p, c->key_b.p, c->cell_start.p,
+                                                                              use_role ? c->s_role.p : nullptr, c->grid.dim[0], c->grid.dim[1],
+                                                                              c->grid.dim[2], (int)n, (float)(rn * rn), c->grid.reach_nms,
+                                                                              U.threshold, U.draws_threshold, nullptr, c->s_state.p, c->counters.p);
     c->launches++;
-    for (int round = 0; round < (int)std::min<int64_t>(n, 1 << 20); ++round) {
-        if ((e = cudaMemsetAsync(c->counters.p + 6, 0, sizeof(unsigned long long), c->stream))) return e;
-        nms_draws_kernel<1><<<blocks, 128, 0, c->stream>>>(c->s_pos.p, c->s_score.p, c->key_b.p, c->cell_start.p, role,
-                                                            c->grid.dim[0], c->grid.dim[1], c->grid.dim[2], (int)n, (float)(rn * rn),
-                                                            c->grid.reach_nms, U.threshold, U.draws_threshold, c->s_state.p, c->counters.p);
-        c->launches++;
+    return cudaGetLastError();
+}
+
+// one resolution round; counters[6] = candidates left undecided by it
+cudaError_t launch_nms_draws_round(kpl_ctx* c, int64_t n, bool use_role, const int32_t* gidx)
+{
+    const kpl_params& U = c->params;
+    cudaError_t e;
+    if ((e = cudaMemsetAsync(c->counters.p + 6, 0, sizeof(unsigned long long), c->stream))) return e;
+    const double rn = (double)U.radius_nms;
+    nms_draws_kernel<1><<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(c->s_pos.p, c->s_score.p, c->key_b.p, c->cell_start.p,
+                                                                              use_role ? c->s_role.p : nullptr, c->grid.dim[0], c->grid.dim[1],
+                                                                              c->grid.dim[2], (int)n, (float)(rn * rn), c->grid.reach_nms,
+                                                                              U.threshold, U.draws_threshold, gidx, c->s_state.p, c->counters.p);
+    c->launches++;
+    c->stats.nms_rounds++;
+    return cudaGetLastError();
+}
+
+cudaError_t launch_nms_draws_flags(kpl_ctx* c, int64_t n, bool use_role)
+{
+    state_to_flag_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(c->s_pos.p, use_role ? c->s_role.p : nullptr, c->s_state.p,
+                                                                            (int)n, c->flag.p);
+    c->launches++;
+    return cudaGetLastError();
+}
+
+// A whole cloud, or a batch of views: each view is a connected component of its own (§5.4 padding layers) that keeps its
+// own index order inside the concatenation, so the rounds over the stacked grid resolve every view at once.
+cudaError_t launch_nms_draws(kpl_ctx* c, int64_t n, bool use_role)
+{
+    cudaError_t e;
+    if ((e = launch_nms_draws_classify(c, n, use_role))) return e;
+    for (int round = 0; round < nms_round_cap(n); ++round) {
+        if ((e = launch_nms_draws_round(c, n, use_role, nullptr))) return e;
         unsigned long long undecided = 0;
         if ((e = cudaMemcpyAsync(&undecided, c->counters.p + 6, sizeof undecided, cudaMemcpyDeviceToHost, c->stream))) return e;
         if ((e = cudaStreamSynchronize(c->stream))) return e;
+        c->syncs++;
         if (undecided == 0) break;
     }
-    state_to_flag_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(c->s_pos.p, c->s_state.p, (int)n, c->flag.p);
-    c->launches++;
-    return cudaGetLastError();
+    return launch_nms_draws_flags(c, n, use_role);
 }
 
 // setNonMaxima(false) (hpp:189-196): every scored point is a keypoint.

@@ -98,9 +98,18 @@ struct kpl_shard {
     DevBuf<float4> loc_xyz;                              // [left halo | owned | right halo]
     DevBuf<uint8_t> role;
     DevBuf<int32_t> gidx;                                // global index of every owned point
+    DevBuf<int32_t> loc_gidx;                            // global index of every local point, [left halo | owned | right halo]
     DevBuf<int32_t> sel_l, sel_r;                        // owned-local indices of the strips
     DevBuf<float4> sbuf_l, sbuf_r;                       // packed position strips
     DevBuf<float> ssc_l, ssc_r;                          // packed score strips
+    DevBuf<int32_t> sgi_l, sgi_r;                        // global indices of the strip points (sent once per resident slab)
+    DevBuf<uint8_t> st_orig;                             // draws-remove NMS states in local original order (halo parts received)
+    // packed state strips, two sets used in turn: an in-process peer copy of round k (on the receiver's stream) may still
+    // read one while round k + 1 packs the other; the exchange of round k + 1 synchronises every stream before round k + 2
+    DevBuf<uint8_t> sst_l[2], sst_r[2];
+    int sst = 0;                                         // the set packed last
+    DevBuf<unsigned long long> und_all;                  // undecided candidates of every rank after a round (NCCL)
+    unsigned long long h_undecided = 0;                  // the same, this rank (in-process group)
     DevBuf<int32_t> kp_local, kp_global, kp_all, kp_sorted;
     DevBuf<uint8_t> sort_tmp;
     DevBuf<ShardRecord> rec, rec_all;
@@ -156,6 +165,26 @@ __global__ void __launch_bounds__(256) pack_scores_kernel(const float* __restric
     const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (k < m) out[k] = owned_scores[sel[k]];
 }
+__global__ void __launch_bounds__(256) pack_states_kernel(const uint8_t* __restrict__ owned_states, const int32_t* __restrict__ sel, int64_t m,
+                                                          uint8_t* __restrict__ out)
+{
+    const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (k < m) out[k] = owned_states[sel[k]];
+}
+// draws-remove states of the owned points, cell-sorted -> local original order (the order the strips are selected in)
+__global__ void __launch_bounds__(256) owned_states_kernel(const float4* __restrict__ s_pos, const uint8_t* __restrict__ s_role,
+                                                           const uint8_t* __restrict__ s_state, int64_t n, uint8_t* __restrict__ st_orig)
+{
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i < n && s_role[i] == KPL_ROLE_OWNED) st_orig[__float_as_uint(s_pos[i].w)] = s_state[i];
+}
+// states of halo points (their owners' decisions) arrived in local original order, as the scores do
+__global__ void __launch_bounds__(256) halo_states_kernel(const float4* __restrict__ s_pos, const uint8_t* __restrict__ s_role,
+                                                          const uint8_t* __restrict__ st_orig, int64_t n, uint8_t* __restrict__ s_state)
+{
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i < n && s_role[i] == KPL_ROLE_HALO) s_state[i] = st_orig[__float_as_uint(s_pos[i].w)];
+}
 // scores of halo points arrived in original (local) order; NMS reads the cell-sorted copy
 __global__ void __launch_bounds__(256) halo_scores_kernel(const float4* __restrict__ s_pos, const uint8_t* __restrict__ s_role,
                                                           const float* __restrict__ score, int64_t n, float* __restrict__ s_score)
@@ -196,6 +225,10 @@ int each_rank(kpl_shard** S, int n, F f)
     return KPL_OK;
 }
 
+// what an exchange moves: positions and scores every detection, draws-remove states every resolution round, global
+// indices once per resident slab
+enum class Strip { positions, scores, states, gidx };
+
 // the buffers of one exchange: the packed strips a rank sends, the ends of its local array that receive
 struct Strips {
     const void *send_l, *send_r;
@@ -203,21 +236,25 @@ struct Strips {
     size_t item;
 };
 
-Strips strips(kpl_shard* t, bool scores)
+Strips strips(kpl_shard* t, Strip kind)
 {
     const int64_t hi = t->n_l + t->n_own;
-    if (scores) return {t->ssc_l.p, t->ssc_r.p, t->ctx->score.p, t->ctx->score.p + hi, sizeof(float)};
-    return {t->sbuf_l.p, t->sbuf_r.p, t->loc_xyz.p, t->loc_xyz.p + hi, sizeof(float4)};
+    switch (kind) {
+    case Strip::scores: return {t->ssc_l.p, t->ssc_r.p, t->ctx->score.p, t->ctx->score.p + hi, sizeof(float)};
+    case Strip::states: return {t->sst_l[t->sst].p, t->sst_r[t->sst].p, t->st_orig.p, t->st_orig.p + hi, sizeof(uint8_t)};
+    case Strip::gidx: return {t->sgi_l.p, t->sgi_r.p, t->loc_gidx.p, t->loc_gidx.p + hi, sizeof(int32_t)};
+    default: return {t->sbuf_l.p, t->sbuf_r.p, t->loc_xyz.p, t->loc_xyz.p + hi, sizeof(float4)};
+    }
 }
 
-// Position strips (scores == false) or score strips with both neighbours: a rank receives the right strip of its left
-// neighbour and the left strip of its right neighbour.  NCCL: grouped ncclSend / ncclRecv on the context stream.
-// In-process group: every stream is synchronised, then peer copies.
-int exchange(kpl_shard** S, int n, bool scores)
+// Strips of one kind with both neighbours: a rank receives the right strip of its left neighbour and the left strip of
+// its right neighbour.  NCCL: grouped ncclSend / ncclRecv on the context stream.  In-process group: every stream is
+// synchronised, then peer copies.
+int exchange(kpl_shard** S, int n, Strip kind)
 {
     kpl_shard* s = S[0];
     if (!s->in_process) {
-        const Strips b = strips(s, scores);
+        const Strips b = strips(s, kind);
         cudaStream_t st = s->ctx->stream;
         KS_NCCL(s->nccl->GroupStart());
         if (s->rank > 0) {
@@ -239,12 +276,12 @@ int exchange(kpl_shard** S, int n, bool scores)
     }
     for (int r = 0; r < n; ++r) {
         kpl_shard* t = S[r];
-        const Strips b = strips(t, scores);
+        const Strips b = strips(t, kind);
         cudaError_t e = cudaSetDevice(t->ctx->device);
         if (!e && r > 0 && t->n_l)
-            e = cudaMemcpyAsync(b.recv_l, strips(S[r - 1], scores).send_r, (size_t)t->n_l * b.item, cudaMemcpyDefault, t->ctx->stream);
+            e = cudaMemcpyAsync(b.recv_l, strips(S[r - 1], kind).send_r, (size_t)t->n_l * b.item, cudaMemcpyDefault, t->ctx->stream);
         if (!e && r < n - 1 && t->n_r)
-            e = cudaMemcpyAsync(b.recv_r, strips(S[r + 1], scores).send_l, (size_t)t->n_r * b.item, cudaMemcpyDefault, t->ctx->stream);
+            e = cudaMemcpyAsync(b.recv_r, strips(S[r + 1], kind).send_l, (size_t)t->n_r * b.item, cudaMemcpyDefault, t->ctx->stream);
         if (e) return sfail(s, KPL_E_CUDA, std::string("peer copy: ") + cudaGetErrorString(e));
     }
     return KPL_OK;
@@ -317,6 +354,36 @@ int phase_score(kpl_shard* s)
     return KPL_OK;
 }
 
+bool draws_remove(const kpl_ctx* c) { return c->params.non_maxima && c->params.draws_remove; }
+
+// the draws-remove states of the owned strip points, packed for the neighbours
+int pack_states(kpl_shard* s)
+{
+    kpl_ctx* c = s->ctx;
+    if (s->send_l + s->send_r == 0) return KPL_OK;
+    owned_states_kernel<<<(unsigned)((s->n_loc + 255) / 256), 256, 0, c->stream>>>(c->s_pos.p, c->s_role.p, c->s_state.p, s->n_loc, s->st_orig.p);
+    const uint8_t* owned = s->st_orig.p + s->n_l;
+    s->sst ^= 1;
+    if (s->send_l) pack_states_kernel<<<(unsigned)((s->send_l + 255) / 256), 256, 0, c->stream>>>(owned, s->sel_l.p, s->send_l, s->sst_l[s->sst].p);
+    if (s->send_r) pack_states_kernel<<<(unsigned)((s->send_r + 255) / 256), 256, 0, c->stream>>>(owned, s->sel_r.p, s->send_r, s->sst_r[s->sst].p);
+    KS_CUDA(cudaGetLastError());
+    c->launches += 1 + (s->send_l > 0) + (s->send_r > 0);
+    return KPL_OK;
+}
+
+// keypoints (owned points only) to global indices, and the rank's record
+int phase_records(kpl_shard* s)
+{
+    kpl_ctx* c = s->ctx;
+    to_global_kernel<<<(unsigned)((s->n_own + 255) / 256), 256, 0, c->stream>>>(s->kp_local.p, c->counters.p, s->gidx.p, s->n_l, s->n_own, s->kp_global.p);
+    record_kernel<<<1, 1, 0, c->stream>>>(c->counters.p, (const uint32_t*)c->d_bbox, s->rec.p);
+    KS_CUDA(cudaGetLastError());
+    c->launches += 2;
+    return KPL_OK;
+}
+
+// Threshold + NMS.  Draws-remove: only the classification here; the resolution rounds need the neighbours' decisions and
+// run over all ranks (nms_draws_rounds), then phase_draws_keypoints.
 int phase_nms(kpl_shard* s)
 {
     kpl_ctx* c = s->ctx;
@@ -324,13 +391,68 @@ int phase_nms(kpl_shard* s)
     KS_CUDA(cudaEventRecord(s->ev[3], c->stream));
     if (s->n_l + s->n_r > 0)
         halo_scores_kernel<<<(unsigned)((s->n_loc + 255) / 256), 256, 0, c->stream>>>(c->s_pos.p, c->s_role.p, c->score.p, s->n_loc, c->s_score.p);
+    c->launches++;
+    if (draws_remove(c)) {
+        KS_CUDA(launch_nms_draws_classify(c, s->n_loc, true));
+        return pack_states(s);
+    }
     int rc = detect_nms_phase(c, true, s->n_loc, s->kp_local.p);
-    if (rc) return rc;
-    to_global_kernel<<<(unsigned)((s->n_own + 255) / 256), 256, 0, c->stream>>>(s->kp_local.p, c->counters.p, s->gidx.p, s->n_l, s->n_own, s->kp_global.p);
-    record_kernel<<<1, 1, 0, c->stream>>>(c->counters.p, (const uint32_t*)c->d_bbox, s->rec.p);
-    KS_CUDA(cudaGetLastError());
-    c->launches += 3;
-    return KPL_OK;
+    return rc ? rc : phase_records(s);
+}
+
+// one draws-remove resolution round of the owned points, on the halo states the last exchange brought in
+int phase_draws_round(kpl_shard* s)
+{
+    kpl_ctx* c = s->ctx;
+    KS_CUDA(cudaSetDevice(c->device));
+    if (s->n_l + s->n_r > 0) {
+        halo_states_kernel<<<(unsigned)((s->n_loc + 255) / 256), 256, 0, c->stream>>>(c->s_pos.p, c->s_role.p, s->st_orig.p, s->n_loc, c->s_state.p);
+        KS_CUDA(cudaGetLastError());
+        c->launches++;
+    }
+    KS_CUDA(launch_nms_draws_round(c, s->n_loc, true, s->loc_gidx.p));
+    if (s->in_process)      // read by the host after the next exchange, which synchronises every stream of the group
+        KS_CUDA(cudaMemcpyAsync(&s->h_undecided, c->counters.p + 6, sizeof s->h_undecided, cudaMemcpyDeviceToHost, c->stream));
+    return pack_states(s);
+}
+
+// The draws-remove rounds over the slabs.  After the classification and after every round, the owned states of the
+// strip points go to the neighbours, so that a halo point always holds its owner's decision (a stale one only postpones
+// a decision).  Every rank stops on the same global count of undecided candidates, within the same cap: no rank is left
+// waiting in a collective.  One host synchronisation per round.
+int nms_draws_rounds(kpl_shard** S, int n)
+{
+    kpl_shard* s = S[0];
+    kpl_ctx* c = s->ctx;
+    if (!draws_remove(c)) return KPL_OK;
+    int rc = exchange(S, n, Strip::states);
+    for (int round = 0; !rc && round < nms_round_cap(s->plan.n_points); ++round) {
+        if ((rc = each_rank(S, n, phase_draws_round)) || (rc = exchange(S, n, Strip::states))) return rc;
+        unsigned long long undecided = 0;
+        if (s->in_process) {
+            for (int r = 0; r < n; ++r) undecided += S[r]->h_undecided;
+        } else {
+            std::vector<unsigned long long> all((size_t)s->world);
+            KS_NCCL(s->nccl->AllGather(c->counters.p + 6, s->und_all.p, 1, ncclUint64, s->comm, c->stream));
+            KS_CUDA(cudaMemcpyAsync(all.data(), s->und_all.p, all.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+            KS_CUDA(cudaStreamSynchronize(c->stream));
+            c->syncs++;
+            for (unsigned long long u : all) undecided += u;
+        }
+        if (undecided == 0) break;
+    }
+    return rc;
+}
+
+// draws-remove: flags of the decided owned points, compaction, records
+int phase_draws_keypoints(kpl_shard* s)
+{
+    kpl_ctx* c = s->ctx;
+    if (!draws_remove(c)) return KPL_OK;
+    KS_CUDA(cudaSetDevice(c->device));
+    KS_CUDA(launch_nms_draws_flags(c, s->n_loc, true));
+    KS_CUDA(launch_compact(c, s->n_loc, s->kp_local.p));
+    return phase_records(s);
 }
 
 // after the records of all ranks reached the host: the same verdict on every rank
@@ -378,7 +500,7 @@ int check_ready(kpl_shard* s)
     // then be two search reaches wide, which no device check can verify after the fact
     if (s->world > 1 && s->ctx->params.normals_mode == KPL_NORMALS_RADIUS && s->plan.normal_support_cells < s->plan.reach_feat)
         return sfail(s, KPL_E_HALO, "radius-mode normals need normal_support_cells >= reach_feat (the whole r_feat ball of every halo point that matters)");
-    return detect_check(s->ctx, s->n_loc, true);
+    return detect_check(s->ctx, s->n_loc, false);
 }
 
 void finish_timings(kpl_shard* s, bool gathered)
@@ -416,8 +538,9 @@ int detect_step(kpl_shard** S, int n, float* const* scores_owned_out, int32_t* k
     kpl_shard* s = S[0];
     kpl_ctx* c = s->ctx;
     int rc;
-    if ((rc = each_rank(S, n, check_ready)) || (rc = each_rank(S, n, phase_pack)) || (rc = exchange(S, n, false)) ||
-        (rc = each_rank(S, n, phase_score)) || (rc = exchange(S, n, true)) || (rc = each_rank(S, n, phase_nms)))
+    if ((rc = each_rank(S, n, check_ready)) || (rc = each_rank(S, n, phase_pack)) || (rc = exchange(S, n, Strip::positions)) ||
+        (rc = each_rank(S, n, phase_score)) || (rc = exchange(S, n, Strip::scores)) || (rc = each_rank(S, n, phase_nms)) ||
+        (rc = nms_draws_rounds(S, n)) || (rc = each_rank(S, n, phase_draws_keypoints)))
         return rc;
     // the records of all ranks to S[0]'s host: all-gathered, or one copy per in-process rank
     if (!s->in_process) {
@@ -611,7 +734,8 @@ int kpl_shard_create(kpl_ctx* ctx, const kpl_slab_plan* plan, int32_t rank, cons
     bool ok = cudaSetDevice(ctx->device) == cudaSuccess;
     for (int i = 0; ok && i < 6; ++i) ok = cudaEventCreate(&s->ev[i]) == cudaSuccess;
     ok = ok && ensure(s->rec, 1) == cudaSuccess && ensure(s->rec_all, (size_t)s->world) == cudaSuccess &&
-         ensure(s->sizes, 2) == cudaSuccess && ensure(s->sizes_all, 2 * (size_t)s->world) == cudaSuccess;
+         ensure(s->sizes, 2) == cudaSuccess && ensure(s->sizes_all, 2 * (size_t)s->world) == cudaSuccess &&
+         ensure(s->und_all, (size_t)s->world) == cudaSuccess;
     if (!ok) { ctx->err = "kpl_shard_create: CUDA resources"; kpl_shard_destroy(s); return KPL_E_CUDA; }
     if (!s->in_process) {
         std::string why;
@@ -646,8 +770,10 @@ void kpl_shard_destroy(kpl_shard* s)
     if (!s) return;
     if (s->ctx) { cudaSetDevice(s->ctx->device); cudaStreamSynchronize(s->ctx->stream); }
     if (s->comm && s->nccl) s->nccl->CommDestroy(s->comm);
-    srelease(s->loc_xyz); srelease(s->role); srelease(s->gidx); srelease(s->sel_l); srelease(s->sel_r);
-    srelease(s->sbuf_l); srelease(s->sbuf_r); srelease(s->ssc_l); srelease(s->ssc_r);
+    srelease(s->loc_xyz); srelease(s->role); srelease(s->gidx); srelease(s->loc_gidx); srelease(s->sel_l); srelease(s->sel_r);
+    srelease(s->sbuf_l); srelease(s->sbuf_r); srelease(s->ssc_l); srelease(s->ssc_r); srelease(s->sgi_l); srelease(s->sgi_r);
+    srelease(s->st_orig); srelease(s->und_all);
+    for (int k = 0; k < 2; ++k) { srelease(s->sst_l[k]); srelease(s->sst_r[k]); }
     srelease(s->kp_local); srelease(s->kp_global); srelease(s->kp_all); srelease(s->kp_sorted); srelease(s->sort_tmp);
     srelease(s->rec); srelease(s->rec_all); srelease(s->sizes); srelease(s->sizes_all);
     for (int i = 0; i < 6; ++i) if (s->ev[i]) cudaEventDestroy(s->ev[i]);
@@ -683,11 +809,18 @@ static int set_slab_local(kpl_shard* s, const float* xyz, int32_t stride, const 
     KS_CUDA(ensure(s->sel_l, sl.size() + 1)); KS_CUDA(ensure(s->sel_r, sr.size() + 1));
     KS_CUDA(ensure(s->sbuf_l, sl.size() + 1)); KS_CUDA(ensure(s->sbuf_r, sr.size() + 1));
     KS_CUDA(ensure(s->ssc_l, sl.size() + 1)); KS_CUDA(ensure(s->ssc_r, sr.size() + 1));
+    for (int k = 0; k < 2; ++k) { KS_CUDA(ensure(s->sst_l[k], sl.size() + 1)); KS_CUDA(ensure(s->sst_r[k], sr.size() + 1)); }
+    KS_CUDA(ensure(s->sgi_l, sl.size() + 1)); KS_CUDA(ensure(s->sgi_r, sr.size() + 1));
+    std::vector<int32_t> gl(sl.size()), gr(sr.size());
+    for (size_t k = 0; k < sl.size(); ++k) gl[k] = gidx[sl[k]];
+    for (size_t k = 0; k < sr.size(); ++k) gr[k] = gidx[sr[k]];
     KS_CUDA(ensure(s->kp_local, (size_t)n_own + 1)); KS_CUDA(ensure(s->kp_global, (size_t)n_own + 1));
     KS_CUDA(cudaMemcpyAsync(s->gidx.p, gidx, (size_t)n_own * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
     if (!sl.empty()) KS_CUDA(cudaMemcpyAsync(s->sel_l.p, sl.data(), sl.size() * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
     if (!sr.empty()) KS_CUDA(cudaMemcpyAsync(s->sel_r.p, sr.data(), sr.size() * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
-    KS_CUDA(cudaStreamSynchronize(c->stream));          // sl / sr / gidx are host buffers of this call
+    if (!gl.empty()) KS_CUDA(cudaMemcpyAsync(s->sgi_l.p, gl.data(), gl.size() * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
+    if (!gr.empty()) KS_CUDA(cudaMemcpyAsync(s->sgi_r.p, gr.data(), gr.size() * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
+    KS_CUDA(cudaStreamSynchronize(c->stream));          // sl / sr / gidx / gl / gr are host buffers of this call
     return KPL_OK;
 }
 
@@ -709,6 +842,10 @@ static int set_slab_layout(kpl_shard* s, int64_t n_l, int64_t n_r)
     KS_CUDA(ensure(s->role, (size_t)s->n_loc));
     KS_CUDA(cudaMemsetAsync(s->role.p, KPL_ROLE_HALO, (size_t)s->n_loc, c->stream));
     KS_CUDA(cudaMemsetAsync(s->role.p + n_l, KPL_ROLE_OWNED, (size_t)s->n_own, c->stream));
+    // global indices: the owned part here, the halo parts by the gidx exchange that follows the layout of every rank
+    KS_CUDA(ensure(s->loc_gidx, (size_t)s->n_loc));
+    KS_CUDA(cudaMemcpyAsync(s->loc_gidx.p + n_l, s->gidx.p, (size_t)s->n_own * sizeof(int32_t), cudaMemcpyDeviceToDevice, c->stream));
+    KS_CUDA(ensure(s->st_orig, (size_t)s->n_loc));
     s->has_slab = true;
     return KPL_OK;
 }
@@ -736,6 +873,7 @@ int kpl_shard_set_slab(kpl_shard* s, const float* xyz, int32_t stride, const int
     KS_CUDA(cudaStreamSynchronize(c->stream));
     rc = set_slab_layout(s, s->rank > 0 ? (int64_t)all[2 * (size_t)(s->rank - 1) + 1] : 0,     // the left neighbour's RIGHT strip
                          s->rank < s->world - 1 ? (int64_t)all[2 * (size_t)(s->rank + 1)] : 0); // the right neighbour's LEFT strip
+    if (!rc) rc = exchange(&s, 1, Strip::gidx);
     return rc ? rc : kpl_shard_upload(s, xyz, stride);
 }
 
@@ -771,13 +909,19 @@ int kpl_shard_detect_group(kpl_shard** S, int32_t world, float** scores_owned_ou
     kpl_shard* s = S[0];                       // errors are reported on rank 0's context
     for (int r = 0; r < world; ++r)
         if (!S[r] || !S[r]->in_process || S[r]->world != world || S[r]->rank != r) return sfail(s, KPL_E_INVALID, "kpl_shard_detect_group: not the ranks 0..world-1 of one in-process group");
-    // first call after set_slab: the strip sizes come from the peers
+    // first call after set_slab: the strip sizes come from the peers, then the global indices of the halo points
+    bool laid_out = false;
     for (int r = 0; r < world; ++r) {
         kpl_shard* t = S[r];
         if (t->has_slab) continue;
         if (t->n_own < 1) return sfail(s, KPL_E_INVALID, "kpl_shard_set_slab was not called on every rank");
         const int rc = set_slab_layout(t, r > 0 ? S[r - 1]->send_r : 0, r < world - 1 ? S[r + 1]->send_l : 0);
         if (rc) return on_rank(S, r, rc);
+        laid_out = true;
+    }
+    if (laid_out) {
+        const int rc = exchange(S, world, Strip::gidx);
+        if (rc) return rc;
     }
     return detect_step(S, world, scores_owned_out, kp_global_out, kp_capacity, n_kp_out);
 }

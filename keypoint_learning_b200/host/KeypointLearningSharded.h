@@ -37,6 +37,7 @@ public:
     void setInputCloud(const PointCloudInConstPtr& cloud) { input_ = cloud; }
     void setNonMaxima(bool v) { for (auto& r : ranks_) r->setNonMaxima(v); }
     void setNonMaximaDrawsRemove(bool v) { for (auto& r : ranks_) r->setNonMaximaDrawsRemove(v); }
+    void setNonMaximaDrawsThreshold(float v) { for (auto& r : ranks_) r->setNonMaximaDrawsThreshold(v); }
     void setPredictionThreshold(double th) { for (auto& r : ranks_) r->setPredictionThreshold(th); }
     void setNonMaxRadius(double v) { for (auto& r : ranks_) r->setNonMaxRadius(v); }
     void setNAnnulus(int n) { for (auto& r : ranks_) r->setNAnnulus(n); }

@@ -241,16 +241,79 @@ class HostSlab:
         return self.local, self.role
 
     def score_strips(self, scores_local):
+        """(to the left neighbour, to the right neighbour): the owned values of the strip points of a local array"""
         own = scores_local[self.n_l:self.n_l + len(self.own)]
         return own[self.sel_l], own[self.sel_r]
 
     def merge_scores(self, scores_local, from_left, from_right):
+        """the local array with its halo parts replaced by what the neighbours sent"""
         out = scores_local.copy()
         if self.n_l:
             out[:self.n_l] = from_left
         if self.n_r:
             out[self.n_l + len(self.own):] = from_right
         return out
+
+    # draws-remove NMS: the state rounds of csrc/shard.cu (states 0 not a keypoint, 1 keypoint, 2 undecided, 3 skipped)
+    state_strips = score_strips
+    merge_states = merge_scores
+
+    def gidx_strips(self):
+        """global indices of the strip points (exchanged once per slab)"""
+        return self.gidx[self.sel_l], self.gidx[self.sel_r]
+
+    def set_local_gidx(self, from_left, from_right):
+        parts = [p for p in (from_left, self.gidx, from_right) if p is not None and len(p)]
+        self.local_gidx = np.concatenate(parts).astype(np.int64)
+        return self.local_gidx
+
+    def draws_classify(self, scores_local, nb_off, nb_idx, th, draws_thr):
+        """States of the owned points (halo points 0, their owners decide them) and the close draws the rounds read.
+        nb_off / nb_idx: the r_nms neighbour lists (self included) of every local point, CSR."""
+        p = self.local.astype(np.float32)
+        sc = np.asarray(scores_local, np.float32)
+        n = len(p)
+        src = np.repeat(np.arange(n), np.diff(nb_off))
+        dst = np.asarray(nb_idx, np.int64)
+        owned = np.zeros(n, bool)
+        owned[self.n_l:self.n_l + len(self.own)] = True
+        above = owned & np.isfinite(sc) & ~(sc.astype(np.float64) < th)
+        beaten = np.zeros(n, bool)
+        np.logical_or.at(beaten, src, sc[src] < sc[dst])
+        draw = (sc[src] == sc[dst]) & (src != dst)
+        d = p[src] - p[dst]
+        dist = np.sqrt(d[:, 0] * d[:, 0] + (d[:, 1] * d[:, 1] + d[:, 2] * d[:, 2]))      # Eigen's norm(): a0 + (a1 + a2)
+        close = draw & (dist < np.float32(draws_thr))
+        has_draw = np.zeros(n, bool); np.logical_or.at(has_draw, src, draw)
+        has_close = np.zeros(n, bool); np.logical_or.at(has_close, src, close)
+        state = np.zeros(n, np.uint8)
+        is_max = above & ~beaten
+        state[is_max & ~has_draw] = 1
+        state[is_max & has_draw & has_close] = 2
+        self._close = (src[close], dst[close])
+        return state
+
+    def draws_round(self, state):
+        """One resolution round of the owned undecided candidates on the states held now (halo: the owners' last
+        decisions).  Returns (new states, owned candidates still undecided)."""
+        i, j = self._close
+        lower = self.local_gidx[j] < self.local_gidx[i]
+        i, j = i[lower], j[lower]
+        n = len(state)
+        active = np.zeros(n, bool); np.logical_or.at(active, i, state[j] == 1)
+        pending = np.zeros(n, bool); np.logical_or.at(pending, i, state[j] == 2)
+        undecided = state == 2
+        undecided[:self.n_l] = False
+        undecided[self.n_l + len(self.own):] = False
+        out = state.copy()
+        out[undecided & active] = 3
+        out[undecided & ~active & ~pending] = 1
+        still = undecided & ~active & pending
+        return out, int(still.sum())
+
+    def draws_keypoints(self, state):
+        """ascending global indices of the owned keypoints"""
+        return self.gidx[np.nonzero(state[self.n_l:self.n_l + len(self.own)] == 1)[0]]
 
     def owned_keypoints(self, kp_local):
         """local keypoint indices (over the assembled cloud) -> ascending global indices of those this rank owns"""
