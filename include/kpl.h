@@ -232,15 +232,17 @@ KPL_API int kpl_detect_batch_device(kpl_ctx* ctx, const void* d_xyz4, const void
 /* The reference is a single process (main_test_detector.cpp:123-187 drives one detector); this is the layer a
  * multi-GPU driver binds to.  The cloud is cut along x at CELL-COLUMN boundaries of the canonical grid of the WHOLE
  * cloud; rank r owns the columns [cuts[r], cuts[r+1]).  Per detection every rank
- *   1. sends its boundary strips (halo = reach(radiusFeatures) + normal_support_cells columns, 16 B per point) to
- *      its two neighbours and receives theirs                                              [ncclSend/ncclRecv]
+ *   1. sends its boundary strips (halo = reach(radiusFeatures) + normal_support_cells columns, 16 B per point, 32 B
+ *      with caller normals) to its two neighbours and receives theirs                      [ncclSend/ncclRecv]
  *   2. builds the grid of [left halo | owned | right halo] with the GLOBAL origin (same cell keys, hence the same
- *      accumulation order, hence bit-identical floats as the single-GPU run), estimates normals for all of it and
- *      scores the points it OWNS -- every point of the cloud is scored exactly once
+ *      accumulation order, hence bit-identical floats as the single-GPU run), estimates normals for all of it (unless
+ *      the caller gave them: kpl_shard_set_slab_normals) and scores the points it OWNS -- every point of the cloud is
+ *      scored exactly once
  *   3. exchanges the 4-byte scores of the strips, so that NMS sees the neighbours' scores  [ncclSend/ncclRecv]
  *   4. runs threshold + NMS for its owned points; rank 0 gathers the ascending GLOBAL keypoint index list.
  * A k-NN normal search that the slab edge would clip fails the call on every rank with KPL_E_HALO (widen
- * normal_support_cells).  draws-remove NMS: every rank classifies and decides its OWNED points only; the states of the
+ * normal_support_cells); with caller normals nothing is estimated, so this cannot happen and a plan with
+ * normal_support_cells = 0 (halo = max(reach_feat, reach_nms)) is the one to use.  draws-remove NMS: every rank classifies and decides its OWNED points only; the states of the
  * strip points (1 B per point) go to the neighbours after the classification and after every resolution round, and all
  * ranks stop on the same global count of undecided candidates -- one host synchronisation per round
  * (kpl_stats.nms_rounds).  The result is the single-GPU one. */
@@ -263,7 +265,7 @@ typedef struct kpl_shard kpl_shard;
 typedef struct kpl_shard_info {
     int64_t n_owned, n_left, n_right;     /* points owned / received from the left / right neighbour              */
     int64_t send_left, send_right;        /* points sent to the neighbours per detection                          */
-    int64_t halo_bytes;                   /* bytes this rank sends per detection (positions + scores)             */
+    int64_t halo_bytes;                   /* bytes this rank sends per detection (positions + scores, + normals when given) */
     int32_t local_dims[3], local_offset[3];
     int32_t rank, world;
     float exchange_ms;                    /* device time of the two exchanges of the last detection               */
@@ -288,13 +290,24 @@ KPL_API int kpl_nccl_unique_id(void* id128_out);
 KPL_API int kpl_shard_create(kpl_ctx* ctx, const kpl_slab_plan* plan, int32_t rank, const void* nccl_id128, kpl_shard** out);
 KPL_API void kpl_shard_destroy(kpl_shard* s);
 /* Replace the plan (same world size) without rebuilding the communicator -- e.g. after KPL_E_HALO, with a plan made
- * for a larger normal_support_cells; kpl_shard_set_slab must follow. */
+ * for a larger normal_support_cells; kpl_shard_set_slab(_normals) must follow (the normals are cleared). */
 KPL_API int kpl_shard_set_plan(kpl_shard* s, const kpl_slab_plan* plan);
 /* The points this rank owns (host, ascending global index; kpl_slab_partition) and their global indices.  Uploads
  * them and exchanges the strip sizes: once per resident slab, not per detection. */
 KPL_API int kpl_shard_set_slab(kpl_shard* s, const float* xyz_owned, int32_t xyz_stride, const int32_t* gidx_owned, int64_t n_owned);
+/* kpl_shard_set_slab plus the caller's normals of the owned points (same order as xyz_owned; 3 floats at normals_stride
+ * bytes, 32 = pcl::Normal).  A non-finite normal is not an error: that point gets no score, as in kpl_detect.
+ * As in kpl_detect, normals_mode, k_normals, flip_normals and viewpoint are then ignored (so is the radius-mode halo
+ * requirement).  The normal strips of the halo travel in the same exchange as the positions.  Every rank must call the
+ * same variant (set_slab or set_slab_normals); otherwise the call fails with KPL_E_INVALID on every rank before any
+ * strip moves (NCCL: here, in the strip-size all-gather; in-process group: in kpl_shard_detect_group).  A later plain
+ * kpl_shard_set_slab returns the rank to estimated normals. */
+KPL_API int kpl_shard_set_slab_normals(kpl_shard* s, const float* xyz_owned, int32_t xyz_stride, const float* normals_owned,
+                                       int32_t normals_stride, const int32_t* gidx_owned, int64_t n_owned);
 /* New coordinates for the same partition (a detection loop that streams its slab from the host every step). */
 KPL_API int kpl_shard_upload(kpl_shard* s, const float* xyz_owned, int32_t xyz_stride);
+/* New normals for the same partition (pairs with kpl_shard_upload); KPL_E_INVALID on a slab set without normals. */
+KPL_API int kpl_shard_upload_normals(kpl_shard* s, const float* normals_owned, int32_t normals_stride);
 /* One detection (all ranks call it).  scores_owned_out: NULL or n_owned floats (host).  kp_global_out (rank 0; NULL
  * elsewhere): ascending global keypoint indices, capacity kp_capacity; *n_kp_out = global keypoint count on every rank. */
 KPL_API int kpl_shard_detect(kpl_shard* s, float* scores_owned_out, int32_t* kp_global_out, int64_t kp_capacity, int64_t* n_kp_out);

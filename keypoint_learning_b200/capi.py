@@ -28,7 +28,7 @@ EXPORTS = ["kpl_create", "kpl_destroy", "kpl_last_error", "kpl_version", "kpl_se
            "kpl_fetch_u8", "kpl_device_count", "kpl_normals_organized", "kpl_detect_batch", "kpl_detect_batch_device",
            "kpl_slab_plan_make", "kpl_slab_partition", "kpl_nccl_unique_id", "kpl_shard_create", "kpl_shard_destroy", "kpl_shard_set_plan",
            "kpl_shard_set_slab", "kpl_shard_upload", "kpl_shard_detect", "kpl_shard_detect_group", "kpl_shard_get_info",
-           "kpl_shard_device_scores"]
+           "kpl_shard_device_scores", "kpl_shard_set_slab_normals", "kpl_shard_upload_normals"]
 KPL_MAX_RANKS = 64
 
 
@@ -120,6 +120,8 @@ def load_library():
     L.kpl_shard_set_plan.argtypes = [vp, C.POINTER(KplSlabPlan)]
     L.kpl_shard_set_slab.argtypes = [vp, f32p, C.c_int32, i32p, C.c_int64]
     L.kpl_shard_upload.argtypes = [vp, f32p, C.c_int32]
+    L.kpl_shard_set_slab_normals.argtypes = [vp, f32p, C.c_int32, f32p, C.c_int32, i32p, C.c_int64]
+    L.kpl_shard_upload_normals.argtypes = [vp, f32p, C.c_int32]
     L.kpl_shard_detect.argtypes = [vp, f32p, i32p, C.c_int64, i64p]
     L.kpl_shard_detect_group.argtypes = [C.POINTER(vp), C.c_int32, C.POINTER(f32p), i32p, C.c_int64, i64p]
     L.kpl_shard_get_info.argtypes = [vp, C.POINTER(KplShardInfo)]

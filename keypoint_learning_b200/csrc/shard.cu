@@ -95,12 +95,15 @@ struct kpl_shard {
     int64_t send_l = 0, send_r = 0;                      // strip sizes sent to the left / right neighbour
     ForcedGrid grid{};                                   // local grid: columns [offset[0], offset[0] + dims[0]) of the global grid
     bool has_slab = false;
+    bool has_nrm = false;                                // the caller's normals (kpl_shard_set_slab_normals) instead of estimated ones
     DevBuf<float4> loc_xyz;                              // [left halo | owned | right halo]
+    DevBuf<float4> loc_nrm;                              // the caller's normals, same layout (has_nrm)
     DevBuf<uint8_t> role;
     DevBuf<int32_t> gidx;                                // global index of every owned point
     DevBuf<int32_t> loc_gidx;                            // global index of every local point, [left halo | owned | right halo]
     DevBuf<int32_t> sel_l, sel_r;                        // owned-local indices of the strips
     DevBuf<float4> sbuf_l, sbuf_r;                       // packed position strips
+    DevBuf<float4> snb_l, snb_r;                         // packed normal strips (has_nrm)
     DevBuf<float> ssc_l, ssc_r;                          // packed score strips
     DevBuf<int32_t> sgi_l, sgi_r;                        // global indices of the strip points (sent once per resident slab)
     DevBuf<uint8_t> st_orig;                             // draws-remove NMS states in local original order (halo parts received)
@@ -158,6 +161,18 @@ __global__ void __launch_bounds__(256) pack_strip_kernel(const float4* __restric
 {
     const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (k < m) out[k] = owned[sel[k]];
+}
+// both records of a strip point when the caller gave the normals: one launch per side, as without them
+__global__ void __launch_bounds__(256) pack_strip_normals_kernel(const float4* __restrict__ owned, const float4* __restrict__ owned_nrm,
+                                                                 const int32_t* __restrict__ sel, int64_t m, float4* __restrict__ out,
+                                                                 float4* __restrict__ out_nrm)
+{
+    const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (k < m) {
+        const int32_t i = sel[k];
+        out[k] = owned[i];
+        out_nrm[k] = owned_nrm[i];
+    }
 }
 __global__ void __launch_bounds__(256) pack_scores_kernel(const float* __restrict__ owned_scores, const int32_t* __restrict__ sel, int64_t m,
                                                           float* __restrict__ out)
@@ -225,8 +240,8 @@ int each_rank(kpl_shard** S, int n, F f)
     return KPL_OK;
 }
 
-// what an exchange moves: positions and scores every detection, draws-remove states every resolution round, global
-// indices once per resident slab
+// what an exchange moves: positions (with the caller's normals, when given) and scores every detection, draws-remove
+// states every resolution round, global indices once per resident slab
 enum class Strip { positions, scores, states, gidx };
 
 // the buffers of one exchange: the packed strips a rank sends, the ends of its local array that receive
@@ -236,14 +251,19 @@ struct Strips {
     size_t item;
 };
 
-Strips strips(kpl_shard* t, Strip kind)
+// the strip sets one exchange of `kind` moves (out[0..return value)): the normal strips travel with the positions
+int strips(kpl_shard* t, Strip kind, Strips* out)
 {
     const int64_t hi = t->n_l + t->n_own;
     switch (kind) {
-    case Strip::scores: return {t->ssc_l.p, t->ssc_r.p, t->ctx->score.p, t->ctx->score.p + hi, sizeof(float)};
-    case Strip::states: return {t->sst_l[t->sst].p, t->sst_r[t->sst].p, t->st_orig.p, t->st_orig.p + hi, sizeof(uint8_t)};
-    case Strip::gidx: return {t->sgi_l.p, t->sgi_r.p, t->loc_gidx.p, t->loc_gidx.p + hi, sizeof(int32_t)};
-    default: return {t->sbuf_l.p, t->sbuf_r.p, t->loc_xyz.p, t->loc_xyz.p + hi, sizeof(float4)};
+    case Strip::scores: out[0] = {t->ssc_l.p, t->ssc_r.p, t->ctx->score.p, t->ctx->score.p + hi, sizeof(float)}; return 1;
+    case Strip::states: out[0] = {t->sst_l[t->sst].p, t->sst_r[t->sst].p, t->st_orig.p, t->st_orig.p + hi, sizeof(uint8_t)}; return 1;
+    case Strip::gidx: out[0] = {t->sgi_l.p, t->sgi_r.p, t->loc_gidx.p, t->loc_gidx.p + hi, sizeof(int32_t)}; return 1;
+    default:
+        out[0] = {t->sbuf_l.p, t->sbuf_r.p, t->loc_xyz.p, t->loc_xyz.p + hi, sizeof(float4)};
+        if (!t->has_nrm) return 1;
+        out[1] = {t->snb_l.p, t->snb_r.p, t->loc_nrm.p, t->loc_nrm.p + hi, sizeof(float4)};
+        return 2;
     }
 }
 
@@ -253,17 +273,20 @@ Strips strips(kpl_shard* t, Strip kind)
 int exchange(kpl_shard** S, int n, Strip kind)
 {
     kpl_shard* s = S[0];
+    Strips b[2], p[2];
     if (!s->in_process) {
-        const Strips b = strips(s, kind);
+        const int nb = strips(s, kind, b);
         cudaStream_t st = s->ctx->stream;
         KS_NCCL(s->nccl->GroupStart());
-        if (s->rank > 0) {
-            if (s->send_l) KS_NCCL(s->nccl->Send(b.send_l, (size_t)s->send_l * b.item, ncclChar, s->rank - 1, s->comm, st));
-            if (s->n_l) KS_NCCL(s->nccl->Recv(b.recv_l, (size_t)s->n_l * b.item, ncclChar, s->rank - 1, s->comm, st));
-        }
-        if (s->rank < s->world - 1) {
-            if (s->send_r) KS_NCCL(s->nccl->Send(b.send_r, (size_t)s->send_r * b.item, ncclChar, s->rank + 1, s->comm, st));
-            if (s->n_r) KS_NCCL(s->nccl->Recv(b.recv_r, (size_t)s->n_r * b.item, ncclChar, s->rank + 1, s->comm, st));
+        for (int k = 0; k < nb; ++k) {
+            if (s->rank > 0) {
+                if (s->send_l) KS_NCCL(s->nccl->Send(b[k].send_l, (size_t)s->send_l * b[k].item, ncclChar, s->rank - 1, s->comm, st));
+                if (s->n_l) KS_NCCL(s->nccl->Recv(b[k].recv_l, (size_t)s->n_l * b[k].item, ncclChar, s->rank - 1, s->comm, st));
+            }
+            if (s->rank < s->world - 1) {
+                if (s->send_r) KS_NCCL(s->nccl->Send(b[k].send_r, (size_t)s->send_r * b[k].item, ncclChar, s->rank + 1, s->comm, st));
+                if (s->n_r) KS_NCCL(s->nccl->Recv(b[k].recv_r, (size_t)s->n_r * b[k].item, ncclChar, s->rank + 1, s->comm, st));
+            }
         }
         KS_NCCL(s->nccl->GroupEnd());
         return KPL_OK;
@@ -276,12 +299,18 @@ int exchange(kpl_shard** S, int n, Strip kind)
     }
     for (int r = 0; r < n; ++r) {
         kpl_shard* t = S[r];
-        const Strips b = strips(t, kind);
+        const int nb = strips(t, kind, b);
         cudaError_t e = cudaSetDevice(t->ctx->device);
-        if (!e && r > 0 && t->n_l)
-            e = cudaMemcpyAsync(b.recv_l, strips(S[r - 1], kind).send_r, (size_t)t->n_l * b.item, cudaMemcpyDefault, t->ctx->stream);
-        if (!e && r < n - 1 && t->n_r)
-            e = cudaMemcpyAsync(b.recv_r, strips(S[r + 1], kind).send_l, (size_t)t->n_r * b.item, cudaMemcpyDefault, t->ctx->stream);
+        if (!e && r > 0 && t->n_l) {
+            strips(S[r - 1], kind, p);
+            for (int k = 0; !e && k < nb; ++k)
+                e = cudaMemcpyAsync(b[k].recv_l, p[k].send_r, (size_t)t->n_l * b[k].item, cudaMemcpyDefault, t->ctx->stream);
+        }
+        if (!e && r < n - 1 && t->n_r) {
+            strips(S[r + 1], kind, p);
+            for (int k = 0; !e && k < nb; ++k)
+                e = cudaMemcpyAsync(b[k].recv_r, p[k].send_l, (size_t)t->n_r * b[k].item, cudaMemcpyDefault, t->ctx->stream);
+        }
         if (e) return sfail(s, KPL_E_CUDA, std::string("peer copy: ") + cudaGetErrorString(e));
     }
     return KPL_OK;
@@ -316,7 +345,7 @@ int gather_keypoints(kpl_shard** S, int n, const std::vector<int64_t>& counts)
 }
 
 // ---- the phases of one detection (everything is enqueued on the context stream) --------------------------------
-// the per-call reset of the rank's context, then its position strips
+// the per-call reset of the rank's context, then its position strips (and normal strips)
 int phase_pack(kpl_shard* s)
 {
     kpl_ctx* c = s->ctx;
@@ -324,12 +353,16 @@ int phase_pack(kpl_shard* s)
     KS_CUDA(cudaSetDevice(c->device));
     KS_CUDA(cudaEventRecord(s->ev[0], c->stream));
     const float4* owned = s->loc_xyz.p + s->n_l;
-    if (s->send_l) {
-        pack_strip_kernel<<<(unsigned)((s->send_l + 255) / 256), 256, 0, c->stream>>>(owned, s->sel_l.p, s->send_l, s->sbuf_l.p);
-        KS_CUDA(cudaGetLastError());
-    }
-    if (s->send_r) {
-        pack_strip_kernel<<<(unsigned)((s->send_r + 255) / 256), 256, 0, c->stream>>>(owned, s->sel_r.p, s->send_r, s->sbuf_r.p);
+    const float4* owned_nrm = s->has_nrm ? s->loc_nrm.p + s->n_l : nullptr;
+    const int64_t m[2] = {s->send_l, s->send_r};
+    const int32_t* sel[2] = {s->sel_l.p, s->sel_r.p};
+    float4* out[2] = {s->sbuf_l.p, s->sbuf_r.p};
+    float4* out_nrm[2] = {s->snb_l.p, s->snb_r.p};
+    for (int k = 0; k < 2; ++k) {
+        if (!m[k]) continue;
+        const unsigned blocks = (unsigned)((m[k] + 255) / 256);
+        if (s->has_nrm) pack_strip_normals_kernel<<<blocks, 256, 0, c->stream>>>(owned, owned_nrm, sel[k], m[k], out[k], out_nrm[k]);
+        else pack_strip_kernel<<<blocks, 256, 0, c->stream>>>(owned, sel[k], m[k], out[k]);
         KS_CUDA(cudaGetLastError());
     }
     return KPL_OK;
@@ -343,8 +376,8 @@ int phase_score(kpl_shard* s)
     int rc = detect_begin(c);
     if (rc) return rc;
     c->launches += 2;
-    if ((rc = prepare_grid(c, s->loc_xyz.p, nullptr, s->role.p, s->n_loc, &s->grid))) return rc;
-    if ((rc = detect_score_phase(c, false, true, s->n_loc))) return rc;
+    if ((rc = prepare_grid(c, s->loc_xyz.p, s->has_nrm ? s->loc_nrm.p : nullptr, s->role.p, s->n_loc, &s->grid))) return rc;
+    if ((rc = detect_score_phase(c, s->has_nrm, true, s->n_loc))) return rc;
     KS_CUDA(cudaEventRecord(s->ev[2], c->stream));
     const float* owned_scores = c->score.p + s->n_l;
     if (s->send_l) pack_scores_kernel<<<(unsigned)((s->send_l + 255) / 256), 256, 0, c->stream>>>(owned_scores, s->sel_l.p, s->send_l, s->ssc_l.p);
@@ -496,9 +529,9 @@ int check_ready(kpl_shard* s)
 {
     if (!s || !s->ctx) return KPL_E_INVALID;
     if (!s->has_slab) return sfail(s, KPL_E_INVALID, "kpl_shard_set_slab was not called");
-    // radius-mode normals (hpp:130-137) need every neighbour within r_feat of a point whose normal matters: the halo must
-    // then be two search reaches wide, which no device check can verify after the fact
-    if (s->world > 1 && s->ctx->params.normals_mode == KPL_NORMALS_RADIUS && s->plan.normal_support_cells < s->plan.reach_feat)
+    // estimated radius-mode normals (hpp:130-137) need every neighbour within r_feat of a point whose normal matters: the
+    // halo must then be two search reaches wide, which no device check can verify after the fact
+    if (s->world > 1 && !s->has_nrm && s->ctx->params.normals_mode == KPL_NORMALS_RADIUS && s->plan.normal_support_cells < s->plan.reach_feat)
         return sfail(s, KPL_E_HALO, "radius-mode normals need normal_support_cells >= reach_feat (the whole r_feat ball of every halo point that matters)");
     return detect_check(s->ctx, s->n_loc, false);
 }
@@ -734,7 +767,7 @@ int kpl_shard_create(kpl_ctx* ctx, const kpl_slab_plan* plan, int32_t rank, cons
     bool ok = cudaSetDevice(ctx->device) == cudaSuccess;
     for (int i = 0; ok && i < 6; ++i) ok = cudaEventCreate(&s->ev[i]) == cudaSuccess;
     ok = ok && ensure(s->rec, 1) == cudaSuccess && ensure(s->rec_all, (size_t)s->world) == cudaSuccess &&
-         ensure(s->sizes, 2) == cudaSuccess && ensure(s->sizes_all, 2 * (size_t)s->world) == cudaSuccess &&
+         ensure(s->sizes, 3) == cudaSuccess && ensure(s->sizes_all, 3 * (size_t)s->world) == cudaSuccess &&
          ensure(s->und_all, (size_t)s->world) == cudaSuccess;
     if (!ok) { ctx->err = "kpl_shard_create: CUDA resources"; kpl_shard_destroy(s); return KPL_E_CUDA; }
     if (!s->in_process) {
@@ -760,7 +793,7 @@ int kpl_shard_set_plan(kpl_shard* s, const kpl_slab_plan* plan)
     if (!s || !plan) return KPL_E_INVALID;
     if (plan->world != s->world) return sfail(s, KPL_E_INVALID, "kpl_shard_set_plan: the communicator was created for another world size");
     s->plan = *plan;
-    s->has_slab = false;
+    s->has_slab = s->has_nrm = false;
     s->n_own = s->n_l = s->n_r = s->n_loc = s->send_l = s->send_r = 0;
     return KPL_OK;
 }
@@ -771,6 +804,7 @@ void kpl_shard_destroy(kpl_shard* s)
     if (s->ctx) { cudaSetDevice(s->ctx->device); cudaStreamSynchronize(s->ctx->stream); }
     if (s->comm && s->nccl) s->nccl->CommDestroy(s->comm);
     srelease(s->loc_xyz); srelease(s->role); srelease(s->gidx); srelease(s->loc_gidx); srelease(s->sel_l); srelease(s->sel_r);
+    srelease(s->loc_nrm); srelease(s->snb_l); srelease(s->snb_r);
     srelease(s->sbuf_l); srelease(s->sbuf_r); srelease(s->ssc_l); srelease(s->ssc_r); srelease(s->sgi_l); srelease(s->sgi_r);
     srelease(s->st_orig); srelease(s->und_all);
     for (int k = 0; k < 2; ++k) { srelease(s->sst_l[k]); srelease(s->sst_r[k]); }
@@ -808,6 +842,7 @@ static int set_slab_local(kpl_shard* s, const float* xyz, int32_t stride, const 
     KS_CUDA(ensure(s->gidx, (size_t)n_own));
     KS_CUDA(ensure(s->sel_l, sl.size() + 1)); KS_CUDA(ensure(s->sel_r, sr.size() + 1));
     KS_CUDA(ensure(s->sbuf_l, sl.size() + 1)); KS_CUDA(ensure(s->sbuf_r, sr.size() + 1));
+    if (s->has_nrm) { KS_CUDA(ensure(s->snb_l, sl.size() + 1)); KS_CUDA(ensure(s->snb_r, sr.size() + 1)); }
     KS_CUDA(ensure(s->ssc_l, sl.size() + 1)); KS_CUDA(ensure(s->ssc_r, sr.size() + 1));
     for (int k = 0; k < 2; ++k) { KS_CUDA(ensure(s->sst_l[k], sl.size() + 1)); KS_CUDA(ensure(s->sst_r[k], sr.size() + 1)); }
     KS_CUDA(ensure(s->sgi_l, sl.size() + 1)); KS_CUDA(ensure(s->sgi_r, sr.size() + 1));
@@ -824,21 +859,28 @@ static int set_slab_local(kpl_shard* s, const float* xyz, int32_t stride, const 
     return KPL_OK;
 }
 
-// [left halo | owned | right halo] once the strip sizes n_l / n_r are known: the local cloud buffer and the roles.
-// An in-process rank's owned points, which kpl_shard_set_slab staged at the start of loc_xyz, move to their place.
+// An in-process rank's owned records, which kpl_shard_set_slab staged at the start of `buf`, move to their place.
+static cudaError_t place_owned(kpl_shard* s, DevBuf<float4>& buf)
+{
+    DevBuf<float4> staged;
+    if (s->in_process) std::swap(staged, buf);
+    cudaError_t e = ensure(buf, (size_t)s->n_loc);
+    if (!e && staged.p) e = cudaMemcpyAsync(buf.p + s->n_l, staged.p, (size_t)s->n_own * sizeof(float4), cudaMemcpyDeviceToDevice, s->ctx->stream);
+    if (!e && staged.p) e = cudaStreamSynchronize(s->ctx->stream);
+    srelease(staged);
+    return e;
+}
+
+// [left halo | owned | right halo] once the strip sizes n_l / n_r are known: the local cloud buffer (and the normal
+// buffer) and the roles.
 static int set_slab_layout(kpl_shard* s, int64_t n_l, int64_t n_r)
 {
     kpl_ctx* c = s->ctx;
     s->n_l = n_l; s->n_r = n_r; s->n_loc = n_l + s->n_own + n_r;
     if (s->n_loc > 2147483000ll) return sfail(s, KPL_E_INVALID, "slab too large");
     KS_CUDA(cudaSetDevice(c->device));
-    DevBuf<float4> staged;
-    if (s->in_process) std::swap(staged, s->loc_xyz);
-    cudaError_t e = ensure(s->loc_xyz, (size_t)s->n_loc);
-    if (!e && staged.p) e = cudaMemcpyAsync(s->loc_xyz.p + n_l, staged.p, (size_t)s->n_own * sizeof(float4), cudaMemcpyDeviceToDevice, c->stream);
-    if (!e && staged.p) e = cudaStreamSynchronize(c->stream);
-    srelease(staged);
-    KS_CUDA(e);
+    KS_CUDA(place_owned(s, s->loc_xyz));
+    if (s->has_nrm) KS_CUDA(place_owned(s, s->loc_nrm));
     KS_CUDA(ensure(s->role, (size_t)s->n_loc));
     KS_CUDA(cudaMemsetAsync(s->role.p, KPL_ROLE_HALO, (size_t)s->n_loc, c->stream));
     KS_CUDA(cudaMemsetAsync(s->role.p + n_l, KPL_ROLE_OWNED, (size_t)s->n_own, c->stream));
@@ -850,31 +892,68 @@ static int set_slab_layout(kpl_shard* s, int64_t n_l, int64_t n_r)
     return KPL_OK;
 }
 
-int kpl_shard_set_slab(kpl_shard* s, const float* xyz, int32_t stride, const int32_t* gidx, int64_t n_own)
+static bool bad_stride(int32_t stride) { return stride < 12 || (stride & 3); }
+
+// host (possibly strided) -> device float4 records, as the single-GPU upload stages them (capi.cu: upload_vec3)
+static cudaError_t upload_records(float4* dst, const float* src, int32_t stride, int64_t n, cudaStream_t st)
 {
-    if (!s) return KPL_E_INVALID;
+    if (stride == 16) return cudaMemcpyAsync(dst, src, (size_t)n * 16, cudaMemcpyHostToDevice, st);
+    return cudaMemcpy2DAsync(dst, 16, src, (size_t)stride, stride >= 16 ? 16 : 12, (size_t)n, cudaMemcpyHostToDevice, st);
+}
+
+// kpl_shard_set_slab with or without the caller's normals (nrm == nullptr: estimated on the device)
+static int set_slab(kpl_shard* s, const float* xyz, int32_t stride, const float* nrm, int32_t nrm_stride, const int32_t* gidx, int64_t n_own)
+{
     s->has_slab = false;
+    s->has_nrm = nrm != nullptr;
     int rc = set_slab_local(s, xyz, stride, gidx, n_own);
     if (rc) return rc;
+    kpl_ctx* c = s->ctx;
     if (s->in_process) {
         // the group driver takes n_l / n_r from the peers; the layout follows there (kpl_shard_detect_group)
         s->n_l = s->n_r = -1;
         KS_CUDA(ensure(s->loc_xyz, (size_t)n_own));
         if (stride == 16) KS_CUDA(cudaMemcpy(s->loc_xyz.p, xyz, (size_t)n_own * 16, cudaMemcpyHostToDevice));
         else KS_CUDA(cudaMemcpy2D(s->loc_xyz.p, 16, xyz, (size_t)stride, 12, (size_t)n_own, cudaMemcpyHostToDevice));
+        if (s->has_nrm) {
+            KS_CUDA(ensure(s->loc_nrm, (size_t)n_own));
+            KS_CUDA(upload_records(s->loc_nrm.p, nrm, nrm_stride, n_own, c->stream));
+            KS_CUDA(cudaStreamSynchronize(c->stream));
+        }
         return KPL_OK;
     }
-    kpl_ctx* c = s->ctx;
-    unsigned long long mine[2] = {(unsigned long long)s->send_l, (unsigned long long)s->send_r};
+    // the strip sizes and whether this rank's normals travel with its positions: every rank must choose alike, or the
+    // strip exchanges would not match
+    unsigned long long mine[3] = {(unsigned long long)s->send_l, (unsigned long long)s->send_r, (unsigned long long)s->has_nrm};
     KS_CUDA(cudaMemcpyAsync(s->sizes.p, mine, sizeof mine, cudaMemcpyHostToDevice, c->stream));
-    KS_NCCL(s->nccl->AllGather(s->sizes.p, s->sizes_all.p, 2, ncclUint64, s->comm, c->stream));
-    std::vector<unsigned long long> all(2 * (size_t)s->world);
+    KS_NCCL(s->nccl->AllGather(s->sizes.p, s->sizes_all.p, 3, ncclUint64, s->comm, c->stream));
+    std::vector<unsigned long long> all(3 * (size_t)s->world);
     KS_CUDA(cudaMemcpyAsync(all.data(), s->sizes_all.p, all.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
     KS_CUDA(cudaStreamSynchronize(c->stream));
-    rc = set_slab_layout(s, s->rank > 0 ? (int64_t)all[2 * (size_t)(s->rank - 1) + 1] : 0,     // the left neighbour's RIGHT strip
-                         s->rank < s->world - 1 ? (int64_t)all[2 * (size_t)(s->rank + 1)] : 0); // the right neighbour's LEFT strip
+    for (int r = 0; r < s->world; ++r)
+        if (all[3 * (size_t)r + 2] != mine[2])
+            return sfail(s, KPL_E_INVALID, "every rank must call kpl_shard_set_slab_normals, or every rank kpl_shard_set_slab");
+    rc = set_slab_layout(s, s->rank > 0 ? (int64_t)all[3 * (size_t)(s->rank - 1) + 1] : 0,     // the left neighbour's RIGHT strip
+                         s->rank < s->world - 1 ? (int64_t)all[3 * (size_t)(s->rank + 1)] : 0); // the right neighbour's LEFT strip
     if (!rc) rc = exchange(&s, 1, Strip::gidx);
-    return rc ? rc : kpl_shard_upload(s, xyz, stride);
+    if (!rc) rc = kpl_shard_upload(s, xyz, stride);
+    return rc || !s->has_nrm ? rc : kpl_shard_upload_normals(s, nrm, nrm_stride);
+}
+
+int kpl_shard_set_slab(kpl_shard* s, const float* xyz, int32_t stride, const int32_t* gidx, int64_t n_own)
+{
+    if (!s) return KPL_E_INVALID;
+    return set_slab(s, xyz, stride, nullptr, 0, gidx, n_own);
+}
+
+int kpl_shard_set_slab_normals(kpl_shard* s, const float* xyz, int32_t stride, const float* normals, int32_t normals_stride,
+                               const int32_t* gidx, int64_t n_own)
+{
+    if (!s) return KPL_E_INVALID;
+    s->has_slab = s->has_nrm = false;
+    if (!normals) return sfail(s, KPL_E_INVALID, "kpl_shard_set_slab_normals: normals_owned is NULL");
+    if (bad_stride(normals_stride)) return sfail(s, KPL_E_INVALID, "normals_stride must be a multiple of 4 and >= 12 bytes");
+    return set_slab(s, xyz, stride, normals, normals_stride, gidx, n_own);
 }
 
 int kpl_shard_upload(kpl_shard* s, const float* xyz, int32_t stride)
@@ -887,6 +966,17 @@ int kpl_shard_upload(kpl_shard* s, const float* xyz, int32_t stride)
     float4* dst = s->loc_xyz.p + s->n_l;
     if (stride == 16) KS_CUDA(cudaMemcpyAsync(dst, xyz, (size_t)s->n_own * 16, cudaMemcpyHostToDevice, c->stream));
     else KS_CUDA(cudaMemcpy2DAsync(dst, 16, xyz, (size_t)stride, 12, (size_t)s->n_own, cudaMemcpyHostToDevice, c->stream));
+    return KPL_OK;
+}
+
+int kpl_shard_upload_normals(kpl_shard* s, const float* normals, int32_t normals_stride)
+{
+    if (!s || !normals) return KPL_E_INVALID;
+    if (!s->has_nrm) return sfail(s, KPL_E_INVALID, "kpl_shard_upload_normals: the slab was not set with normals (kpl_shard_set_slab_normals)");
+    if (!s->has_slab) return sfail(s, KPL_E_INVALID, "kpl_shard_set_slab_normals was not called");
+    if (bad_stride(normals_stride)) return sfail(s, KPL_E_INVALID, "normals_stride must be a multiple of 4 and >= 12 bytes");
+    KS_CUDA(cudaSetDevice(s->ctx->device));
+    KS_CUDA(upload_records(s->loc_nrm.p + s->n_l, normals, normals_stride, s->n_own, s->ctx->stream));
     return KPL_OK;
 }
 
@@ -909,6 +999,9 @@ int kpl_shard_detect_group(kpl_shard** S, int32_t world, float** scores_owned_ou
     kpl_shard* s = S[0];                       // errors are reported on rank 0's context
     for (int r = 0; r < world; ++r)
         if (!S[r] || !S[r]->in_process || S[r]->world != world || S[r]->rank != r) return sfail(s, KPL_E_INVALID, "kpl_shard_detect_group: not the ranks 0..world-1 of one in-process group");
+    for (int r = 1; r < world; ++r)           // the strip exchanges only match when every rank's normals travel, or none
+        if (S[r]->has_nrm != s->has_nrm)
+            return sfail(s, KPL_E_INVALID, "every rank must call kpl_shard_set_slab_normals, or every rank kpl_shard_set_slab");
     // first call after set_slab: the strip sizes come from the peers, then the global indices of the halo points
     bool laid_out = false;
     for (int r = 0; r < world; ++r) {
@@ -932,7 +1025,7 @@ int kpl_shard_get_info(const kpl_shard* s, kpl_shard_info* out)
     memset(out, 0, sizeof *out);
     out->n_owned = s->n_own; out->n_left = std::max<int64_t>(s->n_l, 0); out->n_right = std::max<int64_t>(s->n_r, 0);
     out->send_left = s->send_l; out->send_right = s->send_r;
-    out->halo_bytes = (s->send_l + s->send_r) * (int64_t)(sizeof(float4) + sizeof(float));
+    out->halo_bytes = (s->send_l + s->send_r) * (int64_t)(sizeof(float4) + sizeof(float) + (s->has_nrm ? sizeof(float4) : 0));
     out->local_dims[0] = s->grid.dims[0]; out->local_dims[1] = s->plan.dims[1]; out->local_dims[2] = s->plan.dims[2];
     out->local_offset[0] = s->grid.offset[0];
     out->rank = s->rank; out->world = s->world;

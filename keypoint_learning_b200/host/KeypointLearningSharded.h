@@ -2,8 +2,9 @@
 // the reference driver's `detector->compute(*keypoint)` (src/main_test_detector.cpp:123-187).  The cloud is cut into
 // x slabs (kpl_slab_plan_make), one host thread per GPU drives one rank of the kpl_shard_* entry points of
 // include/kpl.h (NCCL halo + score exchange inside libkpl_b200.so), and the result is the keypoint cloud the
-// single-GPU detector returns, bit for bit.  Normals are estimated on the devices (k-NN, the TestDetector setting
-// :162-169, viewpoint = sensor origin), because a slab needs the normals of its halo as well.
+// single-GPU detector returns, bit for bit.  Without setNormals(), normals are estimated on the devices (k-NN, the
+// TestDetector setting :162-169, viewpoint = sensor origin), each slab for its halo as well; with setNormals() the
+// caller's normals are partitioned like the points and travel with the halo strips (kpl_shard_set_slab_normals).
 //
 // Same setter names as the single-GPU class; every setter is forwarded to all ranks.
 #pragma once
@@ -23,6 +24,8 @@ class ShardedKeypointLearningDetector {
 public:
     typedef KeypointLearningDetector<PointInT, PointOutT> Single;
     typedef typename Single::PointCloudInConstPtr PointCloudInConstPtr;
+    typedef typename Single::PointCloudNConstPtr PointCloudNConstPtr;
+    typedef pcl::Normal NormalT;                              // Single's (the default NormalT of KeypointLearningDetector)
     typedef pcl::PointCloud<PointOutT> PointCloudOut;
 
     // More ranks than devices (e.g. a test on one GPU): the ranks share the devices round-robin and form an in-process
@@ -34,7 +37,13 @@ public:
         for (int g = 0; g < gpus; ++g) ranks_.emplace_back(new Single(0.5f, true, true, 0.0f, 5, 10, g % devices));
     }
     int gpus() const { return gpus_; }
-    void setInputCloud(const PointCloudInConstPtr& cloud) { input_ = cloud; }
+    // as KeypointLearningDetector (impl/KeypointLearning.hpp:49-57): another cloud drops the normals
+    void setInputCloud(const PointCloudInConstPtr& cloud)
+    {
+        if (normals_ && input_ && cloud != input_) normals_.reset();
+        input_ = cloud;
+    }
+    void setNormals(const PointCloudNConstPtr& normals) { normals_ = normals; }
     void setNonMaxima(bool v) { for (auto& r : ranks_) r->setNonMaxima(v); }
     void setNonMaximaDrawsRemove(bool v) { for (auto& r : ranks_) r->setNonMaximaDrawsRemove(v); }
     void setNonMaximaDrawsThreshold(float v) { for (auto& r : ranks_) r->setNonMaximaDrawsThreshold(v); }
@@ -65,6 +74,10 @@ public:
         keypoints_indices_.reset(new pcl::PointIndices);
         if (!input_ || input_->empty()) { std::fprintf(stderr, "[ShardedKeypointLearningDetector::compute] no input cloud\n"); return false; }
         const int64_t n = (int64_t)input_->size();
+        if (normals_ && (int64_t)normals_->size() != n) {       // pcl::KeypointLearningDetector::initCompute (hpp:149-153)
+            std::fprintf(stderr, "[ShardedKeypointLearningDetector::compute] normals given, but the number of normals does not match the number of input points!\n");
+            return false;
+        }
         const float* xyz = reinterpret_cast<const float*>(input_->points.data());
         std::vector<kpl_params> P((size_t)gpus_);
         for (int g = 0; g < gpus_; ++g) {
@@ -82,7 +95,8 @@ public:
         std::vector<int32_t> kp((size_t)n);
         int64_t nkp = 0;
         // a k-NN normal that matters may be clipped by a slab face (KPL_E_HALO, reported by every rank): widen the support
-        for (int support = support_; ; support *= 2) {
+        // (1 after 0).  Given normals need no k-NN support: one plan with support 0, which cannot fail that way.
+        for (int support = normals_ ? 0 : support_; ; support = std::max(support * 2, 1)) {
             int rc = kpl_slab_plan_make(xyz, (int32_t)sizeof(PointInT), n, &P[0], gpus_, support, &plan_);
             if (rc != KPL_OK) {
                 std::fprintf(stderr, "[ShardedKeypointLearningDetector::compute] the cloud cannot be cut into %d slabs with a halo of %d + %d cell columns "
@@ -91,7 +105,7 @@ public:
             }
             rc = run(xyz, n, kp.data(), &nkp);
             if (rc == KPL_OK) break;
-            if (rc != KPL_E_HALO || support > 64) {
+            if (rc != KPL_E_HALO || normals_ || support > 64) {
                 std::fprintf(stderr, "[ShardedKeypointLearningDetector::compute] %s\n", error_.c_str());
                 return false;
             }
@@ -133,10 +147,19 @@ private:
             if (rc) { errs[(size_t)g] = "kpl_slab_partition failed"; return; }
             gidx[(size_t)g].resize((size_t)m);
             std::vector<PointInT> own((size_t)m);
-            for (int64_t k = 0; k < m; ++k) own[(size_t)k] = input_->points[(size_t)gidx[(size_t)g][(size_t)k]];
+            std::vector<NormalT> own_n(normals_ ? (size_t)m : 0);
+            for (int64_t k = 0; k < m; ++k) {
+                own[(size_t)k] = input_->points[(size_t)gidx[(size_t)g][(size_t)k]];
+                if (normals_) own_n[(size_t)k] = normals_->points[(size_t)gidx[(size_t)g][(size_t)k]];
+            }
             scores[(size_t)g].assign((size_t)m, 0.f);
             rc = kpl_shard_create(ctx, &plan_, g, nccl ? id : nullptr, &shards[(size_t)g]);
-            if (!rc) rc = kpl_shard_set_slab(shards[(size_t)g], reinterpret_cast<const float*>(own.data()), (int32_t)sizeof(PointInT), gidx[(size_t)g].data(), m);
+            const float* p = reinterpret_cast<const float*>(own.data());
+            if (!rc && normals_)
+                rc = kpl_shard_set_slab_normals(shards[(size_t)g], p, (int32_t)sizeof(PointInT), reinterpret_cast<const float*>(own_n.data()),
+                                                (int32_t)sizeof(NormalT), gidx[(size_t)g].data(), m);
+            else if (!rc)
+                rc = kpl_shard_set_slab(shards[(size_t)g], p, (int32_t)sizeof(PointInT), gidx[(size_t)g].data(), m);
             if (rc) errs[(size_t)g] = kpl_last_error(ctx);
         };
         auto detect = [&](int g) {
@@ -179,6 +202,7 @@ private:
     bool flip_ = false, share_devices_ = false;
     std::vector<std::unique_ptr<Single>> ranks_;
     PointCloudInConstPtr input_;
+    PointCloudNConstPtr normals_;
     pcl::PointIndicesPtr keypoints_indices_{new pcl::PointIndices};
     std::vector<float> response_;
     kpl_slab_plan plan_;

@@ -5,7 +5,8 @@ handling and the keypoint gather all live in csrc/shard.cu; nothing on the step 
 The reference is a single process (src/main_test_detector.cpp:123-187); this is what a multi-GPU driver of that loop
 uses.  Schedule per detection (see include/kpl.h):
   1. position strips (halo = reach(radiusFeatures) + normal_support_cells columns) to / from the two neighbours
-  2. grid with the GLOBAL origin, normals for everything held, scores for the OWNED points only
+  2. grid with the GLOBAL origin, normals for everything held (estimated, or the caller's: their strips travel with the
+     position strips), scores for the OWNED points only
   3. score strips (4 B / point) to / from the two neighbours
   4. threshold + NMS for the owned points, global keypoint list gathered and sorted on rank 0.
 
@@ -93,11 +94,14 @@ def nccl_unique_id() -> bytes:
 
 class SlabJob:
     """One rank of a sharded detection job on a GPU.  `det` is this rank's KeypointLearningDetector (forest and parameters
-    set); `nccl_id` the 128-byte id shared by all ranks (None: a rank of an in-process group, see detect_group)."""
+    set); `nccl_id` the 128-byte id shared by all ranks (None: a rank of an in-process group, see detect_group).
+    `normals`: None (estimated on the devices) or the caller's (n, >=3) normals of the WHOLE cloud
+    (kpl_shard_set_slab_normals; plan with plan_slabs(..., normal_support_cells=0)).  Every rank must choose alike."""
 
-    def __init__(self, det, xyz, plan: SlabPlan, rank: int, nccl_id: bytes | None):
+    def __init__(self, det, xyz, plan: SlabPlan, rank: int, nccl_id: bytes | None, normals=None):
         self._L = capi.load_library()
         self.det, self.plan, self.rank, self.world = det, plan, int(rank), plan.world
+        self.normals = normals
         det._push()
         self._h = C.c_void_p()
         idbuf = C.create_string_buffer(nccl_id, 128) if nccl_id is not None else None
@@ -105,8 +109,8 @@ class SlabJob:
         self._set_slab(xyz)
 
     def replan(self, xyz, plan: SlabPlan):
-        """kpl_shard_set_plan + kpl_shard_set_slab: a new plan for the same communicator (e.g. a wider k-NN support after
-        KPL_E_HALO)."""
+        """kpl_shard_set_plan + kpl_shard_set_slab(_normals): a new plan for the same communicator (e.g. a wider k-NN support
+        after KPL_E_HALO).  The normals given to the constructor are kept."""
         self.plan = plan
         self._check(self._L.kpl_shard_set_plan(self._h, C.byref(plan.c_plan)))
         self._set_slab(xyz)
@@ -119,8 +123,19 @@ class SlabJob:
         own[:, :3] = a[self.gidx, :3]
         self.host_xyz4 = own                       # callers may replace this by a pinned copy (same contents)
         self.n_owned, self.n_total = len(self.gidx), len(a)
-        self._check(self._L.kpl_shard_set_slab(self._h, own.ctypes.data_as(C.POINTER(C.c_float)), 16,
-                                               self.gidx.ctypes.data_as(C.POINTER(C.c_int32)), len(self.gidx)))
+        f32p, gp = C.POINTER(C.c_float), self.gidx.ctypes.data_as(C.POINTER(C.c_int32))
+        if self.normals is None:
+            self._check(self._L.kpl_shard_set_slab(self._h, own.ctypes.data_as(f32p), 16, gp, len(self.gidx)))
+            return
+        nrm = self._owned_normals(self.normals)
+        self._check(self._L.kpl_shard_set_slab_normals(self._h, own.ctypes.data_as(f32p), 16, nrm.ctypes.data_as(f32p), nrm.shape[1] * 4,
+                                                       gp, len(self.gidx)))
+
+    def _owned_normals(self, normals):
+        a = np.asarray(normals)
+        if a.ndim != 2 or a.shape[1] < 3 or len(a) != self.n_total:
+            raise ValueError("normals must be (n, >=3) for the whole cloud of %d points" % self.n_total)
+        return np.ascontiguousarray(a[self.gidx], np.float32)
 
     def _check(self, rc):
         if rc != 0:
@@ -129,6 +144,12 @@ class SlabJob:
     def upload(self, host_xyz4=None):
         a = self.host_xyz4 if host_xyz4 is None else host_xyz4
         self._check(self._L.kpl_shard_upload(self._h, a.ctypes.data_as(C.POINTER(C.c_float)), a.shape[1] * 4))
+
+    def upload_normals(self, normals):
+        """kpl_shard_upload_normals: new normals of the WHOLE cloud, (n, >=3), for the same partition; replan keeps them."""
+        nrm = self._owned_normals(normals)
+        self._check(self._L.kpl_shard_upload_normals(self._h, nrm.ctypes.data_as(C.POINTER(C.c_float)), nrm.shape[1] * 4))
+        self.normals = normals
 
     def detect(self, scores_out=None, kp_out=None):
         """kpl_shard_detect.  Returns (global keypoint count, ascending global keypoint indices on rank 0 / None)."""
@@ -166,12 +187,13 @@ class SlabJob:
 
 def _widening(detect, jobs, xyz, r_feat, r_nms, cpr, max_support):
     """detect(); on KPL_E_HALO (a k-NN normal that matters was clipped by a slab face -- every rank reports it) re-plan
-    `jobs` with twice the k-NN support and try again.  The support is thereby derived from the data."""
+    `jobs` with twice the k-NN support (1 after 0: a support that stays 0 would clip on every retry) and try again.  The support is
+    thereby derived from the data."""
     while True:
         try:
             return detect()
         except capi.KplError as e:
-            ns = jobs[0].plan.normal_support_cells * 2
+            ns = max(jobs[0].plan.normal_support_cells * 2, 1)
             if e.code != capi.KPL_E_HALO or ns > max_support:
                 raise
             plan = plan_slabs(xyz, r_feat, r_nms, cpr, jobs[0].world, ns)
