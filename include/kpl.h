@@ -228,6 +228,38 @@ KPL_API int kpl_detect_batch(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride,
 KPL_API int kpl_detect_batch_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, const int64_t* view_offsets,
                                     int32_t n_views, void* d_scores, void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out);
 
+/* ---- a batch of ORGANIZED frames of one size (depth-camera streams; the 2.5-D views of BASELINE.json configs[4]) ---- */
+/* n_frames organized frames of width x height points each, row-major, frame after frame (NaN = no measurement); xyz at
+ * xyz_stride bytes per point.
+ * normals: NULL -> pcl::IntegralImageNormalEstimation(SIMPLE_3D_GRADIENT, smoothing_size) per frame (hpp:138-145, as
+ *          kpl_normals_organized), flipped towards viewpoints[3f..3f+2] (viewpoints NULL: params.viewpoint for every
+ *          frame); else the caller's per-pixel normals at normals_stride bytes (viewpoints ignored).
+ * The points with finite x, y, z (pcl::isFinite) of each frame are detected as kpl_detect would detect them alone, in
+ * ascending pixel order: the results of every frame are bit-identical to the single-frame organized path.  normals_mode
+ * and flip_normals are ignored, as on that path.  The integral images of up to 256 MiB of frames ((W+1)(H+1)*24 B per
+ * frame) are built per launch; a larger batch runs in chunks on the stream, without a host round trip between them.
+ * scores_out: NULL or n_frames*width*height floats in pixel order (NaN: non-finite pixel or no finite normal).
+ * kp_idx_out (capacity n_frames*width*height): FRAME-LOCAL pixel indices r*width + c, ascending within a frame;
+ * kp_offsets_out[n_frames + 1]: frame f's keypoints are kp_idx_out[kp_offsets_out[f] .. kp_offsets_out[f+1]).  A frame
+ * without a finite point gets an empty range; a batch without any returns KPL_OK and no keypoint.
+ * kpl_stats describe the detection over the finite points (n_points = their number, n_views = n_frames); in kpl_timings
+ * normals_ms includes the integral images and the compaction, total_ms covers the whole call.  kpl_fetch("normals")
+ * then returns the normals of the finite points, frame after frame.  Host round trips: one for the per-frame finite
+ * counts plus those of kpl_detect_batch_device (plus one for the results).
+ * KPL_E_INVALID: width, height or n_frames < 1, more than 2 147 483 000 points, a smoothing size that is not finite and
+ * > 0, a bad stride, a NULL input or output, a forced grid in the params.  KPL_E_FOREST without a forest. */
+KPL_API int kpl_detect_batch_organized(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals,
+                                       int32_t normals_stride, int32_t width, int32_t height, int32_t n_frames,
+                                       float smoothing_size, const float* viewpoints, float* scores_out,
+                                       int32_t* kp_idx_out, int64_t* kp_offsets_out);
+/* Device-resident frames (float4 per pixel); viewpoints stay a HOST array; d_scores: NULL or n_frames*width*height
+ * floats; d_kp_idx: n_frames*width*height int32; d_kp_offsets: n_frames + 1 int64.  The keypoint offsets are computed on
+ * the device: no round trip beyond those of kpl_detect_batch_device and the per-frame finite counts. */
+KPL_API int kpl_detect_batch_organized_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, int32_t width,
+                                              int32_t height, int32_t n_frames, float smoothing_size,
+                                              const float* viewpoints, void* d_scores, void* d_kp_idx,
+                                              void* d_kp_offsets, int64_t* n_kp_out);
+
 /* ---- ONE large cloud over the GPUs of a node: x slabs + halo over NCCL (BASELINE.json configs[3]) ---------- */
 /* The reference is a single process (main_test_detector.cpp:123-187 drives one detector); this is the layer a
  * multi-GPU driver binds to.  The cloud is cut along x at CELL-COLUMN boundaries of the canonical grid of the WHOLE

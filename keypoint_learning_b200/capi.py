@@ -28,7 +28,8 @@ EXPORTS = ["kpl_create", "kpl_destroy", "kpl_last_error", "kpl_version", "kpl_se
            "kpl_fetch_u8", "kpl_device_count", "kpl_normals_organized", "kpl_detect_batch", "kpl_detect_batch_device",
            "kpl_slab_plan_make", "kpl_slab_partition", "kpl_nccl_unique_id", "kpl_shard_create", "kpl_shard_destroy", "kpl_shard_set_plan",
            "kpl_shard_set_slab", "kpl_shard_upload", "kpl_shard_detect", "kpl_shard_detect_group", "kpl_shard_get_info",
-           "kpl_shard_device_scores", "kpl_shard_set_slab_normals", "kpl_shard_upload_normals"]
+           "kpl_shard_device_scores", "kpl_shard_set_slab_normals", "kpl_shard_upload_normals", "kpl_detect_batch_organized",
+           "kpl_detect_batch_organized_device"]
 KPL_MAX_RANKS = 64
 
 
@@ -128,6 +129,9 @@ def load_library():
     L.kpl_shard_device_scores.argtypes = [vp]; L.kpl_shard_device_scores.restype = vp
     L.kpl_detect_batch.argtypes = [vp, f32p, C.c_int32, f32p, C.c_int32, i64p, C.c_int32, f32p, i32p, i64p]
     L.kpl_detect_batch_device.argtypes = [vp, vp, vp, i64p, C.c_int32, vp, vp, vp, i64p]
+    L.kpl_detect_batch_organized.argtypes = [vp, f32p, C.c_int32, f32p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_float, f32p, f32p,
+                                             i32p, i64p]
+    L.kpl_detect_batch_organized_device.argtypes = [vp, vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_float, f32p, vp, vp, vp, i64p]
     _lib = L
     return L
 
@@ -397,6 +401,45 @@ class KeypointLearningDetector:
             return self.compute()
         finally:
             self._cloud, self._normals = saved
+
+    def computeOrganizedBatch(self, frames, smoothing=5.0, normals=None, viewpoints=None):
+        """kpl_detect_batch_organized: `frames` is (F, height, width, >=3) float32 (NaN = no measurement).  normals: None
+        (integral-image normals of every frame, flipped towards viewpoints[f] -- an (F, 3) array, default the detector's
+        viewpoint) or per-pixel normals of the same (F, height, width, >=3) shape.  Returns (scores list, keypoint pixel index
+        list), one entry per frame: what computeOrganized() (normals None) or compute() on the flattened frame with
+        setNormals (normals given) returns for that frame alone."""
+        a = np.asarray(frames)
+        if a.ndim != 4 or a.shape[3] < 3:
+            raise ValueError("frames must be (n_frames, height, width, >=3) float32")
+        a = np.ascontiguousarray(a, np.float32)
+        nf, h, w, c = a.shape
+        nrm = None
+        if normals is not None:
+            nrm = np.ascontiguousarray(normals, np.float32)
+            if nrm.shape[:3] != (nf, h, w) or nrm.ndim != 4 or nrm.shape[3] < 3:
+                raise ValueError("normals must be (n_frames, height, width, >=3) float32")
+        vp = None if viewpoints is None else np.ascontiguousarray(viewpoints, np.float32).reshape(nf, 3)
+        self._push()
+        n = nf * h * w
+        scores = np.empty(n, np.float32)
+        kp = np.empty(max(n, 1), np.int32)
+        kpo = np.empty(nf + 1, np.int64)
+        self._check(self._L.kpl_detect_batch_organized(self._h, _ptr(a, C.c_float), c * 4, _ptr(nrm, C.c_float),
+                                                       0 if nrm is None else nrm.shape[3] * 4, w, h, nf, float(smoothing), _ptr(vp, C.c_float),
+                                                       _ptr(scores, C.c_float), _ptr(kp, C.c_int32), _ptr(kpo, C.c_int64)))
+        return ([scores[f * h * w:(f + 1) * h * w] for f in range(nf)], [kp[kpo[f]:kpo[f + 1]].copy() for f in range(nf)])
+
+    def detectOrganizedBatchDevice(self, d_xyz4, width, height, n_frames, smoothing=5.0, d_normals4=0, viewpoints=None, d_scores=0,
+                                   d_kp_idx=0, d_kp_offsets=0):
+        """Device-resident organized frames (float4 per pixel): raw device pointers (ints), host viewpoints ((F, 3) or None).
+        Returns the total keypoint count."""
+        vp = None if viewpoints is None else np.ascontiguousarray(viewpoints, np.float32).reshape(int(n_frames), 3)
+        self._push()
+        nkp = C.c_int64(0)
+        self._check(self._L.kpl_detect_batch_organized_device(self._h, C.c_void_p(d_xyz4), C.c_void_p(d_normals4 or None), int(width), int(height),
+                                                              int(n_frames), float(smoothing), _ptr(vp, C.c_float), C.c_void_p(d_scores or None),
+                                                              C.c_void_p(d_kp_idx or None), C.c_void_p(d_kp_offsets or None), C.byref(nkp)))
+        return nkp.value
 
     def computePointsForTrainingFeatures(self, indices=None):
         xyz, xs = _vec3(self._cloud, "cloud")

@@ -121,6 +121,8 @@ void kpl_destroy(kpl_ctx* ctx)
     release(ctx->warp_order); release(ctx->s_pos); release(ctx->s_nrm); release(ctx->feat);
     release(ctx->s_score); release(ctx->score); release(ctx->flag); release(ctx->s_state); release(ctx->kp_idx);
     release(ctx->scratch_f); release(ctx->scratch_i); release(ctx->counters);
+    release(ctx->org_flag); release(ctx->org_pix); release(ctx->org_xyz); release(ctx->org_nrm); release(ctx->org_frame_off);
+    release(ctx->org_kp_off); release(ctx->org_vp); release(ctx->org_score);
     if (ctx->d_bbox) cudaFree(ctx->d_bbox);
     if (ctx->forest.d_nodes) cudaFree(ctx->forest.d_nodes);
     if (ctx->forest.d_roots) cudaFree(ctx->forest.d_roots);
@@ -551,6 +553,66 @@ static int run_detect_batch(kpl_ctx* ctx, const float4* d_xyz, const float4* d_n
     return rc;
 }
 
+// A batch of organized frames of one size: integral-image normals of every frame (or the caller's per-pixel normals),
+// the finite pixels compacted in ascending pixel order, the compacted frames detected as the views of one batch, and the
+// results mapped back to pixel order.  Each frame's view is the cloud the single-frame path (computeOrganized /
+// KeypointLearningDetector::compute) detects after dropping its NaN points, in the same order, so its results are that
+// path's.  One host round trip for the per-frame finite counts, which the batch needs as host view offsets; a frame
+// without a finite point is left out of the batch (views must not be empty) and gets an empty keypoint range.
+static int run_detect_organized_batch(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, int32_t W, int32_t H, int32_t F,
+                                      float smoothing_size, const float* h_viewpoints, float* d_scores_out, int32_t* d_kp_out,
+                                      int64_t* d_kp_offsets_out, int64_t* n_kp_out)
+{
+    const int64_t n = (int64_t)W * H, total = n * F;
+    int rc = detect_check(ctx, total, false);
+    if (rc) return rc;
+    if (ctx->params.grid_forced) return fail(ctx, KPL_E_INVALID, "a forced grid cannot be combined with a batch of frames");
+    ctx->stats.n_views = F;
+    if ((rc = detect_begin(ctx))) return rc;
+    if (!d_nrm) {
+        const float* d_vp = nullptr;
+        if (h_viewpoints) {
+            KPL_CUDA(ensure(ctx->org_vp, (size_t)F * 3));
+            KPL_CUDA(cudaMemcpyAsync(ctx->org_vp.p, h_viewpoints, (size_t)F * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+            d_vp = ctx->org_vp.p;
+        }
+        KPL_CUDA(ensure(ctx->in_nrm, (size_t)total));        // per-pixel normals; the staging buffer is free without caller normals
+        KPL_CUDA(launch_normals_integral_image(ctx, d_xyz, W, H, F, smoothing_size, d_vp, ctx->in_nrm.p));
+        d_nrm = ctx->in_nrm.p;
+    }
+    KPL_CUDA(launch_organized_select(ctx, d_xyz, n, F, d_scores_out));
+    KPL_CUDA(cudaEventRecord(ctx->ev[6], ctx->stream));
+    std::vector<int64_t> frame_off((size_t)F + 1);
+    KPL_CUDA(cudaMemcpyAsync(frame_off.data(), ctx->org_frame_off.p, frame_off.size() * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    KPL_CUDA(cudaStreamSynchronize(ctx->stream));
+    ctx->syncs++;
+    const int64_t m = frame_off[(size_t)F];
+    std::vector<int64_t> view_off(1, 0);
+    for (int32_t f = 0; f < F; ++f)
+        if (frame_off[(size_t)f + 1] > frame_off[(size_t)f]) view_off.push_back(frame_off[(size_t)f + 1]);
+    kpl_timings& T = ctx->timings;
+    if (m == 0) {
+        KPL_CUDA(cudaMemsetAsync(d_kp_offsets_out, 0, ((size_t)F + 1) * sizeof(int64_t), ctx->stream));
+        cudaEventElapsedTime(&T.normals_ms, ctx->ev[0], ctx->ev[6]);
+        T.total_ms = T.normals_ms;
+        ctx->stats.n_points = 0; ctx->stats.kernel_launches = ctx->launches; ctx->stats.host_syncs = ctx->syncs;
+        return KPL_OK;
+    }
+    KPL_CUDA(launch_organized_gather(ctx, d_xyz, d_nrm, m));
+    if ((rc = prepare_grid_batch(ctx, ctx->org_xyz.p, ctx->org_nrm.p, m, view_off.data(), (int)view_off.size() - 1))) return rc;
+    if ((rc = detect_score_phase(ctx, true, false, m))) return rc;
+    if ((rc = detect_nms_phase(ctx, false, m, d_kp_out))) return rc;
+    KPL_CUDA(launch_organized_map_back(ctx, m, n, F, d_scores_out, d_kp_out, d_kp_offsets_out));
+    if ((rc = detect_finish(ctx, m, n_kp_out))) return rc;
+    // the integral images and the compaction are part of the normals stage; the grid stage starts after them
+    float prep = 0.f;
+    cudaEventElapsedTime(&prep, ctx->ev[0], ctx->ev[6]);
+    cudaEventElapsedTime(&T.grid_ms, ctx->ev[6], ctx->ev[1]);
+    T.normals_ms += prep;
+    ctx->stats.n_views = F;
+    return KPL_OK;
+}
+
 // host (possibly strided) -> device float4 staging
 static int upload_vec3(kpl_ctx* ctx, DevBuf<float4>& dst, const float* src, int32_t stride, int64_t n)
 {
@@ -721,6 +783,57 @@ int kpl_detect_batch_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_norm
                             (int32_t*)d_kp_idx, (int64_t*)d_kp_offsets, n_kp_out);
 }
 
+static int check_organized_batch(kpl_ctx* ctx, int32_t width, int32_t height, int32_t n_frames, float smoothing_size)
+{
+    if (width < 1 || height < 1 || n_frames < 1) return fail(ctx, KPL_E_INVALID, "width, height and n_frames must be >= 1");
+    if ((int64_t)width * height * n_frames > 2147483000ll) return fail(ctx, KPL_E_INVALID, "point count out of range");
+    if (!(smoothing_size > 0.f) || !std::isfinite(smoothing_size)) return fail(ctx, KPL_E_INVALID, "normal smoothing size must be > 0");
+    return KPL_OK;
+}
+
+int kpl_detect_batch_organized(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
+                               int32_t width, int32_t height, int32_t n_frames, float smoothing_size, const float* viewpoints,
+                               float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out)
+{
+    if (!ctx) return KPL_E_INVALID;
+    detect_reset(ctx);
+    ctx->stats.n_views = n_frames;
+    if (!xyz || !kp_idx_out || !kp_offsets_out) return fail(ctx, KPL_E_INVALID, "xyz / kp_idx_out / kp_offsets_out is NULL");
+    int rc = check_organized_batch(ctx, width, height, n_frames, smoothing_size);
+    if (rc) return rc;
+    const int64_t total = (int64_t)width * height * n_frames;
+    if ((rc = upload_inputs(ctx, xyz, xyz_stride, normals, normals_stride, nullptr, total))) return rc;
+    KPL_CUDA(ensure(ctx->kp_idx, (size_t)total));
+    KPL_CUDA(ensure(ctx->org_kp_off, (size_t)n_frames + 1));
+    if (scores_out) KPL_CUDA(ensure(ctx->org_score, (size_t)total));
+    int64_t nkp = 0;
+    rc = run_detect_organized_batch(ctx, ctx->in_xyz.p, normals ? ctx->in_nrm.p : nullptr, width, height, n_frames, smoothing_size, viewpoints,
+                                    scores_out ? ctx->org_score.p : nullptr, ctx->kp_idx.p, ctx->org_kp_off.p, &nkp);
+    if (rc) return rc;
+    if (scores_out) KPL_CUDA(cudaMemcpyAsync(scores_out, ctx->org_score.p, (size_t)total * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    if (nkp > 0) KPL_CUDA(cudaMemcpyAsync(kp_idx_out, ctx->kp_idx.p, (size_t)nkp * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    KPL_CUDA(cudaMemcpyAsync(kp_offsets_out, ctx->org_kp_off.p, ((size_t)n_frames + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    KPL_CUDA(cudaStreamSynchronize(ctx->stream));
+    ctx->syncs++; ctx->stats.host_syncs = ctx->syncs;
+    return KPL_OK;
+}
+
+int kpl_detect_batch_organized_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, int32_t width, int32_t height,
+                                      int32_t n_frames, float smoothing_size, const float* viewpoints, void* d_scores, void* d_kp_idx,
+                                      void* d_kp_offsets, int64_t* n_kp_out)
+{
+    if (!ctx) return KPL_E_INVALID;
+    detect_reset(ctx);
+    ctx->stats.n_views = n_frames;
+    if (n_kp_out) *n_kp_out = 0;
+    if (!d_xyz4 || !d_kp_idx || !d_kp_offsets) return fail(ctx, KPL_E_INVALID, "NULL device pointer");
+    int rc = check_organized_batch(ctx, width, height, n_frames, smoothing_size);
+    if (rc) return rc;
+    KPL_CUDA(cudaSetDevice(ctx->device));
+    return run_detect_organized_batch(ctx, (const float4*)d_xyz4, (const float4*)d_normals4, width, height, n_frames, smoothing_size, viewpoints,
+                                      (float*)d_scores, (int32_t*)d_kp_idx, (int64_t*)d_kp_offsets, n_kp_out);
+}
+
 int kpl_normals(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, int64_t n, float* normals_out)
 {
     if (!ctx || (n > 0 && !normals_out)) return KPL_E_INVALID;
@@ -760,7 +873,7 @@ int kpl_normals_organized(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, in
     int rc = upload_inputs(ctx, xyz, xyz_stride, nullptr, 0, nullptr, n);
     if (rc) return rc;
     KPL_CUDA(ensure(ctx->in_nrm, (size_t)n));
-    KPL_CUDA(launch_normals_integral_image(ctx, ctx->in_xyz.p, width, height, smoothing_size, ctx->in_nrm.p));
+    KPL_CUDA(launch_normals_integral_image(ctx, ctx->in_xyz.p, width, height, 1, smoothing_size, nullptr, ctx->in_nrm.p));
     KPL_CUDA(cudaMemcpyAsync(normals_out, ctx->in_nrm.p, (size_t)n * 16, cudaMemcpyDeviceToHost, ctx->stream));
     KPL_CUDA(cudaStreamSynchronize(ctx->stream));
     ctx->syncs++;

@@ -124,6 +124,14 @@ struct kpl_ctx {
     kpl::DevBuf<int32_t> kp_idx;
     kpl::DevBuf<float> scratch_f;                // fetch / reorder scratch
     kpl::DevBuf<int32_t> scratch_i;
+    // kpl_detect_batch_organized: finite-pixel flags, compact index -> pixel index (frame f's pixel p is f*width*height + p),
+    // the compacted positions / normals the detection runs on, the frames' first compacted points (+ their count), the
+    // per-frame viewpoints, and the pixel-order scores / frame keypoint offsets of the host entry point
+    kpl::DevBuf<uint8_t> org_flag;
+    kpl::DevBuf<int32_t> org_pix;
+    kpl::DevBuf<float4> org_xyz, org_nrm;
+    kpl::DevBuf<int64_t> org_frame_off, org_kp_off;
+    kpl::DevBuf<float> org_vp, org_score;
     // [0] feature pairs [1] candidate pairs [2] above th [3] n_kp [4] unscored [5] scored [6] scratch [7] near threshold
     // [8] fragile points [9] clipped k-NN searches (slab edge) [10] scratch [11..15] sizes of the query lists (grid.cu: build_lists)
     kpl::DevBuf<unsigned long long> counters;
@@ -152,7 +160,17 @@ cudaError_t launch_check_normals(kpl_ctx* c, int64_t n, bool use_role);
 bool normals_knn_uses_work_list(const kpl_params& P);
 cudaError_t launch_bbox_init(kpl_ctx* c);
 cudaError_t launch_gather_keypoints(kpl_ctx* c, const float4* d_xyz, const int32_t* d_kp_idx, int64_t nkp, float4* d_out);
-cudaError_t launch_normals_integral_image(kpl_ctx* c, const float4* d_xyz, int W, int H, float smoothing_size, float4* d_out);
+// nframes frames of W x H pixels; d_viewpoints: NULL (params.viewpoint) or 3 device floats per frame
+cudaError_t launch_normals_integral_image(kpl_ctx* c, const float4* d_xyz, int W, int H, int nframes, float smoothing_size,
+                                          const float* d_viewpoints, float4* d_out);
+// organized frames (n pixels each) -> finite pixels in ascending order (org_pix) and org_frame_off; d_scores (NULL or
+// nframes * n floats) is set to NaN
+cudaError_t launch_organized_select(kpl_ctx* c, const float4* d_xyz, int64_t n, int nframes, float* d_scores);
+// the m selected pixels' positions and normals (per pixel) -> org_xyz / org_nrm
+cudaError_t launch_organized_gather(kpl_ctx* c, const float4* d_xyz, const float4* d_nrm, int64_t m);
+// after the detection of the m compacted points: scores to pixel order, keypoints (in place) to frame-local pixel indices,
+// frame keypoint offsets (nframes + 1)
+cudaError_t launch_organized_map_back(kpl_ctx* c, int64_t m, int64_t n, int nframes, float* d_scores, int32_t* d_kp, int64_t* d_kp_off);
 cudaError_t build_lists(kpl_ctx* c, int64_t n, int span_n, bool curve_normals, bool want_features, bool use_role, int64_t longest_first_below);
 cudaError_t launch_count_occupied_cells(kpl_ctx* c, int64_t n, unsigned long long* d_out);
 cudaError_t build_query_list(kpl_ctx* c, int64_t n, const int32_t* d_indices, int64_t m);

@@ -172,20 +172,66 @@ public:
         return m;
     }
 
-    kpl_ctx* context() { return ctx_; }
-
-protected:
-    bool initCompute()
+    // A stream of organized frames of one width x height (a depth camera) in one pass (kpl_detect_batch_organized): for
+    // every frame what compute() returns for it alone with no normals set -- integral-image normals (hpp:138-145) flipped
+    // towards the frame's sensor_origin_, the detection over its finite points.  outputs[f] is frame f's keypoint cloud
+    // (x, y, z, intensity = response); (*indices)[f], when asked for, its keypoint indices.  The input cloud, normals,
+    // response and keypoint indices of the detector are left as they are.
+    bool computeOrganizedBatch(const std::vector<PointCloudInConstPtr>& frames, std::vector<PointCloudOut>& outputs,
+                               std::vector<pcl::PointIndices>* indices = nullptr)
     {
-        if (!ctx_ || !input_) {
+        outputs.assign(frames.size(), PointCloudOut());
+        if (indices) indices->assign(frames.size(), pcl::PointIndices());
+        if (!ctx_ || frames.empty() || !frames[0]) {
             std::fprintf(stderr, "[pcl::%s::initCompute] init failed!\n", name_.c_str());
             return false;
         }
-        if (surface_ && surface_ != input_) {
-            std::fprintf(stderr, "[pcl::%s::initCompute] a search surface other than the input cloud is not supported: normals, response and "
-                                 "neighbour indices share one index space (hpp:203-253,334-342)\n", name_.c_str());
+        const uint32_t W = frames[0]->width, H = frames[0]->height;
+        for (const PointCloudInConstPtr& f : frames)
+            if (!f || !f->isOrganized() || f->width != W || f->height != H || f->size() != (size_t)W * H) {
+                std::fprintf(stderr, "[pcl::%s::initCompute] the frames of a batch must be organized clouds of one width x height\n", name_.c_str());
+                return false;
+            }
+        if (!checkSearch()) return false;
+        const size_t n = (size_t)W * H, F = frames.size();
+        std::vector<PointInT> pts(n * F);
+        std::vector<float> vps(3 * F), scores(n * F);
+        for (size_t f = 0; f < F; ++f) {
+            std::copy(frames[f]->points.begin(), frames[f]->points.end(), pts.begin() + f * n);
+            for (int a = 0; a < 3; ++a) vps[3 * f + a] = frames[f]->sensor_origin_[a];
+        }
+        std::vector<int32_t> idx(n * F);
+        std::vector<int64_t> off(F + 1);
+        if (kpl_set_params(ctx_, &p_) != KPL_OK ||
+            kpl_detect_batch_organized(ctx_, reinterpret_cast<const float*>(pts.data()), (int32_t)sizeof(PointInT), nullptr, 0, (int32_t)W, (int32_t)H,
+                                       (int32_t)F, 5.0f, vps.data(), scores.data(), idx.data(), off.data()) != KPL_OK) {
+            std::fprintf(stderr, "[pcl::%s::compute] %s\n", name_.c_str(), kpl_last_error(ctx_));
             return false;
         }
+        for (size_t f = 0; f < F; ++f) {
+            PointCloudOut& out = outputs[f];
+            for (int64_t k = off[f]; k < off[f + 1]; ++k) {                      // hpp:246-253
+                const int32_t i = idx[(size_t)k];
+                const PointInT& p = frames[f]->points[(size_t)i];
+                PointOutT o;
+                o.x = p.x; o.y = p.y; o.z = p.z;
+                o.intensity = scores[f * n + (size_t)i];
+                out.points.push_back(o);
+                if (indices) (*indices)[f].indices.push_back(i);
+            }
+            out.height = 1;
+            out.width = (uint32_t)out.points.size();
+            out.is_dense = p_.non_maxima ? true : frames[f]->is_dense;             // hpp:192-193,258-260
+        }
+        return true;
+    }
+
+    kpl_ctx* context() { return ctx_; }
+
+protected:
+    // pcl::Keypoint::initCompute's search checks
+    bool checkSearch() const
+    {
         if (p_.radius_features > 0.f && k_ != 0) {   // pcl::Keypoint::initCompute
             std::fprintf(stderr, "[pcl::%s::initCompute] Both radius (%f) and K (%d) defined! Set one of them to zero first and then re-run compute ().\n",
                          name_.c_str(), p_.radius_features, k_);
@@ -198,6 +244,21 @@ protected:
                 std::fprintf(stderr, "[pcl::%s::initCompute] Neither radius nor K defined! Set one of them to zero first and then re-run compute ().\n", name_.c_str());
             return false;
         }
+        return true;
+    }
+
+    bool initCompute()
+    {
+        if (!ctx_ || !input_) {
+            std::fprintf(stderr, "[pcl::%s::initCompute] init failed!\n", name_.c_str());
+            return false;
+        }
+        if (surface_ && surface_ != input_) {
+            std::fprintf(stderr, "[pcl::%s::initCompute] a search surface other than the input cloud is not supported: normals, response and "
+                                 "neighbour indices share one index space (hpp:203-253,334-342)\n", name_.c_str());
+            return false;
+        }
+        if (!checkSearch()) return false;
         if (normals_ && normals_->size() != input_->size()) {
             std::fprintf(stderr, "[pcl::%s::initCompute] normals given, but the number of normals does not match the number of input points!\n", name_.c_str());
             return false;
