@@ -148,6 +148,19 @@ KPL_API int kpl_set_forest(kpl_ctx* ctx, int32_t ntrees, int32_t nnodes, const i
                            int32_t var_count);
 KPL_API int kpl_forest_info(const kpl_ctx* ctx, int32_t* ntrees, int32_t* nnodes, int32_t* var_count, int32_t* max_depth);
 
+/* ---- a SET of forests scored from one feature pass (kpl_detect_forests) ---------------------------- */
+/* The forest set holds forest 0 -- the one kpl_load_forest / kpl_set_forest install, which also drop every other forest --
+ * and up to KPL_MAX_FORESTS - 1 forests appended by kpl_add_forest(_arrays) as forests 1, 2, ...; *index_out (may be NULL)
+ * receives the new forest's index.  Adding needs forest 0 (KPL_E_FOREST without it) and fails with KPL_E_INVALID once the
+ * set is full; a failed add leaves the set as it was.  kpl_forest_info keeps describing forest 0, and every entry point
+ * other than kpl_detect_forests(_device) scores with forest 0 only, whatever else is loaded. */
+#define KPL_MAX_FORESTS 16
+KPL_API int kpl_add_forest(kpl_ctx* ctx, const char* path, int32_t* index_out);
+KPL_API int kpl_add_forest_arrays(kpl_ctx* ctx, int32_t ntrees, int32_t nnodes, const int32_t* roots, const int32_t* var,
+                                  const float* thr, const int32_t* left, const int32_t* right, const float* value,
+                                  int32_t var_count, int32_t* index_out);
+KPL_API int kpl_forest_count(const kpl_ctx* ctx, int32_t* count_out);
+
 /* ---- the hot path, host buffers (what detector->compute() binds to) --------------------------- */
 /* xyz: n points, 3 floats each at xyz_stride bytes (16 = pcl::PointXYZ, 12 = packed).
  * normals: NULL (estimate per params.normals_mode) or n normals, 3 floats each at normals_stride bytes
@@ -210,6 +223,26 @@ KPL_API int kpl_radius_neighbors(kpl_ctx* ctx, const float* xyz, int32_t xyz_str
  * synchronises once at the end to return n_kp. */
 KPL_API int kpl_detect_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, const void* d_role, int64_t n,
                               void* d_scores, void* d_kp_idx, int64_t* n_kp_out);
+
+/* ---- one cloud, every forest of the set (several descriptors' forests, forest sweeps) ---------------- */
+/* The K forests of the set (kpl_forest_count) score one cloud from ONE feature pass: grid, normals and the annuli x bins
+ * histograms are computed once, and the feature kernel walks all K forests from each histogram.  Forest k's results are
+ * bit-identical to kpl_detect on the same cloud with only forest k loaded and params.threshold = thresholds[k]
+ * (thresholds NULL: params.threshold for every forest; compared in double, hpp:207).  Inputs as in kpl_detect, without a
+ * role array; the grid follows the params as in kpl_detect (a forced grid included).  Outputs are forest-major:
+ * scores_out: NULL or K*n floats, forest k's at k*n.  kp_idx_out (capacity K*n): ascending point indices per forest;
+ * kp_offsets_out[K + 1]: forest k's keypoints are kp_idx_out[kp_offsets_out[k] .. kp_offsets_out[k+1]).
+ * Every forest must match annuli*bins (var_count, and no split beyond it): KPL_E_VARCOUNT names the forest.  K*n must not
+ * exceed 2 147 483 000.  kpl_stats: feature_pairs, candidate_pairs and n_scored count the one feature pass;
+ * n_above_threshold, n_near_threshold, n_keypoints, n_fragile_points and nms_rounds are sums over the forests.  With
+ * report_fragile, kpl_fetch_u8("fragile") returns K*n bytes, forest-major.  Host round trips: those of kpl_detect_device
+ * whatever K is (plus one per draws-remove round of each forest, plus one for the results). */
+KPL_API int kpl_detect_forests(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
+                               int64_t n, const double* thresholds, float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out);
+/* Device-resident cloud: d_scores NULL or K*n floats, d_kp_idx K*n int32, d_kp_offsets K + 1 int64, all on the device
+ * (thresholds stays a HOST array of K doubles or NULL); *n_kp_out = keypoints of all forests. */
+KPL_API int kpl_detect_forests_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, int64_t n, const double* thresholds,
+                                      void* d_scores, void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out);
 
 /* ---- a batch of independent views in one pass (BASELINE.json configs[4]) ------------------------ */
 /* TestDetector handles one view per process run (main_test_detector.cpp:142-187); a caller with many small views
@@ -360,7 +393,8 @@ KPL_API int kpl_get_stats(const kpl_ctx* ctx, kpl_stats* s);
 /* Device copies of intermediate results of the last call, for parity tests: what = "normals"
  * (n x 4 floats, original order) or "features" (n x A*B floats, original order). */
 KPL_API int kpl_fetch(kpl_ctx* ctx, const char* what, float* out, int64_t capacity_floats);
-/* Byte masks of the last detect call, original order: what = "fragile" (see kpl_stats.n_fragile_points). */
+/* Byte masks of the last detect call, original order: what = "fragile" (see kpl_stats.n_fragile_points); K*n bytes,
+ * forest-major, after kpl_detect_forests. */
 KPL_API int kpl_fetch_u8(kpl_ctx* ctx, const char* what, uint8_t* out, int64_t capacity);
 
 #ifdef __cplusplus

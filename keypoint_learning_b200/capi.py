@@ -29,8 +29,10 @@ EXPORTS = ["kpl_create", "kpl_destroy", "kpl_last_error", "kpl_version", "kpl_se
            "kpl_slab_plan_make", "kpl_slab_partition", "kpl_nccl_unique_id", "kpl_shard_create", "kpl_shard_destroy", "kpl_shard_set_plan",
            "kpl_shard_set_slab", "kpl_shard_upload", "kpl_shard_detect", "kpl_shard_detect_group", "kpl_shard_get_info",
            "kpl_shard_device_scores", "kpl_shard_set_slab_normals", "kpl_shard_upload_normals", "kpl_detect_batch_organized",
-           "kpl_detect_batch_organized_device"]
+           "kpl_detect_batch_organized_device", "kpl_add_forest", "kpl_add_forest_arrays", "kpl_forest_count", "kpl_detect_forests",
+           "kpl_detect_forests_device"]
 KPL_MAX_RANKS = 64
+KPL_MAX_FORESTS = 16
 
 
 class KplParams(C.Structure):
@@ -98,6 +100,12 @@ def load_library():
     L.kpl_load_forest.argtypes = [vp, C.c_char_p]
     L.kpl_set_forest.argtypes = [vp, C.c_int32, C.c_int32, i32p, i32p, f32p, i32p, i32p, f32p, C.c_int32]
     L.kpl_forest_info.argtypes = [vp, i32p, i32p, i32p, i32p]
+    L.kpl_add_forest.argtypes = [vp, C.c_char_p, i32p]
+    L.kpl_add_forest_arrays.argtypes = [vp, C.c_int32, C.c_int32, i32p, i32p, f32p, i32p, i32p, f32p, C.c_int32, i32p]
+    L.kpl_forest_count.argtypes = [vp, i32p]
+    f64p = C.POINTER(C.c_double)
+    L.kpl_detect_forests.argtypes = [vp, f32p, C.c_int32, f32p, C.c_int32, C.c_int64, f64p, f32p, i32p, i64p]
+    L.kpl_detect_forests_device.argtypes = [vp, vp, vp, C.c_int64, f64p, vp, vp, vp, i64p]
     L.kpl_detect.argtypes = [vp, f32p, C.c_int32, f32p, C.c_int32, u8p, C.c_int64, f32p, i32p, i64p]
     L.kpl_detect_xyzi.argtypes = [vp, f32p, C.c_int32, f32p, C.c_int32, u8p, C.c_int64, f32p, i32p, f32p, i64p]
     L.kpl_normals.argtypes = [vp, f32p, C.c_int32, C.c_int64, f32p]
@@ -175,6 +183,7 @@ class KeypointLearningDetector:
         self._normals = None
         self._kp_idx = np.empty(0, np.int32)
         self._scores = None
+        self._responses = None
         self._xyzi = None
 
     # ---- lifetime
@@ -254,12 +263,34 @@ class KeypointLearningDetector:
         ptr = None if cuda_stream_ptr is None else (int(cuda_stream_ptr) or 1)
         self._check(self._L.kpl_set_stream(self._h, C.c_void_p(ptr)))
 
+    @staticmethod
+    def _forest_args(f):
+        arrays = [np.ascontiguousarray(f["roots"], np.int32), np.ascontiguousarray(f["var"], np.int32), np.ascontiguousarray(f["thr"], np.float32),
+                  np.ascontiguousarray(f["left"], np.int32), np.ascontiguousarray(f["right"], np.int32), np.ascontiguousarray(f["value"], np.float32)]
+        types = [C.c_int32, C.c_int32, C.c_float, C.c_int32, C.c_int32, C.c_float]
+        return arrays, [int(f["ntrees"]), len(f["var"])] + [_ptr(a, t) for a, t in zip(arrays, types)] + [int(f.get("var_count", 0))]
+
     def setForestArrays(self, forest):
-        f = forest
-        self._check(self._L.kpl_set_forest(self._h, int(f["ntrees"]), len(f["var"]), _ptr(np.ascontiguousarray(f["roots"], np.int32), C.c_int32),
-                                           _ptr(np.ascontiguousarray(f["var"], np.int32), C.c_int32), _ptr(np.ascontiguousarray(f["thr"], np.float32), C.c_float),
-                                           _ptr(np.ascontiguousarray(f["left"], np.int32), C.c_int32), _ptr(np.ascontiguousarray(f["right"], np.int32), C.c_int32),
-                                           _ptr(np.ascontiguousarray(f["value"], np.float32), C.c_float), int(f.get("var_count", 0))))
+        keep, args = self._forest_args(forest)
+        self._check(self._L.kpl_set_forest(self._h, *args))
+
+    def addForest(self, path):
+        """kpl_add_forest: append the forest at `path` to the forest set (forest 0 is loadForest's); returns its index."""
+        idx = C.c_int32(-1)
+        self._check(self._L.kpl_add_forest(self._h, os.fsencode(path), C.byref(idx)))
+        return idx.value
+
+    def addForestArrays(self, forest):
+        """kpl_add_forest_arrays: the same from the arrays setForestArrays takes; returns the new forest's index."""
+        keep, args = self._forest_args(forest)
+        idx = C.c_int32(-1)
+        self._check(self._L.kpl_add_forest_arrays(self._h, *args, C.byref(idx)))
+        return idx.value
+
+    def forestCount(self):
+        k = C.c_int32(0)
+        self._check(self._L.kpl_forest_count(self._h, C.byref(k)))
+        return k.value
 
     def forestInfo(self):
         v = [C.c_int32() for _ in range(4)]
@@ -360,6 +391,73 @@ class KeypointLearningDetector:
         self._scores = scores
         self._kp_idx = keep[idx].astype(np.int32)
         return kp, self._kp_idx
+
+    def computeForests(self, thresholds=None):
+        """kpl_detect_forests: every forest of the set over the input cloud, from one feature pass.  thresholds: None (the
+        prediction threshold for every forest) or one per forest.  Returns a list with one (keypoints (n_kp,4) float32,
+        indices (n_kp,) int32) per forest -- what compute() returns with only that forest loaded and that threshold --
+        and keeps the (K, n) responses for getResponses().  A non-dense cloud is compacted and mapped back as in compute()."""
+        if self._cloud is None:
+            raise KplError(1, "no input cloud")
+        xyz, xs = _vec3(self._cloud, "cloud")
+        nrm = ns = None
+        if self._normals is not None:
+            nrm, ns = _vec3(self._normals, "normals")
+            if nrm.shape[0] != xyz.shape[0]:
+                raise KplError(3, "normals given, but the number of normals does not match the number of input points")
+        K = self.forestCount()
+        th = None if thresholds is None else np.ascontiguousarray(thresholds, np.float64)
+        if th is not None and th.shape != (K,):
+            raise ValueError("thresholds must hold one value per forest (%d)" % K)
+        self._push()
+        finite = None
+        scores, kp, kpo = self._detect_forests(xyz, xs, nrm, ns, th, K)
+        if scores is None:                            # KPL_E_NONFINITE: a non-dense cloud
+            finite = np.nonzero(np.isfinite(xyz[:, :3]).all(axis=1))[0]
+            sub = np.ascontiguousarray(xyz[finite])
+            subn = None if nrm is None else np.ascontiguousarray(nrm[finite])
+            sc, kp, kpo = self._detect_forests(sub, xs, subn, ns, th, K)
+            if sc is None:
+                self._check(4)
+            scores = np.full((K, xyz.shape[0]), np.nan, np.float32)
+            scores[:, finite] = sc
+        self._responses = scores
+        out = []
+        for k in range(K):
+            idx = kp[kpo[k]:kpo[k + 1]]
+            idx = (idx if finite is None else finite[idx]).astype(np.int32)
+            pts = np.empty((len(idx), 4), np.float32)
+            pts[:, :3] = xyz[idx, :3]
+            pts[:, 3] = scores[k, idx]
+            out.append((pts, idx))
+        return out
+
+    def _detect_forests(self, xyz, xs, nrm, ns, th, K):
+        n = xyz.shape[0]
+        scores = np.empty((K, n), np.float32)
+        kp = np.empty(max(K * n, 1), np.int32)
+        kpo = np.empty(K + 1, np.int64)
+        rc = self._L.kpl_detect_forests(self._h, _ptr(xyz, C.c_float), xs, _ptr(nrm, C.c_float), ns or 0, n, _ptr(th, C.c_double),
+                                        _ptr(scores, C.c_float), _ptr(kp, C.c_int32), _ptr(kpo, C.c_int64))
+        if rc == 4:
+            return None, None, None
+        self._check(rc)
+        return scores, kp, kpo
+
+    def getResponses(self):
+        """(K, n) responses of the last computeForests()."""
+        return self._responses
+
+    def detectForestsDevice(self, d_xyz4, n, d_normals4=0, thresholds=None, d_scores=0, d_kp_idx=0, d_kp_offsets=0):
+        """kpl_detect_forests_device: raw device pointers (ints); d_scores K*n floats (or 0), d_kp_idx K*n int32, d_kp_offsets
+        K + 1 int64, forest-major.  thresholds: None or one per forest (host).  Returns the keypoint count of all forests."""
+        th = None if thresholds is None else np.ascontiguousarray(thresholds, np.float64)
+        self._push()
+        nkp = C.c_int64(0)
+        self._check(self._L.kpl_detect_forests_device(self._h, C.c_void_p(d_xyz4), C.c_void_p(d_normals4 or None), int(n), _ptr(th, C.c_double),
+                                                      C.c_void_p(d_scores or None), C.c_void_p(d_kp_idx or None),
+                                                      C.c_void_p(d_kp_offsets or None), C.byref(nkp)))
+        return nkp.value
 
     def getKeypointsIndices(self): return self._kp_idx
     def getResponse(self): return self._scores

@@ -9,7 +9,6 @@
 
 namespace kpl {
 int pack_forest(const HostForestArrays& in, std::vector<PackedNode>& nodes, std::vector<int32_t>& roots, int& max_depth, int& max_var, std::string& err);
-cudaError_t launch_all_flags(kpl_ctx* c, int64_t n);
 }
 using namespace kpl;
 
@@ -40,6 +39,14 @@ static float dec_float(uint32_t u)
 
 template <typename T>
 static void release(DevBuf<T>& b) { if (b.p) cudaFree(b.p); b.p = nullptr; b.cap = 0; }
+
+static void free_forest_set(ForestSet& S)
+{
+    if (S.d_nodes) cudaFree(S.d_nodes);
+    if (S.d_roots) cudaFree(S.d_roots);
+    if (S.d_desc) cudaFree(S.d_desc);
+    S = ForestSet();
+}
 
 extern "C" {
 
@@ -126,6 +133,8 @@ void kpl_destroy(kpl_ctx* ctx)
     if (ctx->d_bbox) cudaFree(ctx->d_bbox);
     if (ctx->forest.d_nodes) cudaFree(ctx->forest.d_nodes);
     if (ctx->forest.d_roots) cudaFree(ctx->forest.d_roots);
+    free_forest_set(ctx->forests);
+    release(ctx->forest_off);
     for (int i = 0; i < 8; ++i) if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
     delete ctx;
@@ -167,16 +176,56 @@ int kpl_get_params(const kpl_ctx* ctx, kpl_params* p)
     return KPL_OK;
 }
 
-static int install_forest(kpl_ctx* ctx, const HostForestArrays& H)
+// Uploads a forest set (host arrays complete) and replaces ctx->forests with it; on failure ctx->forests is left as it was.
+static int upload_forest_set(kpl_ctx* ctx, ForestSet& S)
 {
-    std::vector<PackedNode> nodes;
-    std::vector<int32_t> roots;
+    S.d_nodes = nullptr; S.d_roots = nullptr; S.d_desc = nullptr;
+    cudaError_t e = cudaMalloc((void**)&S.d_nodes, S.nodes.size() * sizeof(PackedNode));
+    if (!e) e = cudaMalloc((void**)&S.d_roots, S.roots.size() * sizeof(int32_t));
+    if (!e) e = cudaMalloc((void**)&S.d_desc, S.desc.size() * sizeof(int2));
+    if (!e) e = cudaMemcpy(S.d_nodes, S.nodes.data(), S.nodes.size() * sizeof(PackedNode), cudaMemcpyHostToDevice);
+    if (!e) e = cudaMemcpy(S.d_roots, S.roots.data(), S.roots.size() * sizeof(int32_t), cudaMemcpyHostToDevice);
+    if (!e) e = cudaMemcpy(S.d_desc, S.desc.data(), S.desc.size() * sizeof(int2), cudaMemcpyHostToDevice);
+    if (e) {
+        cudaFree(S.d_nodes); cudaFree(S.d_roots); cudaFree(S.d_desc);
+        return fail(ctx, e == cudaErrorMemoryAllocation ? KPL_E_NOMEM : KPL_E_CUDA, std::string("forest set upload: ") + cudaGetErrorString(e));
+    }
+    free_forest_set(ctx->forests);
+    ctx->forests = std::move(S);
+    return KPL_OK;
+}
+
+// Appends a packed forest to a copy of the set: its roots shifted by the blocks already there (child offsets are relative)
+static void append_forest(ForestSet& S, const Forest& info, const std::vector<PackedNode>& nodes, const std::vector<int32_t>& roots)
+{
+    const int32_t shift = (int32_t)(S.nodes.size() / 4);
+    S.desc.push_back(make_int2((int)S.roots.size(), (int)roots.size()));
+    for (int32_t r : roots) S.roots.push_back(r + shift);
+    S.nodes.insert(S.nodes.end(), nodes.begin(), nodes.end());
+    S.info.push_back(info);
+}
+
+static int pack_checked(kpl_ctx* ctx, const HostForestArrays& H, std::vector<PackedNode>& nodes, std::vector<int32_t>& roots, Forest& info)
+{
     int max_depth = 0, max_var = -1;
     std::string err;
     int rc = pack_forest(H, nodes, roots, max_depth, max_var, err);
     if (rc) return fail(ctx, rc, err);
     if (roots.empty()) return fail(ctx, KPL_E_FOREST, "forest has no trees");
+    info.ntrees = (int32_t)roots.size(); info.nnodes = (int32_t)H.var.size(); info.var_count = H.var_count; info.max_depth = max_depth; info.max_var = max_var;
+    return KPL_OK;
+}
+
+static int install_forest(kpl_ctx* ctx, const HostForestArrays& H)
+{
+    std::vector<PackedNode> nodes;
+    std::vector<int32_t> roots;
+    Forest info;
+    int rc = pack_checked(ctx, H, nodes, roots, info);
+    if (rc) return rc;
     KPL_CUDA(cudaSetDevice(ctx->device));
+    // the forest set restarts with this forest alone: the old one goes first, so that no failure below leaves it behind
+    free_forest_set(ctx->forests);
     Forest& F = ctx->forest;
     if (F.d_nodes) cudaFree(F.d_nodes);
     if (F.d_roots) cudaFree(F.d_roots);
@@ -185,8 +234,28 @@ static int install_forest(kpl_ctx* ctx, const HostForestArrays& H)
     KPL_CUDA(cudaMalloc((void**)&F.d_roots, roots.size() * sizeof(int32_t)));
     KPL_CUDA(cudaMemcpy(F.d_nodes, nodes.data(), nodes.size() * sizeof(PackedNode), cudaMemcpyHostToDevice));
     KPL_CUDA(cudaMemcpy(F.d_roots, roots.data(), roots.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
-    F.ntrees = (int32_t)roots.size(); F.nnodes = (int32_t)H.var.size(); F.var_count = H.var_count; F.max_depth = max_depth; F.max_var = max_var;
+    F.ntrees = info.ntrees; F.nnodes = info.nnodes; F.var_count = info.var_count; F.max_depth = info.max_depth; F.max_var = info.max_var;
     F.roots = roots;
+    ForestSet S;
+    append_forest(S, info, nodes, roots);
+    return upload_forest_set(ctx, S);
+}
+
+static int add_forest(kpl_ctx* ctx, const HostForestArrays& H, int32_t* index_out)
+{
+    if (ctx->forest.ntrees < 1 || ctx->forests.info.empty()) return fail(ctx, KPL_E_FOREST, "no forest 0 loaded: kpl_load_forest / kpl_set_forest come first");
+    if ((int)ctx->forests.info.size() >= KPL_MAX_FORESTS) return fail(ctx, KPL_E_INVALID, "the forest set is full (KPL_MAX_FORESTS)");
+    std::vector<PackedNode> nodes;
+    std::vector<int32_t> roots;
+    Forest info;
+    int rc = pack_checked(ctx, H, nodes, roots, info);
+    if (rc) return rc;
+    KPL_CUDA(cudaSetDevice(ctx->device));
+    ForestSet S;
+    S.info = ctx->forests.info; S.nodes = ctx->forests.nodes; S.roots = ctx->forests.roots; S.desc = ctx->forests.desc;
+    append_forest(S, info, nodes, roots);
+    if ((rc = upload_forest_set(ctx, S))) return rc;
+    if (index_out) *index_out = (int32_t)ctx->forests.info.size() - 1;
     return KPL_OK;
 }
 
@@ -200,15 +269,45 @@ int kpl_load_forest(kpl_ctx* ctx, const char* path)
     return install_forest(ctx, H);
 }
 
-int kpl_set_forest(kpl_ctx* ctx, int32_t ntrees, int32_t nnodes, const int32_t* roots, const int32_t* var, const float* thr,
-                   const int32_t* left, const int32_t* right, const float* value, int32_t var_count)
+static HostForestArrays forest_arrays(int32_t ntrees, int32_t nnodes, const int32_t* roots, const int32_t* var, const float* thr,
+                                      const int32_t* left, const int32_t* right, const float* value, int32_t var_count)
 {
-    if (!ctx || ntrees < 1 || nnodes < 1 || !roots || !var || !thr || !left || !right || !value) return KPL_E_INVALID;
     HostForestArrays H;
     H.roots.assign(roots, roots + ntrees); H.var.assign(var, var + nnodes); H.thr.assign(thr, thr + nnodes);
     H.left.assign(left, left + nnodes); H.right.assign(right, right + nnodes); H.value.assign(value, value + nnodes);
     H.var_count = var_count;
-    return install_forest(ctx, H);
+    return H;
+}
+
+int kpl_set_forest(kpl_ctx* ctx, int32_t ntrees, int32_t nnodes, const int32_t* roots, const int32_t* var, const float* thr,
+                   const int32_t* left, const int32_t* right, const float* value, int32_t var_count)
+{
+    if (!ctx || ntrees < 1 || nnodes < 1 || !roots || !var || !thr || !left || !right || !value) return KPL_E_INVALID;
+    return install_forest(ctx, forest_arrays(ntrees, nnodes, roots, var, thr, left, right, value, var_count));
+}
+
+int kpl_add_forest(kpl_ctx* ctx, const char* path, int32_t* index_out)
+{
+    if (!ctx || !path) return KPL_E_INVALID;
+    HostForestArrays H;
+    std::string err;
+    int rc = parse_forest_yaml(path, H, err);
+    if (rc) return fail(ctx, rc, err);
+    return add_forest(ctx, H, index_out);
+}
+
+int kpl_add_forest_arrays(kpl_ctx* ctx, int32_t ntrees, int32_t nnodes, const int32_t* roots, const int32_t* var, const float* thr,
+                          const int32_t* left, const int32_t* right, const float* value, int32_t var_count, int32_t* index_out)
+{
+    if (!ctx || ntrees < 1 || nnodes < 1 || !roots || !var || !thr || !left || !right || !value) return KPL_E_INVALID;
+    return add_forest(ctx, forest_arrays(ntrees, nnodes, roots, var, thr, left, right, value, var_count), index_out);
+}
+
+int kpl_forest_count(const kpl_ctx* ctx, int32_t* count_out)
+{
+    if (!ctx || !count_out) return KPL_E_INVALID;
+    *count_out = ctx->forest.ntrees > 0 ? (int32_t)ctx->forests.info.size() : 0;
+    return KPL_OK;
 }
 
 int kpl_forest_info(const kpl_ctx* ctx, int32_t* ntrees, int32_t* nnodes, int32_t* var_count, int32_t* max_depth)
@@ -404,6 +503,7 @@ void kpl::detect_reset(kpl_ctx* ctx)
     ctx->syncs = 0;
     ctx->err.clear();
     ctx->last_has_normals = ctx->last_has_features = ctx->last_has_fragile = false;
+    ctx->last_nforests = 1;
     memset(&ctx->timings, 0, sizeof ctx->timings);
     memset(&ctx->stats, 0, sizeof ctx->stats);
     ctx->stats.n_views = 1;
@@ -429,7 +529,7 @@ int detect_check(kpl_ctx* ctx, int64_t n, bool with_role)
 
 // Phase A of a detection: grid (already built by the caller), normals, features + forest -> scores of every point
 // whose role asks for one.  Events 1..4 bracket the stages.
-int detect_score_phase(kpl_ctx* ctx, bool normals_given, bool use_role, int64_t n)
+int detect_score_phase(kpl_ctx* ctx, bool normals_given, bool use_role, int64_t n, bool forest_set)
 {
     const kpl_params& P = ctx->params;
     const int F = P.n_annulus * P.n_bins;
@@ -445,7 +545,7 @@ int detect_score_phase(kpl_ctx* ctx, bool normals_given, bool use_role, int64_t 
     fuse = getenv("KPL_NO_FUSE") == nullptr;
 #endif
     const bool rows = ctx->keep_intermediates || !fuse;
-    KPL_CUDA(launch_features(ctx, n, use_role, fuse, rows));
+    KPL_CUDA(launch_features(ctx, n, use_role, fuse, rows, nullptr, 0, forest_set));
     ctx->last_has_features = rows; ctx->last_F = F;
     ctx->last_has_fragile = fuse && P.report_fragile != 0;
     KPL_CUDA(cudaEventRecord(ctx->ev[3], ctx->stream));
@@ -456,13 +556,22 @@ int detect_score_phase(kpl_ctx* ctx, bool normals_given, bool use_role, int64_t 
     return KPL_OK;
 }
 
+// Threshold + NMS of forest k's scores (slice k of the forest-major scores) into slice k of the keypoint flags.
+static int nms_flags(kpl_ctx* ctx, bool use_role, int64_t n, int k, double th)
+{
+    const kpl_params& P = ctx->params;
+    const int64_t off = (int64_t)k * n;
+    if (P.non_maxima && P.draws_remove) KPL_CUDA(launch_nms_draws(ctx, n, use_role, ctx->s_score.p + off, th, off));
+    else if (P.non_maxima) KPL_CUDA(launch_nms(ctx, n, use_role, ctx->s_score.p + off, th, off));
+    else KPL_CUDA(launch_all_flags(ctx, n, ctx->score.p + off, off));
+    return KPL_OK;
+}
+
 // Phase B: threshold + NMS over the scores in place, ascending keypoint indices into d_kp_out.
 int detect_nms_phase(kpl_ctx* ctx, bool use_role, int64_t n, int32_t* d_kp_out)
 {
-    const kpl_params& P = ctx->params;
-    if (P.non_maxima && P.draws_remove) KPL_CUDA(launch_nms_draws(ctx, n, use_role));
-    else if (P.non_maxima) KPL_CUDA(launch_nms(ctx, n, use_role));
-    else KPL_CUDA(launch_all_flags(ctx, n));
+    int rc = nms_flags(ctx, use_role, n, 0, ctx->params.threshold);
+    if (rc) return rc;
     KPL_CUDA(launch_compact(ctx, n, d_kp_out));
     return KPL_OK;
 }
@@ -527,6 +636,61 @@ static int run_detect(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, co
     if ((rc = detect_score_phase(ctx, d_nrm != nullptr, d_role != nullptr, n))) return rc;
     if ((rc = detect_nms_phase(ctx, d_role != nullptr, n, d_kp_out))) return rc;
     if (d_scores_out) KPL_CUDA(cudaMemcpyAsync(d_scores_out, ctx->score.p, (size_t)n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
+    return detect_finish(ctx, n, n_kp_out);
+}
+
+// Every forest of the set over ONE cloud: one grid, one normal estimation, one feature pass whose tail walks the K forests,
+// then threshold + NMS of each forest's slice (forest-major K x n scores and flags), one compaction of the K x n flags into
+// an ascending list and its split at the forest boundaries k*n by launch_view_ranges.  No host round trip beyond those of
+// run_detect (and one per draws-remove round of each forest).
+static int check_forest_set(kpl_ctx* ctx, int64_t n)
+{
+    const ForestSet& S = ctx->forests;
+    if (ctx->forest.ntrees < 1 || S.info.empty()) return fail(ctx, KPL_E_FOREST, "no forest loaded");
+    const int F = ctx->params.n_annulus * ctx->params.n_bins;
+    for (size_t k = 0; k < S.info.size(); ++k) {
+        char b[160];
+        if (S.info[k].var_count > 0 && S.info[k].var_count != F) {
+            snprintf(b, sizeof b, "annuli*bins does not match the var_count of forest %zu", k);
+            return fail(ctx, KPL_E_VARCOUNT, b);
+        }
+        if (S.info[k].max_var >= F) {
+            snprintf(b, sizeof b, "forest %zu splits on a variable index >= annuli*bins", k);
+            return fail(ctx, KPL_E_VARCOUNT, b);
+        }
+    }
+    if (n > 0 && (int64_t)S.info.size() * n > 2147483000ll) return fail(ctx, KPL_E_INVALID, "forest count x point count out of range");
+    return KPL_OK;
+}
+
+static int run_detect_forests(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, int64_t n, const double* thresholds,
+                              float* d_scores_out, int32_t* d_kp_out, int64_t* d_kp_offsets_out, int64_t* n_kp_out)
+{
+    detect_reset(ctx);
+    if (n_kp_out) *n_kp_out = 0;
+    int rc = check_forest_set(ctx, n);
+    if (rc || (rc = detect_check(ctx, n, false))) return rc;
+    const int K = (int)ctx->forests.info.size();
+    ctx->stats.n_points = n;
+    ctx->last_nforests = K;
+    if (n == 0) {
+        KPL_CUDA(cudaMemsetAsync(d_kp_offsets_out, 0, ((size_t)K + 1) * sizeof(int64_t), ctx->stream));
+        return KPL_OK;
+    }
+    if ((rc = detect_begin(ctx))) return rc;
+    if ((rc = prepare_params_grid(ctx, d_xyz, d_nrm, nullptr, n))) return rc;
+    if ((rc = detect_score_phase(ctx, d_nrm != nullptr, false, n, true))) return rc;
+    KPL_CUDA(ensure(ctx->flag, (size_t)K * n));
+    for (int k = 0; k < K; ++k)
+        if ((rc = nms_flags(ctx, false, n, k, thresholds ? thresholds[k] : ctx->params.threshold))) return rc;
+    KPL_CUDA(launch_compact(ctx, (int64_t)K * n, d_kp_out));
+    // the forest boundaries; a pageable source is staged by cudaMemcpyAsync before it returns, the member keeps it anyway
+    ctx->forest_off_h.resize((size_t)K + 1);
+    for (int k = 0; k <= K; ++k) ctx->forest_off_h[(size_t)k] = (int64_t)k * n;
+    KPL_CUDA(ensure(ctx->forest_off, (size_t)K + 1));
+    KPL_CUDA(cudaMemcpyAsync(ctx->forest_off.p, ctx->forest_off_h.data(), ((size_t)K + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
+    KPL_CUDA(launch_view_ranges(ctx, (int64_t)K * n, d_kp_out, ctx->forest_off.p, K, d_kp_offsets_out));
+    if (d_scores_out) KPL_CUDA(cudaMemcpyAsync(d_scores_out, ctx->score.p, (size_t)K * n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
     return detect_finish(ctx, n, n_kp_out);
 }
 
@@ -681,6 +845,38 @@ int kpl_detect_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, 
     if (n > 0 && (!d_xyz4 || !d_kp_idx)) return fail(ctx, KPL_E_INVALID, "NULL device pointer");
     return run_detect(ctx, (const float4*)d_xyz4, (const float4*)d_normals4, (const uint8_t*)d_role, n, (float*)d_scores,
                       (int32_t*)d_kp_idx, n_kp_out);
+}
+
+int kpl_detect_forests(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride, int64_t n,
+                       const double* thresholds, float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out)
+{
+    if (!ctx) return KPL_E_INVALID;
+    if (!kp_idx_out || !kp_offsets_out) return fail(ctx, KPL_E_INVALID, "kp_idx_out / kp_offsets_out is NULL");
+    int rc = upload_inputs(ctx, xyz, xyz_stride, normals, normals_stride, nullptr, n);
+    if (rc) return rc;
+    const size_t K = ctx->forests.info.size();
+    KPL_CUDA(ensure(ctx->kp_idx, std::max<size_t>(K * (size_t)std::max<int64_t>(n, 0), 1)));
+    KPL_CUDA(ensure(ctx->scratch_f, 2 * (K + 1) + 16));
+    int64_t* d_kp_off = reinterpret_cast<int64_t*>(ctx->scratch_f.p);
+    int64_t nkp = 0;
+    rc = run_detect_forests(ctx, ctx->in_xyz.p, normals ? ctx->in_nrm.p : nullptr, n, thresholds, nullptr, ctx->kp_idx.p, d_kp_off, &nkp);
+    if (rc) return rc;
+    if (n > 0 && scores_out) KPL_CUDA(cudaMemcpyAsync(scores_out, ctx->score.p, K * (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    if (nkp > 0) KPL_CUDA(cudaMemcpyAsync(kp_idx_out, ctx->kp_idx.p, (size_t)nkp * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    KPL_CUDA(cudaMemcpyAsync(kp_offsets_out, d_kp_off, (K + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    KPL_CUDA(cudaStreamSynchronize(ctx->stream));
+    ctx->syncs++; ctx->stats.host_syncs = ctx->syncs;
+    return KPL_OK;
+}
+
+int kpl_detect_forests_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, int64_t n, const double* thresholds,
+                              void* d_scores, void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out)
+{
+    if (!ctx) return KPL_E_INVALID;
+    if (!d_kp_idx || !d_kp_offsets || (n > 0 && !d_xyz4)) return fail(ctx, KPL_E_INVALID, "NULL device pointer");
+    KPL_CUDA(cudaSetDevice(ctx->device));
+    return run_detect_forests(ctx, (const float4*)d_xyz4, (const float4*)d_normals4, n, thresholds, (float*)d_scores, (int32_t*)d_kp_idx,
+                              (int64_t*)d_kp_offsets, n_kp_out);
 }
 
 // Forced grids skip the bounding-box round trip (prepare_grid): entry points other than kpl_detect* read the
@@ -1054,11 +1250,12 @@ int kpl_fetch_u8(kpl_ctx* ctx, const char* what, uint8_t* out, int64_t capacity)
     const int64_t n = ctx->last_n;
     if (n <= 0) return fail(ctx, KPL_E_INVALID, "nothing to fetch");
     if (strcmp(what, "fragile")) return fail(ctx, KPL_E_INVALID, "unknown fetch target");
-    if (capacity < n) return fail(ctx, KPL_E_INVALID, "fetch buffer too small");
-    if (!ctx->last_has_fragile || ctx->fragile.cap < (size_t)n)
+    const int64_t bytes = n * ctx->last_nforests;         // forest-major after kpl_detect_forests
+    if (capacity < bytes) return fail(ctx, KPL_E_INVALID, "fetch buffer too small");
+    if (!ctx->last_has_fragile || ctx->fragile.cap < (size_t)bytes)
         return fail(ctx, KPL_E_INVALID, "the last call did not report fragile splits (kpl_params.report_fragile)");
     KPL_CUDA(cudaSetDevice(ctx->device));
-    KPL_CUDA(cudaMemcpyAsync(out, ctx->fragile.p, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    KPL_CUDA(cudaMemcpyAsync(out, ctx->fragile.p, (size_t)bytes, cudaMemcpyDeviceToHost, ctx->stream));
     KPL_CUDA(cudaStreamSynchronize(ctx->stream));
     return KPL_OK;
 }

@@ -64,6 +64,19 @@ struct Forest {
     int32_t* d_roots = nullptr;
 };
 
+// The forest set of kpl_detect_forests: forest 0 (a copy of kpl_ctx::forest) and the added ones, concatenated into one
+// node array.  pack_forest's child offsets are relative, so a forest moves by shifting its roots by the blocks before it;
+// desc[k] = (first root of forest k, its tree count).
+struct ForestSet {
+    std::vector<Forest> info;             // per forest: ntrees, nnodes, var_count, max_depth, max_var (device pointers unused)
+    std::vector<PackedNode> nodes;        // host copy of the concatenation
+    std::vector<int32_t> roots;           // shifted roots, forest after forest
+    std::vector<int2> desc;
+    PackedNode* d_nodes = nullptr;
+    int32_t* d_roots = nullptr;
+    int2* d_desc = nullptr;
+};
+
 template <typename T>
 struct DevBuf {
     T* p = nullptr;
@@ -87,6 +100,7 @@ struct kpl_ctx {
     cudaStream_t stream = nullptr;
     kpl_params params;
     kpl::Forest forest;
+    kpl::ForestSet forests;                      // kpl_detect_forests: forest 0 + kpl_add_forest*
     kpl::GridDesc grid;
     kpl_timings timings;
     kpl_stats stats;
@@ -116,6 +130,10 @@ struct kpl_ctx {
     kpl::DevBuf<float> s_score, score;           // sorted order / original order
     kpl::DevBuf<uint8_t> flag;                   // keypoint flag, original order
     kpl::DevBuf<uint8_t> fragile;                // near-split flag of the forest walk, original order (forest.cuh)
+    // kpl_detect_forests: scores, flags and fragile flags hold K x n entries, forest-major; forest_off = {0, n, .., K*n}
+    // (host copy kept for the asynchronous upload)
+    kpl::DevBuf<int64_t> forest_off;
+    std::vector<int64_t> forest_off_h;
     kpl::DevBuf<kpl::ViewDesc> views;            // kpl_detect_batch: per-view grids
     kpl::DevBuf<int32_t> layer_view;
     kpl::DevBuf<int64_t> view_offsets;
@@ -142,6 +160,7 @@ struct kpl_ctx {
     float* d_bbox = nullptr;                     // 6 ordered-int encoded floats + flags
     int64_t last_n = 0;
     int last_F = 0;
+    int last_nforests = 1;                       // forests scored by the last call (the fragile mask holds last_nforests x n bytes)
     bool last_has_normals = false, last_has_features = false, last_has_fragile = false;
     bool fast_math = false;                      // feature kernel variant chosen by the arithmetic self-test
     bool keep_intermediates = false;             // kpl_set_keep_intermediates: materialise feature rows in kpl_detect*
@@ -177,18 +196,24 @@ cudaError_t build_query_list(kpl_ctx* c, int64_t n, const int32_t* d_indices, in
 cudaError_t launch_scatter_rows(kpl_ctx* c, const float* d_rows, int64_t m, int width, float* d_out);
 cudaError_t launch_view_ranges(kpl_ctx* c, int64_t n, int32_t* d_kp_idx, const int64_t* d_view_offsets, int nviews, int64_t* d_kp_offsets);
 cudaError_t launch_bbox_views(kpl_ctx* c, const float4* xyz, int64_t n, const int64_t* d_view_offsets, int nviews, uint32_t* d_bbox);
-// qlist != nullptr: features of the m_list listed sorted positions only (rows in list order, c->feat holds m_list x F)
-cudaError_t launch_features(kpl_ctx* c, int64_t n, bool use_role, bool fuse_forest, bool store_rows, const int32_t* d_qlist = nullptr, int64_t m_list = 0);
+// qlist != nullptr: features of the m_list listed sorted positions only (rows in list order, c->feat holds m_list x F).
+// forest_set: the fused tail scores every forest of c->forests (kpl_detect_forests) instead of forest 0.
+cudaError_t launch_features(kpl_ctx* c, int64_t n, bool use_role, bool fuse_forest, bool store_rows, const int32_t* d_qlist = nullptr, int64_t m_list = 0,
+                            bool forest_set = false);
 #ifdef KPL_EXPERIMENTS
 cudaError_t launch_forest(kpl_ctx* c, int64_t n, bool use_role);
 #endif
-cudaError_t launch_nms(kpl_ctx* c, int64_t n, bool use_role);
-cudaError_t launch_nms_draws(kpl_ctx* c, int64_t n, bool use_role);
+// Threshold + NMS of one forest's n sorted scores s_score (th compared in double); the keypoint flags (original order) go to
+// c->flag.p + flag_off.  kpl_detect* pass c->s_score.p, params.threshold and 0; kpl_detect_forests forest k's slice.
+cudaError_t launch_nms(kpl_ctx* c, int64_t n, bool use_role, const float* s_score, double th, int64_t flag_off);
+cudaError_t launch_nms_draws(kpl_ctx* c, int64_t n, bool use_role, const float* s_score, double th, int64_t flag_off);
 // the pieces of launch_nms_draws, for a caller that exchanges halo states between rounds (shard.cu); gidx: global index of
 // every local original index (nullptr: the identity)
-cudaError_t launch_nms_draws_classify(kpl_ctx* c, int64_t n, bool use_role);
-cudaError_t launch_nms_draws_round(kpl_ctx* c, int64_t n, bool use_role, const int32_t* gidx);
-cudaError_t launch_nms_draws_flags(kpl_ctx* c, int64_t n, bool use_role);
+cudaError_t launch_nms_draws_classify(kpl_ctx* c, int64_t n, bool use_role, const float* s_score, double th);
+cudaError_t launch_nms_draws_round(kpl_ctx* c, int64_t n, bool use_role, const int32_t* gidx, const float* s_score, double th);
+cudaError_t launch_nms_draws_flags(kpl_ctx* c, int64_t n, bool use_role, int64_t flag_off);
+// setNonMaxima(false): every scored point of the n original-order scores is a keypoint
+cudaError_t launch_all_flags(kpl_ctx* c, int64_t n, const float* score, int64_t flag_off);
 // resolution rounds of a cloud of n points never exceed this cap (the lowest undecided index resolves in every round)
 inline int nms_round_cap(int64_t n) { return (int)(n < (1 << 20) ? n : (1 << 20)); }
 cudaError_t launch_compact(kpl_ctx* c, int64_t n, int32_t* d_kp_idx_out);
@@ -215,7 +240,8 @@ int detect_check(kpl_ctx* ctx, int64_t n, bool with_role);
 int detect_begin(kpl_ctx* ctx);
 // forced == nullptr: the canonical grid of the cloud's bounding box; cell_override > 0 replaces the canonical cell
 int prepare_grid(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, const uint8_t* d_role, int64_t n, const ForcedGrid* forced, double cell_override = 0.0);
-int detect_score_phase(kpl_ctx* ctx, bool normals_given, bool use_role, int64_t n);
+// forest_set: score with every forest of ctx->forests (kpl_detect_forests)
+int detect_score_phase(kpl_ctx* ctx, bool normals_given, bool use_role, int64_t n, bool forest_set = false);
 int detect_nms_phase(kpl_ctx* ctx, bool use_role, int64_t n, int32_t* d_kp_out);
 int detect_finish(kpl_ctx* ctx, int64_t n, int64_t* n_kp_out);
 

@@ -57,16 +57,16 @@ nms_kernel(const float4* __restrict__ s_pos, const float* __restrict__ s_score, 
     if ((threadIdx.x & 31) == 0 && m) atomicAdd(counters + 7, (unsigned long long)__popc(m));
 }
 
-cudaError_t launch_nms(kpl_ctx* c, int64_t n, bool use_role)
+cudaError_t launch_nms(kpl_ctx* c, int64_t n, bool use_role, const float* s_score, double th, int64_t flag_off)
 {
     const kpl_params& U = c->params;
     cudaError_t e;
-    if ((e = ensure(c->flag, n))) return e;
+    if ((e = ensure(c->flag, (size_t)(flag_off + n)))) return e;
     const double rn = (double)U.radius_nms;
-    nms_kernel<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(c->s_pos.p, c->s_score.p, c->key_b.p, c->cell_start.p,
+    nms_kernel<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(c->s_pos.p, s_score, c->key_b.p, c->cell_start.p,
                                                                    use_role ? c->s_role.p : nullptr,
                                                                    c->grid.dim[0], c->grid.dim[1], c->grid.dim[2], (int)n,
-                                                                   (float)(rn * rn), c->grid.reach_nms, U.threshold, c->flag.p, c->counters.p);
+                                                                   (float)(rn * rn), c->grid.reach_nms, th, c->flag.p + flag_off, c->counters.p);
     c->launches++;
     return cudaGetLastError();
 }
@@ -169,59 +169,61 @@ __global__ void __launch_bounds__(256) state_to_flag_kernel(const float4* __rest
     if (i < n) flag[__float_as_uint(__ldg(&s_pos[i].w))] = s_state[i] == 1 && (!s_role || (s_role[i] & 3) == 3) ? 1 : 0;
 }
 
-cudaError_t launch_nms_draws_classify(kpl_ctx* c, int64_t n, bool use_role)
+cudaError_t launch_nms_draws_classify(kpl_ctx* c, int64_t n, bool use_role, const float* s_score, double th)
 {
     const kpl_params& U = c->params;
     cudaError_t e;
     if ((e = ensure(c->flag, n)) || (e = ensure(c->s_state, n))) return e;
     const double rn = (double)U.radius_nms;
-    nms_draws_kernel<0><<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(c->s_pos.p, c->s_score.p, c->key_b.p, c->cell_start.p,
+    nms_draws_kernel<0><<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(c->s_pos.p, s_score, c->key_b.p, c->cell_start.p,
                                                                               use_role ? c->s_role.p : nullptr, c->grid.dim[0], c->grid.dim[1],
                                                                               c->grid.dim[2], (int)n, (float)(rn * rn), c->grid.reach_nms,
-                                                                              U.threshold, U.draws_threshold, nullptr, c->s_state.p, c->counters.p);
+                                                                              th, U.draws_threshold, nullptr, c->s_state.p, c->counters.p);
     c->launches++;
     return cudaGetLastError();
 }
 
 // one resolution round; counters[6] = candidates left undecided by it
-cudaError_t launch_nms_draws_round(kpl_ctx* c, int64_t n, bool use_role, const int32_t* gidx)
+cudaError_t launch_nms_draws_round(kpl_ctx* c, int64_t n, bool use_role, const int32_t* gidx, const float* s_score, double th)
 {
     const kpl_params& U = c->params;
     cudaError_t e;
     if ((e = cudaMemsetAsync(c->counters.p + 6, 0, sizeof(unsigned long long), c->stream))) return e;
     const double rn = (double)U.radius_nms;
-    nms_draws_kernel<1><<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(c->s_pos.p, c->s_score.p, c->key_b.p, c->cell_start.p,
+    nms_draws_kernel<1><<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(c->s_pos.p, s_score, c->key_b.p, c->cell_start.p,
                                                                               use_role ? c->s_role.p : nullptr, c->grid.dim[0], c->grid.dim[1],
                                                                               c->grid.dim[2], (int)n, (float)(rn * rn), c->grid.reach_nms,
-                                                                              U.threshold, U.draws_threshold, gidx, c->s_state.p, c->counters.p);
+                                                                              th, U.draws_threshold, gidx, c->s_state.p, c->counters.p);
     c->launches++;
     c->stats.nms_rounds++;
     return cudaGetLastError();
 }
 
-cudaError_t launch_nms_draws_flags(kpl_ctx* c, int64_t n, bool use_role)
+cudaError_t launch_nms_draws_flags(kpl_ctx* c, int64_t n, bool use_role, int64_t flag_off)
 {
+    cudaError_t e;
+    if ((e = ensure(c->flag, (size_t)(flag_off + n)))) return e;
     state_to_flag_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(c->s_pos.p, use_role ? c->s_role.p : nullptr, c->s_state.p,
-                                                                            (int)n, c->flag.p);
+                                                                            (int)n, c->flag.p + flag_off);
     c->launches++;
     return cudaGetLastError();
 }
 
 // A whole cloud, or a batch of views: each view is a connected component of its own (§5.4 padding layers) that keeps its
 // own index order inside the concatenation, so the rounds over the stacked grid resolve every view at once.
-cudaError_t launch_nms_draws(kpl_ctx* c, int64_t n, bool use_role)
+cudaError_t launch_nms_draws(kpl_ctx* c, int64_t n, bool use_role, const float* s_score, double th, int64_t flag_off)
 {
     cudaError_t e;
-    if ((e = launch_nms_draws_classify(c, n, use_role))) return e;
+    if ((e = launch_nms_draws_classify(c, n, use_role, s_score, th))) return e;
     for (int round = 0; round < nms_round_cap(n); ++round) {
-        if ((e = launch_nms_draws_round(c, n, use_role, nullptr))) return e;
+        if ((e = launch_nms_draws_round(c, n, use_role, nullptr, s_score, th))) return e;
         unsigned long long undecided = 0;
         if ((e = cudaMemcpyAsync(&undecided, c->counters.p + 6, sizeof undecided, cudaMemcpyDeviceToHost, c->stream))) return e;
         if ((e = cudaStreamSynchronize(c->stream))) return e;
         c->syncs++;
         if (undecided == 0) break;
     }
-    return launch_nms_draws_flags(c, n, use_role);
+    return launch_nms_draws_flags(c, n, use_role, flag_off);
 }
 
 // setNonMaxima(false) (hpp:189-196): every scored point is a keypoint.
@@ -230,11 +232,11 @@ __global__ void __launch_bounds__(256) all_flags_kernel(const float* __restrict_
     int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i < n) flag[i] = isnan(score[i]) ? 0 : 1;
 }
-cudaError_t launch_all_flags(kpl_ctx* c, int64_t n)
+cudaError_t launch_all_flags(kpl_ctx* c, int64_t n, const float* score, int64_t flag_off)
 {
     cudaError_t e;
-    if ((e = ensure(c->flag, n))) return e;
-    all_flags_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(c->score.p, n, c->flag.p);
+    if ((e = ensure(c->flag, (size_t)(flag_off + n)))) return e;
+    all_flags_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(score, n, c->flag.p + flag_off);
     c->launches++;
     return cudaGetLastError();
 }

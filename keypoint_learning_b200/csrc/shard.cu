@@ -426,7 +426,7 @@ int phase_nms(kpl_shard* s)
         halo_scores_kernel<<<(unsigned)((s->n_loc + 255) / 256), 256, 0, c->stream>>>(c->s_pos.p, c->s_role.p, c->score.p, s->n_loc, c->s_score.p);
     c->launches++;
     if (draws_remove(c)) {
-        KS_CUDA(launch_nms_draws_classify(c, s->n_loc, true));
+        KS_CUDA(launch_nms_draws_classify(c, s->n_loc, true, c->s_score.p, c->params.threshold));
         return pack_states(s);
     }
     int rc = detect_nms_phase(c, true, s->n_loc, s->kp_local.p);
@@ -443,7 +443,7 @@ int phase_draws_round(kpl_shard* s)
         KS_CUDA(cudaGetLastError());
         c->launches++;
     }
-    KS_CUDA(launch_nms_draws_round(c, s->n_loc, true, s->loc_gidx.p));
+    KS_CUDA(launch_nms_draws_round(c, s->n_loc, true, s->loc_gidx.p, c->s_score.p, c->params.threshold));
     if (s->in_process)      // read by the host after the next exchange, which synchronises every stream of the group
         KS_CUDA(cudaMemcpyAsync(&s->h_undecided, c->counters.p + 6, sizeof s->h_undecided, cudaMemcpyDeviceToHost, c->stream));
     return pack_states(s);
@@ -483,7 +483,7 @@ int phase_draws_keypoints(kpl_shard* s)
     kpl_ctx* c = s->ctx;
     if (!draws_remove(c)) return KPL_OK;
     KS_CUDA(cudaSetDevice(c->device));
-    KS_CUDA(launch_nms_draws_flags(c, s->n_loc, true));
+    KS_CUDA(launch_nms_draws_flags(c, s->n_loc, true, 0));
     KS_CUDA(launch_compact(c, s->n_loc, s->kp_local.p));
     return phase_records(s);
 }

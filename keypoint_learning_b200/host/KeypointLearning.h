@@ -94,6 +94,16 @@ public:
         kpl_forest_info(ctx_, &ntrees, nullptr, nullptr, nullptr);
         return ntrees != 0;
     }
+    // B200 build only: appends a forest to the set computeForests() scores (loadForest's forest is forest 0 and drops the others)
+    bool addForest(const std::string& path)
+    {
+        if (!ctx_) return false;
+        if (kpl_add_forest(ctx_, path.c_str(), nullptr) != KPL_OK) {
+            std::fprintf(stderr, "[pcl::%s::addForest] impossible to load random forest with path %s (%s)\n", name_.c_str(), path.c_str(), kpl_last_error(ctx_));
+            return false;
+        }
+        return true;
+    }
 
     // pcl::Keypoint::compute -> initCompute / detectKeypoints (impl/KeypointLearning.hpp:116-156,179-263)
     void compute(PointCloudOut& output)
@@ -106,33 +116,20 @@ public:
         if (response_.size() != (size_t)n) response_.resize((size_t)n);
         std::unique_ptr<int32_t[]> idx(new int32_t[(size_t)std::max<int64_t>(n, 1)]);
         int64_t nkp = 0;
-        const float* nrm = normals_ ? reinterpret_cast<const float*>(normals_->points.data()) : nullptr;
         std::unique_ptr<float[]> xyzi(new float[(size_t)std::max<int64_t>(n, 1) * 4]);   // keypoint cloud, gathered on the device
-        int rc = kpl_detect_xyzi(ctx_, reinterpret_cast<const float*>(input_->points.data()), (int32_t)sizeof(PointInT), nrm, (int32_t)sizeof(NormalT),
-                                 nullptr, n, response_.data(), idx.get(), xyzi.get(), &nkp);
-        if (rc == KPL_E_NONFINITE) {
-            // Non-dense clouds (Kinect / organized PCDs carry NaN points; found by the device's bounding-box pass): the
-            // reference's kd-tree ignores them and runForest skips them (hpp:277).  The finite points are compacted,
-            // detected, and the results mapped back; a skipped point has a NaN response and is never a keypoint.
-            std::vector<int32_t> finite;
-            for (int64_t i = 0; i < n; ++i)
-                if (pcl::isFinite(input_->points[(size_t)i])) finite.push_back((int32_t)i);
-            const int64_t m = (int64_t)finite.size();
-            std::vector<PointInT> pts((size_t)m);
-            std::vector<NormalT> nrs(normals_ ? (size_t)m : 0);
-            for (int64_t k = 0; k < m; ++k) {
-                pts[(size_t)k] = input_->points[(size_t)finite[(size_t)k]];
-                if (normals_) nrs[(size_t)k] = normals_->points[(size_t)finite[(size_t)k]];
-            }
-            std::vector<float> sc((size_t)std::max<int64_t>(m, 1));
-            rc = kpl_detect_xyzi(ctx_, reinterpret_cast<const float*>(pts.data()), (int32_t)sizeof(PointInT),
-                                 normals_ ? reinterpret_cast<const float*>(nrs.data()) : nullptr, (int32_t)sizeof(NormalT), nullptr, m, sc.data(), idx.get(),
-                                 xyzi.get(), &nkp);
-            if (rc == KPL_OK) {
-                response_.assign((size_t)n, std::nanf(""));
-                for (int64_t k = 0; k < m; ++k) response_[(size_t)finite[(size_t)k]] = sc[(size_t)k];
-                for (int64_t k = 0; k < nkp; ++k) idx[(size_t)k] = finite[(size_t)idx[(size_t)k]];
-            }
+        std::vector<int32_t> finite;
+        std::vector<float> sc;
+        bool compacted = false;
+        int rc = detectFinite([&](const PointInT* pts, const float* nrm, int64_t m) {
+            float* scores = response_.data();
+            if (compacted) { sc.resize((size_t)std::max<int64_t>(m, 1)); scores = sc.data(); }
+            return kpl_detect_xyzi(ctx_, reinterpret_cast<const float*>(pts), (int32_t)sizeof(PointInT), nrm, (int32_t)sizeof(NormalT), nullptr, m,
+                                   scores, idx.get(), xyzi.get(), &nkp);
+        }, finite, compacted);
+        if (rc == KPL_OK && compacted) {
+            response_.assign((size_t)n, std::nanf(""));
+            for (size_t k = 0; k < finite.size(); ++k) response_[(size_t)finite[k]] = sc[k];
+            for (int64_t k = 0; k < nkp; ++k) idx[(size_t)k] = finite[(size_t)idx[(size_t)k]];
         }
         if (rc != KPL_OK) {
             std::fprintf(stderr, "[pcl::%s::compute] %s\n", name_.c_str(), kpl_last_error(ctx_));
@@ -151,6 +148,59 @@ public:
         output.is_dense = p_.non_maxima ? true : input_->is_dense;               // hpp:192-193,258-260
     }
     pcl::PointIndicesConstPtr getKeypointsIndices() const { return keypoints_indices_; }
+
+    // B200 build only: every forest of the set (loadForest + addForest) over the input cloud from one feature pass
+    // (kpl_detect_forests).  outputs[k] is what compute() returns with only forest k loaded, at threshold (*thresholds)[k]
+    // (default: the prediction threshold); (*indices)[k], when asked for, its keypoint indices.  Non-dense clouds and the
+    // initCompute checks are handled as in compute().  The detector's response and keypoint indices are left as they are.
+    bool computeForests(std::vector<PointCloudOut>& outputs, std::vector<pcl::PointIndices>* indices = nullptr,
+                        const std::vector<double>* thresholds = nullptr)
+    {
+        outputs.clear();
+        if (indices) indices->clear();
+        if (!initCompute()) return false;
+        int32_t K = 0;
+        kpl_forest_count(ctx_, &K);
+        if (thresholds && thresholds->size() != (size_t)K) {
+            std::fprintf(stderr, "[pcl::%s::computeForests] %zu thresholds for %d forests\n", name_.c_str(), thresholds->size(), K);
+            return false;
+        }
+        std::vector<float> scores;
+        std::vector<int32_t> idx, finite;
+        std::vector<int64_t> off((size_t)K + 1);
+        bool compacted = false;
+        int rc = detectFinite([&](const PointInT* pts, const float* nrm, int64_t m) {
+            scores.resize((size_t)K * (size_t)std::max<int64_t>(m, 1));
+            idx.resize((size_t)K * (size_t)std::max<int64_t>(m, 1));
+            return kpl_detect_forests(ctx_, reinterpret_cast<const float*>(pts), (int32_t)sizeof(PointInT), nrm, (int32_t)sizeof(NormalT), m,
+                                      thresholds ? thresholds->data() : nullptr, scores.data(), idx.data(), off.data());
+        }, finite, compacted);
+        if (rc != KPL_OK) {
+            std::fprintf(stderr, "[pcl::%s::compute] %s\n", name_.c_str(), kpl_last_error(ctx_));
+            return false;
+        }
+        const size_t m = compacted ? finite.size() : input_->size();
+        outputs.assign((size_t)K, PointCloudOut());
+        if (indices) indices->assign((size_t)K, pcl::PointIndices());
+        for (size_t k = 0; k < (size_t)K; ++k) {
+            PointCloudOut& out = outputs[k];
+            out.points.reserve((size_t)(off[k + 1] - off[k]));
+            for (int64_t j = off[k]; j < off[k + 1]; ++j) {                     // hpp:246-253
+                const int32_t local = idx[(size_t)j];
+                const int32_t i = compacted ? finite[(size_t)local] : local;
+                const PointInT& p = input_->points[(size_t)i];
+                PointOutT o;
+                o.x = p.x; o.y = p.y; o.z = p.z;
+                o.intensity = scores[k * m + (size_t)local];
+                out.points.push_back(o);
+                if (indices) (*indices)[k].indices.push_back(i);
+            }
+            out.height = 1;
+            out.width = (uint32_t)out.points.size();
+            out.is_dense = p_.non_maxima ? true : input_->is_dense;             // hpp:192-193,258-260
+        }
+        return true;
+    }
     const std::vector<float>& getResponse() const { return response_; }          // the `response` cloud's intensities (hpp:181-187)
 
     // impl/KeypointLearning.hpp:299-318 (cv::Mat -> KplFeatureMatrix)
@@ -229,6 +279,31 @@ public:
     kpl_ctx* context() { return ctx_; }
 
 protected:
+    // detect(points, normals or nullptr, count) on the input cloud.  Non-dense clouds (Kinect / organized PCDs carry NaN
+    // points; found by the device's bounding-box pass, KPL_E_NONFINITE): the reference's kd-tree ignores them and runForest
+    // skips them (hpp:277), so detect runs again on the compacted finite points, whose input indices `finite` then lists
+    // and `compacted` is set.  The caller maps the results back: a skipped point has a NaN response and is never a keypoint.
+    template <typename Detect>
+    int detectFinite(Detect detect, std::vector<int32_t>& finite, bool& compacted)
+    {
+        finite.clear();
+        compacted = false;
+        const int64_t n = (int64_t)input_->size();
+        int rc = detect(input_->points.data(), normals_ ? reinterpret_cast<const float*>(normals_->points.data()) : nullptr, n);
+        if (rc != KPL_E_NONFINITE) return rc;
+        for (int64_t i = 0; i < n; ++i)
+            if (pcl::isFinite(input_->points[(size_t)i])) finite.push_back((int32_t)i);
+        const int64_t m = (int64_t)finite.size();
+        std::vector<PointInT> pts((size_t)m);
+        std::vector<NormalT> nrs(normals_ ? (size_t)m : 0);
+        for (int64_t k = 0; k < m; ++k) {
+            pts[(size_t)k] = input_->points[(size_t)finite[(size_t)k]];
+            if (normals_) nrs[(size_t)k] = normals_->points[(size_t)finite[(size_t)k]];
+        }
+        compacted = true;
+        return detect(pts.data(), normals_ ? reinterpret_cast<const float*>(nrs.data()) : nullptr, m);
+    }
+
     // pcl::Keypoint::initCompute's search checks
     bool checkSearch() const
     {
