@@ -131,8 +131,6 @@ void kpl_destroy(kpl_ctx* ctx)
     release(ctx->org_flag); release(ctx->org_pix); release(ctx->org_xyz); release(ctx->org_nrm); release(ctx->org_frame_off);
     release(ctx->org_kp_off); release(ctx->org_vp); release(ctx->org_score);
     if (ctx->d_bbox) cudaFree(ctx->d_bbox);
-    if (ctx->forest.d_nodes) cudaFree(ctx->forest.d_nodes);
-    if (ctx->forest.d_roots) cudaFree(ctx->forest.d_roots);
     free_forest_set(ctx->forests);
     release(ctx->forest_off);
     for (int i = 0; i < 8; ++i) if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
@@ -196,7 +194,7 @@ static int upload_forest_set(kpl_ctx* ctx, ForestSet& S)
 }
 
 // Appends a packed forest to a copy of the set: its roots shifted by the blocks already there (child offsets are relative)
-static void append_forest(ForestSet& S, const Forest& info, const std::vector<PackedNode>& nodes, const std::vector<int32_t>& roots)
+static void append_forest(ForestSet& S, const ForestInfo& info, const std::vector<PackedNode>& nodes, const std::vector<int32_t>& roots)
 {
     const int32_t shift = (int32_t)(S.nodes.size() / 4);
     S.desc.push_back(make_int2((int)S.roots.size(), (int)roots.size()));
@@ -205,7 +203,7 @@ static void append_forest(ForestSet& S, const Forest& info, const std::vector<Pa
     S.info.push_back(info);
 }
 
-static int pack_checked(kpl_ctx* ctx, const HostForestArrays& H, std::vector<PackedNode>& nodes, std::vector<int32_t>& roots, Forest& info)
+static int pack_checked(kpl_ctx* ctx, const HostForestArrays& H, std::vector<PackedNode>& nodes, std::vector<int32_t>& roots, ForestInfo& info)
 {
     int max_depth = 0, max_var = -1;
     std::string err;
@@ -216,45 +214,28 @@ static int pack_checked(kpl_ctx* ctx, const HostForestArrays& H, std::vector<Pac
     return KPL_OK;
 }
 
-static int install_forest(kpl_ctx* ctx, const HostForestArrays& H)
+// Installs forest 0 alone (replace) or appends a forest to the set.  A forest that does not pack leaves the set as it was.
+static int install_forest(kpl_ctx* ctx, const HostForestArrays& H, bool replace)
 {
     std::vector<PackedNode> nodes;
     std::vector<int32_t> roots;
-    Forest info;
+    ForestInfo info;
     int rc = pack_checked(ctx, H, nodes, roots, info);
     if (rc) return rc;
     KPL_CUDA(cudaSetDevice(ctx->device));
-    // the forest set restarts with this forest alone: the old one goes first, so that no failure below leaves it behind
-    free_forest_set(ctx->forests);
-    Forest& F = ctx->forest;
-    if (F.d_nodes) cudaFree(F.d_nodes);
-    if (F.d_roots) cudaFree(F.d_roots);
-    F.d_nodes = nullptr; F.d_roots = nullptr; F.ntrees = 0;
-    KPL_CUDA(cudaMalloc((void**)&F.d_nodes, nodes.size() * sizeof(PackedNode)));
-    KPL_CUDA(cudaMalloc((void**)&F.d_roots, roots.size() * sizeof(int32_t)));
-    KPL_CUDA(cudaMemcpy(F.d_nodes, nodes.data(), nodes.size() * sizeof(PackedNode), cudaMemcpyHostToDevice));
-    KPL_CUDA(cudaMemcpy(F.d_roots, roots.data(), roots.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
-    F.ntrees = info.ntrees; F.nnodes = info.nnodes; F.var_count = info.var_count; F.max_depth = info.max_depth; F.max_var = info.max_var;
-    F.roots = roots;
     ForestSet S;
+    if (replace) free_forest_set(ctx->forests);     // the old set goes first: a failed upload leaves no forest loaded
+    else { S.info = ctx->forests.info; S.nodes = ctx->forests.nodes; S.roots = ctx->forests.roots; S.desc = ctx->forests.desc; }
     append_forest(S, info, nodes, roots);
     return upload_forest_set(ctx, S);
 }
 
 static int add_forest(kpl_ctx* ctx, const HostForestArrays& H, int32_t* index_out)
 {
-    if (ctx->forest.ntrees < 1 || ctx->forests.info.empty()) return fail(ctx, KPL_E_FOREST, "no forest 0 loaded: kpl_load_forest / kpl_set_forest come first");
+    if (ctx->forests.info.empty()) return fail(ctx, KPL_E_FOREST, "no forest 0 loaded: kpl_load_forest / kpl_set_forest come first");
     if ((int)ctx->forests.info.size() >= KPL_MAX_FORESTS) return fail(ctx, KPL_E_INVALID, "the forest set is full (KPL_MAX_FORESTS)");
-    std::vector<PackedNode> nodes;
-    std::vector<int32_t> roots;
-    Forest info;
-    int rc = pack_checked(ctx, H, nodes, roots, info);
+    int rc = install_forest(ctx, H, false);
     if (rc) return rc;
-    KPL_CUDA(cudaSetDevice(ctx->device));
-    ForestSet S;
-    S.info = ctx->forests.info; S.nodes = ctx->forests.nodes; S.roots = ctx->forests.roots; S.desc = ctx->forests.desc;
-    append_forest(S, info, nodes, roots);
-    if ((rc = upload_forest_set(ctx, S))) return rc;
     if (index_out) *index_out = (int32_t)ctx->forests.info.size() - 1;
     return KPL_OK;
 }
@@ -266,7 +247,7 @@ int kpl_load_forest(kpl_ctx* ctx, const char* path)
     std::string err;
     int rc = parse_forest_yaml(path, H, err);
     if (rc) return fail(ctx, rc, err);
-    return install_forest(ctx, H);
+    return install_forest(ctx, H, true);
 }
 
 static HostForestArrays forest_arrays(int32_t ntrees, int32_t nnodes, const int32_t* roots, const int32_t* var, const float* thr,
@@ -283,7 +264,7 @@ int kpl_set_forest(kpl_ctx* ctx, int32_t ntrees, int32_t nnodes, const int32_t* 
                    const int32_t* left, const int32_t* right, const float* value, int32_t var_count)
 {
     if (!ctx || ntrees < 1 || nnodes < 1 || !roots || !var || !thr || !left || !right || !value) return KPL_E_INVALID;
-    return install_forest(ctx, forest_arrays(ntrees, nnodes, roots, var, thr, left, right, value, var_count));
+    return install_forest(ctx, forest_arrays(ntrees, nnodes, roots, var, thr, left, right, value, var_count), true);
 }
 
 int kpl_add_forest(kpl_ctx* ctx, const char* path, int32_t* index_out)
@@ -306,17 +287,18 @@ int kpl_add_forest_arrays(kpl_ctx* ctx, int32_t ntrees, int32_t nnodes, const in
 int kpl_forest_count(const kpl_ctx* ctx, int32_t* count_out)
 {
     if (!ctx || !count_out) return KPL_E_INVALID;
-    *count_out = ctx->forest.ntrees > 0 ? (int32_t)ctx->forests.info.size() : 0;
+    *count_out = (int32_t)ctx->forests.info.size();
     return KPL_OK;
 }
 
 int kpl_forest_info(const kpl_ctx* ctx, int32_t* ntrees, int32_t* nnodes, int32_t* var_count, int32_t* max_depth)
 {
     if (!ctx) return KPL_E_INVALID;
-    if (ntrees) *ntrees = ctx->forest.ntrees;
-    if (nnodes) *nnodes = ctx->forest.nnodes;
-    if (var_count) *var_count = ctx->forest.var_count;
-    if (max_depth) *max_depth = ctx->forest.max_depth;
+    const ForestInfo F = ctx->forests.info.empty() ? ForestInfo() : ctx->forests.info[0];
+    if (ntrees) *ntrees = F.ntrees;
+    if (nnodes) *nnodes = F.nnodes;
+    if (var_count) *var_count = F.var_count;
+    if (max_depth) *max_depth = F.max_depth;
     return KPL_OK;
 }
 
@@ -511,25 +493,37 @@ void kpl::detect_reset(kpl_ctx* ctx)
 
 namespace kpl {
 
-int detect_check(kpl_ctx* ctx, int64_t n, bool with_role)
+int detect_check(kpl_ctx* ctx, int64_t n, int nforests, bool with_role)
 {
     const kpl_params& P = ctx->params;
+    const std::vector<ForestInfo>& info = ctx->forests.info;
     if (n < 0 || n > 2147483000ll) return fail(ctx, KPL_E_INVALID, "point count out of range");
-    if (ctx->forest.ntrees < 1) return fail(ctx, KPL_E_FOREST, "no forest loaded");
+    if (info.empty()) return fail(ctx, KPL_E_FOREST, "no forest loaded");
     // a caller that drives a slab by itself cannot see the neighbours' decisions, which its own depend on (the kpl_shard_*
     // entry points exchange them between the resolution rounds)
     if (P.draws_remove && P.non_maxima && with_role)
         return fail(ctx, KPL_E_UNSUPPORTED, "draws-remove NMS walks the whole cloud in index order (hpp:233-250): not available with a role array; use the kpl_shard_* entry points");
     const int F = P.n_annulus * P.n_bins;
-    if (ctx->forest.var_count > 0 && ctx->forest.var_count != F) return fail(ctx, KPL_E_VARCOUNT, "annuli*bins does not match the forest's var_count");
-    // whatever var_count says, no split may read beyond the A*B floats of a feature row
-    if (ctx->forest.max_var >= F) return fail(ctx, KPL_E_VARCOUNT, "the forest splits on a variable index >= annuli*bins");
+    for (int k = 0; k < nforests; ++k) {
+        char b[160];
+        if (info[k].var_count > 0 && info[k].var_count != F) {
+            snprintf(b, sizeof b, "annuli*bins does not match the var_count of forest %d", k);
+            return fail(ctx, KPL_E_VARCOUNT, b);
+        }
+        // whatever var_count says, no split may read beyond the A*B floats of a feature row
+        if (info[k].max_var >= F) {
+            snprintf(b, sizeof b, "forest %d splits on a variable index >= annuli*bins", k);
+            return fail(ctx, KPL_E_VARCOUNT, b);
+        }
+    }
+    // scores, flags and fragile flags hold nforests x n entries, forest-major
+    if ((int64_t)nforests * n > 2147483000ll) return fail(ctx, KPL_E_INVALID, "forest count x point count out of range");
     return KPL_OK;
 }
 
 // Phase A of a detection: grid (already built by the caller), normals, features + forest -> scores of every point
 // whose role asks for one.  Events 1..4 bracket the stages.
-int detect_score_phase(kpl_ctx* ctx, bool normals_given, bool use_role, int64_t n, bool forest_set)
+int detect_score_phase(kpl_ctx* ctx, bool normals_given, bool use_role, int64_t n, int nforests)
 {
     const kpl_params& P = ctx->params;
     const int F = P.n_annulus * P.n_bins;
@@ -540,19 +534,12 @@ int detect_score_phase(kpl_ctx* ctx, bool normals_given, bool use_role, int64_t 
     if (rc) return rc;
     KPL_CUDA(launch_check_normals(ctx, n, use_role));
     KPL_CUDA(cudaEventRecord(ctx->ev[2], ctx->stream));
-    bool fuse = true;      // the forest is evaluated in the tail of the feature kernel
-#ifdef KPL_EXPERIMENTS
-    fuse = getenv("KPL_NO_FUSE") == nullptr;
-#endif
-    const bool rows = ctx->keep_intermediates || !fuse;
-    KPL_CUDA(launch_features(ctx, n, use_role, fuse, rows, nullptr, 0, forest_set));
-    ctx->last_has_features = rows; ctx->last_F = F;
-    ctx->last_has_fragile = fuse && P.report_fragile != 0;
+    // the forests are evaluated in the tail of the feature kernel
+    KPL_CUDA(launch_features(ctx, n, use_role, nforests, ctx->keep_intermediates));
+    ctx->last_has_features = ctx->keep_intermediates; ctx->last_F = F;
+    ctx->last_has_fragile = P.report_fragile != 0;
     KPL_CUDA(cudaEventRecord(ctx->ev[3], ctx->stream));
-#ifdef KPL_EXPERIMENTS
-    if (!fuse) KPL_CUDA(launch_forest(ctx, n, use_role));
-#endif
-    KPL_CUDA(cudaEventRecord(ctx->ev[4], ctx->stream));
+    KPL_CUDA(cudaEventRecord(ctx->ev[4], ctx->stream));     // forest_ms: the forests have no stage of their own
     return KPL_OK;
 }
 
@@ -627,13 +614,13 @@ static int run_detect(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, co
 {
     detect_reset(ctx);
     if (n_kp_out) *n_kp_out = 0;
-    int rc = detect_check(ctx, n, d_role != nullptr);
+    int rc = detect_check(ctx, n, 1, d_role != nullptr);
     if (rc) return rc;
     ctx->stats.n_points = n;
     if (n == 0) return KPL_OK;
     if ((rc = detect_begin(ctx))) return rc;
     if ((rc = prepare_params_grid(ctx, d_xyz, d_nrm, d_role, n))) return rc;
-    if ((rc = detect_score_phase(ctx, d_nrm != nullptr, d_role != nullptr, n))) return rc;
+    if ((rc = detect_score_phase(ctx, d_nrm != nullptr, d_role != nullptr, n, 1))) return rc;
     if ((rc = detect_nms_phase(ctx, d_role != nullptr, n, d_kp_out))) return rc;
     if (d_scores_out) KPL_CUDA(cudaMemcpyAsync(d_scores_out, ctx->score.p, (size_t)n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
     return detect_finish(ctx, n, n_kp_out);
@@ -643,34 +630,14 @@ static int run_detect(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, co
 // then threshold + NMS of each forest's slice (forest-major K x n scores and flags), one compaction of the K x n flags into
 // an ascending list and its split at the forest boundaries k*n by launch_view_ranges.  No host round trip beyond those of
 // run_detect (and one per draws-remove round of each forest).
-static int check_forest_set(kpl_ctx* ctx, int64_t n)
-{
-    const ForestSet& S = ctx->forests;
-    if (ctx->forest.ntrees < 1 || S.info.empty()) return fail(ctx, KPL_E_FOREST, "no forest loaded");
-    const int F = ctx->params.n_annulus * ctx->params.n_bins;
-    for (size_t k = 0; k < S.info.size(); ++k) {
-        char b[160];
-        if (S.info[k].var_count > 0 && S.info[k].var_count != F) {
-            snprintf(b, sizeof b, "annuli*bins does not match the var_count of forest %zu", k);
-            return fail(ctx, KPL_E_VARCOUNT, b);
-        }
-        if (S.info[k].max_var >= F) {
-            snprintf(b, sizeof b, "forest %zu splits on a variable index >= annuli*bins", k);
-            return fail(ctx, KPL_E_VARCOUNT, b);
-        }
-    }
-    if (n > 0 && (int64_t)S.info.size() * n > 2147483000ll) return fail(ctx, KPL_E_INVALID, "forest count x point count out of range");
-    return KPL_OK;
-}
-
 static int run_detect_forests(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, int64_t n, const double* thresholds,
                               float* d_scores_out, int32_t* d_kp_out, int64_t* d_kp_offsets_out, int64_t* n_kp_out)
 {
     detect_reset(ctx);
     if (n_kp_out) *n_kp_out = 0;
-    int rc = check_forest_set(ctx, n);
-    if (rc || (rc = detect_check(ctx, n, false))) return rc;
     const int K = (int)ctx->forests.info.size();
+    int rc = detect_check(ctx, n, K, false);
+    if (rc) return rc;
     ctx->stats.n_points = n;
     ctx->last_nforests = K;
     if (n == 0) {
@@ -679,7 +646,7 @@ static int run_detect_forests(kpl_ctx* ctx, const float4* d_xyz, const float4* d
     }
     if ((rc = detect_begin(ctx))) return rc;
     if ((rc = prepare_params_grid(ctx, d_xyz, d_nrm, nullptr, n))) return rc;
-    if ((rc = detect_score_phase(ctx, d_nrm != nullptr, false, n, true))) return rc;
+    if ((rc = detect_score_phase(ctx, d_nrm != nullptr, false, n, K))) return rc;
     KPL_CUDA(ensure(ctx->flag, (size_t)K * n));
     for (int k = 0; k < K; ++k)
         if ((rc = nms_flags(ctx, false, n, k, thresholds ? thresholds[k] : ctx->params.threshold))) return rc;
@@ -701,14 +668,14 @@ static int run_detect_batch(kpl_ctx* ctx, const float4* d_xyz, const float4* d_n
 {
     detect_reset(ctx);
     if (n_kp_out) *n_kp_out = 0;
-    int rc = detect_check(ctx, n, false);
+    int rc = detect_check(ctx, n, 1, false);
     if (rc) return rc;
     if (ctx->params.grid_forced) return fail(ctx, KPL_E_INVALID, "a forced grid cannot be combined with a batch of views");
     ctx->stats.n_points = n; ctx->stats.n_views = nviews;
     if (n == 0) return KPL_OK;
     if ((rc = detect_begin(ctx))) return rc;
     if ((rc = prepare_grid_batch(ctx, d_xyz, d_nrm, n, h_offsets, nviews))) return rc;
-    if ((rc = detect_score_phase(ctx, d_nrm != nullptr, false, n))) return rc;
+    if ((rc = detect_score_phase(ctx, d_nrm != nullptr, false, n, 1))) return rc;
     if ((rc = detect_nms_phase(ctx, false, n, d_kp_out))) return rc;
     KPL_CUDA(launch_view_ranges(ctx, n, d_kp_out, ctx->view_offsets.p, nviews, d_kp_offsets_out));
     if (d_scores_out) KPL_CUDA(cudaMemcpyAsync(d_scores_out, ctx->score.p, (size_t)n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
@@ -728,7 +695,7 @@ static int run_detect_organized_batch(kpl_ctx* ctx, const float4* d_xyz, const f
                                       int64_t* d_kp_offsets_out, int64_t* n_kp_out)
 {
     const int64_t n = (int64_t)W * H, total = n * F;
-    int rc = detect_check(ctx, total, false);
+    int rc = detect_check(ctx, total, 1, false);
     if (rc) return rc;
     if (ctx->params.grid_forced) return fail(ctx, KPL_E_INVALID, "a forced grid cannot be combined with a batch of frames");
     ctx->stats.n_views = F;
@@ -764,7 +731,7 @@ static int run_detect_organized_batch(kpl_ctx* ctx, const float4* d_xyz, const f
     }
     KPL_CUDA(launch_organized_gather(ctx, d_xyz, d_nrm, m));
     if ((rc = prepare_grid_batch(ctx, ctx->org_xyz.p, ctx->org_nrm.p, m, view_off.data(), (int)view_off.size() - 1))) return rc;
-    if ((rc = detect_score_phase(ctx, true, false, m))) return rc;
+    if ((rc = detect_score_phase(ctx, true, false, m, 1))) return rc;
     if ((rc = detect_nms_phase(ctx, false, m, d_kp_out))) return rc;
     KPL_CUDA(launch_organized_map_back(ctx, m, n, F, d_scores_out, d_kp_out, d_kp_offsets_out));
     if ((rc = detect_finish(ctx, m, n_kp_out))) return rc;
@@ -1105,12 +1072,12 @@ int kpl_features(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float
         int32_t* d_idx = reinterpret_cast<int32_t*>(ctx->in_role.p);
         KPL_CUDA(cudaMemcpyAsync(d_idx, indices, (size_t)m * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
         KPL_CUDA(build_query_list(ctx, n, d_idx, m));
-        KPL_CUDA(launch_features(ctx, n, false, false, true, ctx->qlist.p, m));
+        KPL_CUDA(launch_features(ctx, n, false, 0, true, ctx->qlist.p, m));
         KPL_CUDA(ensure(ctx->scratch_f, (size_t)m * F));
         KPL_CUDA(launch_scatter_rows(ctx, ctx->feat.p, m, F, ctx->scratch_f.p));
         d_src = ctx->scratch_f.p;
     } else {
-        KPL_CUDA(launch_features(ctx, n, false, false, true));
+        KPL_CUDA(launch_features(ctx, n, false, 0, true));
         ctx->last_has_features = true; ctx->last_F = F;
         KPL_CUDA(ensure(ctx->scratch_f, (size_t)n * F));
         KPL_CUDA(launch_unsort_rows(ctx, ctx->feat.p, n, F, ctx->scratch_f.p));

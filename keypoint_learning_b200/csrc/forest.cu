@@ -1,73 +1,13 @@
-// forest.cu -- random-forest evaluation: replaces cv::ml::RTrees::predict(feat, result, PREDICT_SUM)
-// and the score line of KeypointLearningDetector::runForest (impl/KeypointLearning.hpp:281-287).
+// forest.cu -- the device layout of a random forest (cv::ml::RTrees), walked by the tail of feature_kernel
+// (features.cu, forest.cuh).
 //
 // Nodes are re-laid out on the host in 32-byte blocks {node, left child, right child} (pack_forest below),
-// so one sector fetched from L2 serves two levels of a walk.  One thread
-// evaluates one point; its feature row sits in shared memory as sf[var][thread] (bank == lane, no
-// conflicts for the data-dependent var), and four trees are walked concurrently per thread so four
-// independent node loads are in flight (the node arrays live in L2 / L1).
+// so one sector fetched from L2 serves two levels of a walk.
 #include <algorithm>
 #include <cmath>
 #include "kpl_internal.h"
-#include "kpl_math.cuh"
-#include "forest.cuh"
 
 namespace kpl {
-
-#ifdef KPL_EXPERIMENTS
-// Stand-alone form of the forest stage (the product path evaluates the forest in the tail of feature_kernel):
-// kept for A/B measurements of the fusion only.
-static constexpr int FOREST_THREADS = 128;
-
-__global__ void __launch_bounds__(FOREST_THREADS)
-forest_kernel(const float* __restrict__ feat, const PackedNode* __restrict__ nodes, const int32_t* __restrict__ roots,
-              int ntrees, int F, int n, const uint8_t* __restrict__ s_role, const float4* __restrict__ s_pos,
-              const float4* __restrict__ s_nrm,
-              float* __restrict__ s_score, float* __restrict__ score, unsigned long long* __restrict__ counters)
-{
-    extern __shared__ __align__(16) float sf[];
-    const int tid = threadIdx.x;
-    const int base = blockIdx.x * FOREST_THREADS;
-    const int rows = min(FOREST_THREADS, n - base);
-    const float* src = feat + (int64_t)base * F;
-    for (int e = tid; e < rows * F; e += FOREST_THREADS) {
-        int row = e / F, f = e - row * F;
-        sf[f * FOREST_THREADS + row] = __ldg(src + e);
-    }
-    __syncthreads();
-    const int i = base + tid;
-    if (i >= n) return;
-    const uint32_t orig = __float_as_uint(__ldg(s_pos + i).w);
-    const float4 qn = __ldg(s_nrm + i);
-    // unscored: halo role, or no finite normal (the reference skips the point, hpp:277)
-    if ((s_role && !(s_role[i] & 1)) || !(isfinite(qn.x) && isfinite(qn.y) && isfinite(qn.z))) {
-        s_score[i] = CUDART_NAN_F;
-        score[orig] = CUDART_NAN_F;
-        return;
-    }
-    bool fragile = false;
-    const float sc = forest_score<false>(sf + tid, FOREST_THREADS, nodes, roots, ntrees, fragile);
-    s_score[i] = sc;
-    score[orig] = sc;
-    (void)counters;
-}
-
-cudaError_t launch_forest(kpl_ctx* c, int64_t n, bool use_role)
-{
-    const int F = c->params.n_annulus * c->params.n_bins;
-    cudaError_t e;
-    if ((e = ensure(c->s_score, n)) || (e = ensure(c->score, n))) return e;
-    size_t smem = (size_t)F * FOREST_THREADS * sizeof(float);
-    if (smem > 227 * 1024) return cudaErrorInvalidValue;
-    if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(forest_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem))) return e;
-    int blocks = (int)((n + FOREST_THREADS - 1) / FOREST_THREADS);
-    forest_kernel<<<blocks, FOREST_THREADS, smem, c->stream>>>(c->feat.p, c->forest.d_nodes, c->forest.d_roots, c->forest.ntrees, F, (int)n,
-                                                               use_role ? c->s_role.p : nullptr, c->s_pos.p, c->s_nrm.p, c->s_score.p, c->score.p,
-                                                               c->counters.p);
-    c->launches++;
-    return cudaGetLastError();
-}
-#endif  // KPL_EXPERIMENTS
 
 // Host side: arbitrary (roots,var,thr,left,right,value) arrays -> 32-byte BLOCKS of four PackedNodes
 // {P, L, R, unused}: a node P of even depth together with its two children.  One 32-byte sector -- the unit

@@ -1,5 +1,5 @@
-// forest.cuh -- per-thread traversal of the packed forest, shared by forest_kernel (forest.cu) and the
-// fused tail of feature_kernel (features.cu).  Semantics: cv::ml::RTrees::predict(.., PREDICT_SUM)
+// forest.cuh -- per-thread traversal of the packed forest (forest.cu), in the tail of feature_kernel
+// (features.cu).  Semantics: cv::ml::RTrees::predict(.., PREDICT_SUM)
 // (OpenCV DTreesImpl::predictTrees: left iff x[var] <= split.c, sum of leaf values) followed by the
 // score line of KeypointLearningDetector::runForest (impl/KeypointLearning.hpp:281-287).
 #pragma once
@@ -14,7 +14,7 @@ namespace kpl {
 static constexpr int TREES_IN_FLIGHT = KPL_TREES_IN_FLIGHT;
 
 // x[var * stride] is feature `var` of this thread's point (a shared-memory column: bank == lane for
-// stride 32 / 128, so the data-dependent var never conflicts).  Four trees are walked concurrently so
+// stride 32, so the data-dependent var never conflicts).  Four trees are walked concurrently so
 // four independent block loads (L2 resident) are in flight per thread; nd[] counts 32-byte blocks.
 //
 // `fragile` reports whether any split DECIDED on the way (the nodes actually visited) had |x[var] - thr| <= 1e-5:

@@ -56,19 +56,16 @@ struct __align__(8) PackedNode {
 };
 static constexpr uint32_t KPL_LEAF_VAR = 1023u;
 
-struct Forest {
+struct ForestInfo {
     int32_t ntrees = 0, nnodes = 0, var_count = 0, max_depth = 0;
     int32_t max_var = -1;                 // largest variable index any split reads (checked against annuli*bins per call)
-    std::vector<int32_t> roots;           // host copy (block index of each root)
-    PackedNode* d_nodes = nullptr;
-    int32_t* d_roots = nullptr;
 };
 
-// The forest set of kpl_detect_forests: forest 0 (a copy of kpl_ctx::forest) and the added ones, concatenated into one
-// node array.  pack_forest's child offsets are relative, so a forest moves by shifting its roots by the blocks before it;
-// desc[k] = (first root of forest k, its tree count).
+// The loaded forests: forest 0 (kpl_load_forest / kpl_set_forest, which every entry point scores with) and the ones
+// kpl_add_forest* appended, concatenated into one node array.  pack_forest's child offsets are relative, so a forest moves
+// by shifting its roots by the blocks before it; desc[k] = (first root of forest k, its tree count).  Empty: no forest loaded.
 struct ForestSet {
-    std::vector<Forest> info;             // per forest: ntrees, nnodes, var_count, max_depth, max_var (device pointers unused)
+    std::vector<ForestInfo> info;
     std::vector<PackedNode> nodes;        // host copy of the concatenation
     std::vector<int32_t> roots;           // shifted roots, forest after forest
     std::vector<int2> desc;
@@ -99,8 +96,7 @@ struct kpl_ctx {
     cudaStream_t own_stream = nullptr;
     cudaStream_t stream = nullptr;
     kpl_params params;
-    kpl::Forest forest;
-    kpl::ForestSet forests;                      // kpl_detect_forests: forest 0 + kpl_add_forest*
+    kpl::ForestSet forests;
     kpl::GridDesc grid;
     kpl_timings timings;
     kpl_stats stats;
@@ -196,13 +192,9 @@ cudaError_t build_query_list(kpl_ctx* c, int64_t n, const int32_t* d_indices, in
 cudaError_t launch_scatter_rows(kpl_ctx* c, const float* d_rows, int64_t m, int width, float* d_out);
 cudaError_t launch_view_ranges(kpl_ctx* c, int64_t n, int32_t* d_kp_idx, const int64_t* d_view_offsets, int nviews, int64_t* d_kp_offsets);
 cudaError_t launch_bbox_views(kpl_ctx* c, const float4* xyz, int64_t n, const int64_t* d_view_offsets, int nviews, uint32_t* d_bbox);
+// nforests: forests 0 .. nforests - 1 of c->forests are scored in the kernel's tail (0: features only, kpl_features).
 // qlist != nullptr: features of the m_list listed sorted positions only (rows in list order, c->feat holds m_list x F).
-// forest_set: the fused tail scores every forest of c->forests (kpl_detect_forests) instead of forest 0.
-cudaError_t launch_features(kpl_ctx* c, int64_t n, bool use_role, bool fuse_forest, bool store_rows, const int32_t* d_qlist = nullptr, int64_t m_list = 0,
-                            bool forest_set = false);
-#ifdef KPL_EXPERIMENTS
-cudaError_t launch_forest(kpl_ctx* c, int64_t n, bool use_role);
-#endif
+cudaError_t launch_features(kpl_ctx* c, int64_t n, bool use_role, int nforests, bool store_rows, const int32_t* d_qlist = nullptr, int64_t m_list = 0);
 // Threshold + NMS of one forest's n sorted scores s_score (th compared in double); the keypoint flags (original order) go to
 // c->flag.p + flag_off.  kpl_detect* pass c->s_score.p, params.threshold and 0; kpl_detect_forests forest k's slice.
 cudaError_t launch_nms(kpl_ctx* c, int64_t n, bool use_role, const float* s_score, double th, int64_t flag_off);
@@ -235,13 +227,14 @@ int grid_reach(double radius, double cell);
 
 // detection phases (capi.cu), shared with the slab-sharded driver (shard.cu); all but detect_reset return kpl_status
 void detect_reset(kpl_ctx* ctx);
+// nforests: the call scores forests 0 .. nforests - 1 (kpl_detect_forests: all of them; every other entry point: 1).
 // with_role: a caller-supplied role array (kpl_detect*), which rules out draws-remove NMS; the kpl_shard_* driver passes false
-int detect_check(kpl_ctx* ctx, int64_t n, bool with_role);
+int detect_check(kpl_ctx* ctx, int64_t n, int nforests, bool with_role);
 int detect_begin(kpl_ctx* ctx);
 // forced == nullptr: the canonical grid of the cloud's bounding box; cell_override > 0 replaces the canonical cell
 int prepare_grid(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, const uint8_t* d_role, int64_t n, const ForcedGrid* forced, double cell_override = 0.0);
-// forest_set: score with every forest of ctx->forests (kpl_detect_forests)
-int detect_score_phase(kpl_ctx* ctx, bool normals_given, bool use_role, int64_t n, bool forest_set = false);
+// scores of forests 0 .. nforests - 1, forest-major
+int detect_score_phase(kpl_ctx* ctx, bool normals_given, bool use_role, int64_t n, int nforests);
 int detect_nms_phase(kpl_ctx* ctx, bool use_role, int64_t n, int32_t* d_kp_out);
 int detect_finish(kpl_ctx* ctx, int64_t n, int64_t* n_kp_out);
 

@@ -377,7 +377,7 @@ int phase_score(kpl_shard* s)
     if (rc) return rc;
     c->launches += 2;
     if ((rc = prepare_grid(c, s->loc_xyz.p, s->has_nrm ? s->loc_nrm.p : nullptr, s->role.p, s->n_loc, &s->grid))) return rc;
-    if ((rc = detect_score_phase(c, s->has_nrm, true, s->n_loc))) return rc;
+    if ((rc = detect_score_phase(c, s->has_nrm, true, s->n_loc, 1))) return rc;
     KS_CUDA(cudaEventRecord(s->ev[2], c->stream));
     const float* owned_scores = c->score.p + s->n_l;
     if (s->send_l) pack_scores_kernel<<<(unsigned)((s->send_l + 255) / 256), 256, 0, c->stream>>>(owned_scores, s->sel_l.p, s->send_l, s->ssc_l.p);
@@ -533,7 +533,7 @@ int check_ready(kpl_shard* s)
     // halo must then be two search reaches wide, which no device check can verify after the fact
     if (s->world > 1 && !s->has_nrm && s->ctx->params.normals_mode == KPL_NORMALS_RADIUS && s->plan.normal_support_cells < s->plan.reach_feat)
         return sfail(s, KPL_E_HALO, "radius-mode normals need normal_support_cells >= reach_feat (the whole r_feat ball of every halo point that matters)");
-    return detect_check(s->ctx, s->n_loc, false);
+    return detect_check(s->ctx, s->n_loc, 1, false);
 }
 
 void finish_timings(kpl_shard* s, bool gathered)

@@ -295,6 +295,33 @@ def test_refusals(kpl):
     nof.close()
 
 
+def test_failed_install_leaves_the_set_alone(kpl):
+    """A malformed kpl_set_forest and a kpl_load_forest of a missing file change nothing: neither the three loaded forests
+    nor what kpl_detect and kpl_detect_forests return."""
+    xyz = _cloud("cheff001")
+    det = _detector(kpl, FORESTS)
+    det.setInputCloud(xyz)
+
+    def results():
+        _, idx = det.compute()
+        out = [det.getResponse().copy(), idx.copy()]
+        res = det.computeForests()
+        return out + [det.getResponses().copy()] + [r[1].copy() for r in res]
+
+    info, before = det.forestInfo(), results()
+    assert len(before[1]) > 0
+    broken = dict(ntrees=1, var=[0, -1, -1], thr=[0.5, 0, 0], left=[1, 0, 0], right=[2, 0, 0], value=[0, 1, 0], roots=[5])   # root out of range
+    with pytest.raises(kpl.KplError) as e:
+        det.setForestArrays(broken)
+    assert e.value.code == KPL_E_FOREST
+    assert not det.loadForest(os.path.join(ROOT, "no-such-forest.yaml.gz"))
+    assert det.forestCount() == 3 and det.forestInfo() == info
+    after = results()
+    for a, b in zip(before, after):
+        assert _same(a, b) if a.dtype == np.float32 else np.array_equal(a, b)
+    det.close()
+
+
 CPP = r"""
 #include <cmath>
 #include <cstdio>

@@ -8,6 +8,8 @@ Medians over --steps calls after two warm-up calls of: wall_ms (host clock aroun
 synchronisation), features_ms (CUDA events around the feature kernel with its fused forest tail; summed over the K calls
 for (b)), nms_ms, host_syncs and kernel_launches.  The script checks that (a) and (b) return identical scores (bits) and
 keypoints, and records the packed size of every forest (32-byte blocks, csrc/forest.cu: pack_forest) and the card.
+--report-fragile times every call with kpl_params.report_fragile on (the feature kernel variant that also flags near-split
+decisions).
 
     python tools/time_forests.py --steps 10 --out profiles/r3_forests.json
 """
@@ -53,10 +55,11 @@ def packed_bytes(path):
     return blocks * 32
 
 
-def detector(K, forests, vp):
+def detector(K, forests, vp, fragile):
     det = K.KeypointLearningDetector()
     det.setNAnnulus(5); det.setNBins(10); det.setNonMaxima(True); det.setNonMaxRadius(R_NMS); det.setNonMaximaDrawsRemove(False)
     det.setPredictionThreshold(TH); det.setRadiusSearch(R_FEAT); det.setNormalsMode(1, k=10, viewpoint=vp)
+    det.setReportFragile(fragile)
     assert det.loadForest(forests[0])
     for f in forests[1:]:
         det.addForest(f)
@@ -72,6 +75,7 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=2)
     ap.add_argument("--workloads", default="scene10m,view1m")
+    ap.add_argument("--report-fragile", action="store_true")
     ap.add_argument("--out")
     a = ap.parse_args()
     import torch
@@ -79,7 +83,7 @@ def main():
         raise SystemExit("no GPU: nothing to measure")
     import keypoint_learning_b200 as K
     from keypoint_learning_b200 import synth
-    out = {"card": card(), "steps": a.steps, "warmup": a.warmup, "threshold": TH,
+    out = {"card": card(), "steps": a.steps, "warmup": a.warmup, "threshold": TH, "report_fragile": a.report_fragile,
            "forests": [{"name": nm, "packed_bytes": packed_bytes(p)} for nm, p in zip(NAMES, FORESTS)], "workloads": {}}
     for wl in a.workloads.split(","):
         if wl == "scene10m":
@@ -90,8 +94,8 @@ def main():
         n = len(xyz)
         x4 = np.ones((n, 4), np.float32); x4[:, :3] = xyz[:, :3]
         d_xyz = torch.from_numpy(x4).cuda()
-        singles = [detector(K, [f], vp) for f in FORESTS]
-        sets = {k: detector(K, FORESTS[:k], vp) for k in (1, 2, 3)}
+        singles = [detector(K, [f], vp, a.report_fragile) for f in FORESTS]
+        sets = {k: detector(K, FORESTS[:k], vp, a.report_fragile) for k in (1, 2, 3)}
         d_sc = torch.empty(3 * n, dtype=torch.float32, device="cuda")
         d_kp = torch.empty(3 * n, dtype=torch.int32, device="cuda")
         d_kpo = torch.empty(4, dtype=torch.int64, device="cuda")
