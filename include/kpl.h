@@ -121,7 +121,7 @@ typedef struct kpl_stats {
                                  (hpp:281) had |x[var] - thr| <= 1e-5: a feature difference of the tolerated
                                  size sends that tree the other way and moves the score by 1/ntrees            */
     int32_t host_syncs;       /* cudaStreamSynchronize calls the last call made                               */
-    int32_t n_views;          /* kpl_detect_batch: views in the call (1 otherwise)                            */
+    int32_t n_views;          /* kpl_detect_batch(_forests): views in the call, frames for the organized batch (1 otherwise) */
 } kpl_stats;
 
 /* ---- lifetime ------------------------------------------------------------------------------- */
@@ -153,7 +153,8 @@ KPL_API int kpl_forest_info(const kpl_ctx* ctx, int32_t* ntrees, int32_t* nnodes
  * and up to KPL_MAX_FORESTS - 1 forests appended by kpl_add_forest(_arrays) as forests 1, 2, ...; *index_out (may be NULL)
  * receives the new forest's index.  Adding needs forest 0 (KPL_E_FOREST without it) and fails with KPL_E_INVALID once the
  * set is full; a failed add leaves the set as it was.  kpl_forest_info keeps describing forest 0, and every entry point
- * other than kpl_detect_forests(_device) scores with forest 0 only, whatever else is loaded. */
+ * other than kpl_detect_forests, kpl_detect_batch_forests and kpl_detect_batch_organized_forests (and their _device
+ * variants) scores with forest 0 only, whatever else is loaded. */
 #define KPL_MAX_FORESTS 16
 KPL_API int kpl_add_forest(kpl_ctx* ctx, const char* path, int32_t* index_out);
 KPL_API int kpl_add_forest_arrays(kpl_ctx* ctx, int32_t ntrees, int32_t nnodes, const int32_t* roots, const int32_t* var,
@@ -260,6 +261,26 @@ KPL_API int kpl_detect_batch(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride,
 /* Same with device-resident clouds; view_offsets stays a HOST array, d_kp_offsets is n_views + 1 int64 on the device. */
 KPL_API int kpl_detect_batch_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, const int64_t* view_offsets,
                                     int32_t n_views, void* d_scores, void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out);
+/* Every forest of the set over a batch of views (evaluating several descriptors' forests over a dataset of views): one
+ * stacked grid, one normal estimation and one feature pass whose tail walks the K forests (kpl_forest_count), then each
+ * forest's NMS.  For forest k and view v the scores (compared as bits) and keypoints are those of kpl_detect_batch on
+ * the same views with only forest k loaded and params.threshold = thresholds[k] (thresholds: NULL or K doubles on the
+ * host, as in kpl_detect_forests).  Outputs are forest-major, then view-major: scores_out NULL or K*n floats, forest k's
+ * at k*n in concatenated point order; kp_idx_out (capacity K*n): VIEW-LOCAL indices, ascending within a range;
+ * kp_offsets_out[K*n_views + 1]: the range of (k, v) is kp_idx_out[kp_offsets_out[k*n_views + v] .. [k*n_views + v + 1]).
+ * Refusals as kpl_detect_batch, plus those of kpl_detect_forests (KPL_E_VARCOUNT names the forest; K*n above
+ * 2 147 483 000 is KPL_E_INVALID before the device is touched).  kpl_stats as kpl_detect_forests, with n_views = n_views;
+ * with report_fragile, kpl_fetch_u8("fragile") returns K*n bytes, forest-major.  Host round trips: those of
+ * kpl_detect_batch(_device) whatever K is (plus one per draws-remove round of each forest); kernel launches: K - 1 more
+ * (one NMS per further forest).  K = 1 is kpl_detect_batch. */
+KPL_API int kpl_detect_batch_forests(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
+                                     const int64_t* view_offsets, int32_t n_views, const double* thresholds,
+                                     float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out);
+/* Device-resident views: d_scores NULL or K*n floats, d_kp_idx K*n int32, d_kp_offsets K*n_views + 1 int64, all on the
+ * device; view_offsets and thresholds stay HOST arrays.  *n_kp_out = keypoints of all forests and views. */
+KPL_API int kpl_detect_batch_forests_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, const int64_t* view_offsets,
+                                            int32_t n_views, const double* thresholds, void* d_scores, void* d_kp_idx,
+                                            void* d_kp_offsets, int64_t* n_kp_out);
 
 /* ---- a batch of ORGANIZED frames of one size (depth-camera streams; the 2.5-D views of BASELINE.json configs[4]) ---- */
 /* n_frames organized frames of width x height points each, row-major, frame after frame (NaN = no measurement); xyz at
@@ -292,6 +313,29 @@ KPL_API int kpl_detect_batch_organized_device(kpl_ctx* ctx, const void* d_xyz4, 
                                               int32_t height, int32_t n_frames, float smoothing_size,
                                               const float* viewpoints, void* d_scores, void* d_kp_idx,
                                               void* d_kp_offsets, int64_t* n_kp_out);
+/* Every forest of the set over a batch of organized frames, from one feature pass (as kpl_detect_batch_forests).  For
+ * forest k and frame f the scores (as bits, NaN payloads included) and keypoints are those of kpl_detect_batch_organized
+ * with only forest k loaded and params.threshold = thresholds[k] (NULL or K doubles on the host).  Forest-major, then
+ * frame-major: scores_out NULL or K*n_frames*width*height floats in pixel order, forest k's at k*n_frames*width*height
+ * (NaN on non-finite pixels in every slice); kp_idx_out (capacity K*n_frames*width*height): FRAME-LOCAL pixel indices,
+ * ascending within a range; kp_offsets_out[K*n_frames + 1]: the range of (k, f) is [kp_offsets_out[k*n_frames + f],
+ * kp_offsets_out[k*n_frames + f + 1]).  A frame without a finite point gets an empty range in every forest; a batch
+ * without any returns KPL_OK, K*n_frames + 1 zero offsets and all-NaN scores.  Refusals as kpl_detect_batch_organized
+ * plus those of kpl_detect_forests (K*n_frames*width*height above 2 147 483 000: KPL_E_INVALID before the device is
+ * touched).  kpl_stats as kpl_detect_forests over the finite points, n_views = n_frames; with report_fragile,
+ * kpl_fetch_u8("fragile") returns K x (finite points) bytes, forest-major.  Host round trips: those of
+ * kpl_detect_batch_organized(_device) whatever K is (plus one per draws-remove round of each forest); kernel launches:
+ * K - 1 more.  K = 1 is kpl_detect_batch_organized. */
+KPL_API int kpl_detect_batch_organized_forests(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals,
+                                               int32_t normals_stride, int32_t width, int32_t height, int32_t n_frames,
+                                               float smoothing_size, const float* viewpoints, const double* thresholds,
+                                               float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out);
+/* Device-resident frames; viewpoints and thresholds stay HOST arrays; d_scores NULL or K*n_frames*width*height floats,
+ * d_kp_idx K*n_frames*width*height int32, d_kp_offsets K*n_frames + 1 int64, all on the device. */
+KPL_API int kpl_detect_batch_organized_forests_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, int32_t width,
+                                                      int32_t height, int32_t n_frames, float smoothing_size,
+                                                      const float* viewpoints, const double* thresholds, void* d_scores,
+                                                      void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out);
 
 /* ---- ONE large cloud over the GPUs of a node: x slabs + halo over NCCL (BASELINE.json configs[3]) ---------- */
 /* The reference is a single process (main_test_detector.cpp:123-187 drives one detector); this is the layer a

@@ -30,7 +30,8 @@ EXPORTS = ["kpl_create", "kpl_destroy", "kpl_last_error", "kpl_version", "kpl_se
            "kpl_shard_set_slab", "kpl_shard_upload", "kpl_shard_detect", "kpl_shard_detect_group", "kpl_shard_get_info",
            "kpl_shard_device_scores", "kpl_shard_set_slab_normals", "kpl_shard_upload_normals", "kpl_detect_batch_organized",
            "kpl_detect_batch_organized_device", "kpl_add_forest", "kpl_add_forest_arrays", "kpl_forest_count", "kpl_detect_forests",
-           "kpl_detect_forests_device"]
+           "kpl_detect_forests_device", "kpl_detect_batch_forests", "kpl_detect_batch_forests_device", "kpl_detect_batch_organized_forests",
+           "kpl_detect_batch_organized_forests_device"]
 KPL_MAX_RANKS = 64
 KPL_MAX_FORESTS = 16
 
@@ -140,6 +141,12 @@ def load_library():
     L.kpl_detect_batch_organized.argtypes = [vp, f32p, C.c_int32, f32p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_float, f32p, f32p,
                                              i32p, i64p]
     L.kpl_detect_batch_organized_device.argtypes = [vp, vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_float, f32p, vp, vp, vp, i64p]
+    L.kpl_detect_batch_forests.argtypes = [vp, f32p, C.c_int32, f32p, C.c_int32, i64p, C.c_int32, f64p, f32p, i32p, i64p]
+    L.kpl_detect_batch_forests_device.argtypes = [vp, vp, vp, i64p, C.c_int32, f64p, vp, vp, vp, i64p]
+    L.kpl_detect_batch_organized_forests.argtypes = [vp, f32p, C.c_int32, f32p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_float, f32p,
+                                                     f64p, f32p, i32p, i64p]
+    L.kpl_detect_batch_organized_forests_device.argtypes = [vp, vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_float, f32p, f64p, vp, vp, vp,
+                                                            i64p]
     _lib = L
     return L
 
@@ -331,9 +338,8 @@ class KeypointLearningDetector:
         self._kp_idx = kp[:nkp.value].copy()
         return self._xyzi[:nkp.value].copy(), self._kp_idx          # the keypoint cloud was gathered on the device
 
-    def computeBatch(self, clouds, normals=None):
-        """kpl_detect_batch: `clouds` is a list of (n_v, >=3) float32 views.  Returns (scores list, keypoint index list),
-        one entry per view, exactly what compute() returns for each view alone."""
+    @staticmethod
+    def _concat_views(clouds, normals):
         arrs = [_vec3(c, "cloud")[0] for c in clouds]
         width = arrs[0].shape[1]
         if any(a.shape[1] != width for a in arrs):
@@ -345,7 +351,38 @@ class KeypointLearningDetector:
         if normals is not None:
             nrm = np.ascontiguousarray(np.concatenate([_vec3(x, "normals")[0] for x in normals]))
             ns = nrm.shape[1] * 4
-        return self.computeBatchConcat(xyz, off, nrm, ns)
+        return xyz, off, nrm, ns
+
+    def _thresholds(self, thresholds):
+        """None, or one float64 threshold per forest of the set (the shape computeForests checks)."""
+        if thresholds is None:
+            return None
+        K = self.forestCount()
+        th = np.ascontiguousarray(thresholds, np.float64)
+        if th.shape != (K,):
+            raise ValueError("thresholds must hold one value per forest (%d)" % K)
+        return th
+
+    def computeBatch(self, clouds, normals=None):
+        """kpl_detect_batch: `clouds` is a list of (n_v, >=3) float32 views.  Returns (scores list, keypoint index list),
+        one entry per view, exactly what compute() returns for each view alone."""
+        return self.computeBatchConcat(*self._concat_views(clouds, normals))
+
+    def computeBatchForests(self, clouds, normals=None, thresholds=None):
+        """kpl_detect_batch_forests: every forest of the set over a batch of views, from one feature pass.  thresholds: None
+        (the prediction threshold for every forest) or one per forest.  Returns out[k][v] = (scores, view-local keypoint
+        indices): what computeBatch() returns for view v with only forest k loaded and threshold k."""
+        th = self._thresholds(thresholds)
+        xyz, off, nrm, ns = self._concat_views(clouds, normals)
+        K, n, nv = self.forestCount(), xyz.shape[0], len(off) - 1
+        self._push()
+        scores = np.empty((max(K, 1), n), np.float32)
+        kp = np.empty(max(K * n, 1), np.int32)
+        kpo = np.empty(K * nv + 1, np.int64)
+        self._check(self._L.kpl_detect_batch_forests(self._h, _ptr(xyz, C.c_float), xyz.shape[1] * 4, _ptr(nrm, C.c_float), ns or 0,
+                                                     _ptr(off, C.c_int64), nv, _ptr(th, C.c_double), _ptr(scores, C.c_float),
+                                                     _ptr(kp, C.c_int32), _ptr(kpo, C.c_int64)))
+        return [[(scores[k, off[v]:off[v + 1]], kp[kpo[k * nv + v]:kpo[k * nv + v + 1]].copy()) for v in range(nv)] for k in range(K)]
 
     def computeBatchConcat(self, xyz, offsets, nrm=None, ns=None, scores_out=None, kp_out=None):
         """kpl_detect_batch on an already concatenated host array (what bench.py times)."""
@@ -368,6 +405,18 @@ class KeypointLearningDetector:
         self._check(self._L.kpl_detect_batch_device(self._h, C.c_void_p(d_xyz4), C.c_void_p(d_normals4 or None), _ptr(off, C.c_int64),
                                                     len(off) - 1, C.c_void_p(d_scores or None), C.c_void_p(d_kp_idx), C.c_void_p(d_kp_offsets),
                                                     C.byref(nkp)))
+        return nkp.value
+
+    def detectBatchForestsDevice(self, d_xyz4, offsets, d_scores=0, d_kp_idx=0, d_kp_offsets=0, d_normals4=0, thresholds=None):
+        """kpl_detect_batch_forests_device: raw device pointers (ints), host offsets; d_scores K*n floats (or 0), d_kp_idx K*n
+        int32, d_kp_offsets K*n_views + 1 int64, forest-major then view-major.  Returns the keypoint count of all forests."""
+        th = self._thresholds(thresholds)
+        self._push()
+        off = np.ascontiguousarray(offsets, np.int64)
+        nkp = C.c_int64(0)
+        self._check(self._L.kpl_detect_batch_forests_device(self._h, C.c_void_p(d_xyz4), C.c_void_p(d_normals4 or None), _ptr(off, C.c_int64),
+                                                            len(off) - 1, _ptr(th, C.c_double), C.c_void_p(d_scores or None),
+                                                            C.c_void_p(d_kp_idx or None), C.c_void_p(d_kp_offsets or None), C.byref(nkp)))
         return nkp.value
 
     def fetchFragile(self, n):
@@ -406,9 +455,7 @@ class KeypointLearningDetector:
             if nrm.shape[0] != xyz.shape[0]:
                 raise KplError(3, "normals given, but the number of normals does not match the number of input points")
         K = self.forestCount()
-        th = None if thresholds is None else np.ascontiguousarray(thresholds, np.float64)
-        if th is not None and th.shape != (K,):
-            raise ValueError("thresholds must hold one value per forest (%d)" % K)
+        th = self._thresholds(thresholds)
         self._push()
         finite = None
         scores, kp, kpo = self._detect_forests(xyz, xs, nrm, ns, th, K)
@@ -506,17 +553,8 @@ class KeypointLearningDetector:
         viewpoint) or per-pixel normals of the same (F, height, width, >=3) shape.  Returns (scores list, keypoint pixel index
         list), one entry per frame: what computeOrganized() (normals None) or compute() on the flattened frame with
         setNormals (normals given) returns for that frame alone."""
-        a = np.asarray(frames)
-        if a.ndim != 4 or a.shape[3] < 3:
-            raise ValueError("frames must be (n_frames, height, width, >=3) float32")
-        a = np.ascontiguousarray(a, np.float32)
+        a, nrm, vp = self._frames(frames, normals, viewpoints)
         nf, h, w, c = a.shape
-        nrm = None
-        if normals is not None:
-            nrm = np.ascontiguousarray(normals, np.float32)
-            if nrm.shape[:3] != (nf, h, w) or nrm.ndim != 4 or nrm.shape[3] < 3:
-                raise ValueError("normals must be (n_frames, height, width, >=3) float32")
-        vp = None if viewpoints is None else np.ascontiguousarray(viewpoints, np.float32).reshape(nf, 3)
         self._push()
         n = nf * h * w
         scores = np.empty(n, np.float32)
@@ -526,6 +564,55 @@ class KeypointLearningDetector:
                                                        0 if nrm is None else nrm.shape[3] * 4, w, h, nf, float(smoothing), _ptr(vp, C.c_float),
                                                        _ptr(scores, C.c_float), _ptr(kp, C.c_int32), _ptr(kpo, C.c_int64)))
         return ([scores[f * h * w:(f + 1) * h * w] for f in range(nf)], [kp[kpo[f]:kpo[f + 1]].copy() for f in range(nf)])
+
+    @staticmethod
+    def _frames(frames, normals, viewpoints):
+        a = np.asarray(frames)
+        if a.ndim != 4 or a.shape[3] < 3:
+            raise ValueError("frames must be (n_frames, height, width, >=3) float32")
+        a = np.ascontiguousarray(a, np.float32)
+        nf, h, w, _ = a.shape
+        nrm = None
+        if normals is not None:
+            nrm = np.ascontiguousarray(normals, np.float32)
+            if nrm.shape[:3] != (nf, h, w) or nrm.ndim != 4 or nrm.shape[3] < 3:
+                raise ValueError("normals must be (n_frames, height, width, >=3) float32")
+        vp = None if viewpoints is None else np.ascontiguousarray(viewpoints, np.float32).reshape(nf, 3)
+        return a, nrm, vp
+
+    def computeOrganizedBatchForests(self, frames, smoothing=5.0, normals=None, viewpoints=None, thresholds=None):
+        """kpl_detect_batch_organized_forests: every forest of the set over a batch of organized frames (arguments as in
+        computeOrganizedBatch), from one feature pass.  thresholds: None or one per forest.  Returns out[k][f] = (pixel-order
+        scores, frame-local keypoint pixel indices): what computeOrganizedBatch() returns for frame f with only forest k
+        loaded and threshold k."""
+        th = self._thresholds(thresholds)
+        a, nrm, vp = self._frames(frames, normals, viewpoints)
+        nf, h, w, c = a.shape
+        K, n = self.forestCount(), nf * h * w
+        self._push()
+        scores = np.empty((max(K, 1), n), np.float32)
+        kp = np.empty(max(K * n, 1), np.int32)
+        kpo = np.empty(K * nf + 1, np.int64)
+        self._check(self._L.kpl_detect_batch_organized_forests(self._h, _ptr(a, C.c_float), c * 4, _ptr(nrm, C.c_float),
+                                                               0 if nrm is None else nrm.shape[3] * 4, w, h, nf, float(smoothing),
+                                                               _ptr(vp, C.c_float), _ptr(th, C.c_double), _ptr(scores, C.c_float),
+                                                               _ptr(kp, C.c_int32), _ptr(kpo, C.c_int64)))
+        return [[(scores[k, f * h * w:(f + 1) * h * w], kp[kpo[k * nf + f]:kpo[k * nf + f + 1]].copy()) for f in range(nf)] for k in range(K)]
+
+    def detectOrganizedBatchForestsDevice(self, d_xyz4, width, height, n_frames, smoothing=5.0, d_normals4=0, viewpoints=None, d_scores=0,
+                                          d_kp_idx=0, d_kp_offsets=0, thresholds=None):
+        """kpl_detect_batch_organized_forests_device: raw device pointers (ints), host viewpoints and thresholds; d_scores
+        K*F*W*H floats (or 0), d_kp_idx K*F*W*H int32, d_kp_offsets K*F + 1 int64.  Returns the keypoint count of all forests."""
+        th = self._thresholds(thresholds)
+        vp = None if viewpoints is None else np.ascontiguousarray(viewpoints, np.float32).reshape(int(n_frames), 3)
+        self._push()
+        nkp = C.c_int64(0)
+        self._check(self._L.kpl_detect_batch_organized_forests_device(self._h, C.c_void_p(d_xyz4), C.c_void_p(d_normals4 or None), int(width),
+                                                                      int(height), int(n_frames), float(smoothing), _ptr(vp, C.c_float),
+                                                                      _ptr(th, C.c_double), C.c_void_p(d_scores or None),
+                                                                      C.c_void_p(d_kp_idx or None), C.c_void_p(d_kp_offsets or None),
+                                                                      C.byref(nkp)))
+        return nkp.value
 
     def detectOrganizedBatchDevice(self, d_xyz4, width, height, n_frames, smoothing=5.0, d_normals4=0, viewpoints=None, d_scores=0,
                                    d_kp_idx=0, d_kp_offsets=0):

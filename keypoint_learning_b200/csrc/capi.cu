@@ -132,7 +132,7 @@ void kpl_destroy(kpl_ctx* ctx)
     release(ctx->org_kp_off); release(ctx->org_vp); release(ctx->org_score);
     if (ctx->d_bbox) cudaFree(ctx->d_bbox);
     free_forest_set(ctx->forests);
-    release(ctx->forest_off);
+    release(ctx->range_off);
     for (int i = 0; i < 8; ++i) if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
     delete ctx;
@@ -554,12 +554,16 @@ static int nms_flags(kpl_ctx* ctx, bool use_role, int64_t n, int k, double th)
     return KPL_OK;
 }
 
-// Phase B: threshold + NMS over the scores in place, ascending keypoint indices into d_kp_out.
-int detect_nms_phase(kpl_ctx* ctx, bool use_role, int64_t n, int32_t* d_kp_out)
+// Phase B: threshold + NMS of every forest's slice of the scores in place, then one compaction of the nforests x n flags:
+// ascending keypoint indices in [0, nforests * n) into d_kp_out.
+int detect_nms_phase(kpl_ctx* ctx, bool use_role, int64_t n, int nforests, const double* thresholds, int32_t* d_kp_out)
 {
-    int rc = nms_flags(ctx, use_role, n, 0, ctx->params.threshold);
-    if (rc) return rc;
-    KPL_CUDA(launch_compact(ctx, n, d_kp_out));
+    KPL_CUDA(ensure(ctx->flag, (size_t)nforests * n));      // before slice 0: a later growth would drop the flags of earlier slices
+    for (int k = 0; k < nforests; ++k) {
+        int rc = nms_flags(ctx, use_role, n, k, thresholds ? thresholds[k] : ctx->params.threshold);
+        if (rc) return rc;
+    }
+    KPL_CUDA(launch_compact(ctx, (int64_t)nforests * n, d_kp_out));
     return KPL_OK;
 }
 
@@ -621,9 +625,27 @@ static int run_detect(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, co
     if ((rc = detect_begin(ctx))) return rc;
     if ((rc = prepare_params_grid(ctx, d_xyz, d_nrm, d_role, n))) return rc;
     if ((rc = detect_score_phase(ctx, d_nrm != nullptr, d_role != nullptr, n, 1))) return rc;
-    if ((rc = detect_nms_phase(ctx, d_role != nullptr, n, d_kp_out))) return rc;
+    if ((rc = detect_nms_phase(ctx, d_role != nullptr, n, 1, nullptr, d_kp_out))) return rc;
     if (d_scores_out) KPL_CUDA(cudaMemcpyAsync(d_scores_out, ctx->score.p, (size_t)n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
     return detect_finish(ctx, n, n_kp_out);
+}
+
+// Boundaries of the (forest, view) ranges of a forest-major keypoint list over K x n points: {k*n + h_view_off[v]} for
+// k < K, v < V, then K*n.  One forest: d_view_off, the view offsets already on the device (no copy).  The host copy is a
+// member: a pageable source is staged by cudaMemcpyAsync before it returns, the member keeps it anyway.
+static int range_bounds(kpl_ctx* ctx, int K, int64_t n, const int64_t* h_view_off, int V, const int64_t* d_view_off, const int64_t** d_out)
+{
+    *d_out = d_view_off;
+    if (K == 1 && d_view_off) return KPL_OK;
+    const size_t nb = (size_t)K * V + 1;
+    ctx->range_off_h.resize(nb);
+    for (int k = 0; k < K; ++k)
+        for (int v = 0; v < V; ++v) ctx->range_off_h[(size_t)k * V + v] = (int64_t)k * n + h_view_off[v];
+    ctx->range_off_h[nb - 1] = (int64_t)K * n;
+    KPL_CUDA(ensure(ctx->range_off, nb));
+    KPL_CUDA(cudaMemcpyAsync(ctx->range_off.p, ctx->range_off_h.data(), nb * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
+    *d_out = ctx->range_off.p;
+    return KPL_OK;
 }
 
 // Every forest of the set over ONE cloud: one grid, one normal estimation, one feature pass whose tail walks the K forests,
@@ -647,38 +669,39 @@ static int run_detect_forests(kpl_ctx* ctx, const float4* d_xyz, const float4* d
     if ((rc = detect_begin(ctx))) return rc;
     if ((rc = prepare_params_grid(ctx, d_xyz, d_nrm, nullptr, n))) return rc;
     if ((rc = detect_score_phase(ctx, d_nrm != nullptr, false, n, K))) return rc;
-    KPL_CUDA(ensure(ctx->flag, (size_t)K * n));
-    for (int k = 0; k < K; ++k)
-        if ((rc = nms_flags(ctx, false, n, k, thresholds ? thresholds[k] : ctx->params.threshold))) return rc;
-    KPL_CUDA(launch_compact(ctx, (int64_t)K * n, d_kp_out));
-    // the forest boundaries; a pageable source is staged by cudaMemcpyAsync before it returns, the member keeps it anyway
-    ctx->forest_off_h.resize((size_t)K + 1);
-    for (int k = 0; k <= K; ++k) ctx->forest_off_h[(size_t)k] = (int64_t)k * n;
-    KPL_CUDA(ensure(ctx->forest_off, (size_t)K + 1));
-    KPL_CUDA(cudaMemcpyAsync(ctx->forest_off.p, ctx->forest_off_h.data(), ((size_t)K + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
-    KPL_CUDA(launch_view_ranges(ctx, (int64_t)K * n, d_kp_out, ctx->forest_off.p, K, d_kp_offsets_out));
+    if ((rc = detect_nms_phase(ctx, false, n, K, thresholds, d_kp_out))) return rc;
+    const int64_t whole[2] = {0, n};
+    const int64_t* d_bounds = nullptr;
+    if ((rc = range_bounds(ctx, K, n, whole, 1, nullptr, &d_bounds))) return rc;
+    KPL_CUDA(launch_view_ranges(ctx, (int64_t)K * n, d_kp_out, d_bounds, K, d_kp_offsets_out));
     if (d_scores_out) KPL_CUDA(cudaMemcpyAsync(d_scores_out, ctx->score.p, (size_t)K * n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
     return detect_finish(ctx, n, n_kp_out);
 }
 
 // A batch of independent views in ONE pass: one stacked grid, one query order, one launch per stage, per-view
 // keypoint ranges -- a 200 k-point view alone is 1.5 waves of the feature kernel and a handful of host round trips.
+// K forests (kpl_detect_batch_forests; thresholds NULL or one per forest) are scored from the one feature pass, each
+// forest's slice gets its own NMS, and the one compacted list is split into the K x V (forest, view) ranges.
 static int run_detect_batch(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, int64_t n, const int64_t* h_offsets, int nviews,
-                            float* d_scores_out, int32_t* d_kp_out, int64_t* d_kp_offsets_out, int64_t* n_kp_out)
+                            int K, const double* thresholds, float* d_scores_out, int32_t* d_kp_out, int64_t* d_kp_offsets_out,
+                            int64_t* n_kp_out)
 {
     detect_reset(ctx);
     if (n_kp_out) *n_kp_out = 0;
-    int rc = detect_check(ctx, n, 1, false);
+    int rc = detect_check(ctx, n, K, false);
     if (rc) return rc;
     if (ctx->params.grid_forced) return fail(ctx, KPL_E_INVALID, "a forced grid cannot be combined with a batch of views");
     ctx->stats.n_points = n; ctx->stats.n_views = nviews;
+    ctx->last_nforests = K;
     if (n == 0) return KPL_OK;
     if ((rc = detect_begin(ctx))) return rc;
     if ((rc = prepare_grid_batch(ctx, d_xyz, d_nrm, n, h_offsets, nviews))) return rc;
-    if ((rc = detect_score_phase(ctx, d_nrm != nullptr, false, n, 1))) return rc;
-    if ((rc = detect_nms_phase(ctx, false, n, d_kp_out))) return rc;
-    KPL_CUDA(launch_view_ranges(ctx, n, d_kp_out, ctx->view_offsets.p, nviews, d_kp_offsets_out));
-    if (d_scores_out) KPL_CUDA(cudaMemcpyAsync(d_scores_out, ctx->score.p, (size_t)n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
+    if ((rc = detect_score_phase(ctx, d_nrm != nullptr, false, n, K))) return rc;
+    if ((rc = detect_nms_phase(ctx, false, n, K, thresholds, d_kp_out))) return rc;
+    const int64_t* d_bounds = nullptr;
+    if ((rc = range_bounds(ctx, K, n, h_offsets, nviews, ctx->view_offsets.p, &d_bounds))) return rc;
+    KPL_CUDA(launch_view_ranges(ctx, (int64_t)K * n, d_kp_out, d_bounds, K * nviews, d_kp_offsets_out));
+    if (d_scores_out) KPL_CUDA(cudaMemcpyAsync(d_scores_out, ctx->score.p, (size_t)K * n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
     rc = detect_finish(ctx, n, n_kp_out);
     ctx->stats.n_views = nviews;
     return rc;
@@ -689,16 +712,19 @@ static int run_detect_batch(kpl_ctx* ctx, const float4* d_xyz, const float4* d_n
 // results mapped back to pixel order.  Each frame's view is the cloud the single-frame path (computeOrganized /
 // KeypointLearningDetector::compute) detects after dropping its NaN points, in the same order, so its results are that
 // path's.  One host round trip for the per-frame finite counts, which the batch needs as host view offsets; a frame
-// without a finite point is left out of the batch (views must not be empty) and gets an empty keypoint range.
+// without a finite point is left out of the batch (views must not be empty) and gets an empty keypoint range.  K forests
+// (kpl_detect_batch_organized_forests) score the inner batch from one feature pass; the results stay forest-major through
+// the map back: K x F x W*H scores, K x F + 1 keypoint offsets.
 static int run_detect_organized_batch(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, int32_t W, int32_t H, int32_t F,
-                                      float smoothing_size, const float* h_viewpoints, float* d_scores_out, int32_t* d_kp_out,
-                                      int64_t* d_kp_offsets_out, int64_t* n_kp_out)
+                                      float smoothing_size, const float* h_viewpoints, int K, const double* thresholds,
+                                      float* d_scores_out, int32_t* d_kp_out, int64_t* d_kp_offsets_out, int64_t* n_kp_out)
 {
     const int64_t n = (int64_t)W * H, total = n * F;
-    int rc = detect_check(ctx, total, 1, false);
+    int rc = detect_check(ctx, total, K, false);
     if (rc) return rc;
     if (ctx->params.grid_forced) return fail(ctx, KPL_E_INVALID, "a forced grid cannot be combined with a batch of frames");
     ctx->stats.n_views = F;
+    ctx->last_nforests = K;
     if ((rc = detect_begin(ctx))) return rc;
     if (!d_nrm) {
         const float* d_vp = nullptr;
@@ -711,7 +737,7 @@ static int run_detect_organized_batch(kpl_ctx* ctx, const float4* d_xyz, const f
         KPL_CUDA(launch_normals_integral_image(ctx, d_xyz, W, H, F, smoothing_size, d_vp, ctx->in_nrm.p));
         d_nrm = ctx->in_nrm.p;
     }
-    KPL_CUDA(launch_organized_select(ctx, d_xyz, n, F, d_scores_out));
+    KPL_CUDA(launch_organized_select(ctx, d_xyz, n, F, K, d_scores_out));
     KPL_CUDA(cudaEventRecord(ctx->ev[6], ctx->stream));
     std::vector<int64_t> frame_off((size_t)F + 1);
     KPL_CUDA(cudaMemcpyAsync(frame_off.data(), ctx->org_frame_off.p, frame_off.size() * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
@@ -723,7 +749,7 @@ static int run_detect_organized_batch(kpl_ctx* ctx, const float4* d_xyz, const f
         if (frame_off[(size_t)f + 1] > frame_off[(size_t)f]) view_off.push_back(frame_off[(size_t)f + 1]);
     kpl_timings& T = ctx->timings;
     if (m == 0) {
-        KPL_CUDA(cudaMemsetAsync(d_kp_offsets_out, 0, ((size_t)F + 1) * sizeof(int64_t), ctx->stream));
+        KPL_CUDA(cudaMemsetAsync(d_kp_offsets_out, 0, ((size_t)K * F + 1) * sizeof(int64_t), ctx->stream));
         cudaEventElapsedTime(&T.normals_ms, ctx->ev[0], ctx->ev[6]);
         T.total_ms = T.normals_ms;
         ctx->stats.n_points = 0; ctx->stats.kernel_launches = ctx->launches; ctx->stats.host_syncs = ctx->syncs;
@@ -731,9 +757,9 @@ static int run_detect_organized_batch(kpl_ctx* ctx, const float4* d_xyz, const f
     }
     KPL_CUDA(launch_organized_gather(ctx, d_xyz, d_nrm, m));
     if ((rc = prepare_grid_batch(ctx, ctx->org_xyz.p, ctx->org_nrm.p, m, view_off.data(), (int)view_off.size() - 1))) return rc;
-    if ((rc = detect_score_phase(ctx, true, false, m, 1))) return rc;
-    if ((rc = detect_nms_phase(ctx, false, m, d_kp_out))) return rc;
-    KPL_CUDA(launch_organized_map_back(ctx, m, n, F, d_scores_out, d_kp_out, d_kp_offsets_out));
+    if ((rc = detect_score_phase(ctx, true, false, m, K))) return rc;
+    if ((rc = detect_nms_phase(ctx, false, m, K, thresholds, d_kp_out))) return rc;
+    KPL_CUDA(launch_organized_map_back(ctx, m, n, F, K, d_scores_out, d_kp_out, d_kp_offsets_out));
     if ((rc = detect_finish(ctx, m, n_kp_out))) return rc;
     // the integral images and the compaction are part of the normals stage; the grid stage starts after them
     float prep = 0.f;
@@ -911,39 +937,76 @@ static int check_view_offsets(kpl_ctx* ctx, const int64_t* view_offsets, int32_t
     return KPL_OK;
 }
 
-int kpl_detect_batch(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
-                     const int64_t* view_offsets, int32_t n_views, float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out)
+// kpl_detect_batch (K = 1) and kpl_detect_batch_forests: host views in, host results out, forest-major.  The forests' call
+// checks its point and forest counts before it touches the device.
+static int detect_batch_host(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
+                             const int64_t* view_offsets, int32_t n_views, int K, const double* thresholds, float* scores_out,
+                             int32_t* kp_idx_out, int64_t* kp_offsets_out)
 {
-    if (!ctx) return KPL_E_INVALID;
     if (!kp_idx_out || !kp_offsets_out) return fail(ctx, KPL_E_INVALID, "kp_idx_out / kp_offsets_out is NULL");
     int64_t n = 0;
     int rc = check_view_offsets(ctx, view_offsets, n_views, n);
     if (rc) return rc;
+    if (K != 1 && (rc = detect_check(ctx, n, K, false))) return rc;
     if ((rc = upload_inputs(ctx, xyz, xyz_stride, normals, normals_stride, nullptr, n))) return rc;
-    KPL_CUDA(ensure(ctx->kp_idx, (size_t)n));
-    KPL_CUDA(ensure(ctx->scratch_f, ((size_t)n_views + 1) * 2 + 16));
+    const size_t nr = (size_t)K * n_views + 1;
+    KPL_CUDA(ensure(ctx->kp_idx, (size_t)K * n));
+    KPL_CUDA(ensure(ctx->scratch_f, nr * 2 + 16));
     int64_t* d_kpo = reinterpret_cast<int64_t*>(ctx->scratch_f.p);
     int64_t nkp = 0;
-    rc = run_detect_batch(ctx, ctx->in_xyz.p, normals ? ctx->in_nrm.p : nullptr, n, view_offsets, n_views, nullptr, ctx->kp_idx.p, d_kpo, &nkp);
+    rc = run_detect_batch(ctx, ctx->in_xyz.p, normals ? ctx->in_nrm.p : nullptr, n, view_offsets, n_views, K, thresholds, nullptr,
+                          ctx->kp_idx.p, d_kpo, &nkp);
     if (rc) return rc;
-    if (scores_out) KPL_CUDA(cudaMemcpyAsync(scores_out, ctx->score.p, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    if (scores_out) KPL_CUDA(cudaMemcpyAsync(scores_out, ctx->score.p, (size_t)K * n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     if (nkp > 0) KPL_CUDA(cudaMemcpyAsync(kp_idx_out, ctx->kp_idx.p, (size_t)nkp * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    KPL_CUDA(cudaMemcpyAsync(kp_offsets_out, d_kpo, ((size_t)n_views + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    KPL_CUDA(cudaMemcpyAsync(kp_offsets_out, d_kpo, nr * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
     KPL_CUDA(cudaStreamSynchronize(ctx->stream));
     ctx->syncs++; ctx->stats.host_syncs = ctx->syncs;
     return KPL_OK;
+}
+
+int kpl_detect_batch(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
+                     const int64_t* view_offsets, int32_t n_views, float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out)
+{
+    if (!ctx) return KPL_E_INVALID;
+    return detect_batch_host(ctx, xyz, xyz_stride, normals, normals_stride, view_offsets, n_views, 1, nullptr, scores_out, kp_idx_out,
+                             kp_offsets_out);
+}
+
+int kpl_detect_batch_forests(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
+                             const int64_t* view_offsets, int32_t n_views, const double* thresholds, float* scores_out,
+                             int32_t* kp_idx_out, int64_t* kp_offsets_out)
+{
+    if (!ctx) return KPL_E_INVALID;
+    detect_reset(ctx);
+    return detect_batch_host(ctx, xyz, xyz_stride, normals, normals_stride, view_offsets, n_views, (int)ctx->forests.info.size(), thresholds,
+                             scores_out, kp_idx_out, kp_offsets_out);
+}
+
+static int detect_batch_dev(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, const int64_t* view_offsets, int32_t n_views, int K,
+                            const double* thresholds, void* d_scores, void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out)
+{
+    if (!d_xyz4 || !d_kp_idx || !d_kp_offsets) return fail(ctx, KPL_E_INVALID, "NULL device pointer");
+    int64_t n = 0;
+    int rc = check_view_offsets(ctx, view_offsets, n_views, n);
+    if (rc) return rc;
+    return run_detect_batch(ctx, (const float4*)d_xyz4, (const float4*)d_normals4, n, view_offsets, n_views, K, thresholds, (float*)d_scores,
+                            (int32_t*)d_kp_idx, (int64_t*)d_kp_offsets, n_kp_out);
 }
 
 int kpl_detect_batch_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, const int64_t* view_offsets, int32_t n_views,
                             void* d_scores, void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out)
 {
     if (!ctx) return KPL_E_INVALID;
-    if (!d_xyz4 || !d_kp_idx || !d_kp_offsets) return fail(ctx, KPL_E_INVALID, "NULL device pointer");
-    int64_t n = 0;
-    int rc = check_view_offsets(ctx, view_offsets, n_views, n);
-    if (rc) return rc;
-    return run_detect_batch(ctx, (const float4*)d_xyz4, (const float4*)d_normals4, n, view_offsets, n_views, (float*)d_scores,
-                            (int32_t*)d_kp_idx, (int64_t*)d_kp_offsets, n_kp_out);
+    return detect_batch_dev(ctx, d_xyz4, d_normals4, view_offsets, n_views, 1, nullptr, d_scores, d_kp_idx, d_kp_offsets, n_kp_out);
+}
+
+int kpl_detect_batch_forests_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, const int64_t* view_offsets, int32_t n_views,
+                                    const double* thresholds, void* d_scores, void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out)
+{
+    if (!ctx) return KPL_E_INVALID;
+    return detect_batch_dev(ctx, d_xyz4, d_normals4, view_offsets, n_views, (int)ctx->forests.info.size(), thresholds, d_scores, d_kp_idx,
+                            d_kp_offsets, n_kp_out);
 }
 
 static int check_organized_batch(kpl_ctx* ctx, int32_t width, int32_t height, int32_t n_frames, float smoothing_size)
@@ -954,38 +1017,58 @@ static int check_organized_batch(kpl_ctx* ctx, int32_t width, int32_t height, in
     return KPL_OK;
 }
 
-int kpl_detect_batch_organized(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
-                               int32_t width, int32_t height, int32_t n_frames, float smoothing_size, const float* viewpoints,
-                               float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out)
+// kpl_detect_batch_organized (K = 1) and kpl_detect_batch_organized_forests: host frames in, host results out,
+// forest-major.  The forests' call checks its point and forest counts before it touches the device.
+static int detect_organized_host(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
+                                 int32_t width, int32_t height, int32_t n_frames, float smoothing_size, const float* viewpoints, int K,
+                                 const double* thresholds, float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out)
 {
-    if (!ctx) return KPL_E_INVALID;
     detect_reset(ctx);
     ctx->stats.n_views = n_frames;
     if (!xyz || !kp_idx_out || !kp_offsets_out) return fail(ctx, KPL_E_INVALID, "xyz / kp_idx_out / kp_offsets_out is NULL");
     int rc = check_organized_batch(ctx, width, height, n_frames, smoothing_size);
     if (rc) return rc;
     const int64_t total = (int64_t)width * height * n_frames;
+    if (K != 1 && (rc = detect_check(ctx, total, K, false))) return rc;
     if ((rc = upload_inputs(ctx, xyz, xyz_stride, normals, normals_stride, nullptr, total))) return rc;
-    KPL_CUDA(ensure(ctx->kp_idx, (size_t)total));
-    KPL_CUDA(ensure(ctx->org_kp_off, (size_t)n_frames + 1));
-    if (scores_out) KPL_CUDA(ensure(ctx->org_score, (size_t)total));
+    const size_t nr = (size_t)K * n_frames + 1;
+    KPL_CUDA(ensure(ctx->kp_idx, (size_t)K * total));
+    KPL_CUDA(ensure(ctx->org_kp_off, nr));
+    if (scores_out) KPL_CUDA(ensure(ctx->org_score, (size_t)K * total));
     int64_t nkp = 0;
     rc = run_detect_organized_batch(ctx, ctx->in_xyz.p, normals ? ctx->in_nrm.p : nullptr, width, height, n_frames, smoothing_size, viewpoints,
-                                    scores_out ? ctx->org_score.p : nullptr, ctx->kp_idx.p, ctx->org_kp_off.p, &nkp);
+                                    K, thresholds, scores_out ? ctx->org_score.p : nullptr, ctx->kp_idx.p, ctx->org_kp_off.p, &nkp);
     if (rc) return rc;
-    if (scores_out) KPL_CUDA(cudaMemcpyAsync(scores_out, ctx->org_score.p, (size_t)total * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    if (scores_out) KPL_CUDA(cudaMemcpyAsync(scores_out, ctx->org_score.p, (size_t)K * total * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     if (nkp > 0) KPL_CUDA(cudaMemcpyAsync(kp_idx_out, ctx->kp_idx.p, (size_t)nkp * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    KPL_CUDA(cudaMemcpyAsync(kp_offsets_out, ctx->org_kp_off.p, ((size_t)n_frames + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    KPL_CUDA(cudaMemcpyAsync(kp_offsets_out, ctx->org_kp_off.p, nr * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
     KPL_CUDA(cudaStreamSynchronize(ctx->stream));
     ctx->syncs++; ctx->stats.host_syncs = ctx->syncs;
     return KPL_OK;
 }
 
-int kpl_detect_batch_organized_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, int32_t width, int32_t height,
-                                      int32_t n_frames, float smoothing_size, const float* viewpoints, void* d_scores, void* d_kp_idx,
-                                      void* d_kp_offsets, int64_t* n_kp_out)
+int kpl_detect_batch_organized(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
+                               int32_t width, int32_t height, int32_t n_frames, float smoothing_size, const float* viewpoints,
+                               float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out)
 {
     if (!ctx) return KPL_E_INVALID;
+    return detect_organized_host(ctx, xyz, xyz_stride, normals, normals_stride, width, height, n_frames, smoothing_size, viewpoints, 1, nullptr,
+                                 scores_out, kp_idx_out, kp_offsets_out);
+}
+
+int kpl_detect_batch_organized_forests(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
+                                       int32_t width, int32_t height, int32_t n_frames, float smoothing_size, const float* viewpoints,
+                                       const double* thresholds, float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out)
+{
+    if (!ctx) return KPL_E_INVALID;
+    return detect_organized_host(ctx, xyz, xyz_stride, normals, normals_stride, width, height, n_frames, smoothing_size, viewpoints,
+                                 (int)ctx->forests.info.size(), thresholds, scores_out, kp_idx_out, kp_offsets_out);
+}
+
+static int detect_organized_dev(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, int32_t width, int32_t height, int32_t n_frames,
+                                float smoothing_size, const float* viewpoints, int K, const double* thresholds, void* d_scores, void* d_kp_idx,
+                                void* d_kp_offsets, int64_t* n_kp_out)
+{
     detect_reset(ctx);
     ctx->stats.n_views = n_frames;
     if (n_kp_out) *n_kp_out = 0;
@@ -994,7 +1077,25 @@ int kpl_detect_batch_organized_device(kpl_ctx* ctx, const void* d_xyz4, const vo
     if (rc) return rc;
     KPL_CUDA(cudaSetDevice(ctx->device));
     return run_detect_organized_batch(ctx, (const float4*)d_xyz4, (const float4*)d_normals4, width, height, n_frames, smoothing_size, viewpoints,
-                                      (float*)d_scores, (int32_t*)d_kp_idx, (int64_t*)d_kp_offsets, n_kp_out);
+                                      K, thresholds, (float*)d_scores, (int32_t*)d_kp_idx, (int64_t*)d_kp_offsets, n_kp_out);
+}
+
+int kpl_detect_batch_organized_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, int32_t width, int32_t height,
+                                      int32_t n_frames, float smoothing_size, const float* viewpoints, void* d_scores, void* d_kp_idx,
+                                      void* d_kp_offsets, int64_t* n_kp_out)
+{
+    if (!ctx) return KPL_E_INVALID;
+    return detect_organized_dev(ctx, d_xyz4, d_normals4, width, height, n_frames, smoothing_size, viewpoints, 1, nullptr, d_scores, d_kp_idx,
+                                d_kp_offsets, n_kp_out);
+}
+
+int kpl_detect_batch_organized_forests_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, int32_t width, int32_t height,
+                                              int32_t n_frames, float smoothing_size, const float* viewpoints, const double* thresholds,
+                                              void* d_scores, void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out)
+{
+    if (!ctx) return KPL_E_INVALID;
+    return detect_organized_dev(ctx, d_xyz4, d_normals4, width, height, n_frames, smoothing_size, viewpoints, (int)ctx->forests.info.size(),
+                                thresholds, d_scores, d_kp_idx, d_kp_offsets, n_kp_out);
 }
 
 int kpl_normals(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, int64_t n, float* normals_out)

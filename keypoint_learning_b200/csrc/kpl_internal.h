@@ -126,10 +126,11 @@ struct kpl_ctx {
     kpl::DevBuf<float> s_score, score;           // sorted order / original order
     kpl::DevBuf<uint8_t> flag;                   // keypoint flag, original order
     kpl::DevBuf<uint8_t> fragile;                // near-split flag of the forest walk, original order (forest.cuh)
-    // kpl_detect_forests: scores, flags and fragile flags hold K x n entries, forest-major; forest_off = {0, n, .., K*n}
-    // (host copy kept for the asynchronous upload)
-    kpl::DevBuf<int64_t> forest_off;
-    std::vector<int64_t> forest_off_h;
+    // kpl_detect_forests / kpl_detect_batch_forests (and the organized batch's inner batch): scores, flags and fragile flags
+    // hold K x n entries, forest-major.  range_off = the K*V + 1 boundaries {k*n + view_offsets[v]} of the (forest, view)
+    // ranges of the keypoint list (host copy kept for the asynchronous upload); a single cloud is V = 1
+    kpl::DevBuf<int64_t> range_off;
+    std::vector<int64_t> range_off_h;
     kpl::DevBuf<kpl::ViewDesc> views;            // kpl_detect_batch: per-view grids
     kpl::DevBuf<int32_t> layer_view;
     kpl::DevBuf<int64_t> view_offsets;
@@ -179,13 +180,15 @@ cudaError_t launch_gather_keypoints(kpl_ctx* c, const float4* d_xyz, const int32
 cudaError_t launch_normals_integral_image(kpl_ctx* c, const float4* d_xyz, int W, int H, int nframes, float smoothing_size,
                                           const float* d_viewpoints, float4* d_out);
 // organized frames (n pixels each) -> finite pixels in ascending order (org_pix) and org_frame_off; d_scores (NULL or
-// nframes * n floats) is set to NaN
-cudaError_t launch_organized_select(kpl_ctx* c, const float4* d_xyz, int64_t n, int nframes, float* d_scores);
+// nforests x nframes * n floats, forest-major) is set to NaN
+cudaError_t launch_organized_select(kpl_ctx* c, const float4* d_xyz, int64_t n, int nframes, int nforests, float* d_scores);
 // the m selected pixels' positions and normals (per pixel) -> org_xyz / org_nrm
 cudaError_t launch_organized_gather(kpl_ctx* c, const float4* d_xyz, const float4* d_nrm, int64_t m);
-// after the detection of the m compacted points: scores to pixel order, keypoints (in place) to frame-local pixel indices,
-// frame keypoint offsets (nframes + 1)
-cudaError_t launch_organized_map_back(kpl_ctx* c, int64_t m, int64_t n, int nframes, float* d_scores, int32_t* d_kp, int64_t* d_kp_off);
+// after the detection of the m compacted points by nforests forests (forest-major K x m scores, keypoints ascending in
+// [0, K*m)): scores to pixel order (forest k's at k * nframes * n), keypoints (in place) to frame-local pixel indices,
+// (forest, frame) keypoint offsets (nforests * nframes + 1)
+cudaError_t launch_organized_map_back(kpl_ctx* c, int64_t m, int64_t n, int nframes, int nforests, float* d_scores, int32_t* d_kp,
+                                      int64_t* d_kp_off);
 cudaError_t build_lists(kpl_ctx* c, int64_t n, int span_n, bool curve_normals, bool want_features, bool use_role, int64_t longest_first_below);
 cudaError_t launch_count_occupied_cells(kpl_ctx* c, int64_t n, unsigned long long* d_out);
 cudaError_t build_query_list(kpl_ctx* c, int64_t n, const int32_t* d_indices, int64_t m);
@@ -227,7 +230,7 @@ int grid_reach(double radius, double cell);
 
 // detection phases (capi.cu), shared with the slab-sharded driver (shard.cu); all but detect_reset return kpl_status
 void detect_reset(kpl_ctx* ctx);
-// nforests: the call scores forests 0 .. nforests - 1 (kpl_detect_forests: all of them; every other entry point: 1).
+// nforests: the call scores forests 0 .. nforests - 1 (the *_forests entry points: all of them; every other entry point: 1).
 // with_role: a caller-supplied role array (kpl_detect*), which rules out draws-remove NMS; the kpl_shard_* driver passes false
 int detect_check(kpl_ctx* ctx, int64_t n, int nforests, bool with_role);
 int detect_begin(kpl_ctx* ctx);
@@ -235,7 +238,9 @@ int detect_begin(kpl_ctx* ctx);
 int prepare_grid(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, const uint8_t* d_role, int64_t n, const ForcedGrid* forced, double cell_override = 0.0);
 // scores of forests 0 .. nforests - 1, forest-major
 int detect_score_phase(kpl_ctx* ctx, bool normals_given, bool use_role, int64_t n, int nforests);
-int detect_nms_phase(kpl_ctx* ctx, bool use_role, int64_t n, int32_t* d_kp_out);
+// threshold + NMS of each of the nforests forest-major score slices (thresholds: NULL = params.threshold, else one per
+// forest), then one compaction of the nforests x n flags into an ascending list of indices in [0, nforests * n)
+int detect_nms_phase(kpl_ctx* ctx, bool use_role, int64_t n, int nforests, const double* thresholds, int32_t* d_kp_out);
 int detect_finish(kpl_ctx* ctx, int64_t n, int64_t* n_kp_out);
 
 template <typename T>

@@ -210,16 +210,18 @@ cudaError_t launch_normals_integral_image(kpl_ctx* c, const float4* d_xyz, int W
 }
 
 // ---- batches of organized frames: finite pixels -> the concatenated views of a batch, and back --------------------
-// Finite flag of every pixel (x, y and z finite: pcl::isFinite, the rule of bbox_kernel); the pixel-order scores start as
-// NaN (the value a point the detection never saw gets, as std::nanf("") in the C++ facade and np.nan in capi.py).
-__global__ void __launch_bounds__(256) org_finite_kernel(const float4* __restrict__ xyz, int64_t total, uint8_t* __restrict__ flag,
+// Finite flag of every pixel (x, y and z finite: pcl::isFinite, the rule of bbox_kernel); the pixel-order scores of all
+// nforests slices start as NaN (the value a point the detection never saw gets, as std::nanf("") in the C++ facade and
+// np.nan in capi.py).
+__global__ void __launch_bounds__(256) org_finite_kernel(const float4* __restrict__ xyz, int64_t total, int nforests, uint8_t* __restrict__ flag,
                                                          float* __restrict__ scores)
 {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= total) return;
     const float4 p = __ldg(xyz + i);
     flag[i] = isfinite(p.x) && isfinite(p.y) && isfinite(p.z);
-    if (scores) scores[i] = __int_as_float(0x7FC00000);
+    if (scores)
+        for (int k = 0; k < nforests; ++k) scores[k * total + i] = __int_as_float(0x7FC00000);
 }
 
 // frame_off[f] = first compacted point of frame f = lower bound of f * n in the ascending pixel list; frame_off[nframes]
@@ -247,41 +249,51 @@ __global__ void __launch_bounds__(256) org_gather_kernel(const float4* __restric
     nrm_c[k] = __ldg(nrm + p);
 }
 
-// kp_off[f] = first keypoint of frame f: the keypoints are ascending compacted indices
+// kp_off[j] = first keypoint of (forest j / nframes, frame j % nframes): the keypoints are ascending indices into the
+// forest-major K x m compacted points, forest k's frame f starts at k*m + frame_off[f] (m = frame_off[nframes]), and
+// j = K * nframes gives K*m, the end of the list
 __global__ void __launch_bounds__(256) org_kp_offsets_kernel(const int32_t* __restrict__ kp, const int32_t* __restrict__ d_nkp,
-                                                             const int64_t* __restrict__ frame_off, int nframes, int64_t* __restrict__ kp_off)
+                                                             const int64_t* __restrict__ frame_off, int nframes, int nforests,
+                                                             int64_t* __restrict__ kp_off)
 {
-    const int f = blockIdx.x * blockDim.x + threadIdx.x;
-    if (f > nframes) return;
-    const int64_t bound = frame_off[f];
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j > nforests * nframes) return;
+    const int k = j / nframes;
+    const int64_t bound = k * frame_off[nframes] + frame_off[j - k * nframes];
     int lo = 0, hi = *d_nkp;
     while (lo < hi) {
         const int mid = (lo + hi) >> 1;
         if ((int64_t)kp[mid] < bound) lo = mid + 1; else hi = mid;
     }
-    kp_off[f] = lo;
+    kp_off[j] = lo;
 }
 
-// compacted scores -> pixel order; keypoints: compacted index -> frame-local pixel index, in place
-__global__ void __launch_bounds__(256) org_map_back_kernel(const int32_t* __restrict__ pix, int64_t m, int64_t n, const float* __restrict__ score_c,
-                                                           float* __restrict__ scores, int32_t* __restrict__ kp, const int32_t* __restrict__ d_nkp)
+// forest-major compacted scores (K x m) -> pixel order (forest k's at k * total, total = nframes * n pixels); keypoints:
+// index c into the K x m compacted points -> frame-local pixel index of point c - (c / m) * m, in place
+__global__ void __launch_bounds__(256) org_map_back_kernel(const int32_t* __restrict__ pix, int64_t m, int64_t n, int64_t total, int64_t km,
+                                                           const float* __restrict__ score_c, float* __restrict__ scores,
+                                                           int32_t* __restrict__ kp, const int32_t* __restrict__ d_nkp)
 {
-    const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (k >= m) return;
-    if (scores) scores[pix[k]] = score_c[k];
-    if (k < *d_nkp) {
-        const int64_t p = pix[kp[k]];
-        kp[k] = (int32_t)(p - p / n * n);
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= km) return;
+    if (scores) {
+        const int64_t k = i / m;
+        scores[k * total + pix[i - k * m]] = score_c[i];
+    }
+    if (i < *d_nkp) {
+        const int64_t c = kp[i];
+        const int64_t p = pix[c - c / m * m];
+        kp[i] = (int32_t)(p - p / n * n);
     }
 }
 
-cudaError_t launch_organized_select(kpl_ctx* c, const float4* d_xyz, int64_t n, int nframes, float* d_scores)
+cudaError_t launch_organized_select(kpl_ctx* c, const float4* d_xyz, int64_t n, int nframes, int nforests, float* d_scores)
 {
     const int64_t total = n * nframes;
     cudaError_t e;
     if ((e = ensure(c->org_flag, (size_t)total)) || (e = ensure(c->org_pix, (size_t)total)) || (e = ensure(c->org_frame_off, (size_t)nframes + 2)))
         return e;
-    org_finite_kernel<<<(unsigned)((total + 255) / 256), 256, 0, c->stream>>>(d_xyz, total, c->org_flag.p, d_scores);
+    org_finite_kernel<<<(unsigned)((total + 255) / 256), 256, 0, c->stream>>>(d_xyz, total, nforests, c->org_flag.p, d_scores);
     thrust::counting_iterator<int32_t> it(0);
     int64_t* d_m = c->org_frame_off.p + nframes + 1;
     size_t bytes = 0;
@@ -303,11 +315,13 @@ cudaError_t launch_organized_gather(kpl_ctx* c, const float4* d_xyz, const float
     return cudaGetLastError();
 }
 
-cudaError_t launch_organized_map_back(kpl_ctx* c, int64_t m, int64_t n, int nframes, float* d_scores, int32_t* d_kp, int64_t* d_kp_off)
+cudaError_t launch_organized_map_back(kpl_ctx* c, int64_t m, int64_t n, int nframes, int nforests, float* d_scores, int32_t* d_kp,
+                                      int64_t* d_kp_off)
 {
     const int32_t* d_nkp = (const int32_t*)(c->counters.p + 3);
-    org_kp_offsets_kernel<<<(nframes + 1 + 255) / 256, 256, 0, c->stream>>>(d_kp, d_nkp, c->org_frame_off.p, nframes, d_kp_off);
-    org_map_back_kernel<<<(unsigned)((m + 255) / 256), 256, 0, c->stream>>>(c->org_pix.p, m, n, c->score.p, d_scores, d_kp, d_nkp);
+    const int64_t km = m * nforests;
+    org_kp_offsets_kernel<<<(nforests * nframes + 1 + 255) / 256, 256, 0, c->stream>>>(d_kp, d_nkp, c->org_frame_off.p, nframes, nforests, d_kp_off);
+    org_map_back_kernel<<<(unsigned)((km + 255) / 256), 256, 0, c->stream>>>(c->org_pix.p, m, n, n * nframes, km, c->score.p, d_scores, d_kp, d_nkp);
     c->launches += 2;
     return cudaGetLastError();
 }

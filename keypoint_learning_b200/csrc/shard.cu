@@ -429,7 +429,7 @@ int phase_nms(kpl_shard* s)
         KS_CUDA(launch_nms_draws_classify(c, s->n_loc, true, c->s_score.p, c->params.threshold));
         return pack_states(s);
     }
-    int rc = detect_nms_phase(c, true, s->n_loc, s->kp_local.p);
+    int rc = detect_nms_phase(c, true, s->n_loc, 1, nullptr, s->kp_local.p);
     return rc ? rc : phase_records(s);
 }
 

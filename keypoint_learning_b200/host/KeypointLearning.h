@@ -230,8 +230,57 @@ public:
     bool computeOrganizedBatch(const std::vector<PointCloudInConstPtr>& frames, std::vector<PointCloudOut>& outputs,
                                std::vector<pcl::PointIndices>* indices = nullptr)
     {
-        outputs.assign(frames.size(), PointCloudOut());
-        if (indices) indices->assign(frames.size(), pcl::PointIndices());
+        return detectOrganizedFrames(frames, 1, outputs, indices, [&](const float* pts, const float* vps, int32_t W, int32_t H, int32_t F,
+                                                                      float* scores, int32_t* idx, int64_t* off) {
+            return kpl_detect_batch_organized(ctx_, pts, (int32_t)sizeof(PointInT), nullptr, 0, W, H, F, 5.0f, vps, scores, idx, off);
+        });
+    }
+
+    // B200 build only: computeOrganizedBatch for every forest of the set (loadForest + addForest) from one feature pass
+    // (kpl_detect_batch_organized_forests).  outputs[k][f] is what computeOrganizedBatch returns for frame f with only forest
+    // k loaded, at threshold (*thresholds)[k] (default: the prediction threshold); (*indices)[k][f], when asked for, its
+    // keypoint indices.  A thresholds vector that does not hold one value per forest is refused.
+    bool computeOrganizedBatchForests(const std::vector<PointCloudInConstPtr>& frames, std::vector<std::vector<PointCloudOut>>& outputs,
+                                      std::vector<std::vector<pcl::PointIndices>>* indices = nullptr,
+                                      const std::vector<double>* thresholds = nullptr)
+    {
+        outputs.clear();
+        if (indices) indices->clear();
+        int32_t K = 0;
+        if (ctx_) kpl_forest_count(ctx_, &K);
+        if (thresholds && thresholds->size() != (size_t)K) {
+            std::fprintf(stderr, "[pcl::%s::computeOrganizedBatchForests] %zu thresholds for %d forests\n", name_.c_str(), thresholds->size(), K);
+            return false;
+        }
+        std::vector<PointCloudOut> flat;
+        std::vector<pcl::PointIndices> flat_idx;
+        const bool ok = detectOrganizedFrames(frames, std::max(K, 1), flat, indices ? &flat_idx : nullptr,
+                                              [&](const float* pts, const float* vps, int32_t W, int32_t H, int32_t F, float* scores, int32_t* idx,
+                                                  int64_t* off) {
+            return kpl_detect_batch_organized_forests(ctx_, pts, (int32_t)sizeof(PointInT), nullptr, 0, W, H, F, 5.0f, vps,
+                                                      thresholds ? thresholds->data() : nullptr, scores, idx, off);
+        });
+        if (!ok) return false;
+        const size_t F = frames.size();
+        for (size_t k = 0; k < (size_t)K; ++k) {
+            outputs.emplace_back(flat.begin() + k * F, flat.begin() + (k + 1) * F);
+            if (indices) indices->emplace_back(flat_idx.begin() + k * F, flat_idx.begin() + (k + 1) * F);
+        }
+        return true;
+    }
+
+    kpl_ctx* context() { return ctx_; }
+
+protected:
+    // The frame checks and packing of computeOrganizedBatch(Forests): detect(points, viewpoints, W, H, F, scores, indices,
+    // offsets) runs K forests over the packed frames; outputs[k * F + f] (and (*indices)[k * F + f]) receive forest k's
+    // keypoints of frame f.
+    template <typename Detect>
+    bool detectOrganizedFrames(const std::vector<PointCloudInConstPtr>& frames, int K, std::vector<PointCloudOut>& outputs,
+                               std::vector<pcl::PointIndices>* indices, Detect detect)
+    {
+        outputs.assign((size_t)K * frames.size(), PointCloudOut());
+        if (indices) indices->assign((size_t)K * frames.size(), pcl::PointIndices());
         if (!ctx_ || frames.empty() || !frames[0]) {
             std::fprintf(stderr, "[pcl::%s::initCompute] init failed!\n", name_.c_str());
             return false;
@@ -245,29 +294,30 @@ public:
         if (!checkSearch()) return false;
         const size_t n = (size_t)W * H, F = frames.size();
         std::vector<PointInT> pts(n * F);
-        std::vector<float> vps(3 * F), scores(n * F);
+        std::vector<float> vps(3 * F), scores((size_t)K * n * F);
         for (size_t f = 0; f < F; ++f) {
             std::copy(frames[f]->points.begin(), frames[f]->points.end(), pts.begin() + f * n);
             for (int a = 0; a < 3; ++a) vps[3 * f + a] = frames[f]->sensor_origin_[a];
         }
-        std::vector<int32_t> idx(n * F);
-        std::vector<int64_t> off(F + 1);
+        std::vector<int32_t> idx((size_t)K * n * F);
+        std::vector<int64_t> off((size_t)K * F + 1);
         if (kpl_set_params(ctx_, &p_) != KPL_OK ||
-            kpl_detect_batch_organized(ctx_, reinterpret_cast<const float*>(pts.data()), (int32_t)sizeof(PointInT), nullptr, 0, (int32_t)W, (int32_t)H,
-                                       (int32_t)F, 5.0f, vps.data(), scores.data(), idx.data(), off.data()) != KPL_OK) {
+            detect(reinterpret_cast<const float*>(pts.data()), vps.data(), (int32_t)W, (int32_t)H, (int32_t)F, scores.data(), idx.data(),
+                   off.data()) != KPL_OK) {
             std::fprintf(stderr, "[pcl::%s::compute] %s\n", name_.c_str(), kpl_last_error(ctx_));
             return false;
         }
-        for (size_t f = 0; f < F; ++f) {
-            PointCloudOut& out = outputs[f];
-            for (int64_t k = off[f]; k < off[f + 1]; ++k) {                      // hpp:246-253
+        for (size_t r = 0; r < (size_t)K * F; ++r) {
+            const size_t f = r % F;
+            PointCloudOut& out = outputs[r];
+            for (int64_t k = off[r]; k < off[r + 1]; ++k) {                      // hpp:246-253
                 const int32_t i = idx[(size_t)k];
                 const PointInT& p = frames[f]->points[(size_t)i];
                 PointOutT o;
                 o.x = p.x; o.y = p.y; o.z = p.z;
-                o.intensity = scores[f * n + (size_t)i];
+                o.intensity = scores[r * n + (size_t)i];
                 out.points.push_back(o);
-                if (indices) (*indices)[f].indices.push_back(i);
+                if (indices) (*indices)[r].indices.push_back(i);
             }
             out.height = 1;
             out.width = (uint32_t)out.points.size();
@@ -276,9 +326,6 @@ public:
         return true;
     }
 
-    kpl_ctx* context() { return ctx_; }
-
-protected:
     // detect(points, normals or nullptr, count) on the input cloud.  Non-dense clouds (Kinect / organized PCDs carry NaN
     // points; found by the device's bounding-box pass, KPL_E_NONFINITE): the reference's kd-tree ignores them and runForest
     // skips them (hpp:277), so detect runs again on the compacted finite points, whose input indices `finite` then lists
