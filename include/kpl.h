@@ -163,6 +163,14 @@ KPL_API int kpl_add_forest_arrays(kpl_ctx* ctx, int32_t ntrees, int32_t nnodes, 
 KPL_API int kpl_forest_count(const kpl_ctx* ctx, int32_t* count_out);
 
 /* ---- the hot path, host buffers (what detector->compute() binds to) --------------------------- */
+/* Every kpl_detect* entry point below, host and device, starts the same way.  It resets kpl_stats, kpl_timings and the
+ * kpl_fetch targets and sets *n_kp_out (where there is one) to 0, so a refused call leaves nothing of an earlier call.
+ * Its refusals then come in one order, and an input with several faults gets the code of the first check it fails:
+ *   1. NULL arguments;
+ *   2. the layout: view_offsets / n_views, or width, height, n_frames and smoothing_size;
+ *   3. the point and forest checks: point count, a forest loaded, each scored forest's var_count, K*n, draws-remove
+ *      with a role array, a forced grid with a batch;
+ *   4. the strides of host arrays. */
 /* xyz: n points, 3 floats each at xyz_stride bytes (16 = pcl::PointXYZ, 12 = packed).
  * normals: NULL (estimate per params.normals_mode) or n normals, 3 floats each at normals_stride bytes
  *          (32 = pcl::Normal).  role: NULL or n bytes of enum kpl_role.

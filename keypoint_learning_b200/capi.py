@@ -498,7 +498,7 @@ class KeypointLearningDetector:
     def detectForestsDevice(self, d_xyz4, n, d_normals4=0, thresholds=None, d_scores=0, d_kp_idx=0, d_kp_offsets=0):
         """kpl_detect_forests_device: raw device pointers (ints); d_scores K*n floats (or 0), d_kp_idx K*n int32, d_kp_offsets
         K + 1 int64, forest-major.  thresholds: None or one per forest (host).  Returns the keypoint count of all forests."""
-        th = None if thresholds is None else np.ascontiguousarray(thresholds, np.float64)
+        th = self._thresholds(thresholds)
         self._push()
         nkp = C.c_int64(0)
         self._check(self._L.kpl_detect_forests_device(self._h, C.c_void_p(d_xyz4), C.c_void_p(d_normals4 or None), int(n), _ptr(th, C.c_double),

@@ -129,7 +129,7 @@ void kpl_destroy(kpl_ctx* ctx)
     release(ctx->s_score); release(ctx->score); release(ctx->flag); release(ctx->s_state); release(ctx->kp_idx);
     release(ctx->scratch_f); release(ctx->scratch_i); release(ctx->counters);
     release(ctx->org_flag); release(ctx->org_pix); release(ctx->org_xyz); release(ctx->org_nrm); release(ctx->org_frame_off);
-    release(ctx->org_kp_off); release(ctx->org_vp); release(ctx->org_score);
+    release(ctx->kp_off); release(ctx->org_vp); release(ctx->org_score);
     if (ctx->d_bbox) cudaFree(ctx->d_bbox);
     free_forest_set(ctx->forests);
     release(ctx->range_off);
@@ -613,98 +613,62 @@ int detect_begin(kpl_ctx* ctx)
 
 }  // namespace kpl
 
+// ------------------------------------------------------------------------------------------------
+// kpl_detect*: one driver behind every entry point
+// ------------------------------------------------------------------------------------------------
+
+// Grid -> scores -> NMS, the body of every detection: the params grid of one cloud (h_view_off NULL; roles allowed) or the
+// stacked grid of nviews views at host offsets h_view_off, then one feature pass whose tail walks K forests, each forest's
+// threshold + NMS on its slice of the forest-major K x n scores, and one compaction into the ascending list d_kp.
+static int detect_body(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, const uint8_t* d_role, int64_t n,
+                       const int64_t* h_view_off, int nviews, int K, const double* thresholds, int32_t* d_kp)
+{
+    int rc = h_view_off ? prepare_grid_batch(ctx, d_xyz, d_nrm, n, h_view_off, nviews) : prepare_params_grid(ctx, d_xyz, d_nrm, d_role, n);
+    if (rc) return rc;
+    if ((rc = detect_score_phase(ctx, d_nrm != nullptr, d_role != nullptr, n, K))) return rc;
+    return detect_nms_phase(ctx, d_role != nullptr, n, K, thresholds, d_kp);
+}
+
+// One cloud, or a batch of independent views in ONE pass (one stacked grid, one query order, one launch per stage -- a
+// 200 k-point view alone is 1.5 waves of the feature kernel and a handful of host round trips).  d_scores: NULL or the
+// K x n scores.  d_kp_off: NULL (kpl_detect*), or the K x nviews + 1 offsets of the (forest, view) ranges, which
+// launch_view_ranges cuts from the one list (view-local indices).  No host round trip beyond those of the grid, the
+// draws-remove rounds and detect_finish.
 static int run_detect(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, const uint8_t* d_role, int64_t n,
-                      float* d_scores_out, int32_t* d_kp_out, int64_t* n_kp_out)
+                      const int64_t* h_view_off, int nviews, int K, const double* thresholds, float* d_scores, int32_t* d_kp,
+                      int64_t* d_kp_off, int64_t* n_kp_out)
 {
-    detect_reset(ctx);
-    if (n_kp_out) *n_kp_out = 0;
-    int rc = detect_check(ctx, n, 1, d_role != nullptr);
-    if (rc) return rc;
-    ctx->stats.n_points = n;
-    if (n == 0) return KPL_OK;
-    if ((rc = detect_begin(ctx))) return rc;
-    if ((rc = prepare_params_grid(ctx, d_xyz, d_nrm, d_role, n))) return rc;
-    if ((rc = detect_score_phase(ctx, d_nrm != nullptr, d_role != nullptr, n, 1))) return rc;
-    if ((rc = detect_nms_phase(ctx, d_role != nullptr, n, 1, nullptr, d_kp_out))) return rc;
-    if (d_scores_out) KPL_CUDA(cudaMemcpyAsync(d_scores_out, ctx->score.p, (size_t)n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
-    return detect_finish(ctx, n, n_kp_out);
-}
-
-// Boundaries of the (forest, view) ranges of a forest-major keypoint list over K x n points: {k*n + h_view_off[v]} for
-// k < K, v < V, then K*n.  One forest: d_view_off, the view offsets already on the device (no copy).  The host copy is a
-// member: a pageable source is staged by cudaMemcpyAsync before it returns, the member keeps it anyway.
-static int range_bounds(kpl_ctx* ctx, int K, int64_t n, const int64_t* h_view_off, int V, const int64_t* d_view_off, const int64_t** d_out)
-{
-    *d_out = d_view_off;
-    if (K == 1 && d_view_off) return KPL_OK;
-    const size_t nb = (size_t)K * V + 1;
-    ctx->range_off_h.resize(nb);
-    for (int k = 0; k < K; ++k)
-        for (int v = 0; v < V; ++v) ctx->range_off_h[(size_t)k * V + v] = (int64_t)k * n + h_view_off[v];
-    ctx->range_off_h[nb - 1] = (int64_t)K * n;
-    KPL_CUDA(ensure(ctx->range_off, nb));
-    KPL_CUDA(cudaMemcpyAsync(ctx->range_off.p, ctx->range_off_h.data(), nb * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
-    *d_out = ctx->range_off.p;
-    return KPL_OK;
-}
-
-// Every forest of the set over ONE cloud: one grid, one normal estimation, one feature pass whose tail walks the K forests,
-// then threshold + NMS of each forest's slice (forest-major K x n scores and flags), one compaction of the K x n flags into
-// an ascending list and its split at the forest boundaries k*n by launch_view_ranges.  No host round trip beyond those of
-// run_detect (and one per draws-remove round of each forest).
-static int run_detect_forests(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, int64_t n, const double* thresholds,
-                              float* d_scores_out, int32_t* d_kp_out, int64_t* d_kp_offsets_out, int64_t* n_kp_out)
-{
-    detect_reset(ctx);
-    if (n_kp_out) *n_kp_out = 0;
-    const int K = (int)ctx->forests.info.size();
-    int rc = detect_check(ctx, n, K, false);
-    if (rc) return rc;
-    ctx->stats.n_points = n;
-    ctx->last_nforests = K;
-    if (n == 0) {
-        KPL_CUDA(cudaMemsetAsync(d_kp_offsets_out, 0, ((size_t)K + 1) * sizeof(int64_t), ctx->stream));
-        return KPL_OK;
-    }
-    if ((rc = detect_begin(ctx))) return rc;
-    if ((rc = prepare_params_grid(ctx, d_xyz, d_nrm, nullptr, n))) return rc;
-    if ((rc = detect_score_phase(ctx, d_nrm != nullptr, false, n, K))) return rc;
-    if ((rc = detect_nms_phase(ctx, false, n, K, thresholds, d_kp_out))) return rc;
-    const int64_t whole[2] = {0, n};
-    const int64_t* d_bounds = nullptr;
-    if ((rc = range_bounds(ctx, K, n, whole, 1, nullptr, &d_bounds))) return rc;
-    KPL_CUDA(launch_view_ranges(ctx, (int64_t)K * n, d_kp_out, d_bounds, K, d_kp_offsets_out));
-    if (d_scores_out) KPL_CUDA(cudaMemcpyAsync(d_scores_out, ctx->score.p, (size_t)K * n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
-    return detect_finish(ctx, n, n_kp_out);
-}
-
-// A batch of independent views in ONE pass: one stacked grid, one query order, one launch per stage, per-view
-// keypoint ranges -- a 200 k-point view alone is 1.5 waves of the feature kernel and a handful of host round trips.
-// K forests (kpl_detect_batch_forests; thresholds NULL or one per forest) are scored from the one feature pass, each
-// forest's slice gets its own NMS, and the one compacted list is split into the K x V (forest, view) ranges.
-static int run_detect_batch(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, int64_t n, const int64_t* h_offsets, int nviews,
-                            int K, const double* thresholds, float* d_scores_out, int32_t* d_kp_out, int64_t* d_kp_offsets_out,
-                            int64_t* n_kp_out)
-{
-    detect_reset(ctx);
-    if (n_kp_out) *n_kp_out = 0;
-    int rc = detect_check(ctx, n, K, false);
-    if (rc) return rc;
-    if (ctx->params.grid_forced) return fail(ctx, KPL_E_INVALID, "a forced grid cannot be combined with a batch of views");
     ctx->stats.n_points = n; ctx->stats.n_views = nviews;
     ctx->last_nforests = K;
-    if (n == 0) return KPL_OK;
-    if ((rc = detect_begin(ctx))) return rc;
-    if ((rc = prepare_grid_batch(ctx, d_xyz, d_nrm, n, h_offsets, nviews))) return rc;
-    if ((rc = detect_score_phase(ctx, d_nrm != nullptr, false, n, K))) return rc;
-    if ((rc = detect_nms_phase(ctx, false, n, K, thresholds, d_kp_out))) return rc;
-    const int64_t* d_bounds = nullptr;
-    if ((rc = range_bounds(ctx, K, n, h_offsets, nviews, ctx->view_offsets.p, &d_bounds))) return rc;
-    KPL_CUDA(launch_view_ranges(ctx, (int64_t)K * n, d_kp_out, d_bounds, K * nviews, d_kp_offsets_out));
-    if (d_scores_out) KPL_CUDA(cudaMemcpyAsync(d_scores_out, ctx->score.p, (size_t)K * n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
-    rc = detect_finish(ctx, n, n_kp_out);
-    ctx->stats.n_views = nviews;
-    return rc;
+    if (n == 0) {       // no runtime call unless there are offsets to zero
+        if (d_kp_off) {
+            KPL_CUDA(cudaSetDevice(ctx->device));
+            KPL_CUDA(cudaMemsetAsync(d_kp_off, 0, ((size_t)K * nviews + 1) * sizeof(int64_t), ctx->stream));
+        }
+        return KPL_OK;
+    }
+    int rc = detect_begin(ctx);
+    if (rc) return rc;
+    if ((rc = detect_body(ctx, d_xyz, d_nrm, d_role, n, h_view_off, nviews, K, thresholds, d_kp))) return rc;
+    if (d_kp_off) {
+        // the boundaries of the (forest, view) ranges: {k*n + h_view_off[v]} for k < K, v < nviews, then K*n.  One forest of
+        // a batch splits at the view offsets the stacked grid holds on the device.  The host copy is a member: a pageable
+        // source is staged by cudaMemcpyAsync before it returns, the member keeps it anyway.
+        const int64_t* d_bounds = ctx->view_offsets.p;
+        if (K > 1 || !h_view_off) {
+            const size_t nb = (size_t)K * nviews + 1;
+            ctx->range_off_h.resize(nb);
+            for (int k = 0; k < K; ++k)
+                for (int v = 0; v < nviews; ++v) ctx->range_off_h[(size_t)k * nviews + v] = (int64_t)k * n + (h_view_off ? h_view_off[v] : 0);
+            ctx->range_off_h[nb - 1] = (int64_t)K * n;
+            KPL_CUDA(ensure(ctx->range_off, nb));
+            KPL_CUDA(cudaMemcpyAsync(ctx->range_off.p, ctx->range_off_h.data(), nb * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
+            d_bounds = ctx->range_off.p;
+        }
+        KPL_CUDA(launch_view_ranges(ctx, (int64_t)K * n, d_kp, d_bounds, K * nviews, d_kp_off));
+    }
+    if (d_scores) KPL_CUDA(cudaMemcpyAsync(d_scores, ctx->score.p, (size_t)K * n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
+    return detect_finish(ctx, n, n_kp_out);
 }
 
 // A batch of organized frames of one size: integral-image normals of every frame (or the caller's per-pixel normals),
@@ -717,15 +681,13 @@ static int run_detect_batch(kpl_ctx* ctx, const float4* d_xyz, const float4* d_n
 // the map back: K x F x W*H scores, K x F + 1 keypoint offsets.
 static int run_detect_organized_batch(kpl_ctx* ctx, const float4* d_xyz, const float4* d_nrm, int32_t W, int32_t H, int32_t F,
                                       float smoothing_size, const float* h_viewpoints, int K, const double* thresholds,
-                                      float* d_scores_out, int32_t* d_kp_out, int64_t* d_kp_offsets_out, int64_t* n_kp_out)
+                                      float* d_scores, int32_t* d_kp, int64_t* d_kp_off, int64_t* n_kp_out)
 {
     const int64_t n = (int64_t)W * H, total = n * F;
-    int rc = detect_check(ctx, total, K, false);
-    if (rc) return rc;
-    if (ctx->params.grid_forced) return fail(ctx, KPL_E_INVALID, "a forced grid cannot be combined with a batch of frames");
     ctx->stats.n_views = F;
     ctx->last_nforests = K;
-    if ((rc = detect_begin(ctx))) return rc;
+    int rc = detect_begin(ctx);
+    if (rc) return rc;
     if (!d_nrm) {
         const float* d_vp = nullptr;
         if (h_viewpoints) {
@@ -737,7 +699,7 @@ static int run_detect_organized_batch(kpl_ctx* ctx, const float4* d_xyz, const f
         KPL_CUDA(launch_normals_integral_image(ctx, d_xyz, W, H, F, smoothing_size, d_vp, ctx->in_nrm.p));
         d_nrm = ctx->in_nrm.p;
     }
-    KPL_CUDA(launch_organized_select(ctx, d_xyz, n, F, K, d_scores_out));
+    KPL_CUDA(launch_organized_select(ctx, d_xyz, n, F, K, d_scores));
     KPL_CUDA(cudaEventRecord(ctx->ev[6], ctx->stream));
     std::vector<int64_t> frame_off((size_t)F + 1);
     KPL_CUDA(cudaMemcpyAsync(frame_off.data(), ctx->org_frame_off.p, frame_off.size() * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
@@ -749,24 +711,22 @@ static int run_detect_organized_batch(kpl_ctx* ctx, const float4* d_xyz, const f
         if (frame_off[(size_t)f + 1] > frame_off[(size_t)f]) view_off.push_back(frame_off[(size_t)f + 1]);
     kpl_timings& T = ctx->timings;
     if (m == 0) {
-        KPL_CUDA(cudaMemsetAsync(d_kp_offsets_out, 0, ((size_t)K * F + 1) * sizeof(int64_t), ctx->stream));
+        KPL_CUDA(cudaMemsetAsync(d_kp_off, 0, ((size_t)K * F + 1) * sizeof(int64_t), ctx->stream));
         cudaEventElapsedTime(&T.normals_ms, ctx->ev[0], ctx->ev[6]);
         T.total_ms = T.normals_ms;
         ctx->stats.n_points = 0; ctx->stats.kernel_launches = ctx->launches; ctx->stats.host_syncs = ctx->syncs;
         return KPL_OK;
     }
     KPL_CUDA(launch_organized_gather(ctx, d_xyz, d_nrm, m));
-    if ((rc = prepare_grid_batch(ctx, ctx->org_xyz.p, ctx->org_nrm.p, m, view_off.data(), (int)view_off.size() - 1))) return rc;
-    if ((rc = detect_score_phase(ctx, true, false, m, K))) return rc;
-    if ((rc = detect_nms_phase(ctx, false, m, K, thresholds, d_kp_out))) return rc;
-    KPL_CUDA(launch_organized_map_back(ctx, m, n, F, K, d_scores_out, d_kp_out, d_kp_offsets_out));
+    if ((rc = detect_body(ctx, ctx->org_xyz.p, ctx->org_nrm.p, nullptr, m, view_off.data(), (int)view_off.size() - 1, K, thresholds, d_kp)))
+        return rc;
+    KPL_CUDA(launch_organized_map_back(ctx, m, n, F, K, d_scores, d_kp, d_kp_off));
     if ((rc = detect_finish(ctx, m, n_kp_out))) return rc;
     // the integral images and the compaction are part of the normals stage; the grid stage starts after them
     float prep = 0.f;
     cudaEventElapsedTime(&prep, ctx->ev[0], ctx->ev[6]);
     cudaEventElapsedTime(&T.grid_ms, ctx->ev[6], ctx->ev[1]);
     T.normals_ms += prep;
-    ctx->stats.n_views = F;
     return KPL_OK;
 }
 
@@ -795,34 +755,134 @@ static int upload_inputs(kpl_ctx* ctx, const float* xyz, int32_t xs, const float
     return KPL_OK;
 }
 
+// Where a call's points come from: one cloud of n points on the params grid (kpl_detect*, kpl_detect_forests*), n_views
+// views at host view_offsets (kpl_detect_batch*), or n_views organized frames of width x height pixels
+// (kpl_detect_batch_organized*).
+enum class Layout { Cloud, Views, Frames };
+
+// One kpl_detect* call as its entry point passes it on: host arrays (xyz / normals at their strides) for the host entry
+// points, float4 device arrays for the _device ones.
+struct DetectCall {
+    const void* xyz; int32_t xyz_stride; const void* normals; int32_t normals_stride;
+    const uint8_t* role = nullptr;                  // a cloud only
+    int64_t n = 0;                                  // a cloud's points; detect_prologue counts those of a batch
+    Layout layout = Layout::Cloud;
+    const int64_t* view_offsets = nullptr;          // views: n_views + 1 host offsets
+    int32_t n_views = 1;                            // views or frames
+    int32_t width = 0, height = 0; float smoothing = 0.f; const float* viewpoints = nullptr;      // frames
+    bool all_forests = false;                       // the *_forests entry points score the whole set, the others forest 0
+    int K = 1; const double* thresholds = nullptr;  // K: set by detect_prologue
+    bool offsets = false;                           // the call returns the K x n_views + 1 keypoint offsets
+    void *scores = nullptr, *kp = nullptr, *kp_offsets = nullptr; float* kp_xyzi = nullptr;
+
+    DetectCall(const void* x, int32_t xs, const void* nrm, int32_t ns) : xyz(x), xyz_stride(xs), normals(nrm), normals_stride(ns) {}
+    DetectCall& cloud(int64_t n_, const uint8_t* role_ = nullptr) { n = n_; role = role_; return *this; }
+    DetectCall& views(const int64_t* off, int32_t nv) { layout = Layout::Views; view_offsets = off; n_views = nv; offsets = true; return *this; }
+    DetectCall& frames(int32_t w, int32_t h, int32_t f, float s, const float* vp)
+    {
+        layout = Layout::Frames; width = w; height = h; n_views = f; smoothing = s; viewpoints = vp; offsets = true;
+        return *this;
+    }
+    DetectCall& forests(const double* th) { all_forests = true; thresholds = th; offsets = true; return *this; }
+    DetectCall& out(void* s, void* k, void* ko, float* xyzi = nullptr) { scores = s; kp = k; kp_offsets = ko; kp_xyzi = xyzi; return *this; }
+};
+
+// The start of every kpl_detect* entry point.  The reset comes first, so that a refused call leaves nothing of the
+// previous one; then the refusals in the order kpl.h states: NULL arguments, layout, detect_check (with the forced grid a
+// batch cannot use).  The strides of a host call are checked last, by its upload.
+static int detect_prologue(kpl_ctx* ctx, DetectCall& c, int64_t* n_kp_out)
+{
+    if (!ctx) return KPL_E_INVALID;
+    detect_reset(ctx);
+    if (n_kp_out) *n_kp_out = 0;
+    if (c.all_forests) c.K = (int)ctx->forests.info.size();
+    const bool points = c.layout != Layout::Cloud || c.n > 0;       // a batch holds at least one point
+    if ((points && !c.xyz) || ((points || c.offsets) && !c.kp) || (c.offsets && !c.kp_offsets))
+        return fail(ctx, KPL_E_INVALID, "NULL input or output array");
+    if (c.layout == Layout::Views) {
+        const int64_t* off = c.view_offsets;
+        if (c.n_views < 1 || !off) return fail(ctx, KPL_E_INVALID, "view_offsets / n_views missing");
+        if (off[0] != 0) return fail(ctx, KPL_E_INVALID, "view_offsets[0] must be 0");
+        for (int32_t v = 0; v < c.n_views; ++v)
+            if (off[v + 1] <= off[v]) return fail(ctx, KPL_E_INVALID, "view_offsets must be strictly ascending (empty views are not allowed)");
+        c.n = off[c.n_views];
+    } else if (c.layout == Layout::Frames) {
+        if (c.width < 1 || c.height < 1 || c.n_views < 1) return fail(ctx, KPL_E_INVALID, "width, height and n_frames must be >= 1");
+        c.n = (int64_t)c.width * c.height * c.n_views;
+        if (c.n > 2147483000ll) return fail(ctx, KPL_E_INVALID, "point count out of range");
+        if (!(c.smoothing > 0.f) || !std::isfinite(c.smoothing)) return fail(ctx, KPL_E_INVALID, "normal smoothing size must be > 0");
+    }
+    int rc = detect_check(ctx, c.n, c.K, c.role != nullptr);
+    if (rc) return rc;
+    if (c.layout != Layout::Cloud && ctx->params.grid_forced) return fail(ctx, KPL_E_INVALID, "a forced grid cannot be combined with a batch");
+    return KPL_OK;
+}
+
+// A call whose arrays are on the device, past its prologue.  The drivers set the device before their first runtime call.
+static int run_call(kpl_ctx* ctx, const DetectCall& c, int64_t* n_kp_out)
+{
+    const float4 *xyz = (const float4*)c.xyz, *nrm = (const float4*)c.normals;
+    float* scores = (float*)c.scores;
+    int32_t* kp = (int32_t*)c.kp;
+    int64_t* kp_off = (int64_t*)c.kp_offsets;
+    if (c.layout == Layout::Frames)
+        return run_detect_organized_batch(ctx, xyz, nrm, c.width, c.height, c.n_views, c.smoothing, c.viewpoints, c.K, c.thresholds, scores, kp,
+                                          kp_off, n_kp_out);
+    return run_detect(ctx, xyz, nrm, c.role, c.n, c.view_offsets, c.n_views, c.K, c.thresholds, scores, kp, kp_off, n_kp_out);
+}
+
+static int detect_device(kpl_ctx* ctx, DetectCall c, int64_t* n_kp_out)
+{
+    const int rc = detect_prologue(ctx, c, n_kp_out);
+    return rc ? rc : run_call(ctx, c, n_kp_out);
+}
+
+// Host arrays in, host results out: the n points staged (every pixel of the frames), the driver, then the copies of the
+// K x n scores (the pixel-order org_score of frames, ctx->score otherwise), the keypoints, kpl_detect_xyzi's keypoint
+// cloud and the offsets, and one synchronisation.  A cloud without points and offsets has nothing to copy back.
+static int detect_host(kpl_ctx* ctx, DetectCall c, int64_t* n_kp_out)
+{
+    int rc = detect_prologue(ctx, c, n_kp_out);
+    if (rc || (rc = upload_inputs(ctx, (const float*)c.xyz, c.xyz_stride, (const float*)c.normals, c.normals_stride, c.role, c.n))) return rc;
+    const int64_t n = c.n;
+    const size_t noff = c.offsets ? (size_t)c.K * c.n_views + 1 : 0;
+    if (n > 0) KPL_CUDA(ensure(ctx->kp_idx, (size_t)c.K * n));
+    if (noff) KPL_CUDA(ensure(ctx->kp_off, noff));
+    float* d_scores = nullptr;
+    if (c.layout == Layout::Frames && c.scores) {
+        KPL_CUDA(ensure(ctx->org_score, (size_t)c.K * n));
+        d_scores = ctx->org_score.p;
+    }
+    DetectCall staged = c;
+    staged.xyz = ctx->in_xyz.p; staged.normals = c.normals ? ctx->in_nrm.p : nullptr; staged.role = c.role ? ctx->in_role.p : nullptr;
+    staged.out(d_scores, ctx->kp_idx.p, noff ? ctx->kp_off.p : nullptr);
+    int64_t nkp = 0;
+    if ((rc = run_call(ctx, staged, &nkp))) return rc;
+    if (n == 0 && !noff) return KPL_OK;
+    if (c.scores && n > 0)
+        KPL_CUDA(cudaMemcpyAsync(c.scores, d_scores ? d_scores : ctx->score.p, (size_t)c.K * n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    if (nkp > 0) KPL_CUDA(cudaMemcpyAsync(c.kp, ctx->kp_idx.p, (size_t)nkp * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    if (nkp > 0 && c.kp_xyzi) {
+        // the keypoint cloud of hpp:246-253 (x, y, z of the input point, intensity = its response), gathered on the
+        // device: a host-side gather of ~1e5 scattered rows out of a 160 MB array costs milliseconds of cache misses
+        KPL_CUDA(ensure(ctx->scratch_f, (size_t)nkp * 4));
+        KPL_CUDA(launch_gather_keypoints(ctx, ctx->in_xyz.p, ctx->kp_idx.p, nkp, (float4*)ctx->scratch_f.p));
+        KPL_CUDA(cudaMemcpyAsync(c.kp_xyzi, ctx->scratch_f.p, (size_t)nkp * 16, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    if (noff) KPL_CUDA(cudaMemcpyAsync(c.kp_offsets, ctx->kp_off.p, noff * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    KPL_CUDA(cudaStreamSynchronize(ctx->stream));
+    ctx->syncs++; ctx->stats.host_syncs = ctx->syncs; ctx->stats.kernel_launches = ctx->launches;
+    if (n_kp_out) *n_kp_out = nkp;
+    return KPL_OK;
+}
+
 extern "C" {
 
 int kpl_detect_xyzi(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
                     const uint8_t* role, int64_t n, float* scores_out, int32_t* kp_idx_out, float* kp_xyzi_out, int64_t* n_kp_out)
 {
-    if (!ctx) return KPL_E_INVALID;
-    if (n > 0 && !kp_idx_out) return fail(ctx, KPL_E_INVALID, "kp_idx_out is NULL");
-    int rc = upload_inputs(ctx, xyz, xyz_stride, normals, normals_stride, role, n);
-    if (rc) return rc;
-    if (n > 0) KPL_CUDA(ensure(ctx->kp_idx, (size_t)n));
-    int64_t nkp = 0;
-    rc = run_detect(ctx, ctx->in_xyz.p, normals ? ctx->in_nrm.p : nullptr, role ? ctx->in_role.p : nullptr, n, nullptr, ctx->kp_idx.p, &nkp);
-    if (rc) return rc;
-    if (n > 0) {
-        if (scores_out) KPL_CUDA(cudaMemcpyAsync(scores_out, ctx->score.p, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-        if (nkp > 0) KPL_CUDA(cudaMemcpyAsync(kp_idx_out, ctx->kp_idx.p, (size_t)nkp * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-        if (nkp > 0 && kp_xyzi_out) {
-            // the keypoint cloud of hpp:246-253 (x, y, z of the input point, intensity = its response), gathered on the
-            // device: a host-side gather of ~1e5 scattered rows out of a 160 MB array costs milliseconds of cache misses
-            KPL_CUDA(ensure(ctx->scratch_f, (size_t)nkp * 4));
-            KPL_CUDA(launch_gather_keypoints(ctx, ctx->in_xyz.p, ctx->kp_idx.p, nkp, (float4*)ctx->scratch_f.p));
-            KPL_CUDA(cudaMemcpyAsync(kp_xyzi_out, ctx->scratch_f.p, (size_t)nkp * 16, cudaMemcpyDeviceToHost, ctx->stream));
-        }
-        KPL_CUDA(cudaStreamSynchronize(ctx->stream));
-        ctx->syncs++; ctx->stats.host_syncs = ctx->syncs; ctx->stats.kernel_launches = ctx->launches;
-    }
-    if (n_kp_out) *n_kp_out = nkp;
-    return KPL_OK;
+    DetectCall c(xyz, xyz_stride, normals, normals_stride);
+    return detect_host(ctx, c.cloud(n, role).out(scores_out, kp_idx_out, nullptr, kp_xyzi_out), n_kp_out);
 }
 
 int kpl_detect(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
@@ -834,42 +894,83 @@ int kpl_detect(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* 
 int kpl_detect_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, const void* d_role, int64_t n,
                       void* d_scores, void* d_kp_idx, int64_t* n_kp_out)
 {
-    if (!ctx) return KPL_E_INVALID;
-    if (n > 0 && (!d_xyz4 || !d_kp_idx)) return fail(ctx, KPL_E_INVALID, "NULL device pointer");
-    return run_detect(ctx, (const float4*)d_xyz4, (const float4*)d_normals4, (const uint8_t*)d_role, n, (float*)d_scores,
-                      (int32_t*)d_kp_idx, n_kp_out);
+    DetectCall c(d_xyz4, 16, d_normals4, 16);
+    return detect_device(ctx, c.cloud(n, (const uint8_t*)d_role).out(d_scores, d_kp_idx, nullptr), n_kp_out);
 }
 
 int kpl_detect_forests(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride, int64_t n,
                        const double* thresholds, float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out)
 {
-    if (!ctx) return KPL_E_INVALID;
-    if (!kp_idx_out || !kp_offsets_out) return fail(ctx, KPL_E_INVALID, "kp_idx_out / kp_offsets_out is NULL");
-    int rc = upload_inputs(ctx, xyz, xyz_stride, normals, normals_stride, nullptr, n);
-    if (rc) return rc;
-    const size_t K = ctx->forests.info.size();
-    KPL_CUDA(ensure(ctx->kp_idx, std::max<size_t>(K * (size_t)std::max<int64_t>(n, 0), 1)));
-    KPL_CUDA(ensure(ctx->scratch_f, 2 * (K + 1) + 16));
-    int64_t* d_kp_off = reinterpret_cast<int64_t*>(ctx->scratch_f.p);
-    int64_t nkp = 0;
-    rc = run_detect_forests(ctx, ctx->in_xyz.p, normals ? ctx->in_nrm.p : nullptr, n, thresholds, nullptr, ctx->kp_idx.p, d_kp_off, &nkp);
-    if (rc) return rc;
-    if (n > 0 && scores_out) KPL_CUDA(cudaMemcpyAsync(scores_out, ctx->score.p, K * (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    if (nkp > 0) KPL_CUDA(cudaMemcpyAsync(kp_idx_out, ctx->kp_idx.p, (size_t)nkp * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    KPL_CUDA(cudaMemcpyAsync(kp_offsets_out, d_kp_off, (K + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-    KPL_CUDA(cudaStreamSynchronize(ctx->stream));
-    ctx->syncs++; ctx->stats.host_syncs = ctx->syncs;
-    return KPL_OK;
+    DetectCall c(xyz, xyz_stride, normals, normals_stride);
+    return detect_host(ctx, c.cloud(n).forests(thresholds).out(scores_out, kp_idx_out, kp_offsets_out), nullptr);
 }
 
 int kpl_detect_forests_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, int64_t n, const double* thresholds,
                               void* d_scores, void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out)
 {
-    if (!ctx) return KPL_E_INVALID;
-    if (!d_kp_idx || !d_kp_offsets || (n > 0 && !d_xyz4)) return fail(ctx, KPL_E_INVALID, "NULL device pointer");
-    KPL_CUDA(cudaSetDevice(ctx->device));
-    return run_detect_forests(ctx, (const float4*)d_xyz4, (const float4*)d_normals4, n, thresholds, (float*)d_scores, (int32_t*)d_kp_idx,
-                              (int64_t*)d_kp_offsets, n_kp_out);
+    DetectCall c(d_xyz4, 16, d_normals4, 16);
+    return detect_device(ctx, c.cloud(n).forests(thresholds).out(d_scores, d_kp_idx, d_kp_offsets), n_kp_out);
+}
+
+int kpl_detect_batch(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
+                     const int64_t* view_offsets, int32_t n_views, float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out)
+{
+    DetectCall c(xyz, xyz_stride, normals, normals_stride);
+    return detect_host(ctx, c.views(view_offsets, n_views).out(scores_out, kp_idx_out, kp_offsets_out), nullptr);
+}
+
+int kpl_detect_batch_forests(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
+                             const int64_t* view_offsets, int32_t n_views, const double* thresholds, float* scores_out,
+                             int32_t* kp_idx_out, int64_t* kp_offsets_out)
+{
+    DetectCall c(xyz, xyz_stride, normals, normals_stride);
+    return detect_host(ctx, c.views(view_offsets, n_views).forests(thresholds).out(scores_out, kp_idx_out, kp_offsets_out), nullptr);
+}
+
+int kpl_detect_batch_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, const int64_t* view_offsets, int32_t n_views,
+                            void* d_scores, void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out)
+{
+    DetectCall c(d_xyz4, 16, d_normals4, 16);
+    return detect_device(ctx, c.views(view_offsets, n_views).out(d_scores, d_kp_idx, d_kp_offsets), n_kp_out);
+}
+
+int kpl_detect_batch_forests_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, const int64_t* view_offsets, int32_t n_views,
+                                    const double* thresholds, void* d_scores, void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out)
+{
+    DetectCall c(d_xyz4, 16, d_normals4, 16);
+    return detect_device(ctx, c.views(view_offsets, n_views).forests(thresholds).out(d_scores, d_kp_idx, d_kp_offsets), n_kp_out);
+}
+
+int kpl_detect_batch_organized(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
+                               int32_t width, int32_t height, int32_t n_frames, float smoothing_size, const float* viewpoints,
+                               float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out)
+{
+    DetectCall c(xyz, xyz_stride, normals, normals_stride);
+    return detect_host(ctx, c.frames(width, height, n_frames, smoothing_size, viewpoints).out(scores_out, kp_idx_out, kp_offsets_out), nullptr);
+}
+
+int kpl_detect_batch_organized_forests(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
+                                       int32_t width, int32_t height, int32_t n_frames, float smoothing_size, const float* viewpoints,
+                                       const double* thresholds, float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out)
+{
+    DetectCall c(xyz, xyz_stride, normals, normals_stride);
+    return detect_host(ctx, c.frames(width, height, n_frames, smoothing_size, viewpoints).forests(thresholds).out(scores_out, kp_idx_out, kp_offsets_out), nullptr);
+}
+
+int kpl_detect_batch_organized_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, int32_t width, int32_t height,
+                                      int32_t n_frames, float smoothing_size, const float* viewpoints, void* d_scores, void* d_kp_idx,
+                                      void* d_kp_offsets, int64_t* n_kp_out)
+{
+    DetectCall c(d_xyz4, 16, d_normals4, 16);
+    return detect_device(ctx, c.frames(width, height, n_frames, smoothing_size, viewpoints).out(d_scores, d_kp_idx, d_kp_offsets), n_kp_out);
+}
+
+int kpl_detect_batch_organized_forests_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, int32_t width, int32_t height,
+                                              int32_t n_frames, float smoothing_size, const float* viewpoints, const double* thresholds,
+                                              void* d_scores, void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out)
+{
+    DetectCall c(d_xyz4, 16, d_normals4, 16);
+    return detect_device(ctx, c.frames(width, height, n_frames, smoothing_size, viewpoints).forests(thresholds).out(d_scores, d_kp_idx, d_kp_offsets), n_kp_out);
 }
 
 // Forced grids skip the bounding-box round trip (prepare_grid): entry points other than kpl_detect* read the
@@ -927,176 +1028,6 @@ static int prepare_knn_grid(kpl_ctx* ctx, int64_t n)
     return KPL_OK;
 }
 
-static int check_view_offsets(kpl_ctx* ctx, const int64_t* view_offsets, int32_t n_views, int64_t& n)
-{
-    if (n_views < 1 || !view_offsets) return fail(ctx, KPL_E_INVALID, "view_offsets / n_views missing");
-    if (view_offsets[0] != 0) return fail(ctx, KPL_E_INVALID, "view_offsets[0] must be 0");
-    for (int32_t v = 0; v < n_views; ++v)
-        if (view_offsets[v + 1] <= view_offsets[v]) return fail(ctx, KPL_E_INVALID, "view_offsets must be strictly ascending (empty views are not allowed)");
-    n = view_offsets[n_views];
-    return KPL_OK;
-}
-
-// kpl_detect_batch (K = 1) and kpl_detect_batch_forests: host views in, host results out, forest-major.  The forests' call
-// checks its point and forest counts before it touches the device.
-static int detect_batch_host(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
-                             const int64_t* view_offsets, int32_t n_views, int K, const double* thresholds, float* scores_out,
-                             int32_t* kp_idx_out, int64_t* kp_offsets_out)
-{
-    if (!kp_idx_out || !kp_offsets_out) return fail(ctx, KPL_E_INVALID, "kp_idx_out / kp_offsets_out is NULL");
-    int64_t n = 0;
-    int rc = check_view_offsets(ctx, view_offsets, n_views, n);
-    if (rc) return rc;
-    if (K != 1 && (rc = detect_check(ctx, n, K, false))) return rc;
-    if ((rc = upload_inputs(ctx, xyz, xyz_stride, normals, normals_stride, nullptr, n))) return rc;
-    const size_t nr = (size_t)K * n_views + 1;
-    KPL_CUDA(ensure(ctx->kp_idx, (size_t)K * n));
-    KPL_CUDA(ensure(ctx->scratch_f, nr * 2 + 16));
-    int64_t* d_kpo = reinterpret_cast<int64_t*>(ctx->scratch_f.p);
-    int64_t nkp = 0;
-    rc = run_detect_batch(ctx, ctx->in_xyz.p, normals ? ctx->in_nrm.p : nullptr, n, view_offsets, n_views, K, thresholds, nullptr,
-                          ctx->kp_idx.p, d_kpo, &nkp);
-    if (rc) return rc;
-    if (scores_out) KPL_CUDA(cudaMemcpyAsync(scores_out, ctx->score.p, (size_t)K * n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    if (nkp > 0) KPL_CUDA(cudaMemcpyAsync(kp_idx_out, ctx->kp_idx.p, (size_t)nkp * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    KPL_CUDA(cudaMemcpyAsync(kp_offsets_out, d_kpo, nr * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-    KPL_CUDA(cudaStreamSynchronize(ctx->stream));
-    ctx->syncs++; ctx->stats.host_syncs = ctx->syncs;
-    return KPL_OK;
-}
-
-int kpl_detect_batch(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
-                     const int64_t* view_offsets, int32_t n_views, float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out)
-{
-    if (!ctx) return KPL_E_INVALID;
-    return detect_batch_host(ctx, xyz, xyz_stride, normals, normals_stride, view_offsets, n_views, 1, nullptr, scores_out, kp_idx_out,
-                             kp_offsets_out);
-}
-
-int kpl_detect_batch_forests(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
-                             const int64_t* view_offsets, int32_t n_views, const double* thresholds, float* scores_out,
-                             int32_t* kp_idx_out, int64_t* kp_offsets_out)
-{
-    if (!ctx) return KPL_E_INVALID;
-    detect_reset(ctx);
-    return detect_batch_host(ctx, xyz, xyz_stride, normals, normals_stride, view_offsets, n_views, (int)ctx->forests.info.size(), thresholds,
-                             scores_out, kp_idx_out, kp_offsets_out);
-}
-
-static int detect_batch_dev(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, const int64_t* view_offsets, int32_t n_views, int K,
-                            const double* thresholds, void* d_scores, void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out)
-{
-    if (!d_xyz4 || !d_kp_idx || !d_kp_offsets) return fail(ctx, KPL_E_INVALID, "NULL device pointer");
-    int64_t n = 0;
-    int rc = check_view_offsets(ctx, view_offsets, n_views, n);
-    if (rc) return rc;
-    return run_detect_batch(ctx, (const float4*)d_xyz4, (const float4*)d_normals4, n, view_offsets, n_views, K, thresholds, (float*)d_scores,
-                            (int32_t*)d_kp_idx, (int64_t*)d_kp_offsets, n_kp_out);
-}
-
-int kpl_detect_batch_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, const int64_t* view_offsets, int32_t n_views,
-                            void* d_scores, void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out)
-{
-    if (!ctx) return KPL_E_INVALID;
-    return detect_batch_dev(ctx, d_xyz4, d_normals4, view_offsets, n_views, 1, nullptr, d_scores, d_kp_idx, d_kp_offsets, n_kp_out);
-}
-
-int kpl_detect_batch_forests_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, const int64_t* view_offsets, int32_t n_views,
-                                    const double* thresholds, void* d_scores, void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out)
-{
-    if (!ctx) return KPL_E_INVALID;
-    return detect_batch_dev(ctx, d_xyz4, d_normals4, view_offsets, n_views, (int)ctx->forests.info.size(), thresholds, d_scores, d_kp_idx,
-                            d_kp_offsets, n_kp_out);
-}
-
-static int check_organized_batch(kpl_ctx* ctx, int32_t width, int32_t height, int32_t n_frames, float smoothing_size)
-{
-    if (width < 1 || height < 1 || n_frames < 1) return fail(ctx, KPL_E_INVALID, "width, height and n_frames must be >= 1");
-    if ((int64_t)width * height * n_frames > 2147483000ll) return fail(ctx, KPL_E_INVALID, "point count out of range");
-    if (!(smoothing_size > 0.f) || !std::isfinite(smoothing_size)) return fail(ctx, KPL_E_INVALID, "normal smoothing size must be > 0");
-    return KPL_OK;
-}
-
-// kpl_detect_batch_organized (K = 1) and kpl_detect_batch_organized_forests: host frames in, host results out,
-// forest-major.  The forests' call checks its point and forest counts before it touches the device.
-static int detect_organized_host(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
-                                 int32_t width, int32_t height, int32_t n_frames, float smoothing_size, const float* viewpoints, int K,
-                                 const double* thresholds, float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out)
-{
-    detect_reset(ctx);
-    ctx->stats.n_views = n_frames;
-    if (!xyz || !kp_idx_out || !kp_offsets_out) return fail(ctx, KPL_E_INVALID, "xyz / kp_idx_out / kp_offsets_out is NULL");
-    int rc = check_organized_batch(ctx, width, height, n_frames, smoothing_size);
-    if (rc) return rc;
-    const int64_t total = (int64_t)width * height * n_frames;
-    if (K != 1 && (rc = detect_check(ctx, total, K, false))) return rc;
-    if ((rc = upload_inputs(ctx, xyz, xyz_stride, normals, normals_stride, nullptr, total))) return rc;
-    const size_t nr = (size_t)K * n_frames + 1;
-    KPL_CUDA(ensure(ctx->kp_idx, (size_t)K * total));
-    KPL_CUDA(ensure(ctx->org_kp_off, nr));
-    if (scores_out) KPL_CUDA(ensure(ctx->org_score, (size_t)K * total));
-    int64_t nkp = 0;
-    rc = run_detect_organized_batch(ctx, ctx->in_xyz.p, normals ? ctx->in_nrm.p : nullptr, width, height, n_frames, smoothing_size, viewpoints,
-                                    K, thresholds, scores_out ? ctx->org_score.p : nullptr, ctx->kp_idx.p, ctx->org_kp_off.p, &nkp);
-    if (rc) return rc;
-    if (scores_out) KPL_CUDA(cudaMemcpyAsync(scores_out, ctx->org_score.p, (size_t)K * total * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    if (nkp > 0) KPL_CUDA(cudaMemcpyAsync(kp_idx_out, ctx->kp_idx.p, (size_t)nkp * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    KPL_CUDA(cudaMemcpyAsync(kp_offsets_out, ctx->org_kp_off.p, nr * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-    KPL_CUDA(cudaStreamSynchronize(ctx->stream));
-    ctx->syncs++; ctx->stats.host_syncs = ctx->syncs;
-    return KPL_OK;
-}
-
-int kpl_detect_batch_organized(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
-                               int32_t width, int32_t height, int32_t n_frames, float smoothing_size, const float* viewpoints,
-                               float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out)
-{
-    if (!ctx) return KPL_E_INVALID;
-    return detect_organized_host(ctx, xyz, xyz_stride, normals, normals_stride, width, height, n_frames, smoothing_size, viewpoints, 1, nullptr,
-                                 scores_out, kp_idx_out, kp_offsets_out);
-}
-
-int kpl_detect_batch_organized_forests(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, const float* normals, int32_t normals_stride,
-                                       int32_t width, int32_t height, int32_t n_frames, float smoothing_size, const float* viewpoints,
-                                       const double* thresholds, float* scores_out, int32_t* kp_idx_out, int64_t* kp_offsets_out)
-{
-    if (!ctx) return KPL_E_INVALID;
-    return detect_organized_host(ctx, xyz, xyz_stride, normals, normals_stride, width, height, n_frames, smoothing_size, viewpoints,
-                                 (int)ctx->forests.info.size(), thresholds, scores_out, kp_idx_out, kp_offsets_out);
-}
-
-static int detect_organized_dev(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, int32_t width, int32_t height, int32_t n_frames,
-                                float smoothing_size, const float* viewpoints, int K, const double* thresholds, void* d_scores, void* d_kp_idx,
-                                void* d_kp_offsets, int64_t* n_kp_out)
-{
-    detect_reset(ctx);
-    ctx->stats.n_views = n_frames;
-    if (n_kp_out) *n_kp_out = 0;
-    if (!d_xyz4 || !d_kp_idx || !d_kp_offsets) return fail(ctx, KPL_E_INVALID, "NULL device pointer");
-    int rc = check_organized_batch(ctx, width, height, n_frames, smoothing_size);
-    if (rc) return rc;
-    KPL_CUDA(cudaSetDevice(ctx->device));
-    return run_detect_organized_batch(ctx, (const float4*)d_xyz4, (const float4*)d_normals4, width, height, n_frames, smoothing_size, viewpoints,
-                                      K, thresholds, (float*)d_scores, (int32_t*)d_kp_idx, (int64_t*)d_kp_offsets, n_kp_out);
-}
-
-int kpl_detect_batch_organized_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, int32_t width, int32_t height,
-                                      int32_t n_frames, float smoothing_size, const float* viewpoints, void* d_scores, void* d_kp_idx,
-                                      void* d_kp_offsets, int64_t* n_kp_out)
-{
-    if (!ctx) return KPL_E_INVALID;
-    return detect_organized_dev(ctx, d_xyz4, d_normals4, width, height, n_frames, smoothing_size, viewpoints, 1, nullptr, d_scores, d_kp_idx,
-                                d_kp_offsets, n_kp_out);
-}
-
-int kpl_detect_batch_organized_forests_device(kpl_ctx* ctx, const void* d_xyz4, const void* d_normals4, int32_t width, int32_t height,
-                                              int32_t n_frames, float smoothing_size, const float* viewpoints, const double* thresholds,
-                                              void* d_scores, void* d_kp_idx, void* d_kp_offsets, int64_t* n_kp_out)
-{
-    if (!ctx) return KPL_E_INVALID;
-    return detect_organized_dev(ctx, d_xyz4, d_normals4, width, height, n_frames, smoothing_size, viewpoints, (int)ctx->forests.info.size(),
-                                thresholds, d_scores, d_kp_idx, d_kp_offsets, n_kp_out);
-}
 
 int kpl_normals(kpl_ctx* ctx, const float* xyz, int32_t xyz_stride, int64_t n, float* normals_out)
 {

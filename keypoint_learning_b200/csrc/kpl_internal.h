@@ -139,13 +139,14 @@ struct kpl_ctx {
     kpl::DevBuf<int32_t> kp_idx;
     kpl::DevBuf<float> scratch_f;                // fetch / reorder scratch
     kpl::DevBuf<int32_t> scratch_i;
+    kpl::DevBuf<int64_t> kp_off;                 // keypoint offsets of the host entry points that return them
     // kpl_detect_batch_organized: finite-pixel flags, compact index -> pixel index (frame f's pixel p is f*width*height + p),
     // the compacted positions / normals the detection runs on, the frames' first compacted points (+ their count), the
-    // per-frame viewpoints, and the pixel-order scores / frame keypoint offsets of the host entry point
+    // per-frame viewpoints, and the pixel-order scores of the host entry point
     kpl::DevBuf<uint8_t> org_flag;
     kpl::DevBuf<int32_t> org_pix;
     kpl::DevBuf<float4> org_xyz, org_nrm;
-    kpl::DevBuf<int64_t> org_frame_off, org_kp_off;
+    kpl::DevBuf<int64_t> org_frame_off;
     kpl::DevBuf<float> org_vp, org_score;
     // [0] feature pairs [1] candidate pairs [2] above th [3] n_kp [4] unscored [5] scored [6] scratch [7] near threshold
     // [8] fragile points [9] clipped k-NN searches (slab edge) [10] scratch [11..15] sizes of the query lists (grid.cu: build_lists)
