@@ -154,7 +154,7 @@ KPL_API int kpl_forest_info(const kpl_ctx* ctx, int32_t* ntrees, int32_t* nnodes
  * receives the new forest's index.  Adding needs forest 0 (KPL_E_FOREST without it) and fails with KPL_E_INVALID once the
  * set is full; a failed add leaves the set as it was.  kpl_forest_info keeps describing forest 0, and every entry point
  * other than kpl_detect_forests, kpl_detect_batch_forests and kpl_detect_batch_organized_forests (and their _device
- * variants) scores with forest 0 only, whatever else is loaded. */
+ * variants) and kpl_shard_detect_forests(_group) scores with forest 0 only, whatever else is loaded. */
 #define KPL_MAX_FORESTS 16
 KPL_API int kpl_add_forest(kpl_ctx* ctx, const char* path, int32_t* index_out);
 KPL_API int kpl_add_forest_arrays(kpl_ctx* ctx, int32_t ntrees, int32_t nnodes, const int32_t* roots, const int32_t* var,
@@ -432,8 +432,39 @@ KPL_API int kpl_shard_detect(kpl_shard* s, float* scores_owned_out, int32_t* kp_
  * (entries may be NULL), the global list lands in kp_global_out. */
 KPL_API int kpl_shard_detect_group(kpl_shard** shards, int32_t world, float** scores_owned_out, int32_t* kp_global_out,
                                    int64_t kp_capacity, int64_t* n_kp_out);
+/* Every forest of the set (kpl_forest_count = K) over the slab-sharded cloud, from ONE position exchange, ONE grid / normal
+ * estimation and ONE feature pass per rank (several descriptors' forests on a large scene).  For every forest k the owned
+ * scores (as bits, NaN included) and the keypoints are those of kpl_shard_detect with only forest k loaded and
+ * params.threshold = thresholds[k], and so those of kpl_detect_forests on the whole cloud -- with estimated or caller
+ * normals, plain NMS, draws-remove NMS or non_maxima = 0.  K = 1 returns what kpl_shard_detect returns.
+ * thresholds: NULL (params.threshold for every forest) or K host doubles.
+ * scores_owned_out: NULL or K*n_owned floats, forest-major (forest k's owned scores at k*n_owned, in the order given to
+ * kpl_shard_set_slab).  kp_global_out (rank 0; NULL elsewhere): ascending GLOBAL indices per forest, capacity kp_capacity;
+ * kp_offsets_out: NULL or K + 1 int64 (on every rank that passes it): forest k's keypoints are
+ * kp_global_out[kp_offsets_out[k] .. kp_offsets_out[k+1]).  *n_kp_out = keypoints of all forests, on every rank.
+ * Each strip point's score moves as K floats in the one score exchange; draws-remove NMS runs forest after forest, each
+ * with its own state exchanges and resolution rounds.
+ * Refusals, in this order: NULL arguments; K * plan.n_points above 2 147 483 000 (KPL_E_INVALID, before the device is
+ * touched); the checks of kpl_detect_forests on every rank (KPL_E_FOREST without a forest, KPL_E_VARCOUNT names the
+ * forest); ranks whose forest count, forests (compared by a digest of each) or thresholds differ: KPL_E_INVALID on every
+ * rank before any strip moves (NCCL: one all-gather of a small descriptor and one host synchronisation; in-process group:
+ * compared on the host); kp_capacity below the total: KPL_E_INVALID on rank 0.  KPL_E_HALO and KPL_E_GRID as in
+ * kpl_shard_detect.  kpl_stats per rank as kpl_detect_forests: feature_pairs, candidate_pairs and n_scored count the one
+ * feature pass; n_above_threshold, n_near_threshold, n_keypoints (the rank's own), n_fragile_points and nms_rounds are sums
+ * over the forests.  kpl_shard_info.halo_bytes counts 4*K score bytes per strip point after this call.
+ * Host synchronisations (NCCL rank): those of kpl_shard_detect, plus one for the descriptor, plus one per draws-remove
+ * round of each further forest (an in-process group also synchronises its streams at every peer-copy exchange: one more
+ * state exchange per further forest and one per round).  Kernel launches: those of kpl_shard_detect, plus each further
+ * forest's NMS (plain: one launch; draws-remove: its classification, state packing, rounds and flags), plus one launch on
+ * rank 0 that turns the sorted (forest, global index) keys back into global indices. */
+KPL_API int kpl_shard_detect_forests(kpl_shard* s, const double* thresholds, float* scores_owned_out, int32_t* kp_global_out,
+                                     int64_t kp_capacity, int64_t* kp_offsets_out, int64_t* n_kp_out);
+/* The same for the ranks of an in-process group (outputs as in kpl_shard_detect_group; kp_offsets_out K + 1 int64). */
+KPL_API int kpl_shard_detect_forests_group(kpl_shard** shards, int32_t world, const double* thresholds, float** scores_owned_out,
+                                           int32_t* kp_global_out, int64_t kp_capacity, int64_t* kp_offsets_out, int64_t* n_kp_out);
 KPL_API int kpl_shard_get_info(const kpl_shard* s, kpl_shard_info* out);
-/* Device pointer of the owned scores of the last detection (n_owned floats), for callers that keep results on the GPU. */
+/* Device pointer of the owned scores of the last detection (n_owned floats), for callers that keep results on the GPU;
+ * after kpl_shard_detect_forests, forest 0's owned scores. */
 KPL_API const void* kpl_shard_device_scores(const kpl_shard* s);
 
 /* ---- introspection --------------------------------------------------------------------------- */

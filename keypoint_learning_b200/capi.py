@@ -31,7 +31,7 @@ EXPORTS = ["kpl_create", "kpl_destroy", "kpl_last_error", "kpl_version", "kpl_se
            "kpl_shard_device_scores", "kpl_shard_set_slab_normals", "kpl_shard_upload_normals", "kpl_detect_batch_organized",
            "kpl_detect_batch_organized_device", "kpl_add_forest", "kpl_add_forest_arrays", "kpl_forest_count", "kpl_detect_forests",
            "kpl_detect_forests_device", "kpl_detect_batch_forests", "kpl_detect_batch_forests_device", "kpl_detect_batch_organized_forests",
-           "kpl_detect_batch_organized_forests_device"]
+           "kpl_detect_batch_organized_forests_device", "kpl_shard_detect_forests", "kpl_shard_detect_forests_group"]
 KPL_MAX_RANKS = 64
 KPL_MAX_FORESTS = 16
 
@@ -134,6 +134,8 @@ def load_library():
     L.kpl_shard_upload_normals.argtypes = [vp, f32p, C.c_int32]
     L.kpl_shard_detect.argtypes = [vp, f32p, i32p, C.c_int64, i64p]
     L.kpl_shard_detect_group.argtypes = [C.POINTER(vp), C.c_int32, C.POINTER(f32p), i32p, C.c_int64, i64p]
+    L.kpl_shard_detect_forests.argtypes = [vp, f64p, f32p, i32p, C.c_int64, i64p, i64p]
+    L.kpl_shard_detect_forests_group.argtypes = [C.POINTER(vp), C.c_int32, f64p, C.POINTER(f32p), i32p, C.c_int64, i64p, i64p]
     L.kpl_shard_get_info.argtypes = [vp, C.POINTER(KplShardInfo)]
     L.kpl_shard_device_scores.argtypes = [vp]; L.kpl_shard_device_scores.restype = vp
     L.kpl_detect_batch.argtypes = [vp, f32p, C.c_int32, f32p, C.c_int32, i64p, C.c_int32, f32p, i32p, i64p]

@@ -211,6 +211,8 @@ static int pack_checked(kpl_ctx* ctx, const HostForestArrays& H, std::vector<Pac
     if (rc) return fail(ctx, rc, err);
     if (roots.empty()) return fail(ctx, KPL_E_FOREST, "forest has no trees");
     info.ntrees = (int32_t)roots.size(); info.nnodes = (int32_t)H.var.size(); info.var_count = H.var_count; info.max_depth = max_depth; info.max_var = max_var;
+    info.digest = fnv1a64(roots.data(), roots.size() * sizeof(int32_t), fnv1a64(nodes.data(), nodes.size() * sizeof(PackedNode)));
+    info.digest = fnv1a64(&H.var_count, sizeof H.var_count, info.digest);
     return KPL_OK;
 }
 

@@ -59,7 +59,16 @@ static constexpr uint32_t KPL_LEAF_VAR = 1023u;
 struct ForestInfo {
     int32_t ntrees = 0, nnodes = 0, var_count = 0, max_depth = 0;
     int32_t max_var = -1;                 // largest variable index any split reads (checked against annuli*bins per call)
+    uint64_t digest = 0;                  // of the packed nodes and roots: the ranks of a sharded call compare their forests by it
 };
+
+// 64-bit FNV-1a of n bytes, continuing from h
+inline uint64_t fnv1a64(const void* p, size_t n, uint64_t h = 14695981039346656037ull)
+{
+    const unsigned char* b = static_cast<const unsigned char*>(p);
+    for (size_t i = 0; i < n; ++i) h = (h ^ b[i]) * 1099511628211ull;
+    return h;
+}
 
 // The loaded forests: forest 0 (kpl_load_forest / kpl_set_forest, which every entry point scores with) and the ones
 // kpl_add_forest* appended, concatenated into one node array.  pack_forest's child offsets are relative, so a forest moves

@@ -78,10 +78,18 @@ inline const float* point_at(const float* xyz, int32_t stride, int64_t i)
 
 // One record per rank, all-gathered at the end of a detection so that every rank takes the same decision.
 struct ShardRecord {
-    unsigned long long n_kp;       // keypoints among the owned points
+    unsigned long long n_kp;       // keypoints among the owned points (all forests of the call)
     unsigned long long clipped;    // k-NN searches clipped by a slab face (KPL_E_HALO)
     unsigned long long bad_grid;   // a point outside the forced grid / not finite
     unsigned long long reserved;
+    unsigned long long n_kp_forest[KPL_MAX_FORESTS];   // the same per forest (the first K entries)
+};
+
+// What the ranks of a kpl_shard_detect_forests call must agree on before any strip moves: strips of K score slices, the
+// same forests, the same thresholds.
+struct ShardDesc {
+    unsigned long long K, thresholds;
+    unsigned long long forest[KPL_MAX_FORESTS];
 };
 
 struct kpl_shard {
@@ -116,8 +124,13 @@ struct kpl_shard {
     DevBuf<int32_t> kp_local, kp_global, kp_all, kp_sorted;
     DevBuf<uint8_t> sort_tmp;
     DevBuf<ShardRecord> rec, rec_all;
+    DevBuf<ShardDesc> desc, desc_all;
     DevBuf<unsigned long long> sizes, sizes_all;
     std::vector<ShardRecord> h_rec;
+    // the call in flight: K forest-major score slices (kpl_shard_detect: 1), the thresholds (NULL: params.threshold), the
+    // forest whose draws-remove rounds run; last_K is kept for kpl_shard_get_info
+    int K = 1, fk = 0, last_K = 1;
+    const double* th = nullptr;
     cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     float exchange_ms = 0.f, gather_ms = 0.f;
 };
@@ -174,11 +187,14 @@ __global__ void __launch_bounds__(256) pack_strip_normals_kernel(const float4* _
         out_nrm[k] = owned_nrm[i];
     }
 }
+// the strip points' scores of K forest-major slices (stride n_loc) -> K packed slices of m
 __global__ void __launch_bounds__(256) pack_scores_kernel(const float* __restrict__ owned_scores, const int32_t* __restrict__ sel, int64_t m,
-                                                          float* __restrict__ out)
+                                                          int64_t n_loc, int K, float* __restrict__ out)
 {
-    const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (k < m) out[k] = owned_scores[sel[k]];
+    const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (t >= m * K) return;
+    const int64_t k = t / m, j = t - k * m;
+    out[t] = owned_scores[k * n_loc + sel[j]];
 }
 __global__ void __launch_bounds__(256) pack_states_kernel(const uint8_t* __restrict__ owned_states, const int32_t* __restrict__ sel, int64_t m,
                                                           uint8_t* __restrict__ out)
@@ -200,26 +216,58 @@ __global__ void __launch_bounds__(256) halo_states_kernel(const float4* __restri
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i < n && s_role[i] == KPL_ROLE_HALO) s_state[i] = st_orig[__float_as_uint(s_pos[i].w)];
 }
-// scores of halo points arrived in original (local) order; NMS reads the cell-sorted copy
+// scores of halo points arrived in original (local) order in each of the K slices; NMS reads the cell-sorted copy.  The
+// original-order entry of a halo point becomes NaN again: only the owner flags a point, also when every scored point is a
+// keypoint (non_maxima = 0 reads the original-order scores)
 __global__ void __launch_bounds__(256) halo_scores_kernel(const float4* __restrict__ s_pos, const uint8_t* __restrict__ s_role,
-                                                          const float* __restrict__ score, int64_t n, float* __restrict__ s_score)
+                                                          float* __restrict__ score, int64_t n, int K, float* __restrict__ s_score)
 {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (i < n && s_role[i] == KPL_ROLE_HALO) s_score[i] = score[__float_as_uint(s_pos[i].w)];
+    if (i >= n || s_role[i] != KPL_ROLE_HALO) return;
+    const int64_t o = __float_as_uint(s_pos[i].w);
+    for (int k = 0; k < K; ++k) {
+        s_score[k * n + i] = score[k * n + o];
+        score[k * n + o] = __int_as_float(0x7FFFFFFF);
+    }
 }
+// local keypoint l = k * n_loc + i (forest k, local point i) -> key k * N + global index, ascending like l; K = 1: the
+// global index
 __global__ void __launch_bounds__(256) to_global_kernel(const int32_t* __restrict__ kp_local, const unsigned long long* __restrict__ counters,
-                                                        const int32_t* __restrict__ gidx, int64_t n_l, int64_t n, int32_t* __restrict__ kp_global)
+                                                        const int32_t* __restrict__ gidx, int64_t n_l, int64_t n_loc, int64_t N, int64_t n,
+                                                        int32_t* __restrict__ kp_global)
 {
-    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    const int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     const int64_t cnt = (int64_t)(counters[3] & 0xFFFFFFFFull);
-    if (i < n && i < cnt) kp_global[i] = gidx[kp_local[i] - n_l];
+    if (j >= n || j >= cnt) return;
+    const int64_t l = kp_local[j], k = l / n_loc;
+    kp_global[j] = (int32_t)(k * N + gidx[l - k * n_loc - n_l]);
 }
-__global__ void record_kernel(const unsigned long long* __restrict__ counters, const uint32_t* __restrict__ bbox, ShardRecord* __restrict__ rec)
+// the rank's record; the keypoints of forest k are the local list's entries in [k * n_loc, (k + 1) * n_loc)
+__global__ void record_kernel(const unsigned long long* __restrict__ counters, const uint32_t* __restrict__ bbox, const int32_t* __restrict__ kp_local,
+                              int64_t n_loc, int K, ShardRecord* __restrict__ rec)
 {
-    rec->n_kp = counters[3] & 0xFFFFFFFFull;
+    const int32_t cnt = (int32_t)(counters[3] & 0xFFFFFFFFull);
+    rec->n_kp = (unsigned long long)cnt;
     rec->clipped = counters[9];
     rec->bad_grid = bbox[7];
     rec->reserved = 0;
+    int32_t lo = 0;
+    for (int k = 0; k < K; ++k) {
+        int32_t a = lo, b = cnt;
+        if (k < K - 1)
+            while (a < b) {
+                const int32_t mid = (a + b) >> 1;
+                if ((int64_t)kp_local[mid] < (int64_t)(k + 1) * n_loc) a = mid + 1; else b = mid;
+            }
+        rec->n_kp_forest[k] = (unsigned long long)(b - lo);
+        lo = b;
+    }
+}
+// sorted keys k * N + global index -> global indices (K > 1; the offsets of the forests come from the records)
+__global__ void __launch_bounds__(256) strip_forest_kernel(int32_t* __restrict__ kp, int64_t n, int32_t N)
+{
+    const int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (j < n) kp[j] %= N;
 }
 
 // ---- transport -------------------------------------------------------------------------------------------------
@@ -251,12 +299,18 @@ struct Strips {
     size_t item;
 };
 
-// the strip sets one exchange of `kind` moves (out[0..return value)): the normal strips travel with the positions
+// the strip sets one exchange of `kind` moves (out[0..return value), at most KPL_MAX_FORESTS): the normal strips travel
+// with the positions, the scores of forest k go from packed slice k into slice k of the local scores
 int strips(kpl_shard* t, Strip kind, Strips* out)
 {
     const int64_t hi = t->n_l + t->n_own;
     switch (kind) {
-    case Strip::scores: out[0] = {t->ssc_l.p, t->ssc_r.p, t->ctx->score.p, t->ctx->score.p + hi, sizeof(float)}; return 1;
+    case Strip::scores:
+        for (int k = 0; k < t->K; ++k) {
+            float* sc = t->ctx->score.p + (int64_t)k * t->n_loc;
+            out[k] = {t->ssc_l.p + (int64_t)k * t->send_l, t->ssc_r.p + (int64_t)k * t->send_r, sc, sc + hi, sizeof(float)};
+        }
+        return t->K;
     case Strip::states: out[0] = {t->sst_l[t->sst].p, t->sst_r[t->sst].p, t->st_orig.p, t->st_orig.p + hi, sizeof(uint8_t)}; return 1;
     case Strip::gidx: out[0] = {t->sgi_l.p, t->sgi_r.p, t->loc_gidx.p, t->loc_gidx.p + hi, sizeof(int32_t)}; return 1;
     default:
@@ -273,7 +327,7 @@ int strips(kpl_shard* t, Strip kind, Strips* out)
 int exchange(kpl_shard** S, int n, Strip kind)
 {
     kpl_shard* s = S[0];
-    Strips b[2], p[2];
+    Strips b[KPL_MAX_FORESTS], p[KPL_MAX_FORESTS];
     if (!s->in_process) {
         const int nb = strips(s, kind, b);
         cudaStream_t st = s->ctx->stream;
@@ -373,15 +427,22 @@ int phase_score(kpl_shard* s)
     kpl_ctx* c = s->ctx;
     KS_CUDA(cudaSetDevice(c->device));
     KS_CUDA(cudaEventRecord(s->ev[1], c->stream));
+    // K slices of score strips and of keypoints (set_slab sized them for one)
+    const size_t K = (size_t)s->K;
+    KS_CUDA(ensure(s->ssc_l, K * s->send_l + 1)); KS_CUDA(ensure(s->ssc_r, K * s->send_r + 1));
+    KS_CUDA(ensure(s->kp_local, K * s->n_own + 1)); KS_CUDA(ensure(s->kp_global, K * s->n_own + 1));
     int rc = detect_begin(c);
     if (rc) return rc;
     c->launches += 2;
+    c->last_nforests = s->last_K = s->K;
     if ((rc = prepare_grid(c, s->loc_xyz.p, s->has_nrm ? s->loc_nrm.p : nullptr, s->role.p, s->n_loc, &s->grid))) return rc;
-    if ((rc = detect_score_phase(c, s->has_nrm, true, s->n_loc, 1))) return rc;
+    if ((rc = detect_score_phase(c, s->has_nrm, true, s->n_loc, s->K))) return rc;
     KS_CUDA(cudaEventRecord(s->ev[2], c->stream));
     const float* owned_scores = c->score.p + s->n_l;
-    if (s->send_l) pack_scores_kernel<<<(unsigned)((s->send_l + 255) / 256), 256, 0, c->stream>>>(owned_scores, s->sel_l.p, s->send_l, s->ssc_l.p);
-    if (s->send_r) pack_scores_kernel<<<(unsigned)((s->send_r + 255) / 256), 256, 0, c->stream>>>(owned_scores, s->sel_r.p, s->send_r, s->ssc_r.p);
+    if (s->send_l)
+        pack_scores_kernel<<<(unsigned)((K * s->send_l + 255) / 256), 256, 0, c->stream>>>(owned_scores, s->sel_l.p, s->send_l, s->n_loc, s->K, s->ssc_l.p);
+    if (s->send_r)
+        pack_scores_kernel<<<(unsigned)((K * s->send_r + 255) / 256), 256, 0, c->stream>>>(owned_scores, s->sel_r.p, s->send_r, s->n_loc, s->K, s->ssc_r.p);
     KS_CUDA(cudaGetLastError());
     c->launches += 2;
     return KPL_OK;
@@ -404,36 +465,49 @@ int pack_states(kpl_shard* s)
     return KPL_OK;
 }
 
-// keypoints (owned points only) to global indices, and the rank's record
+// keypoints (owned points only) to global indices (keys k * N + global index with K forests), and the rank's record
 int phase_records(kpl_shard* s)
 {
     kpl_ctx* c = s->ctx;
-    to_global_kernel<<<(unsigned)((s->n_own + 255) / 256), 256, 0, c->stream>>>(s->kp_local.p, c->counters.p, s->gidx.p, s->n_l, s->n_own, s->kp_global.p);
-    record_kernel<<<1, 1, 0, c->stream>>>(c->counters.p, (const uint32_t*)c->d_bbox, s->rec.p);
+    const int64_t m = (int64_t)s->K * s->n_own;
+    to_global_kernel<<<(unsigned)((m + 255) / 256), 256, 0, c->stream>>>(s->kp_local.p, c->counters.p, s->gidx.p, s->n_l, s->n_loc,
+                                                                        s->plan.n_points, m, s->kp_global.p);
+    record_kernel<<<1, 1, 0, c->stream>>>(c->counters.p, (const uint32_t*)c->d_bbox, s->kp_local.p, s->n_loc, s->K, s->rec.p);
     KS_CUDA(cudaGetLastError());
     c->launches += 2;
     return KPL_OK;
 }
 
-// Threshold + NMS.  Draws-remove: only the classification here; the resolution rounds need the neighbours' decisions and
-// run over all ranks (nms_draws_rounds), then phase_draws_keypoints.
+double threshold(const kpl_shard* s, int k) { return s->th ? s->th[k] : s->ctx->params.threshold; }
+
+// draws-remove: the classification of forest fk's slice, then the states of the strip points packed for the neighbours
+int draws_classify(kpl_shard* s)
+{
+    kpl_ctx* c = s->ctx;
+    KS_CUDA(launch_nms_draws_classify(c, s->n_loc, true, c->s_score.p + (int64_t)s->fk * s->n_loc, threshold(s, s->fk)));
+    return pack_states(s);
+}
+
+// Threshold + NMS of the K slices.  Draws-remove: only the classification of forest 0 here; the resolution rounds need the
+// neighbours' decisions and run over all ranks (nms_draws), forest after forest.
 int phase_nms(kpl_shard* s)
 {
     kpl_ctx* c = s->ctx;
     KS_CUDA(cudaSetDevice(c->device));             // an in-process group drives ranks on several devices from one thread
     KS_CUDA(cudaEventRecord(s->ev[3], c->stream));
     if (s->n_l + s->n_r > 0)
-        halo_scores_kernel<<<(unsigned)((s->n_loc + 255) / 256), 256, 0, c->stream>>>(c->s_pos.p, c->s_role.p, c->score.p, s->n_loc, c->s_score.p);
+        halo_scores_kernel<<<(unsigned)((s->n_loc + 255) / 256), 256, 0, c->stream>>>(c->s_pos.p, c->s_role.p, c->score.p, s->n_loc, s->K, c->s_score.p);
     c->launches++;
     if (draws_remove(c)) {
-        KS_CUDA(launch_nms_draws_classify(c, s->n_loc, true, c->s_score.p, c->params.threshold));
-        return pack_states(s);
+        KS_CUDA(ensure(c->flag, (size_t)s->K * s->n_loc));    // before slice 0: a later growth would drop the flags of earlier slices
+        s->fk = 0;
+        return draws_classify(s);
     }
-    int rc = detect_nms_phase(c, true, s->n_loc, 1, nullptr, s->kp_local.p);
+    int rc = detect_nms_phase(c, true, s->n_loc, s->K, s->th, s->kp_local.p);
     return rc ? rc : phase_records(s);
 }
 
-// one draws-remove resolution round of the owned points, on the halo states the last exchange brought in
+// one draws-remove resolution round of the owned points of forest fk, on the halo states the last exchange brought in
 int phase_draws_round(kpl_shard* s)
 {
     kpl_ctx* c = s->ctx;
@@ -443,21 +517,20 @@ int phase_draws_round(kpl_shard* s)
         KS_CUDA(cudaGetLastError());
         c->launches++;
     }
-    KS_CUDA(launch_nms_draws_round(c, s->n_loc, true, s->loc_gidx.p, c->s_score.p, c->params.threshold));
+    KS_CUDA(launch_nms_draws_round(c, s->n_loc, true, s->loc_gidx.p, c->s_score.p + (int64_t)s->fk * s->n_loc, threshold(s, s->fk)));
     if (s->in_process)      // read by the host after the next exchange, which synchronises every stream of the group
         KS_CUDA(cudaMemcpyAsync(&s->h_undecided, c->counters.p + 6, sizeof s->h_undecided, cudaMemcpyDeviceToHost, c->stream));
     return pack_states(s);
 }
 
-// The draws-remove rounds over the slabs.  After the classification and after every round, the owned states of the
-// strip points go to the neighbours, so that a halo point always holds its owner's decision (a stale one only postpones
-// a decision).  Every rank stops on the same global count of undecided candidates, within the same cap: no rank is left
-// waiting in a collective.  One host synchronisation per round.
+// The draws-remove rounds of one forest over the slabs.  After the classification and after every round, the owned states
+// of the strip points go to the neighbours, so that a halo point always holds its owner's decision (a stale one only
+// postpones a decision).  Every rank stops on the same global count of undecided candidates, within the same cap: no rank
+// is left waiting in a collective.  One host synchronisation per round.
 int nms_draws_rounds(kpl_shard** S, int n)
 {
     kpl_shard* s = S[0];
     kpl_ctx* c = s->ctx;
-    if (!draws_remove(c)) return KPL_OK;
     int rc = exchange(S, n, Strip::states);
     for (int round = 0; !rc && round < nms_round_cap(s->plan.n_points); ++round) {
         if ((rc = each_rank(S, n, phase_draws_round)) || (rc = exchange(S, n, Strip::states))) return rc;
@@ -477,15 +550,26 @@ int nms_draws_rounds(kpl_shard** S, int n)
     return rc;
 }
 
-// draws-remove: flags of the decided owned points, compaction, records
+// draws-remove: flags of forest fk's decided owned points into slice fk; then the next forest's classification, or after
+// the last forest one compaction of the K slices and the records
 int phase_draws_keypoints(kpl_shard* s)
 {
     kpl_ctx* c = s->ctx;
-    if (!draws_remove(c)) return KPL_OK;
     KS_CUDA(cudaSetDevice(c->device));
-    KS_CUDA(launch_nms_draws_flags(c, s->n_loc, true, 0));
-    KS_CUDA(launch_compact(c, s->n_loc, s->kp_local.p));
+    KS_CUDA(launch_nms_draws_flags(c, s->n_loc, true, (int64_t)s->fk * s->n_loc));
+    if (++s->fk < s->K) return draws_classify(s);
+    KS_CUDA(launch_compact(c, (int64_t)s->K * s->n_loc, s->kp_local.p));
     return phase_records(s);
+}
+
+// draws-remove NMS of the K forests, one after the other, as on one GPU (capi.cu: nms_flags)
+int nms_draws(kpl_shard** S, int n)
+{
+    if (!draws_remove(S[0]->ctx)) return KPL_OK;
+    int rc = KPL_OK;
+    for (int k = 0; !rc && k < S[0]->K; ++k)
+        if (!(rc = nms_draws_rounds(S, n))) rc = each_rank(S, n, phase_draws_keypoints);
+    return rc;
 }
 
 // after the records of all ranks reached the host: the same verdict on every rank
@@ -514,8 +598,8 @@ int sort_keypoints(kpl_shard* s, int64_t total)
 {
     kpl_ctx* c = s->ctx;
     if (total <= 0) return KPL_OK;
-    int end_bit = 1;
-    while (end_bit < 32 && (1ll << end_bit) < s->plan.n_points) end_bit++;
+    int end_bit = 1;                                // keys below K * N
+    while (end_bit < 32 && (1ll << end_bit) < (int64_t)s->K * s->plan.n_points) end_bit++;
     size_t bytes = 0;
     cub::DeviceRadixSort::SortKeys(nullptr, bytes, (const uint32_t*)s->kp_all.p, (uint32_t*)s->kp_sorted.p, (int)total, 0, end_bit, c->stream);
     KS_CUDA(ensure(s->sort_tmp, bytes));
@@ -533,7 +617,56 @@ int check_ready(kpl_shard* s)
     // halo must then be two search reaches wide, which no device check can verify after the fact
     if (s->world > 1 && !s->has_nrm && s->ctx->params.normals_mode == KPL_NORMALS_RADIUS && s->plan.normal_support_cells < s->plan.reach_feat)
         return sfail(s, KPL_E_HALO, "radius-mode normals need normal_support_cells >= reach_feat (the whole r_feat ball of every halo point that matters)");
-    return detect_check(s->ctx, s->n_loc, 1, false);
+    return detect_check(s->ctx, s->n_loc, s->K, false);
+}
+
+// The descriptor of a rank's call: its forest count, the digests of its forests, a digest of the thresholds it applies
+ShardDesc describe(const kpl_shard* s)
+{
+    ShardDesc d;
+    memset(&d, 0, sizeof d);
+    d.K = (unsigned long long)s->K;
+    uint64_t h = fnv1a64(nullptr, 0);
+    for (int k = 0; k < s->K; ++k) {
+        const double t = threshold(s, k);
+        h = fnv1a64(&t, sizeof t, h);
+        d.forest[k] = s->ctx->forests.info[(size_t)k].digest;
+    }
+    d.thresholds = h;
+    return d;
+}
+
+// One verdict over the descriptors of all ranks, whichever transport brought them: ranks that would exchange strips of
+// different sizes (or score other forests) are refused before any strip moves
+int agreement(kpl_shard* s, const ShardDesc* all, int world)
+{
+    for (int r = 1; r < world; ++r)
+        if (memcmp(&all[r], &all[0], sizeof(ShardDesc))) {
+            char b[200];
+            snprintf(b, sizeof b, "kpl_shard_detect_forests: rank %d holds another forest count, other forests or other thresholds than rank 0", r);
+            return sfail(s, KPL_E_INVALID, b);
+        }
+    return KPL_OK;
+}
+
+// The descriptors to S[0]'s host: one all-gather and one host synchronisation (NCCL), or read on the host (in-process)
+int agree(kpl_shard** S, int n)
+{
+    kpl_shard* s = S[0];
+    kpl_ctx* c = s->ctx;
+    std::vector<ShardDesc> all((size_t)s->world);
+    if (s->in_process) {
+        for (int r = 0; r < n; ++r) all[(size_t)r] = describe(S[r]);
+    } else {
+        const ShardDesc mine = describe(s);
+        KS_CUDA(ensure(s->desc, 1)); KS_CUDA(ensure(s->desc_all, (size_t)s->world));
+        KS_CUDA(cudaMemcpyAsync(s->desc.p, &mine, sizeof mine, cudaMemcpyHostToDevice, c->stream));
+        KS_NCCL(s->nccl->AllGather(s->desc.p, s->desc_all.p, sizeof(ShardDesc), ncclChar, s->comm, c->stream));
+        KS_CUDA(cudaMemcpyAsync(all.data(), s->desc_all.p, all.size() * sizeof(ShardDesc), cudaMemcpyDeviceToHost, c->stream));
+        KS_CUDA(cudaStreamSynchronize(c->stream));
+        c->syncs++;
+    }
+    return agreement(s, all.data(), s->world);
 }
 
 void finish_timings(kpl_shard* s, bool gathered)
@@ -551,8 +684,11 @@ int copy_out(kpl_shard* s, float* scores_owned_out, int32_t* kp_global_out, int6
 {
     kpl_ctx* c = s->ctx;
     KS_CUDA(cudaSetDevice(c->device));
-    if (scores_owned_out)
+    if (scores_owned_out && s->K == 1)
         KS_CUDA(cudaMemcpyAsync(scores_owned_out, c->score.p + s->n_l, (size_t)s->n_own * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    else if (scores_owned_out)      // the owned part of each of the K slices, forest-major
+        KS_CUDA(cudaMemcpy2DAsync(scores_owned_out, (size_t)s->n_own * sizeof(float), c->score.p + s->n_l, (size_t)s->n_loc * sizeof(float),
+                                  (size_t)s->n_own * sizeof(float), (size_t)s->K, cudaMemcpyDeviceToHost, c->stream));
     if (s->rank == 0 && kp_global_out && total > 0) {
         if (kp_capacity < total) return sfail(s, KPL_E_INVALID, "kp_global_out is too small");
         KS_CUDA(cudaMemcpyAsync(kp_global_out, s->kp_sorted.p, (size_t)total * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
@@ -564,16 +700,23 @@ int copy_out(kpl_shard* s, float* scores_owned_out, int32_t* kp_global_out, int6
     return KPL_OK;
 }
 
-// One sharded detection over the ranks S[0..n) of this call.  The verdict over the records of all ranks comes before a
-// rank-local error of detect_finish, so that every rank returns the same status.
-int detect_step(kpl_shard** S, int n, float* const* scores_owned_out, int32_t* kp_global_out, int64_t kp_capacity, int64_t* n_kp_out)
+// One sharded detection over the ranks S[0..n) of this call: forest 0 (kpl_shard_detect), or every forest of the set at
+// the thresholds (NULL: params.threshold), from one feature pass (kpl_shard_detect_forests).  The verdict over the records
+// of all ranks comes before a rank-local error of detect_finish, so that every rank returns the same status.
+int detect_step(kpl_shard** S, int n, bool forests, const double* thresholds, float* const* scores_owned_out, int32_t* kp_global_out,
+                int64_t kp_capacity, int64_t* kp_offsets_out, int64_t* n_kp_out)
 {
     kpl_shard* s = S[0];
     kpl_ctx* c = s->ctx;
-    int rc;
-    if ((rc = each_rank(S, n, check_ready)) || (rc = each_rank(S, n, phase_pack)) || (rc = exchange(S, n, Strip::positions)) ||
-        (rc = each_rank(S, n, phase_score)) || (rc = exchange(S, n, Strip::scores)) || (rc = each_rank(S, n, phase_nms)) ||
-        (rc = nms_draws_rounds(S, n)) || (rc = each_rank(S, n, phase_draws_keypoints)))
+    int rc = each_rank(S, n, [&](kpl_shard* t) {
+        t->K = forests ? (int)t->ctx->forests.info.size() : 1;
+        t->th = thresholds;
+        if ((int64_t)t->K * t->plan.n_points > 2147483000ll) return sfail(t, KPL_E_INVALID, "forest count x point count out of range");
+        return (int)KPL_OK;
+    });
+    if (rc || (rc = each_rank(S, n, check_ready)) || (rc = each_rank(S, n, phase_pack)) || (forests && (rc = agree(S, n))) ||
+        (rc = exchange(S, n, Strip::positions)) || (rc = each_rank(S, n, phase_score)) || (rc = exchange(S, n, Strip::scores)) ||
+        (rc = each_rank(S, n, phase_nms)) || (rc = nms_draws(S, n)))
         return rc;
     // the records of all ranks to S[0]'s host: all-gathered, or one copy per in-process rank
     if (!s->in_process) {
@@ -596,12 +739,24 @@ int detect_step(kpl_shard** S, int n, float* const* scores_owned_out, int32_t* k
     if ((rc = verdict(s, total, counts))) return rc;                   // identical on every rank: nobody is left waiting in a collective
     if (local_err) return on_rank(S, err_rank, local_err);
     if (n_kp_out) *n_kp_out = total;
+    if (kp_offsets_out) {                   // forest k's keypoints of all ranks, which the sort keeps together
+        kp_offsets_out[0] = 0;
+        for (int k = 0; k < s->K; ++k) {
+            kp_offsets_out[k + 1] = kp_offsets_out[k];
+            for (int r = 0; r < s->world; ++r) kp_offsets_out[k + 1] += (int64_t)s->h_rec[(size_t)r].n_kp_forest[k];
+        }
+    }
     // keypoint lists to rank 0 (sizes are known everywhere now), then one sort into ascending global index
     KS_CUDA(cudaSetDevice(c->device));
     KS_CUDA(cudaEventRecord(s->ev[4], c->stream));
     if (s->rank == 0) { KS_CUDA(ensure(s->kp_all, (size_t)total + 1)); KS_CUDA(ensure(s->kp_sorted, (size_t)total + 1)); }
     if ((rc = gather_keypoints(S, n, counts))) return rc;
     if (s->rank == 0 && (rc = sort_keypoints(s, total))) return rc;
+    if (s->rank == 0 && s->K > 1 && total > 0) {
+        strip_forest_kernel<<<(unsigned)((total + 255) / 256), 256, 0, c->stream>>>(s->kp_sorted.p, total, (int32_t)s->plan.n_points);
+        KS_CUDA(cudaGetLastError());
+        c->launches++;
+    }
     KS_CUDA(cudaEventRecord(s->ev[5], c->stream));
     for (int r = 0; r < n; ++r) {
         rc = copy_out(S[r], scores_owned_out ? scores_owned_out[r] : nullptr, r == 0 ? kp_global_out : nullptr, kp_capacity, total);
@@ -809,7 +964,7 @@ void kpl_shard_destroy(kpl_shard* s)
     srelease(s->st_orig); srelease(s->und_all);
     for (int k = 0; k < 2; ++k) { srelease(s->sst_l[k]); srelease(s->sst_r[k]); }
     srelease(s->kp_local); srelease(s->kp_global); srelease(s->kp_all); srelease(s->kp_sorted); srelease(s->sort_tmp);
-    srelease(s->rec); srelease(s->rec_all); srelease(s->sizes); srelease(s->sizes_all);
+    srelease(s->rec); srelease(s->rec_all); srelease(s->desc); srelease(s->desc_all); srelease(s->sizes); srelease(s->sizes_all);
     for (int i = 0; i < 6; ++i) if (s->ev[i]) cudaEventDestroy(s->ev[i]);
     delete s;
 }
@@ -985,14 +1140,23 @@ int kpl_shard_detect(kpl_shard* s, float* scores_owned_out, int32_t* kp_global_o
     if (!s) return KPL_E_INVALID;
     if (n_kp_out) *n_kp_out = 0;
     if (s->in_process) return sfail(s, KPL_E_INVALID, "ranks of an in-process group are driven by kpl_shard_detect_group");
-    return detect_step(&s, 1, &scores_owned_out, kp_global_out, kp_capacity, n_kp_out);
+    return detect_step(&s, 1, false, nullptr, &scores_owned_out, kp_global_out, kp_capacity, nullptr, n_kp_out);
+}
+
+int kpl_shard_detect_forests(kpl_shard* s, const double* thresholds, float* scores_owned_out, int32_t* kp_global_out, int64_t kp_capacity,
+                             int64_t* kp_offsets_out, int64_t* n_kp_out)
+{
+    if (!s) return KPL_E_INVALID;
+    if (n_kp_out) *n_kp_out = 0;
+    if (s->in_process) return sfail(s, KPL_E_INVALID, "ranks of an in-process group are driven by kpl_shard_detect_forests_group");
+    return detect_step(&s, 1, true, thresholds, &scores_owned_out, kp_global_out, kp_capacity, kp_offsets_out, n_kp_out);
 }
 
 // All ranks of an in-process group from one host thread: the same phases, strips moved by peer copies.  The streams
 // of the ranks are synchronised between phases (this is the path for hosts without NCCL and for single-GPU tests,
 // not the fast path).
-int kpl_shard_detect_group(kpl_shard** S, int32_t world, float** scores_owned_out, int32_t* kp_global_out, int64_t kp_capacity,
-                           int64_t* n_kp_out)
+static int detect_group(kpl_shard** S, int32_t world, bool forests, const double* thresholds, float** scores_owned_out, int32_t* kp_global_out,
+                        int64_t kp_capacity, int64_t* kp_offsets_out, int64_t* n_kp_out)
 {
     if (!S || world < 1 || !S[0]) return KPL_E_INVALID;
     if (n_kp_out) *n_kp_out = 0;
@@ -1016,7 +1180,19 @@ int kpl_shard_detect_group(kpl_shard** S, int32_t world, float** scores_owned_ou
         const int rc = exchange(S, world, Strip::gidx);
         if (rc) return rc;
     }
-    return detect_step(S, world, scores_owned_out, kp_global_out, kp_capacity, n_kp_out);
+    return detect_step(S, world, forests, thresholds, scores_owned_out, kp_global_out, kp_capacity, kp_offsets_out, n_kp_out);
+}
+
+int kpl_shard_detect_group(kpl_shard** S, int32_t world, float** scores_owned_out, int32_t* kp_global_out, int64_t kp_capacity,
+                           int64_t* n_kp_out)
+{
+    return detect_group(S, world, false, nullptr, scores_owned_out, kp_global_out, kp_capacity, nullptr, n_kp_out);
+}
+
+int kpl_shard_detect_forests_group(kpl_shard** S, int32_t world, const double* thresholds, float** scores_owned_out, int32_t* kp_global_out,
+                                   int64_t kp_capacity, int64_t* kp_offsets_out, int64_t* n_kp_out)
+{
+    return detect_group(S, world, true, thresholds, scores_owned_out, kp_global_out, kp_capacity, kp_offsets_out, n_kp_out);
 }
 
 int kpl_shard_get_info(const kpl_shard* s, kpl_shard_info* out)
@@ -1025,7 +1201,7 @@ int kpl_shard_get_info(const kpl_shard* s, kpl_shard_info* out)
     memset(out, 0, sizeof *out);
     out->n_owned = s->n_own; out->n_left = std::max<int64_t>(s->n_l, 0); out->n_right = std::max<int64_t>(s->n_r, 0);
     out->send_left = s->send_l; out->send_right = s->send_r;
-    out->halo_bytes = (s->send_l + s->send_r) * (int64_t)(sizeof(float4) + sizeof(float) + (s->has_nrm ? sizeof(float4) : 0));
+    out->halo_bytes = (s->send_l + s->send_r) * (int64_t)(sizeof(float4) + sizeof(float) * s->last_K + (s->has_nrm ? sizeof(float4) : 0));
     out->local_dims[0] = s->grid.dims[0]; out->local_dims[1] = s->plan.dims[1]; out->local_dims[2] = s->plan.dims[2];
     out->local_offset[0] = s->grid.offset[0];
     out->rank = s->rank; out->world = s->world;

@@ -163,6 +163,24 @@ class SlabJob:
                                              0 if kp is None else kp.size, C.byref(n)))
         return n.value, (kp[:n.value] if self.rank == 0 else None)
 
+    def detect_forests(self, thresholds=None, scores_out=None):
+        """kpl_shard_detect_forests: every forest of the set from one feature pass.  thresholds: None (the prediction
+        threshold for every forest) or one per forest.  scores_out: None or K * n_owned float32, forest-major.  Returns
+        (keypoints of all forests, K + 1 offsets, [K ascending global index arrays] on rank 0 / None)."""
+        self.det._push()
+        th = self.det._thresholds(thresholds)
+        K = self.det.forestCount()
+        n = C.c_int64(0)
+        off = np.zeros(K + 1, np.int64)
+        kp = np.empty(max(K, 1) * self.n_total, np.int32) if self.rank == 0 else None
+        if scores_out is not None and (scores_out.dtype != np.float32 or scores_out.size < K * self.n_owned):
+            raise ValueError("scores_out must be float32[%d] (forests x owned points)" % (K * self.n_owned))
+        self._check(self._L.kpl_shard_detect_forests(self._h, None if th is None else th.ctypes.data_as(C.POINTER(C.c_double)),
+                                                     None if scores_out is None else scores_out.ctypes.data_as(C.POINTER(C.c_float)),
+                                                     None if kp is None else kp.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                     0 if kp is None else kp.size, off.ctypes.data_as(C.POINTER(C.c_int64)), C.byref(n)))
+        return n.value, off, ([kp[off[k]:off[k + 1]].copy() for k in range(K)] if self.rank == 0 else None)
+
     def info(self):
         i = capi.KplShardInfo()
         self._check(self._L.kpl_shard_get_info(self._h, C.byref(i)))
@@ -209,6 +227,39 @@ def detect_widening(job, xyz, r_feat, r_nms, cpr, max_support=64, **kw):
 def detect_group_widening(jobs, xyz, r_feat, r_nms, cpr, max_support=64, want_scores=True):
     """detect_group() with the widening loop of _widening for an in-process group."""
     return _widening(lambda: detect_group(jobs, want_scores), jobs, xyz, r_feat, r_nms, cpr, max_support)
+
+
+def detect_forests_widening(job, xyz, r_feat, r_nms, cpr, max_support=64, **kw):
+    """job.detect_forests() with the widening loop of _widening."""
+    return _widening(lambda: job.detect_forests(**kw), [job], xyz, r_feat, r_nms, cpr, max_support)
+
+
+def detect_group_forests_widening(jobs, xyz, r_feat, r_nms, cpr, max_support=64, thresholds=None, want_scores=True):
+    """detect_group_forests() with the widening loop of _widening for an in-process group."""
+    return _widening(lambda: detect_group_forests(jobs, thresholds, want_scores), jobs, xyz, r_feat, r_nms, cpr, max_support)
+
+
+def detect_group_forests(jobs, thresholds=None, want_scores=True):
+    """kpl_shard_detect_forests_group: every forest of the set over an in-process group, from one feature pass.
+    thresholds: None or one per forest.  Returns ([K ascending global keypoint index arrays], [per-rank K x n_owned scores])."""
+    L = capi.load_library()
+    world = len(jobs)
+    for j in jobs:
+        j.det._push()
+    th = jobs[0].det._thresholds(thresholds)
+    K = jobs[0].det.forestCount()
+    hs = (C.c_void_p * world)(*[j._h for j in jobs])
+    scores = [np.empty((max(K, 1), j.n_owned), np.float32) for j in jobs] if want_scores else None
+    f32p = C.POINTER(C.c_float)
+    sc_ptrs = (f32p * world)(*[s.ctypes.data_as(f32p) for s in scores]) if want_scores else None
+    kp = np.empty(max(K, 1) * jobs[0].n_total, np.int32)
+    off = np.zeros(K + 1, np.int64)
+    n = C.c_int64(0)
+    rc = L.kpl_shard_detect_forests_group(hs, world, None if th is None else th.ctypes.data_as(C.POINTER(C.c_double)), sc_ptrs,
+                                          kp.ctypes.data_as(C.POINTER(C.c_int32)), kp.size, off.ctypes.data_as(C.POINTER(C.c_int64)), C.byref(n))
+    if rc != 0:
+        raise capi.KplError(rc, (L.kpl_last_error(jobs[0].det._h) or b"").decode())
+    return [kp[off[k]:off[k + 1]].copy() for k in range(K)], scores
 
 
 def detect_group(jobs, want_scores=True):
